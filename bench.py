@@ -39,6 +39,8 @@ B_POINT_A, B_LINE_A = 412, 204            # mode A: inputs + r/J outputs per fac
 B_POINT_IN, B_LINE_IN = 44, 76            # mode B inputs per factor
 WORKLOAD = ("cfg2: 4096 EuRoC-shaped windows/GPU (11 poses, 150 features, ~560 ProjectionFactors + 110 "
             "LineProjectionFactors each): Evaluate + loss correction + H/b assembly")
+# --dump-outputs: the full H/b of 4096 windows is ~0.5 GB, so a fixed, seeded sample of windows is written
+DUMP_BYTES, DUMP_SEED = 32 << 20, 0x5EED + 7
 
 
 def window_bytes(P, F):
@@ -98,6 +100,26 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+def dump_windows(W, n):
+    """The n of W windows --dump-outputs writes: all of them, or the first n of a fixed permutation, sorted (samples of different
+    sizes over the same W are nested, so a dump with more arrays per window still shares its windows with a smaller one)."""
+    return np.arange(W) if n >= W else np.sort(np.random.default_rng(DUMP_SEED).permutation(W)[:n])
+
+
+def dump_outputs(dirname, outputs):
+    """Writes outputs {name: [W, ...] float64} as dirname/<name>.npy, every array restricted to the same windows: all of them when
+    they fit DUMP_BYTES, else dump_windows(W, n) (same arguments, same windows).  Returns what was written."""
+    W = next(iter(outputs.values())).shape[0]
+    per_window = sum(v[0].nbytes for v in outputs.values())
+    n = min(W, max(1, DUMP_BYTES // per_window))
+    sel = dump_windows(W, n)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in outputs.items():
+        np.save(os.path.join(dirname, k + ".npy"), np.ascontiguousarray(v[sel]))
+    return {"dir": os.path.abspath(dirname), "arrays": sorted(outputs), "windows": int(n), "of_windows": W,
+            "sample": "all windows" if n == W else f"numpy default_rng({DUMP_SEED}).permutation({W})[:{n}], sorted"}
+
+
 def dist_env():
     return int(os.environ.get("RANK", 0)), int(os.environ.get("LOCAL_RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
 
@@ -149,12 +171,7 @@ def run_reference(args):
     batch, _ = synth.with_line_map(synth.make_windows(args.windows, seed=0x5EED + 2, f32_obs=True), cfg)   # the native arm's rank-0 batch
     steps, warm = args.steps, args.warmup
     bufs = batch.alloc_out(flags, fill=0.0)
-    t0 = time.perf_counter()
-    orc.linearize_batch(cfg, batch, flags, nthreads=nthreads, out=bufs)
-    dt1 = time.perf_counter() - t0
-    if dt1 * (steps + warm) > 240.0:     # keep the whole run within a few minutes on a slow host
-        steps = max(3, int(240.0 / dt1) - warm)
-    for _ in range(max(warm - 1, 0)):
+    for _ in range(warm):
         orc.linearize_batch(cfg, batch, flags, nthreads=nthreads, out=bufs)
     t0 = time.perf_counter()
     for _ in range(steps):
@@ -164,7 +181,7 @@ def run_reference(args):
     val = factors * steps / dt
     sample = (f"all {batch.W} windows per step ({factors} factors): Evaluate + Cauchy correction + ThreadsConstructA-rule dense A/b + "
               f"landmark Schur complement; {steps} timed steps")
-    print(json.dumps({
+    res = {
         "impl": "reference", "metric": "linearized_factors_per_s", "value": val, "unit": "factors/s", "n_gpus": args.gpus,
         "steps": steps, "warmup": warm, "ms_per_step": dt / steps * 1e3, "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -173,7 +190,10 @@ def run_reference(args):
         "e2e": {"value": val, "unit": "factors/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "note": "the reference needs Eigen/Ceres/ROS and cannot be built here; this is the dependency-free oracle port of its "
                 "CPU algorithm, std::thread over windows on all host threads",
-    }))
+    }
+    if args.dump_outputs:
+        res["dump_outputs"] = dump_outputs(args.dump_outputs, bufs)
+    print(json.dumps(res))
 
 
 def nccl_bootstrap(torch, dist, world, rank):
@@ -225,6 +245,9 @@ def main():
     ap.add_argument("--skip-extras", action="store_true", help="only the headline linearise metric")
     ap.add_argument("--skip-cpu", action="store_true")
     ap.add_argument("--only-assoc", action="store_true", help="profiling aid: of the extra objects only `assoc` (implies a small headline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step (H_pp, H_lp, H_ll, b_p, "
+                                                          "b_l of rank 0; the reference arm also S, g) as DIR/<name>.npy, float64, "
+                                                          "at most 32 MB")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -348,8 +371,10 @@ def main():
                 "ncu_dram_bytes_per_launch": ncu_traffic, "peak_source": peak_src,
                 "algorithmic_bytes_per_launch": dom_bytes, "avg_launch_ms": dom_ms / dom_n,
                 "step_algorithmic_bytes": step_bytes, "step_frac": step_bytes / (ms_step * 1e-3) / 1e9 / hbm_peak,
-                "kernel_ms_per_step": {k: v[0] / K for k, v in prof.items()}}
+                "kernel_ms_per_step": {k: v[0] / K for k, v in prof.items()},
+                "kernel_launches_timed": {k: v[1] for k, v in prof.items()}}
     H_dev = {k: fetch(shapes[k], d_out[k]) for k in d_out}     # this run's device-resident outputs, for the parity check
+    dumped = dump_outputs(args.dump_outputs, H_dev) if args.dump_outputs and rank == 0 else None
 
     # ------------------------------------------------------------------ e2e: the drop-in call, pinned host buffers
     pins = {k: pkg.pinned_like(v) for k, v in batch.arrays().items() if v is not None}
@@ -403,6 +428,8 @@ def main():
                       "l2": "inputs+outputs per step (%.0f MB) exceed the 126 MB L2" % (step_bytes / 1e6),
                       "parallelism": f"{world} GPU(s), windows sharded, no data-path collective"},
            "roofline": roofline, "e2e": e2e, "e2e_hb": e2e_hb, "gpu_launches": gpu_launches, "clocks": clocks}
+    if dumped:
+        out["dump_outputs"] = dumped
 
     # ------------------------------------------------------------------ CPU baseline + parity of THIS run's outputs (rank 0, N=1)
     if do_cpu:
