@@ -22,6 +22,12 @@
  *                             (evaluated by their owners; their r / J blocks are inputs here), ThreadsConstructA rule :141-172
  *   viml_gn_step           <- one solver iteration of ceres::Solve  estimator.cpp:1888-1905 (normal equations, Schur elimination of
  *                             the landmarks, dense solve, PoseLocalParameterization::Plus  pose_local_parameterization.cpp:3-19)
+ *   viml_inertial_evaluate <- IMUFactor::Evaluate               vins_estimator/src/factor/imu_factor.h:19-181
+ *                             IntegrationBase::evaluate         vins_estimator/src/factor/integration_base.h
+ *                             MarginalizationFactor::Evaluate   marginalization_factor.cpp:335-384
+ *                             (pre-integration itself stays with the host)
+ *   viml_gn_step_vi        <- viml_gn_step over the window's whole problem: the IMU and prior factors evaluated on the device at
+ *                             x (system) and at x+ (cost[1] = f(x+))
  *   viml_fov_update / viml_fov_slide / VIML_FOV_CACHED
  *                          <- the per-slot FoV lists the estimator keeps between frames: UpdateLinesInFoV at frame entry
  *                             (estimator.cpp:342) and their shifts in slideWindowWithLinesFoV (estimator.cpp:2148, :2160, :2218)
@@ -279,6 +285,75 @@ typedef struct viml_gn_out {
 
 int viml_gn_step(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state /* [W][X] or NULL */,
                  const viml_gn_options* opt, const viml_gn_out* out, uint32_t flags);
+
+/* ---- the window's IMU factors and the prior, evaluated on the device --------------------------------------------------
+ * IMUFactor::Evaluate + IntegrationBase::evaluate (vins_estimator/src/factor/imu_factor.h:19-181, integration_base.h) and
+ * MarginalizationFactor::Evaluate (marginalization_factor.cpp:335-384) at the current state.  IMU pre-integration stays with the
+ * host (IntegrationBase::push_back / midPointIntegration / repropagate): its outputs are inputs here, and so is sqrt_info
+ * = LLT(covariance.inverse()).matrixL().transpose(), which the reference recomputes in every Evaluate but which depends on the
+ * pre-integration's covariance alone (fixed during a solve).  The library does not invert the badly scaled 15 x 15 covariance.
+ *
+ * Parameter blocks of a window: pose p (7 values, tangent columns 6p .. 6p+5), the extrinsic (tangent 6P .. 6P+5) and an extra
+ * state of X values per window (tangent D + k for value k, D = 6(P+1)), e.g. the speed-bias blocks [V, Ba, Bg] (9 values each).
+ * IMU factor k couples pose imu_pose[k][0] (i), the 9 extra values at imu_sb[k][0], pose imu_pose[k][1] (j) and the 9 at
+ * imu_sb[k][1]; its reduced block is 15 x 30 over the tangent columns [pose_i(6) | sb_i(9) | pose_j(6) | sb_j(9)].
+ * The prior of window w (prior_n[w] = n_w > 0) has n_w rows; block b (prior_block[w][b] = {kind, index, size, first column}) maps its
+ * local columns first .. first + local - 1 (local = 6 for a size-7 pose / extrinsic block, else size) to the block's tangent
+ * columns; the blocks cover [0, n_w) exactly once.  Extra blocks are vectors (size != 7, size <= VIML_PRIOR_X0_STRIDE): index is their offset
+ * in the extra state.
+ * The host-pointer flavour validates them (VIML_ERR_INVALID: pose indices in [0, P), i != j, speed-bias offsets with sb + 9 <= X
+ * and disjoint, n_w <= n_max, block kinds / sizes / columns as above, D + X <= 232).  The device flavour reads no input back: it
+ * checks what the struct fields alone tell (D + X <= 232, X >= 9 when there are IMU factors, extra_state given when X > 0, no
+ * null array), clamps pose and block indices, and leaves the rest to the caller.                                            */
+#define VIML_BLOCK_POSE 0   /* pose `index` of the window: 7 values                          */
+#define VIML_BLOCK_EX 1     /* the extrinsic: 7 values (index unused)                        */
+#define VIML_BLOCK_EXTRA 2  /* `size` values at offset `index` of the window's extra state    */
+#define VIML_PRIOR_X0_STRIDE 9   /* values per kept block in prior_x0: a speed-bias block (9) is the largest a prior keeps */
+
+typedef struct viml_inertial_factors {
+  int32_t extra_dim;                 /* X: extra state per window [W][X]                                                  */
+  int32_t reserved0;
+  double gravity[3];                 /* G (parameters.cpp: G.z() = g_norm)                                                */
+  /* IMUFactor : SizedCostFunction<15, 7, 9, 7, 9> (imu_factor.h)                                                        */
+  int64_t n_imu;                     /* NI                                                                                */
+  const int32_t* imu_window_offset;  /* [W+1], imu_window_offset[W] == NI                                                 */
+  const int32_t* imu_pose;           /* [NI][2]  pose i, pose j                                                           */
+  const int32_t* imu_sb;             /* [NI][2]  offsets of speed-bias i / j = [V, Ba, Bg] in the extra state             */
+  const double* imu_preint;          /* [NI][17] sum_dt, delta_p[3], delta_q[4] (x y z w), delta_v[3], linearized_ba[3], linearized_bg[3] */
+  const double* imu_jacobian;        /* [NI][15][15] ROW-major pre_integration->jacobian (Eigen stores it column-major)    */
+  const double* imu_sqrt_info;       /* [NI][15][15] row-major LLT(covariance.inverse()).matrixL().transpose()            */
+  /* MarginalizationFactor (last_marginalization_info): at most one per window                                           */
+  int32_t prior_n_max;               /* stride: n_w <= prior_n_max                                                        */
+  int32_t prior_max_blocks;          /* stride of the block lists                                                         */
+  const int32_t* prior_n;            /* [W] n_w, 0 = the window has no prior                                              */
+  const double* prior_jacobian;      /* [W][n_max][n_max] linearized_jacobians (the leading n_w x n_w block is read)      */
+  const double* prior_residual;      /* [W][n_max]        linearized_residuals                                            */
+  const int32_t* prior_n_blocks;     /* [W]                                                                               */
+  const int32_t* prior_block;        /* [W][max_blocks][4] kind, index, global size, first column (keep_block_idx - m)    */
+  const double* prior_x0;            /* [W][max_blocks][VIML_PRIOR_X0_STRIDE] keep_block_data (first `size` values used)  */
+} viml_inertial_factors;
+
+/* Ceres Evaluate layouts, row-major; column 6 of a pose block is exactly 0.  Any pointer may be NULL (= not wanted). */
+typedef struct viml_inertial_out {
+  double* imu_residual;    /* [NI][15]    */
+  double* imu_jac_pose_i;  /* [NI][15][7] */
+  double* imu_jac_sb_i;    /* [NI][15][9] */
+  double* imu_jac_pose_j;  /* [NI][15][7] */
+  double* imu_jac_sb_j;    /* [NI][15][9] */
+  double* prior_residual;  /* [W][n_max] (first n_w written; the prior's Jacobian is its input, marginalization_factor.cpp:371-380) */
+} viml_inertial_out;
+
+/* Mode A for these factors: r and J at the state (poses / ex_pose of `state`, extra_state [W][X]).  Only n_windows,
+ * poses_per_window, poses and ex_pose of `state` are read.  Pointers follow VIML_PTRS_DEVICE.                             */
+int viml_inertial_evaluate(viml_ctx* ctx, const viml_window_batch* state, const double* extra_state, const viml_inertial_factors* vi,
+                           const viml_inertial_out* out, uint32_t flags);
+/* viml_gn_step with the window's prior and IMU factors as its dense-block factors, evaluated on the device: at x for Sx, gx and
+ * cost[0]; at x+ for cost[1], which is then f(x+) exactly:  1/2 sum rho(|r|^2) over the visual factors + 1/2 sum |r|^2 over the
+ * IMU and prior factors (the reference gives both a NULL loss, estimator.cpp:1927, :1939).  Per window the dense factors are the
+ * prior first, then the IMU factors in input order.  Everything else is viml_gn_step's contract (the model decrease, unsolved
+ * windows returned unchanged); extra_state is required when X > 0.  With VIML_PTRS_DEVICE the call does not synchronise.     */
+int viml_gn_step_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
+                    const viml_gn_options* opt, const viml_gn_out* out, uint32_t flags);
 
 /* ---- dense marginalisation (marginalization_factor.cpp:264-293) --------------------------------
  * Per problem k: A [pos][pos] row-major, b [pos], marginalised block = leading m rows, kept n = pos-m.

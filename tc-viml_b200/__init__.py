@@ -27,6 +27,7 @@ ABI_SYMBOLS = (
     "viml_marginalize_batch", "viml_line_associate", "viml_assoc_stats", "viml_allreduce_hb",
     "viml_load_line_map", "viml_reduced_system", "viml_reduced_from_schur", "viml_gn_step",
     "viml_fov_update", "viml_fov_slide", "viml_track_gate", "viml_triangulate_batch",
+    "viml_inertial_evaluate", "viml_gn_step_vi",
 )
 
 
@@ -85,6 +86,10 @@ def load_library():
                                             C.POINTER(_abi.ReducedOut), C.c_uint32]
     lib.viml_gn_step.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.DenseFactors), C.c_void_p,
                                  C.POINTER(_abi.GnOptions), C.POINTER(_abi.GnOut), C.c_uint32]
+    lib.viml_inertial_evaluate.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.c_void_p, C.POINTER(_abi.InertialFactors),
+                                           C.POINTER(_abi.InertialOut), C.c_uint32]
+    lib.viml_gn_step_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.InertialFactors), C.c_void_p,
+                                    C.POINTER(_abi.GnOptions), C.POINTER(_abi.GnOut), C.c_uint32]
     _LIB = lib
     return lib
 
@@ -252,6 +257,43 @@ class Context:
         o.extra = _abi.ptr(res["extra"]) if X > 0 else None
         self._check(self.lib.viml_gn_step(self.h, C.byref(s), C.byref(d) if d is not None else None, _abi.ptr(ex), C.byref(opt),
                                           C.byref(o), flags & ~PTRS_DEVICE))
+        return res
+
+    def inertial_evaluate(self, batch, extra, vi):
+        """viml_inertial_evaluate with host buffers at the state (batch.poses, batch.ex_pose, extra [W, X]): dict of the
+        viml_inertial_out arrays (imu_residual [NI,15], imu_jac_pose_i [NI,15,7], imu_jac_sb_i [NI,15,9], imu_jac_pose_j,
+        imu_jac_sb_j, prior_residual [W,n_max]; prior rows past n_w are NaN)."""
+        NI, W = vi.NI, batch.W
+        res = {"imu_residual": np.full((NI, 15), np.nan), "imu_jac_pose_i": np.full((NI, 15, 7), np.nan),
+               "imu_jac_sb_i": np.full((NI, 15, 9), np.nan), "imu_jac_pose_j": np.full((NI, 15, 7), np.nan),
+               "imu_jac_sb_j": np.full((NI, 15, 9), np.nan), "prior_residual": np.full((W, vi.n_max), np.nan)}
+        s = batch.struct()
+        ex = None if extra is None else np.ascontiguousarray(extra, dtype=np.float64)
+        v = vi.struct()
+        o = _abi.InertialOut()
+        for k in _abi.INERTIAL_OUT_FIELDS:
+            setattr(o, k, _abi.ptr(res[k]) if res[k].size else None)
+        self._check(self.lib.viml_inertial_evaluate(self.h, C.byref(s), _abi.ptr(ex), C.byref(v), C.byref(o), 0))
+        return res
+
+    def gn_step_vi(self, batch, vi, extra, flags, lam=0.0, obs_table=False, line_table=False):
+        """viml_gn_step_vi with host buffers: dict(poses, ex_pose, inv_depth, extra, dx, cost, solved)."""
+        X = vi.X
+        W, Dx = batch.W, batch.D + X
+        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
+               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan),
+               "dx": np.full((W, Dx), np.nan), "cost": np.full((W, 3), np.nan), "solved": np.full(W, -1, dtype=np.int32)}
+        s, _keep = self._batch_struct(batch, obs_table, line_table)
+        v = vi.struct()
+        ex = None if extra is None else np.ascontiguousarray(extra, dtype=np.float64)
+        opt = _abi.GnOptions()
+        opt.lambda_ = float(lam)
+        o = _abi.GnOut()
+        for k in ("poses", "ex_pose", "inv_depth", "dx", "cost", "solved"):
+            setattr(o, k, _abi.ptr(res[k]))
+        o.extra = _abi.ptr(res["extra"]) if X > 0 else None
+        self._check(self.lib.viml_gn_step_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), C.byref(opt), C.byref(o),
+                                             flags & ~PTRS_DEVICE))
         return res
 
     def linearize(self, batch, flags, out=None, obs_table=False, line_table=False):

@@ -22,6 +22,8 @@ S_PACKED = 0x20
 PTRS_DEVICE = 0x100
 FOV_CACHED = 0x200
 FOV_SLOTS = 11
+BLOCK_POSE, BLOCK_EX, BLOCK_EXTRA = 0, 1, 2
+PRIOR_X0_STRIDE = 9
 
 c_double_p = C.POINTER(C.c_double)
 c_float_p = C.POINTER(C.c_float)
@@ -144,6 +146,107 @@ class Dense:
         for k in a:
             setattr(s, k, ptr(a[k]))
         return s
+
+
+class InertialFactors(C.Structure):
+    """viml_inertial_factors — the window's IMU factors (pre-integration outputs) and the prior of the last marginalisation."""
+
+    _fields_ = [("extra_dim", C.c_int32), ("reserved0", C.c_int32), ("gravity", C.c_double * 3), ("n_imu", C.c_int64),
+                ("imu_window_offset", C.c_void_p), ("imu_pose", C.c_void_p), ("imu_sb", C.c_void_p), ("imu_preint", C.c_void_p),
+                ("imu_jacobian", C.c_void_p), ("imu_sqrt_info", C.c_void_p),
+                ("prior_n_max", C.c_int32), ("prior_max_blocks", C.c_int32), ("prior_n", C.c_void_p), ("prior_jacobian", C.c_void_p),
+                ("prior_residual", C.c_void_p), ("prior_n_blocks", C.c_void_p), ("prior_block", C.c_void_p), ("prior_x0", C.c_void_p)]
+
+
+INERTIAL_OUT_FIELDS = ("imu_residual", "imu_jac_pose_i", "imu_jac_sb_i", "imu_jac_pose_j", "imu_jac_sb_j", "prior_residual")
+
+
+class InertialOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in INERTIAL_OUT_FIELDS]
+
+
+class Inertial:
+    """Host-side container of one viml_inertial_factors (numpy arrays, shapes as in viml.h).
+
+    imu_preint rows are [sum_dt, delta_p(3), delta_q(4, x y z w), delta_v(3), linearized_ba(3), linearized_bg(3)]; imu_jacobian and
+    imu_sqrt_info are row-major 15 x 15.  prior_block rows are [kind, index, size, first column]."""
+
+    INT_FIELDS = ("imu_window_offset", "imu_pose", "imu_sb", "prior_n", "prior_n_blocks", "prior_block")
+    FIELDS = ("imu_window_offset", "imu_pose", "imu_sb", "imu_preint", "imu_jacobian", "imu_sqrt_info",
+              "prior_n", "prior_jacobian", "prior_residual", "prior_n_blocks", "prior_block", "prior_x0")
+
+    def __init__(self, W, P, extra_dim, gravity, imu_window_offset, imu_pose, imu_sb, imu_preint, imu_jacobian, imu_sqrt_info,
+                 prior_n, prior_jacobian, prior_residual, prior_n_blocks, prior_block, prior_x0):
+        self.W, self.P, self.X = int(W), int(P), int(extra_dim)
+        self.gravity = np.asarray(gravity, dtype=np.float64).reshape(3)
+        loc = dict(locals())
+        for k in self.FIELDS:
+            setattr(self, k, np.ascontiguousarray(loc[k], dtype=np.int32 if k in self.INT_FIELDS else np.float64))
+        self.imu_pose = self.imu_pose.reshape(-1, 2)
+        self.imu_sb = self.imu_sb.reshape(-1, 2)
+        self.imu_preint = self.imu_preint.reshape(-1, 17)
+        self.imu_jacobian = self.imu_jacobian.reshape(-1, 15, 15)
+        self.imu_sqrt_info = self.imu_sqrt_info.reshape(-1, 15, 15)
+        n_max = self.prior_jacobian.shape[1] if self.prior_jacobian.ndim == 3 else 0
+        self.prior_jacobian = self.prior_jacobian.reshape(self.W, n_max, n_max)
+        self.prior_residual = self.prior_residual.reshape(self.W, n_max)
+        self.prior_block = self.prior_block.reshape(self.W, -1, 4)
+        self.prior_x0 = self.prior_x0.reshape(self.W, -1, PRIOR_X0_STRIDE)
+        assert self.imu_window_offset.shape == (self.W + 1,) and self.prior_n.shape == (self.W,)
+
+    NI = property(lambda s: int(s.imu_pose.shape[0]))
+    n_max = property(lambda s: int(s.prior_jacobian.shape[1]))
+    max_blocks = property(lambda s: int(s.prior_block.shape[1]))
+    D = property(lambda s: 6 * (s.P + 1))
+
+    def arrays(self):
+        return {k: getattr(self, k) for k in self.FIELDS}
+
+    def struct(self, arrays=None):
+        a = self.arrays() if arrays is None else arrays
+        s = InertialFactors()
+        s.extra_dim, s.n_imu = self.X, self.NI
+        for k in range(3):
+            s.gravity[k] = float(self.gravity[k])
+        s.prior_n_max, s.prior_max_blocks = self.n_max, self.max_blocks
+        for k in self.FIELDS:
+            setattr(s, k, ptr(a[k]))
+        return s
+
+    def imu_window(self):
+        return np.repeat(np.arange(self.W), np.diff(self.imu_window_offset))
+
+    def imu_columns(self, k):
+        """Tangent columns of IMU factor k's reduced 15 x 30 block: [pose_i(6) | sb_i(9) | pose_j(6) | sb_j(9)]."""
+        (i, j), (si, sj) = self.imu_pose[k], self.imu_sb[k]
+        D = self.D
+        return np.concatenate([6 * i + np.arange(6), D + si + np.arange(9), 6 * j + np.arange(6), D + sj + np.arange(9)])
+
+    def prior_columns(self, w):
+        """Tangent column of each of the n_w local columns of window w's prior."""
+        n = int(self.prior_n[w])
+        cols = np.full(n, -1, dtype=np.int64)
+        for kind, idx, size, first in self.prior_block[w, :self.prior_n_blocks[w]]:
+            local = 6 if size == 7 else size
+            t0 = 6 * idx if kind == BLOCK_POSE else 6 * self.P if kind == BLOCK_EX else self.D + idx
+            cols[first:first + local] = t0 + np.arange(local)
+        return cols
+
+    def to_dense(self, ev):
+        """The viml_dense_factors of an evaluation (dict of the viml_inertial_out arrays): per window the prior, then its IMU factors
+        in input order — the order viml_gn_step_vi assembles them in."""
+        fs = []
+        win = self.imu_window()
+        for w in range(self.W):
+            n = int(self.prior_n[w])
+            if n > 0:
+                fs.append((w, ev["prior_residual"][w, :n], self.prior_jacobian[w, :n, :n], self.prior_columns(w)))
+            for k in range(self.imu_window_offset[w], self.imu_window_offset[w + 1]):
+                J = np.concatenate([ev["imu_jac_pose_i"][k][:, :6], ev["imu_jac_sb_i"][k], ev["imu_jac_pose_j"][k][:, :6],
+                                    ev["imu_jac_sb_j"][k]], axis=1)
+                fs.append((w, ev["imu_residual"][k], J, self.imu_columns(k)))
+        assert all(f[0] == w for f, w in zip(fs, sorted(f[0] for f in fs)))
+        return Dense(self.W, self.X, fs)
 
 
 def ptr(a):

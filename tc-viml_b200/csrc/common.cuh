@@ -167,6 +167,43 @@ struct DenseArgs {  // device pointers only; viml_dense_factors
   const double* jacobian;
 };
 
+struct InertialArgs {  // device pointers only; viml_inertial_factors plus the state they are evaluated at
+  int W, P, D, X;
+  int64_t NI;
+  double G[3];
+  const int32_t* imu_window_offset;
+  const int32_t* imu_pose;
+  const int32_t* imu_sb;
+  const double* imu_preint;
+  const double* imu_jacobian;
+  const double* imu_sqrt_info;
+  int n_max, max_blocks;
+  const int32_t* prior_n;
+  const double* prior_jacobian;
+  const double* prior_residual;
+  const int32_t* prior_n_blocks;
+  const int32_t* prior_block;
+  const double* prior_x0;
+  const double* poses;    // [W][P][7]
+  const double* ex_pose;  // [W][7]
+  const double* extra;    // [W][X] (may be null when X == 0)
+};
+
+// The dense-factor CSR of the evaluated IMU / prior factors (per window: the prior, then the IMU factors).  Sized on the host from
+// NI, W and n_max alone: factors <= W + NI, rows <= W n_max + 15 NI, columns <= W n_max + 30 NI, Jacobian <= W n_max^2 + 450 NI.
+struct InertialCsr {
+  int32_t* window_offset;  // [W+1]
+  int64_t *row_offset, *col_offset, *jac_offset;   // [W+NI+1]
+  int32_t* col_index;
+  double* residual;
+  double* jacobian;        // null: residuals only
+};
+
+// inertial_kernels.cu.  offsets = true builds window_offset / *_offset / col_index of `csr` (the structure does not depend on the
+// state); the residuals (and the Jacobian when csr.jacobian is set) are written for the state of `v`.  `out` (nullable fields) takes
+// the Ceres layouts.
+int viml_launch_inertial(viml_ctx* ctx, const InertialArgs& v, const viml_inertial_out& out, const InertialCsr& csr, bool offsets);
+
 // linearize_kernels.cu
 int viml_launch_linearize(viml_ctx* ctx, const LinearizeArgs& a);
 int viml_launch_prep(viml_ctx* ctx, const LinearizeArgs& a);   // pose cache of the state in `a` only

@@ -1,5 +1,6 @@
 // gn_api.cu — C-ABI entry points for the reduced system of the whole window (dense-block factors: prior, IMU) and one
 // Gauss-Newton / Levenberg-Marquardt iteration on it, plus the line_3d.txt map reader.  See include/viml.h.
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
@@ -71,14 +72,125 @@ int check_batch(viml_ctx* ctx, const viml_window_batch* in) {
   return VIML_OK;
 }
 
+// viml_inertial_factors: null checks always, index / size validation on the host-pointer path (the device path reads nothing back).
+int check_inertial(viml_ctx* ctx, const viml_inertial_factors* vi, int W, int P, bool dev) {
+  if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
+  const int X = vi->extra_dim, D = 6 * (P + 1), n_max = vi->prior_n_max, mb = vi->prior_max_blocks;
+  const int64_t NI = vi->n_imu;
+  if (X < 0 || D + X > 232) return fail(ctx, VIML_ERR_INVALID, "inertial factors: extra_dim out of range (D + extra_dim <= 232)");
+  if (NI < 0 || n_max < 0 || mb < 0) return fail(ctx, VIML_ERR_INVALID, "inertial factors: negative size");
+  if (NI > 0 && (!vi->imu_window_offset || !vi->imu_pose || !vi->imu_sb || !vi->imu_preint || !vi->imu_jacobian || !vi->imu_sqrt_info))
+    return fail(ctx, VIML_ERR_INVALID, "inertial factors: null IMU array");
+  if (n_max > 0 && (!vi->prior_n || !vi->prior_jacobian || !vi->prior_residual || !vi->prior_n_blocks || (mb > 0 && (!vi->prior_block || !vi->prior_x0))))
+    return fail(ctx, VIML_ERR_INVALID, "inertial factors: null prior array");
+  // read from the struct alone, so both flavours check it: an IMU factor reads two 9-value speed-bias blocks of the extra state
+  if (NI > 0 && X < 9) return fail(ctx, VIML_ERR_INVALID, "IMU factors need extra_dim >= 9 (two speed-bias blocks of 9 values)");
+  if (dev || W == 0) return VIML_OK;
+  if (NI > 0) {
+    const int32_t* off = vi->imu_window_offset;
+    if (off[0] != 0 || off[W] != NI) return fail(ctx, VIML_ERR_INVALID, "IMU factors: imu_window_offset is not a CSR of the factor list");
+    for (int w = 0; w < W; ++w)
+      if (off[w + 1] < off[w]) return fail(ctx, VIML_ERR_INVALID, "IMU factors: imu_window_offset decreases");
+    for (int64_t k = 0; k < NI; ++k) {
+      const int i = vi->imu_pose[2 * k], j = vi->imu_pose[2 * k + 1], si = vi->imu_sb[2 * k], sj = vi->imu_sb[2 * k + 1];
+      if (i < 0 || i >= P || j < 0 || j >= P || i == j) return fail(ctx, VIML_ERR_INVALID, "IMU factor: pose index outside [0, P) or i == j");
+      if (si < 0 || si + 9 > X || sj < 0 || sj + 9 > X) return fail(ctx, VIML_ERR_INVALID, "IMU factor: speed-bias block outside the extra state (sb + 9 <= X)");
+      if (si + 9 > sj && sj + 9 > si) return fail(ctx, VIML_ERR_INVALID, "IMU factor: speed-bias blocks i and j overlap");
+    }
+  }
+  if (n_max > 0) {
+    std::vector<int> col_mark, tan_mark(D + X);
+    for (int w = 0; w < W; ++w) {
+      const int n = vi->prior_n[w];
+      if (n < 0 || n > n_max) return fail(ctx, VIML_ERR_INVALID, "prior: n_w outside [0, prior_n_max]");
+      if (n == 0) continue;
+      const int nb = vi->prior_n_blocks[w];
+      if (nb < 0 || nb > mb) return fail(ctx, VIML_ERR_INVALID, "prior: block count outside [0, prior_max_blocks]");
+      col_mark.assign(n, 0);
+      std::fill(tan_mark.begin(), tan_mark.end(), 0);
+      for (int b = 0; b < nb; ++b) {
+        const int32_t* blk = vi->prior_block + ((size_t)w * mb + b) * 4;
+        const int kind = blk[0], idx = blk[1], size = blk[2], first = blk[3];
+        int tcol;
+        if (kind == VIML_BLOCK_POSE || kind == VIML_BLOCK_EX) {
+          if (size != 7) return fail(ctx, VIML_ERR_INVALID, "prior: a pose / extrinsic block must have size 7");
+          if (kind == VIML_BLOCK_POSE && (idx < 0 || idx >= P)) return fail(ctx, VIML_ERR_INVALID, "prior: pose index outside [0, P)");
+          tcol = kind == VIML_BLOCK_POSE ? 6 * idx : 6 * P;
+        } else if (kind == VIML_BLOCK_EXTRA) {
+          if (size < 1 || size == 7 || size > VIML_PRIOR_X0_STRIDE || idx < 0 || idx + size > X)
+            return fail(ctx, VIML_ERR_INVALID, "prior: extra block outside the extra state (or of size 7, or above VIML_PRIOR_X0_STRIDE)");
+          tcol = D + idx;
+        } else {
+          return fail(ctx, VIML_ERR_INVALID, "prior: unknown block kind");
+        }
+        const int local = size == 7 ? 6 : size;
+        if (first < 0 || first + local > n) return fail(ctx, VIML_ERR_INVALID, "prior: block columns outside [0, n_w)");
+        for (int t = 0; t < local; ++t) {
+          if (col_mark[first + t]++ || tan_mark[tcol + t]++) return fail(ctx, VIML_ERR_INVALID, "prior: blocks overlap");
+        }
+      }
+      for (int c = 0; c < n; ++c)
+        if (!col_mark[c]) return fail(ctx, VIML_ERR_INVALID, "prior: the blocks do not cover [0, n_w)");
+    }
+  }
+  return VIML_OK;
+}
+
+// Stages viml_inertial_factors into *out (the Stager keeps the addresses of its fields: commit() fills them in); the state
+// pointers are left to the caller.
+void stage_inertial(Stager& st, const viml_inertial_factors* vi, int W, int P, InertialArgs* out) {
+  InertialArgs& v = *out;
+  v = InertialArgs{};
+  v.W = W, v.P = P, v.D = 6 * (P + 1), v.X = vi->extra_dim, v.NI = vi->n_imu;
+  for (int k = 0; k < 3; ++k) v.G[k] = vi->gravity[k];
+  v.n_max = vi->prior_n_max, v.max_blocks = vi->prior_max_blocks;
+  const size_t NI = (size_t)v.NI, n_max = (size_t)v.n_max, mb = (size_t)v.max_blocks;
+  st.in(NI ? vi->imu_window_offset : nullptr, NI ? (size_t)W + 1 : 0, &v.imu_window_offset);
+  st.in(vi->imu_pose, NI * 2, &v.imu_pose);
+  st.in(vi->imu_sb, NI * 2, &v.imu_sb);
+  st.in(vi->imu_preint, NI * 17, &v.imu_preint);
+  st.in(vi->imu_jacobian, NI * 225, &v.imu_jacobian);
+  st.in(vi->imu_sqrt_info, NI * 225, &v.imu_sqrt_info);
+  if (n_max) {
+    st.in(vi->prior_n, (size_t)W, &v.prior_n);
+    st.in(vi->prior_jacobian, (size_t)W * n_max * n_max, &v.prior_jacobian);
+    st.in(vi->prior_residual, (size_t)W * n_max, &v.prior_residual);
+    st.in(vi->prior_n_blocks, (size_t)W, &v.prior_n_blocks);
+    st.in(vi->prior_block, (size_t)W * mb * 4, &v.prior_block);
+    st.in(vi->prior_x0, (size_t)W * mb * VIML_PRIOR_X0_STRIDE, &v.prior_x0);
+  }
+}
+
+// Scratch of the dense-factor CSR of the evaluated IMU / prior factors (bounds in common.cuh).
+void stage_inertial_csr(Stager& st, const InertialArgs& v, InertialCsr* csr, double** residual_plus) {
+  const size_t W = (size_t)v.W, NI = (size_t)v.NI, n_max = (size_t)v.n_max;
+  st.out((int32_t*)nullptr, W + 1, &csr->window_offset);
+  st.out((int64_t*)nullptr, W + NI + 1, &csr->row_offset);
+  st.out((int64_t*)nullptr, W + NI + 1, &csr->col_offset);
+  st.out((int64_t*)nullptr, W + NI + 1, &csr->jac_offset);
+  st.out((int32_t*)nullptr, W * n_max + 30 * NI + 1, &csr->col_index);
+  st.out((double*)nullptr, W * n_max + 15 * NI + 1, &csr->residual);
+  st.out((double*)nullptr, W * n_max * n_max + 450 * NI + 1, &csr->jacobian);
+  st.out((double*)nullptr, W * n_max + 15 * NI + 1, residual_plus);
+}
+
 // Shared core of viml_reduced_system / viml_gn_step.
+// With `vi` the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at x+
+// (cost[1], exactly); `dense` is then ignored.
 int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
-        const viml_gn_options* opt, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags) {
+        const viml_gn_options* opt, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags,
+        const viml_inertial_factors* vi = nullptr) {
   int rc = check_batch(ctx, in);
   if (rc != VIML_OK) return rc;
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
   const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
-  const int X = dense ? dense->extra_dim : 0, Dx = D + X;
+  if (vi) {
+    dense = nullptr;
+    rc = check_inertial(ctx, vi, W, P, (flags & VIML_PTRS_DEVICE) != 0);
+    if (rc != VIML_OK) return rc;
+    if (vi->extra_dim > 0 && !extra_state) return fail(ctx, VIML_ERR_INVALID, "viml_gn_step_vi: extra_dim > 0 needs extra_state");
+  }
+  const int X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, Dx = D + X;
   const int64_t ND = dense ? dense->n_factors : 0;
   if (X < 0 || ND < 0 || Dx > 232) return fail(ctx, VIML_ERR_INVALID, "dense factors: extra_dim out of range (D + extra_dim <= 232)");
   if (ND > 0 && (!dense->window_offset || !dense->row_offset || !dense->col_offset || !dense->jac_offset || !dense->col_index ||
@@ -170,6 +282,13 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
     st.in(dense->residual, (size_t)n_rows, &dn.residual);
     st.in(dense->jacobian, (size_t)n_jac, &dn.jacobian);
   }
+  InertialArgs va{};
+  InertialCsr csr{};
+  double* res_plus = nullptr;   // residuals of the IMU / prior factors at x+
+  if (vi) {
+    stage_inertial(st, vi, W, P, &va);
+    stage_inertial_csr(st, va, &csr, &res_plus);
+  }
   // scratch (host == nullptr) and outputs
   double *cache = nullptr, *Sx = nullptr, *gx = nullptr, *dxv = nullptr, *cost = nullptr;
   double *o_poses = nullptr, *o_ex = nullptr, *o_dep = nullptr, *o_extra = nullptr;
@@ -210,6 +329,14 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   }
   rc = viml_launch_linearize(ctx, a);
   if (rc != VIML_OK) return rc;
+  if (vi) {   // the dense-block factors at x, in the CSR every kernel below reads
+    va.poses = a.poses, va.ex_pose = a.ex_pose, va.extra = d_extra;
+    rc = viml_launch_inertial(ctx, va, viml_inertial_out{}, csr, true);
+    if (rc != VIML_OK) return rc;
+    dn.ND = (int64_t)W + va.NI;   // an upper bound: the kernels read ND only as "any dense factors"
+    dn.window_offset = csr.window_offset, dn.row_offset = csr.row_offset, dn.col_offset = csr.col_offset;
+    dn.jac_offset = csr.jac_offset, dn.col_index = csr.col_index, dn.residual = csr.residual, dn.jacobian = csr.jacobian;
+  }
   // a step that does not have to hand Sx / gx to the caller builds and solves the reduced system in one kernel
   bool fused = false;
   if (step && !(rout && (rout->Sx || rout->gx))) {
@@ -234,7 +361,19 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
     LinearizeArgs a2 = a;
     a2.poses = o_poses, a2.ex_pose = o_ex, a2.inv_depth = o_dep;
     rc = viml_launch_prep(ctx, a2);
-    if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dn, dxv, 1, cost);
+    if (rc != VIML_OK) return rc;
+    if (vi) {   // f(x+): the IMU / prior residuals re-evaluated at x+ (same CSR structure), 1/2 |r|^2 without the linear model
+      InertialArgs vp = va;
+      vp.poses = o_poses, vp.ex_pose = o_ex, vp.extra = o_extra;
+      InertialCsr cp = csr;
+      cp.residual = res_plus, cp.jacobian = nullptr;
+      rc = viml_launch_inertial(ctx, vp, viml_inertial_out{}, cp, false);
+      DenseArgs dp = dn;
+      dp.residual = res_plus;
+      if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, 1, cost);
+    } else {
+      rc = viml_launch_cost(ctx, a2, dn, dxv, 1, cost);
+    }
     if (rc != VIML_OK) return rc;
   }
   return st.finish();
@@ -308,6 +447,52 @@ int viml_gn_step(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_fa
   if (!ctx) return VIML_ERR_INVALID;
   if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
   return run(ctx, in, dense, extra_state, opt, nullptr, out, flags);
+}
+
+int viml_gn_step_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
+                    const viml_gn_options* opt, const viml_gn_out* out, uint32_t flags) {
+  if (!ctx) return VIML_ERR_INVALID;
+  if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
+  if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
+  return run(ctx, in, nullptr, extra_state, opt, nullptr, out, flags, vi);
+}
+
+int viml_inertial_evaluate(viml_ctx* ctx, const viml_window_batch* state, const double* extra_state, const viml_inertial_factors* vi,
+                           const viml_inertial_out* out, uint32_t flags) {
+  if (!ctx) return VIML_ERR_INVALID;
+  if (!state || !out) return fail(ctx, VIML_ERR_INVALID, "viml_inertial_evaluate: null arguments");
+  const int W = state->n_windows, P = state->poses_per_window;
+  if (W < 0 || P < 1 || P > 255) return fail(ctx, VIML_ERR_INVALID, "window batch sizes out of range");
+  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
+  int rc = check_inertial(ctx, vi, W, P, dev);
+  if (rc != VIML_OK) return rc;
+  if (W > 0 && (!state->poses || !state->ex_pose)) return fail(ctx, VIML_ERR_INVALID, "null input array");
+  if (vi->extra_dim > 0 && !extra_state) return fail(ctx, VIML_ERR_INVALID, "viml_inertial_evaluate: extra_dim > 0 needs extra_state");
+  if (W == 0) return VIML_OK;
+  VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
+  Stager st{ctx, dev};
+  InertialArgs v;
+  stage_inertial(st, vi, W, P, &v);
+  st.in(state->poses, (size_t)W * P * 7, &v.poses);
+  st.in(state->ex_pose, (size_t)W * 7, &v.ex_pose);
+  st.in(extra_state, extra_state ? (size_t)W * v.X : 0, &v.extra);
+  const size_t NI = (size_t)v.NI;
+  viml_inertial_out o{};
+  st.out(out->imu_residual, out->imu_residual ? NI * 15 : 0, &o.imu_residual);
+  st.out(out->imu_jac_pose_i, out->imu_jac_pose_i ? NI * 105 : 0, &o.imu_jac_pose_i);
+  st.out(out->imu_jac_sb_i, out->imu_jac_sb_i ? NI * 135 : 0, &o.imu_jac_sb_i);
+  st.out(out->imu_jac_pose_j, out->imu_jac_pose_j ? NI * 105 : 0, &o.imu_jac_pose_j);
+  st.out(out->imu_jac_sb_j, out->imu_jac_sb_j ? NI * 135 : 0, &o.imu_jac_sb_j);
+  st.out(out->prior_residual, out->prior_residual ? (size_t)W * v.n_max : 0, &o.prior_residual);
+  rc = st.commit();
+  if (rc != VIML_OK) return rc;
+  // host flavour: the staged prior residuals start as a copy of the caller's buffer, so that rows past n_w keep its content
+  if (!dev && out->prior_residual)
+    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(o.prior_residual, out->prior_residual, (size_t)W * v.n_max * sizeof(double), cudaMemcpyHostToDevice,
+                                       ctx->stream));
+  rc = viml_launch_inertial(ctx, v, o, InertialCsr{}, false);
+  if (rc != VIML_OK) return rc;
+  return st.finish();
 }
 
 int viml_triangulate_batch(viml_ctx* ctx, const viml_triangulate_in* in, double init_depth, double* depth, uint32_t flags) {

@@ -398,3 +398,123 @@ def make_dense_factors(batch, seed=5):
         c0 = np.concatenate([np.arange(6), D + np.arange(9)])
         fs.append((w, 0.01 * rng.standard_normal(15), np.diag(200.0 + 50.0 * rng.uniform(size=15)), c0))
     return Dense(W, X, fs)
+
+
+# ---- IMU factors and the prior of a window, as inputs of viml_inertial_evaluate / viml_gn_step_vi ------------------------------
+def _qmul(a, b):
+    """Hamilton product of [..., (x, y, z, w)] quaternions."""
+    ax, ay, az, aw = np.moveaxis(a, -1, 0)
+    bx, by, bz, bw = np.moveaxis(b, -1, 0)
+    return np.stack([aw * bx + ax * bw + ay * bz - az * by, aw * by + ay * bw + az * bx - ax * bz,
+                     aw * bz + az * bw + ax * by - ay * bx, aw * bw - ax * bx - ay * by - az * bz], -1)
+
+
+def _qconj(q):
+    return np.concatenate([-q[..., :3], q[..., 3:]], -1) / (q * q).sum(-1, keepdims=True)
+
+
+def _rot(q):
+    """toRotationMatrix of an (x, y, z, w) quaternion (no normalisation)."""
+    x, y, z, w = q
+    return np.array([[1 - 2 * (y * y + z * z), 2 * (x * y - w * z), 2 * (x * z + w * y)],
+                     [2 * (x * y + w * z), 1 - 2 * (x * x + z * z), 2 * (y * z - w * x)],
+                     [2 * (x * z - w * y), 2 * (y * z + w * x), 1 - 2 * (x * x + y * y)]])
+
+
+def make_inertial_factors(batch, seed=11, realistic=False, no_imu=(), no_prior=(), extra_pad=0, n_max=None, noise=1e-3):
+    """(Inertial, extra_state [W, X]) for a window batch: one IMU factor per consecutive pose pair and one prior per window, the way
+    Estimator::optimization adds them (estimator.cpp:1717-1733).
+
+    The extra state holds a speed-bias block [V, Ba, Bg] per pose (offset 9 p), plus `extra_pad` values no factor touches.  The
+    pre-integrated deltas are formed from the batch's poses with the chosen velocities and biases (so the residuals are small),
+    plus `noise`; linearized_ba / linearized_bg differ from the state's biases so the bias corrections are exercised; the
+    pre-integration Jacobian takes its first-order closed forms (dp_dba = -R dt^2 / 2, dq_dbg = -dt I, dv_dba = -R dt, ...) plus
+    jitter; sqrt_info = LLT(covariance^-1).matrixL()^T of an SPD covariance.  By default the covariance is scaled like
+    make_dense_factors (entries of sqrt_info of order 10^2: the reduced system stays well conditioned); realistic=True takes the
+    EuRoC noise densities (acc_n 0.08, gyr_n 0.004, acc_w 4e-5, gyr_w 2e-6: bias rows of the covariance near 1e-11).
+    The prior covers [pose 1 .. P-1, extrinsic, speed-bias 1] (n = 6 P + 9, 75 at P = 11) with x0 near the state; windows in
+    no_imu / no_prior carry none.  n_max (default n) is the prior stride."""
+    from ._abi import BLOCK_EX, BLOCK_EXTRA, BLOCK_POSE, PRIOR_X0_STRIDE, Inertial
+    rng = np.random.default_rng(seed)
+    W, P = batch.W, batch.P
+    X = 9 * P + extra_pad
+    G = np.array([0.0, 0.0, 9.81])
+    extra = np.zeros((W, X))
+    sb = extra[:, :9 * P].reshape(W, P, 9)
+    sb[..., 0:3] = 0.5 * rng.standard_normal((W, P, 3))
+    sb[..., 3:6] = 0.05 * rng.standard_normal((W, P, 3))
+    sb[..., 6:9] = 0.005 * rng.standard_normal((W, P, 3))
+    if extra_pad:
+        extra[:, 9 * P:] = rng.standard_normal((W, extra_pad))
+    pose_list, sb_list, pre, jac, info, off = [], [], [], [], [], [0]
+    for w in range(W):
+        pairs = [] if w in no_imu else [(p, p + 1) for p in range(P - 1)]
+        for (i, j) in pairs:
+            dt = rng.uniform(0.05, 0.15)
+            xi, xj = batch.poses[w, i], batch.poses[w, j]
+            qi, qj = xi[3:7], xj[3:7]
+            Ri = _rot(qi)
+            RiT = np.linalg.inv(Ri)
+            Vi, Bai, Bgi = sb[w, i, 0:3], sb[w, i, 3:6], sb[w, i, 6:9]
+            Vj = sb[w, j, 0:3]
+            J = np.eye(15) + 0.01 * rng.standard_normal((15, 15))
+            J[0:3, 9:12] = -0.5 * RiT * dt * dt + 1e-4 * rng.standard_normal((3, 3))
+            J[0:3, 12:15] = 0.01 * dt * rng.standard_normal((3, 3))
+            J[3:6, 12:15] = -dt * np.eye(3) + 1e-3 * rng.standard_normal((3, 3))
+            J[6:9, 9:12] = -RiT * dt + 1e-3 * rng.standard_normal((3, 3))
+            J[6:9, 12:15] = 0.01 * dt * rng.standard_normal((3, 3))
+            lin_ba = Bai + 0.02 * rng.standard_normal(3)
+            lin_bg = Bgi + 0.002 * rng.standard_normal(3)
+            dba, dbg = Bai - lin_ba, Bgi - lin_bg
+            dp = RiT @ (0.5 * G * dt * dt + xj[:3] - xi[:3] - Vi * dt) - J[0:3, 9:12] @ dba - J[0:3, 12:15] @ dbg
+            dv = RiT @ (G * dt + Vj - Vi) - J[6:9, 9:12] @ dba - J[6:9, 12:15] @ dbg
+            corr = np.concatenate([0.5 * (J[3:6, 12:15] @ dbg), [1.0]])
+            qij = _qmul(_qconj(qi), qj)
+            dq = _qmul(qij, _qconj(corr))
+            dq = _qmul(dq, np.concatenate([0.5 * noise * rng.standard_normal(3), [1.0]]))
+            dq /= np.linalg.norm(dq)
+            dp = dp + noise * rng.standard_normal(3)
+            dv = dv + noise * rng.standard_normal(3)
+            pre.append(np.concatenate([[dt], dp, dq, dv, lin_ba, lin_bg]))
+            jac.append(J)
+            if realistic:
+                acc_n, gyr_n, acc_w, gyr_w = 0.08, 0.004, 4e-5, 2e-6
+                sig2 = np.concatenate([np.full(3, acc_n ** 2 * dt ** 3), np.full(3, gyr_n ** 2 * dt), np.full(3, acc_n ** 2 * dt),
+                                       np.full(3, acc_w ** 2 * dt), np.full(3, gyr_w ** 2 * dt)])
+            else:
+                sig2 = (0.01 * (1.0 + rng.uniform(size=15))) ** 2
+            A = rng.standard_normal((15, 15)) * 0.1
+            C = np.sqrt(sig2)[:, None] * (np.eye(15) + 0.1 * (A + A.T)) * np.sqrt(sig2)[None, :]
+            C = 0.5 * (C + C.T) + np.diag(sig2) * 0.05
+            L = np.linalg.cholesky(np.linalg.inv(C))
+            info.append(L.T)
+            pose_list.append((i, j))
+            sb_list.append((9 * i, 9 * j))
+        off.append(len(pre))
+    n = 6 * (P - 1) + 6 + 9
+    nm = n if n_max is None else int(n_max)
+    blocks = [(BLOCK_POSE, p, 7, 6 * (p - 1)) for p in range(1, P)] + [(BLOCK_EX, 0, 7, 6 * (P - 1)), (BLOCK_EXTRA, 9, 9, 6 * P)]
+    mb = len(blocks)
+    prior_n = np.array([0 if w in no_prior else n for w in range(W)], dtype=np.int32)
+    pj, pr = np.zeros((W, nm, nm)), np.zeros((W, nm))
+    pblk, px0 = np.zeros((W, mb, 4), dtype=np.int32), np.zeros((W, mb, PRIOR_X0_STRIDE))
+    for w in range(W):
+        J = 20.0 * rng.standard_normal((n, n)) + np.diag(250.0 + 50.0 * rng.uniform(size=n))
+        pj[w, :n, :n] = J
+        pr[w, :n] = 0.05 * rng.standard_normal(n)
+        pblk[w] = np.array(blocks, dtype=np.int32)
+        for b, (kind, idx, size, first) in enumerate(blocks):
+            x = batch.poses[w, idx] if kind == BLOCK_POSE else batch.ex_pose[w] if kind == BLOCK_EX else extra[w, idx:idx + size]
+            x0 = np.array(x, dtype=np.float64).copy()
+            if size == 7:
+                x0[:3] += 0.01 * rng.standard_normal(3)
+                x0[3:7] = _qmul(x0[3:7], np.concatenate([0.005 * rng.standard_normal(3), [1.0]]))
+                x0[3:7] /= np.linalg.norm(x0[3:7])
+            else:
+                x0 = x0 + 0.01 * rng.standard_normal(size)
+            px0[w, b, :size] = x0
+    NI = len(pre)
+    vi = Inertial(W, P, X, G, np.array(off, dtype=np.int32), np.array(pose_list, dtype=np.int32).reshape(NI, 2),
+                  np.array(sb_list, dtype=np.int32).reshape(NI, 2), np.array(pre).reshape(NI, 17), np.array(jac).reshape(NI, 15, 15),
+                  np.array(info).reshape(NI, 15, 15), prior_n, pj, pr, np.full(W, mb, dtype=np.int32), pblk, px0)
+    return vi, extra
