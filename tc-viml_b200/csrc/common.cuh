@@ -81,7 +81,6 @@ struct viml_ctx {
   int64_t fov_words = 0;
   unsigned long long* d_assoc_stats = nullptr;  // {gate tests, gated pairs, overlap-scored, distance-scored} of the last association call
   DeviceArena in_arena, out_arena, scratch, scratch2, scratch3, gn_in, gn_out, s_full;
-  bool schur_splitk = false;   // VIML_SCHUR_SPLITK=1: round-1 split-K Schur kernel instead of the TMA-pipelined one
   // pinned staging of the small-batch host path (one H2D, one D2H per call)
   char *h_stage_in = nullptr, *h_stage_out = nullptr;
   size_t h_stage_in_cap = 0, h_stage_out_cap = 0;
@@ -154,6 +153,10 @@ struct LinearizeArgs {  // device pointers only
   double sqrt_info, cauchy_a, inv_cauchy_a2, fx, fy, cx, cy;
   uint32_t flags;
 };
+
+// Largest reduced system a Gauss-Newton step takes, Dx = D + extra_dim (viml.h): its tiled Cholesky keeps the lower triangle in
+// shared memory (linearize_kernels.cu checks the size at compile time).
+constexpr int kMaxDx = 232;
 
 struct DenseArgs {  // device pointers only; viml_dense_factors
   int X;          // extra tangent columns behind the D pose / extrinsic columns

@@ -77,7 +77,7 @@ int check_inertial(viml_ctx* ctx, const viml_inertial_factors* vi, int W, int P,
   if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
   const int X = vi->extra_dim, D = 6 * (P + 1), n_max = vi->prior_n_max, mb = vi->prior_max_blocks;
   const int64_t NI = vi->n_imu;
-  if (X < 0 || D + X > 232) return fail(ctx, VIML_ERR_INVALID, "inertial factors: extra_dim out of range (D + extra_dim <= 232)");
+  if (X < 0 || D + X > kMaxDx) return fail(ctx, VIML_ERR_INVALID, "inertial factors: extra_dim out of range (D + extra_dim <= 232)");
   if (NI < 0 || n_max < 0 || mb < 0) return fail(ctx, VIML_ERR_INVALID, "inertial factors: negative size");
   if (NI > 0 && (!vi->imu_window_offset || !vi->imu_pose || !vi->imu_sb || !vi->imu_preint || !vi->imu_jacobian || !vi->imu_sqrt_info))
     return fail(ctx, VIML_ERR_INVALID, "inertial factors: null IMU array");
@@ -174,6 +174,48 @@ void stage_inertial_csr(Stager& st, const InertialArgs& v, InertialCsr* csr, dou
   st.out((double*)nullptr, W * n_max + 15 * NI + 1, residual_plus);
 }
 
+// viml_dense_factors of W windows over Dx tangent columns: ND and the arrays of *dn (the Stager keeps the addresses of its fields).
+// The kernels index row_offset, jac_offset, the Jacobian and the Sx columns through window_offset, the offsets and col_index: the
+// host flavour checks all of them; the device flavour reads back the three totals, which size the staged arrays.
+int stage_dense(viml_ctx* ctx, Stager& st, const viml_dense_factors* dense, int W, int Dx, DenseArgs* dn) {
+  const int64_t ND = dense ? dense->n_factors : 0;
+  dn->ND = ND;
+  if (ND == 0) return VIML_OK;
+  if (!dense->window_offset || !dense->row_offset || !dense->col_offset || !dense->jac_offset || !dense->col_index || !dense->residual ||
+      !dense->jacobian)
+    return fail(ctx, VIML_ERR_INVALID, "dense factors: null array");
+  int64_t n_rows = 0, n_cols = 0, n_jac = 0;
+  if (st.dev) {   // totals are the last prefix entries: three 8-byte reads from the device
+    int64_t t[3];
+    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[0], dense->row_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[1], dense->col_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[2], dense->jac_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    n_rows = t[0], n_cols = t[1], n_jac = t[2];
+  } else {
+    const int32_t* off = dense->window_offset;
+    if (off[0] != 0 || off[W] != ND) return fail(ctx, VIML_ERR_INVALID, "dense factors: window_offset is not a CSR of the factor list");
+    for (int w = 0; w < W; ++w)
+      if (off[w + 1] < off[w]) return fail(ctx, VIML_ERR_INVALID, "dense factors: window_offset decreases");
+    n_rows = dense->row_offset[ND], n_cols = dense->col_offset[ND], n_jac = dense->jac_offset[ND];
+    for (int64_t k = 0; k < n_cols; ++k)
+      if (dense->col_index[k] < 0 || dense->col_index[k] >= Dx) return fail(ctx, VIML_ERR_INVALID, "dense factors: col_index out of range");
+    for (int64_t k = 0; k < ND; ++k) {
+      const int64_t n = dense->row_offset[k + 1] - dense->row_offset[k], c = dense->col_offset[k + 1] - dense->col_offset[k];
+      if (n < 0 || c < 0 || dense->jac_offset[k + 1] - dense->jac_offset[k] != n * c)
+        return fail(ctx, VIML_ERR_INVALID, "dense factors: jac_offset does not match rows x columns");
+    }
+  }
+  st.in(dense->window_offset, (size_t)W + 1, &dn->window_offset);
+  st.in(dense->row_offset, (size_t)ND + 1, &dn->row_offset);
+  st.in(dense->col_offset, (size_t)ND + 1, &dn->col_offset);
+  st.in(dense->jac_offset, (size_t)ND + 1, &dn->jac_offset);
+  st.in(dense->col_index, (size_t)n_cols, &dn->col_index);
+  st.in(dense->residual, (size_t)n_rows, &dn->residual);
+  st.in(dense->jacobian, (size_t)n_jac, &dn->jacobian);
+  return VIML_OK;
+}
+
 // Shared core of viml_reduced_system / viml_gn_step.
 // With `vi` the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at x+
 // (cost[1], exactly); `dense` is then ignored.
@@ -192,10 +234,7 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   }
   const int X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, Dx = D + X;
   const int64_t ND = dense ? dense->n_factors : 0;
-  if (X < 0 || ND < 0 || Dx > 232) return fail(ctx, VIML_ERR_INVALID, "dense factors: extra_dim out of range (D + extra_dim <= 232)");
-  if (ND > 0 && (!dense->window_offset || !dense->row_offset || !dense->col_offset || !dense->jac_offset || !dense->col_index ||
-                 !dense->residual || !dense->jacobian))
-    return fail(ctx, VIML_ERR_INVALID, "dense factors: null array");
+  if (X < 0 || ND < 0 || Dx > kMaxDx) return fail(ctx, VIML_ERR_INVALID, "dense factors: extra_dim out of range (D + extra_dim <= 232)");
   const bool step = gout != nullptr;
   if (step && !(gout->poses && gout->ex_pose && (F == 0 || gout->inv_depth) && gout->cost && gout->solved))
     return fail(ctx, VIML_ERR_INVALID, "viml_gn_step needs poses, ex_pose, inv_depth, cost and solved outputs");
@@ -204,31 +243,11 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   if (W == 0) return VIML_OK;
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
   const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
-  int64_t n_rows = 0, n_cols = 0, n_jac = 0;
-  if (ND > 0) {
-    if (dev) {   // totals are the last prefix entries: three 8-byte reads from the device
-      int64_t t[3];
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[0], dense->row_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[1], dense->col_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[2], dense->jac_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-      n_rows = t[0], n_cols = t[1], n_jac = t[2];
-    } else {
-      n_rows = dense->row_offset[ND], n_cols = dense->col_offset[ND], n_jac = dense->jac_offset[ND];
-      if (dense->window_offset[0] != 0 || dense->window_offset[W] != ND)
-        return fail(ctx, VIML_ERR_INVALID, "dense factors: window_offset is not a CSR of the factor list");
-      for (int64_t k = 0; k < n_cols; ++k)
-        if (dense->col_index[k] < 0 || dense->col_index[k] >= Dx)
-          return fail(ctx, VIML_ERR_INVALID, "dense factors: col_index out of range");
-      for (int64_t k = 0; k < ND; ++k) {
-        const int64_t n = dense->row_offset[k + 1] - dense->row_offset[k], c = dense->col_offset[k + 1] - dense->col_offset[k];
-        if (n < 0 || c < 0 || dense->jac_offset[k + 1] - dense->jac_offset[k] != n * c)
-          return fail(ctx, VIML_ERR_INVALID, "dense factors: jac_offset does not match rows x columns");
-      }
-    }
-  }
-
   Stager st{ctx, dev};
+  DenseArgs dn{};
+  dn.X = X;
+  rc = stage_dense(ctx, st, dense, W, Dx, &dn);
+  if (rc != VIML_OK) return rc;
   LinearizeArgs a{};
   a.W = W, a.P = P, a.F = F, a.D = D, a.NP = NP, a.NL = NL, a.pf_begin = 0, a.lf_begin = 0, a.NL_stride = NL;
   a.sqrt_info = ctx->cfg.sqrt_info, a.cauchy_a = ctx->cfg.cauchy_a, a.inv_cauchy_a2 = 1.0 / (ctx->cfg.cauchy_a * ctx->cfg.cauchy_a);
@@ -271,17 +290,6 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   }
   const double* d_extra = nullptr;
   st.in(extra_state, extra_state ? (size_t)W * X : 0, &d_extra);
-  DenseArgs dn{};
-  dn.X = X, dn.ND = ND;
-  if (ND > 0) {
-    st.in(dense->window_offset, (size_t)W + 1, &dn.window_offset);
-    st.in(dense->row_offset, (size_t)ND + 1, &dn.row_offset);
-    st.in(dense->col_offset, (size_t)ND + 1, &dn.col_offset);
-    st.in(dense->jac_offset, (size_t)ND + 1, &dn.jac_offset);
-    st.in(dense->col_index, (size_t)n_cols, &dn.col_index);
-    st.in(dense->residual, (size_t)n_rows, &dn.residual);
-    st.in(dense->jacobian, (size_t)n_jac, &dn.jacobian);
-  }
   InertialArgs va{};
   InertialCsr csr{};
   double* res_plus = nullptr;   // residuals of the IMU / prior factors at x+
@@ -396,46 +404,20 @@ int viml_reduced_from_schur(viml_ctx* ctx, int32_t W, int32_t D, const double* S
   const int64_t ND = dense ? dense->n_factors : 0;
   if (W < 0 || D < 1 || X < 0 || ND < 0 || !S || !g || !out || !out->Sx || !out->gx)
     return fail(ctx, VIML_ERR_INVALID, "viml_reduced_from_schur: bad arguments");
-  if (ND > 0 && (!dense->window_offset || !dense->row_offset || !dense->col_offset || !dense->jac_offset || !dense->col_index ||
-                 !dense->residual || !dense->jacobian))
-    return fail(ctx, VIML_ERR_INVALID, "dense factors: null array");
   if (W == 0) return VIML_OK;
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
-  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
-  int64_t n_rows = 0, n_cols = 0, n_jac = 0;
-  if (ND > 0) {
-    if (dev) {
-      int64_t t[3];
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[0], dense->row_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[1], dense->col_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&t[2], dense->jac_offset + ND, 8, cudaMemcpyDeviceToHost, ctx->stream));
-      VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-      n_rows = t[0], n_cols = t[1], n_jac = t[2];
-    } else {
-      n_rows = dense->row_offset[ND], n_cols = dense->col_offset[ND], n_jac = dense->jac_offset[ND];
-      for (int64_t k = 0; k < n_cols; ++k)
-        if (dense->col_index[k] < 0 || dense->col_index[k] >= Dx) return fail(ctx, VIML_ERR_INVALID, "dense factors: col_index out of range");
-    }
-  }
-  Stager st{ctx, dev};
+  Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
   const double *dS = nullptr, *dg = nullptr;
   st.in(S, (size_t)W * D * D, &dS);
   st.in(g, (size_t)W * D, &dg);
   DenseArgs dn{};
-  dn.X = X, dn.ND = ND;
-  if (ND > 0) {
-    st.in(dense->window_offset, (size_t)W + 1, &dn.window_offset);
-    st.in(dense->row_offset, (size_t)ND + 1, &dn.row_offset);
-    st.in(dense->col_offset, (size_t)ND + 1, &dn.col_offset);
-    st.in(dense->jac_offset, (size_t)ND + 1, &dn.jac_offset);
-    st.in(dense->col_index, (size_t)n_cols, &dn.col_index);
-    st.in(dense->residual, (size_t)n_rows, &dn.residual);
-    st.in(dense->jacobian, (size_t)n_jac, &dn.jacobian);
-  }
+  dn.X = X;
+  int rc = stage_dense(ctx, st, dense, W, Dx, &dn);
+  if (rc != VIML_OK) return rc;
   double *Sx = nullptr, *gx = nullptr;
   st.out(out->Sx, (size_t)W * Dx * Dx, &Sx);
   st.out(out->gx, (size_t)W * Dx, &gx);
-  int rc = st.commit();
+  rc = st.commit();
   if (rc != VIML_OK) return rc;
   rc = viml_launch_reduced(ctx, W, D, dn, dS, dg, Sx, gx);
   if (rc != VIML_OK) return rc;

@@ -96,8 +96,8 @@ __global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const
 // diagonal).  Right-looking blocked factorisation: per tile column K (1) warp 0 factors the diagonal tile, (2) one thread per row
 // solves the panel rows against it, (3) the trailing tiles take A[I][J] -= L[I][K] L[J][K]^T as two DMMA steps each, dealt
 // round-robin to warps 1..7 while warp 0 updates and factors the next diagonal tile (look-ahead).  22 tile columns and ~44 barriers
-// for Dx = 171 instead of 171 columns and ~510 barriers in solve_kernel below, and the O(n^3) part runs on the FP64 tensor pipe.
-// Forward / backward substitution tile by tile.
+// for Dx = 171, and the O(n^3) part runs on the FP64 tensor pipe.  Forward / backward substitution tile by tile.
+// solved[w] = 0 when a pivot is not positive (dx = 0 then).  cost[3w + 2] = -gx.dx - 1/2 dx.Sx.dx (undamped model).
 // FUSED: the matrix is not read from Sx but built in place — embed(S) plus the window's dense-block factors (J^T J as DMMA tiles
 // from a staged Jacobian, like reduced_kernel) — so that Sx never makes its 234 KB round trip through HBM; the model decrease then
 // uses A x = -g:  x^T Sx x = -g.x - lambda sum d_i x_i^2  with d the undamped diagonal.
@@ -381,90 +381,6 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
   if (tid == 0) {
     double t = 0.0;
     for (int k = 0; k < 8; ++k) t += s_red[k];
-    cost[3 * (size_t)w + 2] = t;
-    solved[w] = ok ? 1 : 0;
-  }
-}
-
-// dx = -(Sx + lambda diag(Sx))^-1 gx by Cholesky in shared memory (packed lower triangle), one CTA per window.
-// solved[w] = 0 when a pivot is not positive (dx = 0 then).  cost[3w + 2] = -gx.dx - 1/2 dx.Sx.dx (undamped model).
-__global__ void __launch_bounds__(256) solve_kernel(int Dx, double lambda, const double* __restrict__ Sx, const double* __restrict__ gx,
-                                                    double* __restrict__ dx, int32_t* __restrict__ solved, double* __restrict__ cost) {
-  extern __shared__ __align__(16) double sm[];
-  __shared__ int s_ok;
-  __shared__ double s_red[8];
-  const int w = blockIdx.x, tid = threadIdx.x, NT = blockDim.x;
-  double* __restrict__ L = sm;                              // packed: L[i][j] at i(i+1)/2 + j, j <= i
-  double* __restrict__ y = sm + (size_t)Dx * (Dx + 1) / 2;   // right-hand side / solution
-  const double* __restrict__ A = Sx + (size_t)w * Dx * Dx;
-  for (int e = tid; e < Dx * Dx; e += NT) {
-    const int i = e / Dx, j = e - i * Dx;
-    if (j <= i) L[i * (i + 1) / 2 + j] = (i == j) ? A[e] * (1.0 + lambda) : 0.5 * (A[e] + A[(size_t)j * Dx + i]);
-  }
-  for (int e = tid; e < Dx; e += NT) y[e] = -gx[(size_t)w * Dx + e];
-  if (tid == 0) s_ok = 1;
-  __syncthreads();
-  for (int j = 0; j < Dx; ++j) {
-    const double d = L[j * (j + 1) / 2 + j];
-    if (!(d > 0.0) || !isfinite(d)) {   // uniform: every thread reads the same value
-      if (tid == 0) s_ok = 0;
-      break;
-    }
-    const double sd = sqrt(d), inv = 1.0 / sd;
-    __syncthreads();
-    for (int i = j + tid; i < Dx; i += NT) L[i * (i + 1) / 2 + j] = (i == j) ? sd : L[i * (i + 1) / 2 + j] * inv;
-    __syncthreads();
-    // trailing update L[i][k] -= L[i][j] L[k][j], j < k <= i, as 16 x 16 thread tiles over the (i, k) triangle: every thread
-    // gets the same number of entries whatever its row
-    {
-      const int ti = tid >> 4, tk = tid & 15, n = Dx - j - 1;
-      for (int i0 = 0; i0 < n; i0 += 16) {
-        const int i = j + 1 + i0 + ti;
-        const double lij = i < Dx ? L[i * (i + 1) / 2 + j] : 0.0;
-        for (int k0 = 0; k0 <= i0; k0 += 16) {
-          const int k = j + 1 + k0 + tk;
-          if (i < Dx && k <= i) L[i * (i + 1) / 2 + k] -= lij * L[k * (k + 1) / 2 + j];
-        }
-      }
-    }
-    __syncthreads();
-  }
-  __syncthreads();
-  const bool ok = s_ok != 0;
-  if (ok) {
-    // forward L z = y, backward L^T x = z (column-oriented, one barrier per column)
-    for (int j = 0; j < Dx; ++j) {
-      if (tid == 0) y[j] /= L[j * (j + 1) / 2 + j];
-      __syncthreads();
-      const double yj = y[j];
-      for (int i = j + 1 + tid; i < Dx; i += NT) y[i] -= L[i * (i + 1) / 2 + j] * yj;
-      __syncthreads();
-    }
-    for (int j = Dx - 1; j >= 0; --j) {
-      if (tid == 0) y[j] /= L[j * (j + 1) / 2 + j];
-      __syncthreads();
-      const double yj = y[j];
-      for (int i = tid; i < j; i += NT) y[i] -= L[j * (j + 1) / 2 + i] * yj;
-      __syncthreads();
-    }
-  }
-  // model decrease with the undamped Sx
-  double part = 0.0;
-  for (int i = tid; i < Dx; i += NT) {
-    const double xi = ok ? y[i] : 0.0;
-    double sx = 0.0;
-    if (ok)
-      for (int c = 0; c < Dx; ++c) sx = fma(A[(size_t)i * Dx + c], y[c], sx);
-    part += -gx[(size_t)w * Dx + i] * xi - 0.5 * xi * sx;
-    dx[(size_t)w * Dx + i] = xi;
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
-  if ((tid & 31) == 0) s_red[tid >> 5] = part;
-  __syncthreads();
-  if (tid == 0) {
-    double t = 0.0;
-    for (int k = 0; k < NT / 32; ++k) t += s_red[k];
     cost[3 * (size_t)w + 2] = t;
     solved[w] = ok ? 1 : 0;
   }

@@ -670,20 +670,19 @@ int viml_launch_reduced(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const 
   return VIML_OK;
 }
 
+// Shared memory of solve_tiled_kernel<false> for a Dx x Dx system: the lower triangle of 8 x 8 tiles and the right-hand side.
+constexpr size_t gn_solve_smem(int Dx) {
+  const size_t NB = (Dx + 7) / 8;
+  return (NB * (NB + 1) / 2 * 64 + NB * 8) * sizeof(double);
+}
+static_assert(gn_solve_smem(kMaxDx) <= 220 * 1024, "the tiled Cholesky of the largest reduced system must fit in shared memory");
+
 int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const double* Sx, const double* gx, double* dx, int32_t* solved,
                          double* cost) {
-  const int NB = (Dx + 7) / 8;
-  const size_t smem_t = ((size_t)NB * (NB + 1) / 2 * 64 + (size_t)NB * 8) * sizeof(double);
+  const size_t smem = gn_solve_smem(Dx);
   LaunchScope ls(ctx, K_GN);
-  if (smem_t <= 220 * 1024 && Dx <= 256 - 8 && !getenv("VIML_GN_UNBLOCKED")) {   // tiled factorisation on the tensor pipe
-    VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
-    gn::solve_tiled_kernel<false><<<W, 256, smem_t, ctx->stream>>>(Dx, lambda, Sx, gx, dx, solved, cost, 0, DenseArgs{}, nullptr, nullptr);
-    VIML_TRY_CUDA(ctx, cudaGetLastError());
-    return VIML_OK;
-  }
-  const size_t smem = ((size_t)Dx * (Dx + 1) / 2 + Dx) * sizeof(double);
-  VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  gn::solve_kernel<<<W, 256, smem, ctx->stream>>>(Dx, lambda, Sx, gx, dx, solved, cost);
+  VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  gn::solve_tiled_kernel<false><<<W, 256, smem, ctx->stream>>>(Dx, lambda, Sx, gx, dx, solved, cost, 0, DenseArgs{}, nullptr, nullptr);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
@@ -694,7 +693,7 @@ int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& d
                                  double* dx, int32_t* solved, double* cost) {
   const int Dx = D + dn.X, NB = (Dx + 7) / 8;
   const size_t smem = ((size_t)NB * (NB + 1) / 2 * 64 + 3 * (size_t)NB * 8 + gn::kFusedStage) * sizeof(double);
-  if (smem > 224 * 1024 || Dx > 256 - 8 || getenv("VIML_GN_UNBLOCKED") || getenv("VIML_GN_UNFUSED")) return VIML_ERR_UNSUPPORTED;
+  if (smem > 224 * 1024) return VIML_ERR_UNSUPPORTED;
   LaunchScope ls(ctx, K_GN);
   VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   gn::solve_tiled_kernel<true><<<W, 256, smem, ctx->stream>>>(Dx, lambda, nullptr, nullptr, dx, solved, cost, D, dn, S, g);

@@ -8,11 +8,11 @@
 // It is a SYRK: D x D output, contraction over the F landmarks — the one GEMM-shaped piece of the hot path
 // (2 D^2 F flop over D F 8 bytes, ~18 flop/B at D = 72), so it goes to the FP64 tensor pipe.  tcgen05 has no
 // FP64 kind; on sm_100a the FP64 MMA is still mma.sync (DMMA in SASS).
-// Three kernels: schur_tma_kernel (D <= 72, the sliding window: TMA + mbarrier producer/consumer pipeline, warps own output tiles;
-// the default), schur_splitk_kernel (its round-1 predecessor, VIML_SCHUR_SPLITK=1) and schur_dmma_kernel (D > 72: one CTA per
-// (72 x 72 output tile, window), 8 warps share the 81 8x8 sub-tiles — 45 on the diagonal, where only the upper triangle is computed
-// and mirrored; W staged through shared memory in chunks of 32 landmarks with a row stride of 76 doubles, conflict-free fragment
-// loads; with the band plan of extent_kernel / order_kernel a tile only visits the landmarks that touch it).
+// Two kernels: schur_tma_kernel (D <= 72, the sliding window: TMA + mbarrier producer/consumer pipeline, warps own output tiles)
+// and schur_dmma_kernel (D > 72: one CTA per (72 x 72 output tile, window), 8 warps share the 81 8x8 sub-tiles — 45 on the
+// diagonal, where only the upper triangle is computed and mirrored; W staged through shared memory in chunks of 32 landmarks with
+// a row stride of 76 doubles, conflict-free fragment loads; with the band plan of extent_kernel / order_kernel a tile only visits
+// the landmarks that touch it).
 #include "common.cuh"
 
 namespace {
@@ -248,147 +248,6 @@ __global__ void __launch_bounds__(256) ex_block_kernel(int F, int D, const doubl
   }
 }
 
-// ---- D <= 72 (one tile, the sliding-window case): split-K over the 8 warps ------------------------------------
-// Each warp owns every 8x8 sub-tile of the upper triangle (45 x 2 accumulator registers per lane) for its share
-// of the landmarks: one row fragment per 8-column block is loaded once per 4 landmarks and feeds both operand
-// roles (A = W^T/L, B = W) of up to 9 MMAs each, there is no block barrier in the main loop, and the next
-// 4 rows are prefetched into registers while the current ones are multiplied.  The 8 partial triangles are summed
-// through shared memory at the end.
-constexpr int kSplitStageLd = 76;
-constexpr int kSplitAcc = 45 * 64 + 72;   // doubles per warp slab: 45 upper-triangle 8x8 sub-tiles + g
-__global__ void __launch_bounds__(SWARPS * 32) schur_splitk_kernel(int W, int F, int D, const double* __restrict__ H_pp,
-                                                                   const double* __restrict__ H_lp,
-                                                                   const double* __restrict__ H_ll,
-                                                                   const double* __restrict__ b_p,
-                                                                   const double* __restrict__ b_l, double* __restrict__ S,
-                                                                   double* __restrict__ g, double eps) {
-  __shared__ double stage[SWARPS][4 * kSplitStageLd + 8];   // 4 landmark rows (padded stride) + inv[4] + b[4]
-  extern __shared__ double sAcc[];                           // [SWARPS][kSplitAcc]: every warp's 45 sub-tiles + g
-  // persistent: one CTA per SM walks the windows; the first landmark rows of the NEXT window are fetched before the
-  // epilogue of the current one, so neither the CTA launch nor the first HBM round trip is exposed per window
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int kq = lane & 3, mq = lane >> 2;
-  double* st = stage[warp];
-  const int nsteps = (F + 3) / 4;
-  // register prefetch of one step: 4 rows x 72 columns = 288 doubles = 9 per lane, plus L and b for lanes 0..3
-  double pre[9], preL = 0.0, preB = 0.0;
-  const double* __restrict__ Hl = nullptr;
-  const double* __restrict__ Ll = nullptr;
-  const double* __restrict__ Bl = nullptr;
-  auto window = [&](int w) {
-    Hl = H_lp + (size_t)w * F * D, Ll = H_ll + (size_t)w * F, Bl = b_l + (size_t)w * F;
-  };
-  auto fetch = [&](int step) {
-    const int l0 = 4 * step;
-#pragma unroll
-    for (int q = 0; q < 9; ++q) {
-      const int e = q * 32 + lane, r = e / 72, c = e % 72;
-      pre[q] = (l0 + r < F && c < D) ? Hl[(size_t)(l0 + r) * D + c] : 0.0;
-    }
-    if (lane < 4) {
-      preL = l0 + lane < F ? Ll[l0 + lane] : 0.0;
-      preB = l0 + lane < F ? Bl[l0 + lane] : 0.0;
-    }
-  };
-  if ((int)blockIdx.x < W) {
-    window(blockIdx.x);
-    if (warp < nsteps) fetch(warp);
-  }
-  for (int w = blockIdx.x; w < W; w += gridDim.x) {
-  double acc[45][2];
-#pragma unroll
-  for (int i = 0; i < 45; ++i) acc[i][0] = acc[i][1] = 0.0;
-  double gacc[3] = {0.0, 0.0, 0.0};
-  for (int step = warp; step < nsteps; step += SWARPS) {
-#pragma unroll
-    for (int q = 0; q < 9; ++q) {
-      const int e = q * 32 + lane, r = e / 72, c = e % 72;
-      st[r * kSplitStageLd + c] = pre[q];
-    }
-    if (lane < 4) {
-      st[4 * kSplitStageLd + lane] = (preL > eps) ? 1.0 / preL : 0.0;
-      st[4 * kSplitStageLd + 4 + lane] = preB;
-    }
-    __syncwarp();
-    if (step + SWARPS < nsteps) fetch(step + SWARPS);
-    const double inv = st[4 * kSplitStageLd + kq];
-    double fb[9], fa[9];
-#pragma unroll
-    for (int t = 0; t < 9; ++t) {
-      fb[t] = st[kq * kSplitStageLd + 8 * t + mq];
-      fa[t] = fb[t] * inv;
-    }
-    int idx = 0;
-#pragma unroll
-    for (int tr = 0; tr < 9; ++tr)
-#pragma unroll
-      for (int tc = tr; tc < 9; ++tc, ++idx) dmma(acc[idx][0], acc[idx][1], fa[tr], fb[tc]);
-    // g: lanes own rows lane, lane+32, lane+64
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const double s = st[4 * kSplitStageLd + k] * st[4 * kSplitStageLd + 4 + k];
-#pragma unroll
-      for (int q = 0; q < 3; ++q)
-        if (lane + 32 * q < 72) gacc[q] = fma(st[k * kSplitStageLd + lane + 32 * q], s, gacc[q]);
-    }
-    __syncwarp();
-  }
-  if (w + (int)gridDim.x < W) {   // first step of the next window, in flight during the epilogue
-    window(w + gridDim.x);
-    if (warp < nsteps) fetch(warp);
-  }
-  // cross-warp reduction (once per window): every warp parks its partial sums in its own slab (no turn-taking),
-  // the S / g writers add the SWARPS slabs
-  {
-    double* mine = sAcc + warp * kSplitAcc;
-#pragma unroll
-    for (int i = 0; i < 45; ++i)
-      *reinterpret_cast<double2*>(mine + i * 64 + mq * 8 + 2 * kq) = make_double2(acc[i][0], acc[i][1]);
-#pragma unroll
-    for (int q = 0; q < 3; ++q)
-      if (lane + 32 * q < 72) mine[45 * 64 + lane + 32 * q] = gacc[q];
-  }
-  // H_pp of this window is fetched while the slabs settle (the accumulator registers are free now): the S loop
-  // below then has no global-load latency on its critical path
-  const double* __restrict__ Hp = H_pp + (size_t)w * D * D;
-  double* __restrict__ So = S + (size_t)w * D * D;
-  constexpr int kHp = (72 * 72 + SWARPS * 32 - 1) / (SWARPS * 32);
-  double hp[kHp];
-#pragma unroll
-  for (int i = 0; i < kHp; ++i) {
-    const int e = tid + i * SWARPS * 32;
-    hp[i] = e < D * D ? Hp[e] : 0.0;
-  }
-  __syncthreads();
-  // slabs 1.. are folded into slab 0 in slab order (consecutive threads, consecutive words: conflict-free); the
-  // symmetric read-out below, whose lower-triangle half is strided, then touches one slab instead of SWARPS
-  for (int off = tid; off < kSplitAcc; off += SWARPS * 32) {
-    double v = sAcc[off];
-#pragma unroll
-    for (int k = 1; k < SWARPS; ++k) v += sAcc[k * kSplitAcc + off];
-    sAcc[off] = v;
-  }
-  __syncthreads();
-#pragma unroll
-  for (int i = 0; i < kHp; ++i) {
-    const int e = tid + i * SWARPS * 32;
-    if (e >= D * D) break;
-    const int r = e / D, c = e % D;
-    const int rr = r <= c ? r : c, cc = r <= c ? c : r;     // value lives in the upper triangle
-    const int tr = rr >> 3, tc = cc >> 3;
-    // sub-tile index in the (tr <= tc) enumeration: sum_{k<tr} (9-k) + (tc - tr)
-    const int idx = tr * 9 - (tr * (tr - 1)) / 2 + (tc - tr);
-    // a diagonal sub-tile holds the full 8x8 (both triangles were computed)
-    const int off = tr == tc ? idx * 64 + (r & 7) * 8 + (c & 7) : idx * 64 + (rr & 7) * 8 + (cc & 7);
-    So[e] = hp[i] - sAcc[off];
-  }
-  for (int e = tid; e < D; e += SWARPS * 32) {
-    g[(size_t)w * D + e] = b_p[(size_t)w * D + e] - sAcc[45 * 64 + e];
-  }
-  __syncthreads();   // the slabs and the stages are reused by the next window
-  }
-}
-
 // ---- DMMA peak (for the roofline denominator of this kernel) ----
 __global__ void __launch_bounds__(256) dmma_peak_kernel(double* out, double a, double b, int iters) {
   double c[8][2];
@@ -410,11 +269,11 @@ __global__ void __launch_bounds__(256) dmma_peak_kernel(double* out, double a, d
 // through a ring of shared-memory stages with cp.async.bulk (TMA bulk copy, one 8*D-byte row per copy into a stride of 76
 // doubles: conflict-free fragment loads) completing on mbarriers; 1/L and b come from a small pre-pass (schur_inv_kernel,
 // rows padded to whole stages).  The consumers OWN output sub-tiles, so the contraction over the landmarks needs no cross-warp
-// reduction (the split-K kernel above spent half of a 150-landmark window in that epilogue) and no CTA-wide barrier: S is a
-// symmetric 9 x 9 grid of 8x8 tiles, and on the torus every unordered pair of tile indices is (w, (w + d) mod 9) for exactly one
-// w in 0..8 and d in 0..4 — warp w computes those five tiles (one A fragment, five B fragments, five DMMA per step of four
-// landmarks; every warp runs the same code) and writes each with its mirror.  g[8w..8w+7] rides along on the A fragment: one FMA
-// per step and lane, summed over the four k-lanes at the end of the window.
+// reduction and no CTA-wide barrier: S is a symmetric 9 x 9 grid of 8x8 tiles, and on the torus every unordered pair of tile
+// indices is (w, (w + d) mod 9) for exactly one w in 0..8 and d in 0..4 — warp w computes those five tiles (one A fragment, five
+// B fragments, five DMMA per step of four landmarks; every warp runs the same code) and writes each with its mirror.  g[8w..8w+7]
+// rides along on the A fragment: one FMA per step and lane, summed over the four k-lanes at the end of the window.  Without
+// landmarks (F = 0) there are no chunks: the producer issues nothing and the consumers write S = H_pp, g = b_p.
 constexpr int kTmaStageL = 32;                         // landmarks per stage
 constexpr int kTmaStageD = kTmaStageL * LDW + 2 * kTmaStageL;   // doubles per stage: rows + 1/L + b
 constexpr int kTmaStages = 4;
@@ -582,12 +441,12 @@ __global__ void __launch_bounds__(kTmaThreads, 2) schur_tma_kernel(int W, int F,
 int viml_launch_schur(viml_ctx* ctx, int W, int F, int D, const double* H_pp, const double* H_lp, const double* H_ll,
                       const double* b_p, const double* b_l, double* S, double* g, double eps) {
   const int ntile = (D + TS - 1) / TS;
-  if (ntile == 1 && F > 0 && !ctx->schur_splitk) {   // sliding-window case: TMA-pipelined kernel, warps own output tiles
+  if (ntile == 1) {   // sliding-window case: TMA-pipelined kernel, warps own output tiles
     const int Fp = (F + kTmaStageL - 1) / kTmaStageL * kTmaStageL;
     VIML_TRY_CUDA(ctx, ctx->scratch2.reserve(2 * DeviceArena::padded((size_t)W * Fp * 8)));
     double* invp = ctx->scratch2.take<double>((size_t)W * Fp);
     double* blp = ctx->scratch2.take<double>((size_t)W * Fp);
-    {
+    if (Fp > 0) {   // F == 0: nothing to pad, and a grid of 0 blocks is a launch error
       LaunchScope ls(ctx, K_SCHUR);
       schur_inv_kernel<<<(unsigned)(((size_t)W * Fp + 255) / 256), 256, 0, ctx->stream>>>(W, F, Fp, H_ll, b_l, eps, invp, blp);
     }
@@ -596,14 +455,6 @@ int viml_launch_schur(viml_ctx* ctx, int W, int F, int D, const double* H_pp, co
     const int grid = W < 2 * ctx->sm_count ? W : 2 * ctx->sm_count;
     LaunchScope ls(ctx, K_SCHUR);
     schur_tma_kernel<<<(unsigned)grid, kTmaThreads, smem, ctx->stream>>>(W, F, Fp, D, H_pp, H_lp, invp, blp, b_p, S, g);
-    return VIML_OK;
-  }
-  if (ntile == 1) {   // split-K variant (VIML_SCHUR_SPLITK=1, or no landmarks): one persistent CTA per SM
-    LaunchScope ls(ctx, K_SCHUR);
-    const int smem = SWARPS * kSplitAcc * (int)sizeof(double);
-    if (cudaFuncSetAttribute(schur_splitk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return VIML_ERR_CUDA;
-    const int grid = W < ctx->sm_count ? W : ctx->sm_count;
-    schur_splitk_kernel<<<(unsigned)grid, SWARPS * 32, smem, ctx->stream>>>(W, F, D, H_pp, H_lp, H_ll, b_p, b_l, S, g, eps);
     return VIML_OK;
   }
   dim3 grid((unsigned)(ntile * (ntile + 1) / 2), (unsigned)W);

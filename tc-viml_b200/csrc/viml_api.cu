@@ -73,7 +73,6 @@ int viml_create(viml_ctx** out, const viml_config* cfg, int device) {
   ctx->nan_angle_passes = !(3.1415926 > cfg->angle_th);
   if (const char* e = getenv("VIML_FORCE_GENERIC")) ctx->force_generic = e[0] == '1';  // test hook
   if (const char* e = getenv("VIML_BRUTE_CULL")) ctx->brute_cull = e[0] == '1';
-  if (const char* e = getenv("VIML_SCHUR_SPLITK")) ctx->schur_splitk = e[0] == '1';
   if (cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaStreamCreateWithFlags(&ctx->copy_stream2, cudaStreamNonBlocking) != cudaSuccess ||

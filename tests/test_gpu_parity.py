@@ -135,6 +135,17 @@ def test_fused_path_extremes(pkg, orc, ctx, cfg):
                            b.lf_window_offset, b.lf_frame, b.lf_geom)
     got, _ = check_linearize(pkg, orc, ctx, cfg, only_lines, abi.OUT_HB | abi.LOSS_CAUCHY)
     assert np.all(got["H_lp"] == 0.0) and np.all(got["H_ll"] == 0.0)
+    # no landmarks at all (F = 0): nothing to eliminate, S and g are H_pp and b_p bit for bit (full and packed S)
+    no_feats = abi.Batch(b.poses, b.ex_pose, np.zeros((b.W, 0)), np.zeros(5, dtype=np.int32), b.pf_idx[:0], b.pf_obs[:0],
+                         b.lf_window_offset, b.lf_frame, b.lf_geom)
+    got, _ = check_linearize(pkg, orc, ctx, cfg, no_feats, abi.OUT_HB | abi.OUT_SCHUR | abi.LOSS_CAUCHY)
+    assert np.array_equal(got["S"], got["H_pp"]) and np.array_equal(got["g"], got["b_p"])
+    bufs = no_feats.alloc_out(abi.OUT_HB | abi.OUT_SCHUR)
+    del bufs["S"]
+    bufs["S_packed"] = np.full(no_feats.out_shapes()["S_packed"], np.nan)
+    ctx.linearize(no_feats, abi.OUT_HB | abi.OUT_SCHUR | abi.S_PACKED | abi.LOSS_CAUCHY, out=bufs)
+    iu = np.triu_indices(no_feats.D)
+    assert np.array_equal(bufs["S_packed"], bufs["H_pp"][:, iu[0], iu[1]]) and np.array_equal(bufs["g"], bufs["b_p"])
     # one pose pair carries every factor (all features start in frame 0 and are seen once more, in frame 1)
     b = synth.make_windows(3, seed=125, P=11, F=150, all_start_zero=True, max_len=2)
     check_linearize(pkg, orc, ctx, cfg, b, hb)
@@ -225,6 +236,27 @@ def test_bad_arguments(pkg, ctx, cfg):
     assert lib.viml_linearize_batch(ctx.h, None, C.byref(o), abi.OUT_HB) == abi.VIML_ERR_INVALID
     s.poses_per_window = 0
     assert lib.viml_linearize_batch(ctx.h, C.byref(s), C.byref(o), abi.OUT_RESIDUAL_JACOBIAN) == abi.VIML_ERR_INVALID
+    # dense factors through host pointers: the CSR the kernels index through is checked before anything is launched
+    b3 = pkg.synth.make_windows(3, seed=110)
+    dense = pkg.synth.make_dense_factors(b3)
+    Dx = b3.D + dense.X
+    bs = b3.struct()
+    S, g = np.zeros((b3.W, b3.D, b3.D)), np.zeros((b3.W, b3.D))
+    Sx, gx = np.zeros((b3.W, Dx, Dx)), np.zeros((b3.W, Dx))
+    ro = abi.ReducedOut()
+    ro.Sx, ro.gx = abi.ptr(Sx), abi.ptr(gx)
+    wo = dense.window_offset
+    for field, i, val in (("jac_offset", 1, dense.jac_offset[1] + 1),   # a step != rows x columns
+                          ("window_offset", -1, wo[-1] - 1),            # last entry != n_factors
+                          ("window_offset", 1, wo[2] + 1),              # decreases in the middle
+                          ("col_index", 0, Dx)):                        # column outside [0, Dx)
+        arrs = {k: v.copy() for k, v in dense.arrays().items()}
+        arrs[field][i] = val
+        d = dense.struct(arrs)
+        assert lib.viml_reduced_system(ctx.h, C.byref(bs), C.byref(d), C.byref(ro), 0) == abi.VIML_ERR_INVALID
+        assert field.encode() in lib.viml_last_error(ctx.h)
+        assert lib.viml_reduced_from_schur(ctx.h, b3.W, b3.D, abi.ptr(S), abi.ptr(g), C.byref(d), C.byref(ro), 0) == abi.VIML_ERR_INVALID
+        assert field.encode() in lib.viml_last_error(ctx.h)
 
 
 def test_observation_table_input(pkg, orc, ctx, cfg):
@@ -464,14 +496,14 @@ def block_err(got, ref, bounds):
     return worst
 
 
-def test_reduced_system_and_gn_step(pkg, orc, ctx, cfg):
+def check_reduced_system_and_gn_step(pkg, orc, ctx, cfg, b, flags):
+    """viml_reduced_system and viml_gn_step (lambda = 0 and 1e-3) on batch b with make_dense's factors against the oracle;
+    returns (dense, extra)."""
     from oracle import gn_oracle
-    abi, synth = pkg._abi, pkg.synth
-    b = synth.make_windows(12, seed=141)
+    abi = pkg._abi
     dense = make_dense(pkg, b)
     P, D, X = b.P, b.D, dense.X
     bounds = [6 * k for k in range(P + 2)] + [D + 9 * k for k in range(1, P + 1)]
-    flags = abi.LOSS_CAUCHY
     Sx, gx = ctx.reduced_system(b, dense, flags)
     rSx, rgx, _ = gn_oracle.reduced_system(cfg, b, dense, flags)
     assert block_err(Sx, rSx, bounds) < TOL and block_err(gx, rgx, bounds) < TOL
@@ -497,6 +529,18 @@ def test_reduced_system_and_gn_step(pkg, orc, ctx, cfg):
         # identical accept / reject decisions, and the step does decrease the cost on these windows
         assert np.array_equal(got["cost"][:, 1] < got["cost"][:, 0], ref["cost"][:, 1] < ref["cost"][:, 0])
         assert (got["cost"][:, 2] > 0).all()
+    return dense, extra
+
+
+def test_reduced_system_and_gn_step(pkg, orc, ctx, cfg):
+    from oracle import gn_oracle
+    abi, synth = pkg._abi, pkg.synth
+    flags = abi.LOSS_CAUCHY
+    b = synth.make_windows(12, seed=141)
+    dense, extra = check_reduced_system_and_gn_step(pkg, orc, ctx, cfg, b, flags)
+    # P = 13: Dx = 201 is too large for the step's single kernel (reduced_kernel, then the tiled solve), and H / b come from the
+    # generic atomic kernels (P > 12)
+    check_reduced_system_and_gn_step(pkg, orc, ctx, cfg, synth.make_windows(12, seed=141, P=13), flags)
     # a few iterations from a perturbed state converge (cost decreases monotonically when every step is accepted)
     cur = b
     costs = []
