@@ -228,7 +228,11 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
  *
  * viml_reduced_system:  Sx = embed(S) + sum_k J_k^T J_k,  gx = embed(g) + sum_k J_k^T r_k   ([W][Dx][Dx], [W][Dx], Dx = D + X),
  * with S, g the landmark-eliminated system of the window's ProjectionFactors / LineProjectionFactors (viml_linearize_batch,
- * VIML_OUT_SCHUR; VIML_LOSS_CAUCHY in `flags` applies to those).  dense == NULL gives the embedding alone.               */
+ * VIML_OUT_SCHUR; VIML_LOSS_CAUCHY in `flags` applies to those).  dense == NULL gives the embedding alone.
+ * The host-pointer flavour validates the arrays (VIML_ERR_INVALID: offsets that start at 0, window_offset a non-decreasing CSR of
+ * the factors, jac_offset steps of n_k * c_k, col_index in [0, D+X) and without a column repeated inside a factor).  The device
+ * flavour reads back only the three totals: the rest, col_index distinct inside a factor included, is the caller's to keep.  A
+ * repeated column there gives a step that depends on which kernel solves it.                                              */
 typedef struct viml_dense_factors {
   int32_t extra_dim;             /* X                                              */
   int32_t reserved0;

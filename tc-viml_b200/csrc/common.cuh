@@ -221,7 +221,8 @@ int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const doub
                          double* cost);
 int viml_launch_gn_update(viml_ctx* ctx, const LinearizeArgs& a, int X, const double* extra_in, const double* dx, const int32_t* solved,
                           double* o_poses, double* o_ex, double* o_dep, double* o_extra);
-int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, int slot, double* cost);
+int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, const int32_t* solved, int slot,
+                     double* cost);
 // schur_kernels.cu
 int viml_launch_schur(viml_ctx* ctx, int W, int F, int D, const double* H_pp, const double* H_lp, const double* H_ll,
                       const double* b_p, const double* b_l, double* S, double* g, double eps);

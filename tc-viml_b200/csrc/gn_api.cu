@@ -197,14 +197,26 @@ int stage_dense(viml_ctx* ctx, Stager& st, const viml_dense_factors* dense, int 
     if (off[0] != 0 || off[W] != ND) return fail(ctx, VIML_ERR_INVALID, "dense factors: window_offset is not a CSR of the factor list");
     for (int w = 0; w < W; ++w)
       if (off[w + 1] < off[w]) return fail(ctx, VIML_ERR_INVALID, "dense factors: window_offset decreases");
+    if (dense->row_offset[0] != 0 || dense->col_offset[0] != 0 || dense->jac_offset[0] != 0)
+      return fail(ctx, VIML_ERR_INVALID, "dense factors: row_offset, col_offset and jac_offset must start at 0");
     n_rows = dense->row_offset[ND], n_cols = dense->col_offset[ND], n_jac = dense->jac_offset[ND];
     for (int64_t k = 0; k < n_cols; ++k)
       if (dense->col_index[k] < 0 || dense->col_index[k] >= Dx) return fail(ctx, VIML_ERR_INVALID, "dense factors: col_index out of range");
     for (int64_t k = 0; k < ND; ++k) {
       const int64_t n = dense->row_offset[k + 1] - dense->row_offset[k], c = dense->col_offset[k + 1] - dense->col_offset[k];
-      if (n < 0 || c < 0 || dense->jac_offset[k + 1] - dense->jac_offset[k] != n * c)
+      if (n < 0 || c < 0 || dense->row_offset[k + 1] > n_rows || dense->col_offset[k + 1] > n_cols)
+        return fail(ctx, VIML_ERR_INVALID, "dense factors: row_offset and col_offset must be non-decreasing up to their totals");
+      if (dense->jac_offset[k + 1] - dense->jac_offset[k] != n * c)
         return fail(ctx, VIML_ERR_INVALID, "dense factors: jac_offset does not match rows x columns");
     }
+    // only now that every factor's columns lie inside [0, n_cols): the fused kernel keeps the lower triangle only and adds a
+    // diagonal tile's a >= b half, so a column repeated inside a factor would count once there and twice in reduced_kernel
+    std::vector<int64_t> seen(Dx, -1);
+    for (int64_t k = 0; k < ND; ++k)
+      for (int64_t a = dense->col_offset[k]; a < dense->col_offset[k + 1]; ++a) {
+        if (seen[dense->col_index[a]] == k) return fail(ctx, VIML_ERR_INVALID, "dense factors: col_index repeats a column inside a factor");
+        seen[dense->col_index[a]] = k;
+      }
   }
   st.in(dense->window_offset, (size_t)W + 1, &dn->window_offset);
   st.in(dense->row_offset, (size_t)ND + 1, &dn->row_offset);
@@ -348,7 +360,7 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   // a step that does not have to hand Sx / gx to the caller builds and solves the reduced system in one kernel
   bool fused = false;
   if (step && !(rout && (rout->Sx || rout->gx))) {
-    rc = viml_launch_cost(ctx, a, dn, nullptr, 0, cost);
+    rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, cost);
     if (rc != VIML_OK) return rc;
     rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, opt ? opt->lambda : 0.0, dxv, solved, cost);
     if (rc == VIML_OK) fused = true;
@@ -361,7 +373,7 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   if (step) {
     rc = VIML_OK;
     if (!fused) {
-      rc = viml_launch_cost(ctx, a, dn, nullptr, 0, cost);
+      rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, cost);
       if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, opt ? opt->lambda : 0.0, Sx, gx, dxv, solved, cost);
     }
     if (rc == VIML_OK) rc = viml_launch_gn_update(ctx, a, X, d_extra, dxv, solved, o_poses, o_ex, o_dep, o_extra);
@@ -378,9 +390,9 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
       rc = viml_launch_inertial(ctx, vp, viml_inertial_out{}, cp, false);
       DenseArgs dp = dn;
       dp.residual = res_plus;
-      if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, 1, cost);
+      if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, nullptr, 1, cost);
     } else {
-      rc = viml_launch_cost(ctx, a2, dn, dxv, 1, cost);
+      rc = viml_launch_cost(ctx, a2, dn, dxv, solved, 1, cost);
     }
     if (rc != VIML_OK) return rc;
   }

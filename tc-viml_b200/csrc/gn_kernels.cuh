@@ -352,12 +352,13 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
       __syncthreads();
     }
   }
-  // model decrease with the undamped Sx: -g.x - x.Sx x / 2
+  // model decrease with the undamped Sx: -g.x - x.Sx x / 2 (exactly 0 for a window that was not solved, even when its system
+  // holds a NaN or an infinity)
   double part = 0.0;
   if (FUSED) {   // (Sx + lambda diag d) x = -g  =>  x.Sx x = -g.x - lambda sum d_i x_i^2
     for (int i = tid; i < Dx; i += 256) {
       const double xi = ok ? y[i] : 0.0;
-      part += -0.5 * gv[i] * xi + 0.5 * lambda * dv[i] * xi * xi;
+      if (ok) part += -0.5 * gv[i] * xi + 0.5 * lambda * dv[i] * xi * xi;
       dx[(size_t)w * Dx + i] = xi;
     }
   } else {       // a warp per row of Sx (coalesced), lanes over the columns
@@ -369,7 +370,7 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
       for (int o = 16; o > 0; o >>= 1) sx += __shfl_xor_sync(0xffffffffu, sx, o);
       const double xi = ok ? y[i] : 0.0;
       if (lane == 0) {
-        part += -gx[(size_t)w * Dx + i] * xi - 0.5 * xi * sx;
+        if (ok) part += -gx[(size_t)w * Dx + i] * xi - 0.5 * xi * sx;
         dx[(size_t)w * Dx + i] = xi;
       }
     }
@@ -425,17 +426,23 @@ __global__ void __launch_bounds__(128) update_kernel(LinearizeArgs A, int X, con
       for (int c = 0; c < D; ++c) s = fma(row[c], d[c], s);
       dl = -s / hll;
     }
-    o_dep[(size_t)w * F + l] = lam + dl;
+    o_dep[(size_t)w * F + l] = ok ? lam + dl : lam;   // not lam + 0.0, which turns -0.0 into +0.0
   }
   if (o_extra)
-    for (int e = tid; e < X; e += blockDim.x) o_extra[(size_t)w * X + e] = (extra_in ? extra_in[(size_t)w * X + e] : 0.0) + (ok ? d[D + e] : 0.0);
+    for (int e = tid; e < X; e += blockDim.x) {
+      const double x = extra_in ? extra_in[(size_t)w * X + e] : 0.0;
+      o_extra[(size_t)w * X + e] = ok ? x + d[D + e] : x;
+    }
 }
 
 // cost[3w + slot] = 1/2 sum rho(|r|^2) over the window's point and line factors at the state of A (pose cache ready)
-// + 1/2 sum |r_k + J_k dx|^2 over its dense-block factors (dx == nullptr: at the linearisation point).
-__global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn, const double* __restrict__ dx, int slot, double* __restrict__ cost) {
+// + 1/2 sum |r_k + J_k dx|^2 over its dense-block factors (dx == nullptr, or a window the step did not solve: at the
+// linearisation point, so that cost[1] == cost[0] even when a Jacobian holds a NaN).
+__global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn, const double* __restrict__ dx,
+                                                   const int32_t* __restrict__ solved, int slot, double* __restrict__ cost) {
   __shared__ double s_red[4];
   const int w = blockIdx.x, tid = threadIdx.x, Dx = A.D + dn.X;
+  const bool moved = dx != nullptr && solved[w] != 0;
   const bool cauchy = (A.flags & VIML_LOSS_CAUCHY) != 0;
   LinearizeArgs R = A;
   R.flags &= ~VIML_LOSS_CAUCHY;   // raw residuals: rho is applied here, not the Jacobian correction
@@ -472,7 +479,7 @@ __global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn
       const int32_t* __restrict__ ci = dn.col_index + dn.col_offset[k];
       for (int q = tid; q < n; q += blockDim.x) {
         double v = r[q];
-        if (dx)
+        if (moved)
           for (int a = 0; a < c; ++a) v = fma(J[(size_t)q * c + a], dx[(size_t)w * Dx + ci[a]], v);
         acc += v * v;
       }

@@ -709,9 +709,10 @@ int viml_launch_gn_update(viml_ctx* ctx, const LinearizeArgs& a, int X, const do
   return VIML_OK;
 }
 
-int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, int slot, double* cost) {
+int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, const int32_t* solved, int slot,
+                     double* cost) {
   LaunchScope ls(ctx, K_GN);
-  gn::cost_kernel<<<a.W, 128, 0, ctx->stream>>>(a, dn, dx, slot, cost);
+  gn::cost_kernel<<<a.W, 128, 0, ctx->stream>>>(a, dn, dx, solved, slot, cost);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }

@@ -249,7 +249,10 @@ def test_bad_arguments(pkg, ctx, cfg):
     for field, i, val in (("jac_offset", 1, dense.jac_offset[1] + 1),   # a step != rows x columns
                           ("window_offset", -1, wo[-1] - 1),            # last entry != n_factors
                           ("window_offset", 1, wo[2] + 1),              # decreases in the middle
-                          ("col_index", 0, Dx)):                        # column outside [0, Dx)
+                          ("col_index", 0, Dx),                         # column outside [0, Dx)
+                          ("col_index", 1, dense.col_index[0]),         # a column repeated inside factor 0
+                          ("col_offset", 0, 1),                         # offsets that do not start at 0
+                          ("col_offset", 1, dense.col_offset[-1] + 7)):  # past the total, then back down
         arrs = {k: v.copy() for k, v in dense.arrays().items()}
         arrs[field][i] = val
         d = dense.struct(arrs)
