@@ -28,6 +28,8 @@
  *                             (pre-integration itself stays with the host)
  *   viml_gn_step_vi        <- viml_gn_step over the window's whole problem: the IMU and prior factors evaluated on the device at
  *                             x (system) and at x+ (cost[1] = f(x+))
+ *   viml_solve_vi          <- ceres::Solve of the window's whole problem  estimator.cpp:1888-1905 (TrustRegionMinimizer with
+ *                             LevenbergMarquardtStrategy; every step is viml_gn_step_vi's; deviations at the declaration)
  *   viml_fov_update / viml_fov_slide / VIML_FOV_CACHED
  *                          <- the per-slot FoV lists the estimator keeps between frames: UpdateLinesInFoV at frame entry
  *                             (estimator.cpp:342) and their shifts in slideWindowWithLinesFoV (estimator.cpp:2148, :2160, :2218)
@@ -358,6 +360,68 @@ int viml_inertial_evaluate(viml_ctx* ctx, const viml_window_batch* state, const 
  * windows returned unchanged); extra_state is required when X > 0.  With VIML_PTRS_DEVICE the call does not synchronise.     */
 int viml_gn_step_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
                     const viml_gn_options* opt, const viml_gn_out* out, uint32_t flags);
+
+/* ---- a whole Levenberg-Marquardt solve per window, on the device --------------------------------------------------------
+ * Replaces the ceres::Solve call of Estimator::OptimizationWithLine (estimator.cpp:1888-1905) for the window's whole problem: the
+ * trust-region loop of Ceres' TrustRegionMinimizer with its default LevenbergMarquardtStrategy, restated from Ceres' documented
+ * behaviour (not pinned against its source).  Every window keeps its own radius and stops on its own.  Per window:
+ *   f(x0) is computed first; if it is not finite the window stops with VIML_SOLVE_FAILURE after 0 iterations, state unchanged.
+ *   state: x, radius = initial_radius, decrease_factor = 2, counters.  Each iteration of a running window:
+ *   1. lambda = 1 / radius; the step viml_gn_step_vi takes at x with that lambda gives f(x), f(x+), the model decrease m, solved.
+ *   2. invalid (solved == 0, f(x+) not finite, or !(m > 0)): consecutive_invalid += 1, radius /= decrease_factor,
+ *      decrease_factor *= 2; FAILURE when consecutive_invalid > max_consecutive_invalid.
+ *   3. otherwise consecutive_invalid = 0, then in order:
+ *      |dx| <= parameter_tolerance (|x| + parameter_tolerance)  -> PARAMETER_TOL at x (dx: the reduced step and the landmark
+ *         increments x+ - x; |x| over every state value: 7 per pose, 7 for the extrinsic, the inverse depths, the extra state);
+ *      |f(x) - f(x+)| <= function_tolerance f(x)                 -> FUNCTION_TOL at x;
+ *      rho = (f(x) - f(x+)) / m;  rho > min_relative_decrease: accept (x = x+), t = 2 rho - 1,
+ *         radius = min(max_radius, radius / max(1/3, 1 - t^3)), decrease_factor = 2;
+ *      else reject: radius /= decrease_factor, decrease_factor *= 2.
+ *   4. iterations += 1; a window still running stops with MIN_RADIUS when radius < min_radius, else with NO_CONVERGENCE when
+ *      iterations == max_iterations.
+ * A stopped window's state, counters and outputs never change again.  The policy arithmetic is plain IEEE binary64 without fused
+ * multiply-adds, so a scalar restatement reproduces it bit for bit.
+ * Deviations from Ceres' Solve as the reference configures it:
+ *   - the strategy is LEVENBERG_MARQUARDT; the reference asks for DOGLEG, which needs the full-space gradient and the Cauchy point;
+ *   - the damping is viml_gn_step's lambda diag(Sx) on the landmark-reduced system (Ceres damps J^T J before the elimination and
+ *     clamps the diagonal to [1e-6, 1e32]);
+ *   - no gradient tolerance (the full-problem gradient is not formed) and no max_solver_time.
+ * Input validation is viml_gn_step_vi's, plus the options below and the required outputs.  W == 0 returns VIML_OK.  With
+ * VIML_PTRS_DEVICE the call neither synchronises nor reads anything back: all max_iterations rounds are enqueued on the context
+ * stream, and rounds after every window has stopped do only the ungated work (linearisation, Schur step, IMU / prior evaluation).  */
+typedef struct viml_solve_options {
+  int32_t max_iterations;           /* > 0; every computed step counts, accepted or not   (ceres: max_num_iterations, 50)         */
+  int32_t max_consecutive_invalid;  /* >= 0                                                (max_num_consecutive_invalid_steps, 5)  */
+  double initial_radius;            /* 0 < min_radius <= initial_radius <= max_radius, all finite  (initial_trust_region_radius, 1e4) */
+  double max_radius;                /*                                                     (max_trust_region_radius, 1e16)          */
+  double min_radius;                /*                                                     (min_trust_region_radius, 1e-32)         */
+  double min_relative_decrease;     /* >= 0                                                (min_relative_decrease, 1e-3)            */
+  double function_tolerance;        /* >= 0                                                (function_tolerance, 1e-6)               */
+  double parameter_tolerance;       /* >= 0                                                (parameter_tolerance, 1e-8)              */
+} viml_solve_options;
+
+#define VIML_SOLVE_NO_CONVERGENCE 0   /* max_iterations reached */
+#define VIML_SOLVE_FUNCTION_TOL 1
+#define VIML_SOLVE_PARAMETER_TOL 2
+#define VIML_SOLVE_MIN_RADIUS 3
+#define VIML_SOLVE_FAILURE 4          /* f(x0) not finite, or more than max_consecutive_invalid invalid steps in a row */
+
+typedef struct viml_solve_out {
+  double* poses;        /* [W][P][7]  the final state */
+  double* ex_pose;      /* [W][7]                     */
+  double* inv_depth;    /* [W][F]     (required when F > 0) */
+  double* extra;        /* [W][X]     (required when X > 0) */
+  int32_t* status;      /* [W] VIML_SOLVE_*          */
+  int32_t* iterations;  /* [W] steps computed        */
+  int32_t* accepted;    /* [W] steps accepted        */
+  double* cost;         /* [W][2] f(x0), f(final state) */
+  double* radius;       /* [W] final radius, or NULL */
+  double* trace;        /* [W][max_iterations][4] or NULL: f(x), f(x+), model decrease, lambda of every step; NaN rows after
+                           the window stopped */
+} viml_solve_out;
+
+int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
+                  const viml_solve_options* opt, const viml_solve_out* out, uint32_t flags);
 
 /* ---- dense marginalisation (marginalization_factor.cpp:264-293) --------------------------------
  * Per problem k: A [pos][pos] row-major, b [pos], marginalised block = leading m rows, kept n = pos-m.

@@ -27,7 +27,7 @@ ABI_SYMBOLS = (
     "viml_marginalize_batch", "viml_line_associate", "viml_assoc_stats", "viml_allreduce_hb",
     "viml_load_line_map", "viml_reduced_system", "viml_reduced_from_schur", "viml_gn_step",
     "viml_fov_update", "viml_fov_slide", "viml_track_gate", "viml_triangulate_batch",
-    "viml_inertial_evaluate", "viml_gn_step_vi",
+    "viml_inertial_evaluate", "viml_gn_step_vi", "viml_solve_vi",
 )
 
 
@@ -90,6 +90,8 @@ def load_library():
                                            C.POINTER(_abi.InertialOut), C.c_uint32]
     lib.viml_gn_step_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.InertialFactors), C.c_void_p,
                                     C.POINTER(_abi.GnOptions), C.POINTER(_abi.GnOut), C.c_uint32]
+    lib.viml_solve_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.InertialFactors), C.c_void_p,
+                                  C.POINTER(_abi.SolveOptions), C.POINTER(_abi.SolveOut), C.c_uint32]
     _LIB = lib
     return lib
 
@@ -294,6 +296,41 @@ class Context:
         o.extra = _abi.ptr(res["extra"]) if X > 0 else None
         self._check(self.lib.viml_gn_step_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), C.byref(opt), C.byref(o),
                                              flags & ~PTRS_DEVICE))
+        return res
+
+    @staticmethod
+    def solve_options(max_iterations=50, max_consecutive_invalid=5, initial_radius=1e4, max_radius=1e16, min_radius=1e-32,
+                      min_relative_decrease=1e-3, function_tolerance=1e-6, parameter_tolerance=1e-8):
+        """viml_solve_options; the defaults are ceres::Solver::Options'."""
+        o = _abi.SolveOptions()
+        o.max_iterations, o.max_consecutive_invalid = int(max_iterations), int(max_consecutive_invalid)
+        o.initial_radius, o.max_radius, o.min_radius = float(initial_radius), float(max_radius), float(min_radius)
+        o.min_relative_decrease, o.function_tolerance = float(min_relative_decrease), float(function_tolerance)
+        o.parameter_tolerance = float(parameter_tolerance)
+        return o
+
+    def solve_vi(self, batch, vi, extra, flags, max_iterations=50, max_consecutive_invalid=5, initial_radius=1e4,
+                 max_radius=1e16, min_radius=1e-32, min_relative_decrease=1e-3, function_tolerance=1e-6, parameter_tolerance=1e-8,
+                 obs_table=False, line_table=False):
+        """viml_solve_vi with host buffers: dict(poses, ex_pose, inv_depth, extra, status, iterations, accepted, cost [W,2],
+        radius [W], trace [W,max_iterations,4])."""
+        X, W = vi.X, batch.W
+        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
+               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan),
+               "status": np.full(W, -1, dtype=np.int32), "iterations": np.full(W, -1, dtype=np.int32),
+               "accepted": np.full(W, -1, dtype=np.int32), "cost": np.full((W, 2), np.nan), "radius": np.full(W, np.nan),
+               "trace": np.full((W, max(int(max_iterations), 0), 4), -1.0)}
+        s, _keep = self._batch_struct(batch, obs_table, line_table)
+        v = vi.struct()
+        ex = None if extra is None else np.ascontiguousarray(extra, dtype=np.float64)
+        opt = self.solve_options(max_iterations, max_consecutive_invalid, initial_radius, max_radius, min_radius,
+                                 min_relative_decrease, function_tolerance, parameter_tolerance)
+        o = _abi.SolveOut()
+        for k in _abi.SOLVE_OUT_FIELDS:
+            setattr(o, k, _abi.ptr(res[k]))
+        o.extra = _abi.ptr(res["extra"]) if X > 0 else None
+        self._check(self.lib.viml_solve_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), C.byref(opt), C.byref(o),
+                                           flags & ~PTRS_DEVICE))
         return res
 
     def linearize(self, batch, flags, out=None, obs_table=False, line_table=False):

@@ -24,6 +24,7 @@ FOV_CACHED = 0x200
 FOV_SLOTS = 11
 BLOCK_POSE, BLOCK_EX, BLOCK_EXTRA = 0, 1, 2
 PRIOR_X0_STRIDE = 9
+SOLVE_NO_CONVERGENCE, SOLVE_FUNCTION_TOL, SOLVE_PARAMETER_TOL, SOLVE_MIN_RADIUS, SOLVE_FAILURE = 0, 1, 2, 3, 4
 
 c_double_p = C.POINTER(C.c_double)
 c_float_p = C.POINTER(C.c_float)
@@ -114,6 +115,21 @@ class GnOptions(C.Structure):
 class GnOut(C.Structure):
     _fields_ = [("poses", C.c_void_p), ("ex_pose", C.c_void_p), ("inv_depth", C.c_void_p), ("extra", C.c_void_p),
                 ("dx", C.c_void_p), ("cost", C.c_void_p), ("solved", C.c_void_p)]
+
+
+class SolveOptions(C.Structure):
+    """viml_solve_options — the trust-region loop of viml_solve_vi (Ceres' defaults in Context.solve_vi)."""
+
+    _fields_ = [("max_iterations", C.c_int32), ("max_consecutive_invalid", C.c_int32), ("initial_radius", C.c_double),
+                ("max_radius", C.c_double), ("min_radius", C.c_double), ("min_relative_decrease", C.c_double),
+                ("function_tolerance", C.c_double), ("parameter_tolerance", C.c_double)]
+
+
+SOLVE_OUT_FIELDS = ("poses", "ex_pose", "inv_depth", "extra", "status", "iterations", "accepted", "cost", "radius", "trace")
+
+
+class SolveOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in SOLVE_OUT_FIELDS]
 
 
 class Dense:

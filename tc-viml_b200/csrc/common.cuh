@@ -215,14 +215,39 @@ int viml_launch_expand_obs(viml_ctx* ctx, const LinearizeArgs& a, const void* fe
 // line table -> the nine lf_geom planes for the line-factor range of `a` (a.lf_geom is the destination, absolute factor ids)
 int viml_launch_expand_lines(viml_ctx* ctx, const LinearizeArgs& a, const int32_t* lf_map_index, const float* lf_seg2d);
 int viml_launch_reduced(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double* Sx, double* gx);
+// lambda_w (nullable): a damping per window instead of `lambda`; running (nullable): only windows with running[w] != 0 are solved,
+// updated and costed (the others are left untouched).
 int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double lambda,
-                                 double* dx, int32_t* solved, double* cost);
+                                 double* dx, int32_t* solved, double* cost, const double* lambda_w = nullptr,
+                                 const int32_t* running = nullptr);
 int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const double* Sx, const double* gx, double* dx, int32_t* solved,
-                         double* cost);
+                         double* cost, const double* lambda_w = nullptr, const int32_t* running = nullptr);
 int viml_launch_gn_update(viml_ctx* ctx, const LinearizeArgs& a, int X, const double* extra_in, const double* dx, const int32_t* solved,
-                          double* o_poses, double* o_ex, double* o_dep, double* o_extra);
+                          double* o_poses, double* o_ex, double* o_dep, double* o_extra, const int32_t* running = nullptr);
 int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, const int32_t* solved, int slot,
-                     double* cost);
+                     double* cost, const int32_t* running = nullptr);
+
+// viml_solve_vi: the trust-region state of one window between rounds (written by policy_kernel only).
+struct SolveState {
+  double radius, decrease_factor;
+  double f0, f;                 // f(x0), f at the current state x
+  int32_t consecutive_invalid, iterations, accepted, status;
+};
+struct SolveArgs {  // device pointers only
+  viml_solve_options opt;
+  int P, F, X, Dx;
+  SolveState* state;            // [W]
+  int32_t* running;             // [W] read by the gated kernels of the next round
+  double* lambda_w;             // [W] 1 / radius for the next round
+  double *x_poses, *x_ex, *x_dep, *x_extra;              // the current state x
+  const double *p_poses, *p_ex, *p_dep, *p_extra;        // x+ of this round
+  const double* dx;             // [W][Dx] this round's reduced step
+  const double* cost;           // [W][3]  this round's f(x), f(x+), model decrease
+  const int32_t* solved;        // [W]
+  viml_solve_out out;           // device pointers (radius, trace nullable)
+};
+// One CTA per window: applies the policy of viml.h to this round's step (round 0 also starts the state from the options).
+int viml_launch_solve_policy(viml_ctx* ctx, int W, const SolveArgs& s, int round);
 // schur_kernels.cu
 int viml_launch_schur(viml_ctx* ctx, int W, int F, int D, const double* H_pp, const double* H_lp, const double* H_ll,
                       const double* b_p, const double* b_l, double* S, double* g, double eps);

@@ -1,6 +1,7 @@
 // gn_api.cu — C-ABI entry points for the reduced system of the whole window (dense-block factors: prior, IMU) and one
 // Gauss-Newton / Levenberg-Marquardt iteration on it, plus the line_3d.txt map reader.  See include/viml.h.
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
@@ -228,39 +229,43 @@ int stage_dense(viml_ctx* ctx, Stager& st, const viml_dense_factors* dense, int 
   return VIML_OK;
 }
 
-// Shared core of viml_reduced_system / viml_gn_step.
-// With `vi` the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at x+
-// (cost[1], exactly); `dense` is then ignored.
-int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
-        const viml_gn_options* opt, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags,
-        const viml_inertial_factors* vi = nullptr) {
-  int rc = check_batch(ctx, in);
-  if (rc != VIML_OK) return rc;
+// Everything one Gauss-Newton step enqueues (device pointers), staged once: viml_gn_step / viml_gn_step_vi enqueue one step,
+// viml_solve_vi one per round.  The state the step starts from is a.poses, a.ex_pose, a.inv_depth and extra; x+ goes to o_*.
+struct StepPlan {
+  int W, X, Dx;
+  bool vi, want_sx;   // the dense-block factors are the IMU / prior factors; the caller asked for Sx or gx
+  LinearizeArgs a;
+  DenseArgs dn;
+  InertialArgs va;
+  InertialCsr csr;
+  double* res_plus;   // residuals of the IMU / prior factors at x+
+  const double* extra;
+  double *Sx, *gx, *dx, *cost;
+  int32_t* solved;
+  double *o_poses, *o_ex, *o_dep, *o_extra;
+  // observation / line tables expanded on the device once (viml.h, viml_window_batch)
+  bool obs_table, obs_f32, line_table;
+  const double *fobs, *obsj;
+  const float *fobs32, *obsj32, *lseg;
+  const int32_t* lidx;
+  double *obs, *geom;   // their expansions
+};
+
+// Checks what viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi share and stages their inputs, scratch and the
+// outputs of `rout` / `gout` (null fields: device scratch) into `st`.  The caller commits `st`, then calls expand_tables().
+int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
+               const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags, const viml_inertial_factors* vi, StepPlan* s) {
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
   const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
-  if (vi) {
-    dense = nullptr;
-    rc = check_inertial(ctx, vi, W, P, (flags & VIML_PTRS_DEVICE) != 0);
-    if (rc != VIML_OK) return rc;
-    if (vi->extra_dim > 0 && !extra_state) return fail(ctx, VIML_ERR_INVALID, "viml_gn_step_vi: extra_dim > 0 needs extra_state");
-  }
-  const int X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, Dx = D + X;
-  const int64_t ND = dense ? dense->n_factors : 0;
-  if (X < 0 || ND < 0 || Dx > kMaxDx) return fail(ctx, VIML_ERR_INVALID, "dense factors: extra_dim out of range (D + extra_dim <= 232)");
-  const bool step = gout != nullptr;
-  if (step && !(gout->poses && gout->ex_pose && (F == 0 || gout->inv_depth) && gout->cost && gout->solved))
-    return fail(ctx, VIML_ERR_INVALID, "viml_gn_step needs poses, ex_pose, inv_depth, cost and solved outputs");
-  if (step && X > 0 && !gout->extra) return fail(ctx, VIML_ERR_INVALID, "viml_gn_step: extra_dim > 0 needs the extra output");
-  if (!step && !(rout && rout->Sx && rout->gx)) return fail(ctx, VIML_ERR_INVALID, "viml_reduced_system needs Sx and gx");
-  if (W == 0) return VIML_OK;
-  VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
-  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
-  Stager st{ctx, dev};
-  DenseArgs dn{};
-  dn.X = X;
-  rc = stage_dense(ctx, st, dense, W, Dx, &dn);
+  const bool dev = st.dev;
+  *s = StepPlan{};
+  s->W = W, s->X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, s->Dx = D + s->X;
+  s->vi = vi != nullptr, s->want_sx = rout && (rout->Sx || rout->gx);
+  const int X = s->X, Dx = s->Dx;
+  s->dn.X = X;
+  int rc = stage_dense(ctx, st, dense, W, Dx, &s->dn);
   if (rc != VIML_OK) return rc;
-  LinearizeArgs a{};
+  LinearizeArgs& a = s->a;
   a.W = W, a.P = P, a.F = F, a.D = D, a.NP = NP, a.NL = NL, a.pf_begin = 0, a.lf_begin = 0, a.NL_stride = NL;
   a.sqrt_info = ctx->cfg.sqrt_info, a.cauchy_a = ctx->cfg.cauchy_a, a.inv_cauchy_a2 = 1.0 / (ctx->cfg.cauchy_a * ctx->cfg.cauchy_a);
   a.fx = ctx->cfg.fx, a.fy = ctx->cfg.fy, a.cx = ctx->cfg.cx, a.cy = ctx->cfg.cy;
@@ -270,52 +275,39 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   st.in(in->inv_depth, (size_t)W * F, &a.inv_depth);
   st.in(in->pf_window_offset, (size_t)W + 1, &a.pf_window_offset);
   st.in(in->pf_idx, (size_t)NP, &a.pf_idx);
-  const bool obs_table = !in->pf_obs && NP > 0;   // observations as a per-feature table (viml.h): expanded on the device
-  const bool obs_f32 = obs_table && !(in->feat_obs && in->pf_obs_j);
-  const double *d_fobs = nullptr, *d_obsj = nullptr;
-  const float *d_fobs32 = nullptr, *d_obsj32 = nullptr;
-  double* d_obs = nullptr;
-  if (obs_f32) {
-    st.in(in->feat_obs_f32, (size_t)W * F * 2, &d_fobs32);
-    st.in(in->pf_obs_j_f32, (size_t)NP * 2, &d_obsj32);
-  } else if (obs_table) {
-    st.in(in->feat_obs, (size_t)W * F * 2, &d_fobs);
-    st.in(in->pf_obs_j, (size_t)NP * 2, &d_obsj);
+  s->obs_table = !in->pf_obs && NP > 0;   // observations as a per-feature table (viml.h): expanded on the device
+  s->obs_f32 = s->obs_table && !(in->feat_obs && in->pf_obs_j);
+  if (s->obs_f32) {
+    st.in(in->feat_obs_f32, (size_t)W * F * 2, &s->fobs32);
+    st.in(in->pf_obs_j_f32, (size_t)NP * 2, &s->obsj32);
+  } else if (s->obs_table) {
+    st.in(in->feat_obs, (size_t)W * F * 2, &s->fobs);
+    st.in(in->pf_obs_j, (size_t)NP * 2, &s->obsj);
   } else {
     st.in(in->pf_obs, (size_t)NP * 4, &a.pf_obs);
   }
   st.in(in->pf_pts_i_z, in->pf_pts_i_z ? (size_t)NP : 0, &a.pf_pts_i_z);
   st.in(in->lf_window_offset, NL > 0 ? (size_t)W + 1 : 0, &a.lf_window_offset);
   st.in(in->lf_frame, (size_t)NL, &a.lf_frame);
-  const bool line_table = NL > 0 && !in->lf_geom;   // line factors as (map line, 2D segment): expanded on the device
-  const int32_t* d_lidx = nullptr;
-  const float* d_lseg = nullptr;
-  double* d_geom = nullptr;
-  if (line_table) {
+  s->line_table = NL > 0 && !in->lf_geom;   // line factors as (map line, 2D segment): expanded on the device
+  if (s->line_table) {
     if (!dev)
       for (int64_t k = 0; k < NL; ++k)
         if (in->lf_map_index[k] < 0 || in->lf_map_index[k] >= ctx->n_map) return fail(ctx, VIML_ERR_INVALID, "line factor: map index outside the map");
-    st.in(in->lf_map_index, (size_t)NL, &d_lidx);
-    st.in(in->lf_seg2d_f32, (size_t)NL * 4, &d_lseg);
+    st.in(in->lf_map_index, (size_t)NL, &s->lidx);
+    st.in(in->lf_seg2d_f32, (size_t)NL * 4, &s->lseg);
   } else {
     st.in(in->lf_geom, (size_t)NL * 9, &a.lf_geom);
   }
-  const double* d_extra = nullptr;
-  st.in(extra_state, extra_state ? (size_t)W * X : 0, &d_extra);
-  InertialArgs va{};
-  InertialCsr csr{};
-  double* res_plus = nullptr;   // residuals of the IMU / prior factors at x+
+  st.in(extra_state, extra_state ? (size_t)W * X : 0, &s->extra);
   if (vi) {
-    stage_inertial(st, vi, W, P, &va);
-    stage_inertial_csr(st, va, &csr, &res_plus);
+    stage_inertial(st, vi, W, P, &s->va);
+    stage_inertial_csr(st, s->va, &s->csr, &s->res_plus);
   }
   // scratch (host == nullptr) and outputs
-  double *cache = nullptr, *Sx = nullptr, *gx = nullptr, *dxv = nullptr, *cost = nullptr;
-  double *o_poses = nullptr, *o_ex = nullptr, *o_dep = nullptr, *o_extra = nullptr;
-  int32_t* solved = nullptr;
-  st.out((double*)nullptr, (size_t)W * (P * kPoseCache + kExCache), &cache);
-  if (obs_table) st.out((double*)nullptr, (size_t)NP * 4, &d_obs);
-  if (line_table) st.out((double*)nullptr, (size_t)NL * 9, &d_geom);
+  st.out((double*)nullptr, (size_t)W * (P * kPoseCache + kExCache), &a.cache);
+  if (s->obs_table) st.out((double*)nullptr, (size_t)NP * 4, &s->obs);
+  if (s->line_table) st.out((double*)nullptr, (size_t)NL * 9, &s->geom);
   st.out((double*)nullptr, (size_t)W * D * D, &a.out.H_pp);
   st.out((double*)nullptr, (size_t)W * F * D, &a.out.H_lp);
   st.out((double*)nullptr, (size_t)W * F, &a.out.H_ll);
@@ -323,80 +315,151 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   st.out((double*)nullptr, (size_t)W * F, &a.out.b_l);
   st.out((double*)nullptr, (size_t)W * D * D, &a.out.S);
   st.out((double*)nullptr, (size_t)W * D, &a.out.g);
-  st.out(rout ? rout->Sx : nullptr, (size_t)W * Dx * Dx, &Sx);
-  st.out(rout ? rout->gx : nullptr, (size_t)W * Dx, &gx);
-  if (step) {
-    st.out(gout->dx, (size_t)W * Dx, &dxv);
-    st.out(gout->cost, (size_t)W * 3, &cost);
-    st.out(gout->solved, (size_t)W, &solved);
-    st.out(gout->poses, (size_t)W * P * 7, &o_poses);
-    st.out(gout->ex_pose, (size_t)W * 7, &o_ex);
-    st.out(gout->inv_depth, (size_t)W * F, &o_dep);
-    if (X > 0) st.out(gout->extra, (size_t)W * X, &o_extra);
+  st.out(rout ? rout->Sx : nullptr, (size_t)W * Dx * Dx, &s->Sx);
+  st.out(rout ? rout->gx : nullptr, (size_t)W * Dx, &s->gx);
+  if (gout) {
+    st.out(gout->dx, (size_t)W * Dx, &s->dx);
+    st.out(gout->cost, (size_t)W * 3, &s->cost);
+    st.out(gout->solved, (size_t)W, &s->solved);
+    st.out(gout->poses, (size_t)W * P * 7, &s->o_poses);
+    st.out(gout->ex_pose, (size_t)W * 7, &s->o_ex);
+    st.out(gout->inv_depth, (size_t)W * F, &s->o_dep);
+    if (X > 0) st.out(gout->extra, (size_t)W * X, &s->o_extra);
   }
-  rc = st.commit();
-  if (rc != VIML_OK) return rc;
-  a.cache = cache;
-  if (obs_table) {
-    a.pf_obs = d_obs;
-    rc = obs_f32 ? viml_launch_expand_obs(ctx, a, d_fobs32, d_obsj32, true) : viml_launch_expand_obs(ctx, a, d_fobs, d_obsj, false);
+  return VIML_OK;
+}
+
+// The observation and line tables of the batch, expanded into the per-factor arrays every step reads (after st.commit()).
+int expand_tables(viml_ctx* ctx, StepPlan& s) {
+  if (s.obs_table) {
+    s.a.pf_obs = s.obs;
+    const int rc = s.obs_f32 ? viml_launch_expand_obs(ctx, s.a, s.fobs32, s.obsj32, true)
+                             : viml_launch_expand_obs(ctx, s.a, s.fobs, s.obsj, false);
     if (rc != VIML_OK) return rc;
   }
-  if (line_table) {
-    a.lf_geom = d_geom;
-    rc = viml_launch_expand_lines(ctx, a, d_lidx, d_lseg);
-    if (rc != VIML_OK) return rc;
+  if (s.line_table) {
+    s.a.lf_geom = s.geom;
+    return viml_launch_expand_lines(ctx, s.a, s.lidx, s.lseg);
   }
-  rc = viml_launch_linearize(ctx, a);
+  return VIML_OK;
+}
+
+// One step at the state of s.a / s.extra: the reduced system (Sx, gx when the caller asked for them) and, with s.cost set, the
+// solve, the update into s.o_* and the costs.  lambda_w / running: see viml_launch_gn_reduced_solve (nullptr: `lambda`, every window).
+// With s.vi the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at
+// x+ (cost[1], exactly); s.dn is then replaced by their CSR.
+int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* lambda_w, const int32_t* running) {
+  const LinearizeArgs& a = s.a;
+  const int W = s.W, D = a.D, X = s.X, Dx = s.Dx;
+  const bool step = s.cost != nullptr;
+  int rc = viml_launch_linearize(ctx, a);
   if (rc != VIML_OK) return rc;
-  if (vi) {   // the dense-block factors at x, in the CSR every kernel below reads
-    va.poses = a.poses, va.ex_pose = a.ex_pose, va.extra = d_extra;
-    rc = viml_launch_inertial(ctx, va, viml_inertial_out{}, csr, true);
+  DenseArgs dn = s.dn;
+  InertialArgs va = s.va;
+  if (s.vi) {   // the dense-block factors at x, in the CSR every kernel below reads
+    va.poses = a.poses, va.ex_pose = a.ex_pose, va.extra = s.extra;
+    rc = viml_launch_inertial(ctx, va, viml_inertial_out{}, s.csr, true);
     if (rc != VIML_OK) return rc;
     dn.ND = (int64_t)W + va.NI;   // an upper bound: the kernels read ND only as "any dense factors"
-    dn.window_offset = csr.window_offset, dn.row_offset = csr.row_offset, dn.col_offset = csr.col_offset;
-    dn.jac_offset = csr.jac_offset, dn.col_index = csr.col_index, dn.residual = csr.residual, dn.jacobian = csr.jacobian;
+    dn.window_offset = s.csr.window_offset, dn.row_offset = s.csr.row_offset, dn.col_offset = s.csr.col_offset;
+    dn.jac_offset = s.csr.jac_offset, dn.col_index = s.csr.col_index, dn.residual = s.csr.residual, dn.jacobian = s.csr.jacobian;
   }
   // a step that does not have to hand Sx / gx to the caller builds and solves the reduced system in one kernel
   bool fused = false;
-  if (step && !(rout && (rout->Sx || rout->gx))) {
-    rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, cost);
+  if (step && !s.want_sx) {
+    rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
     if (rc != VIML_OK) return rc;
-    rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, opt ? opt->lambda : 0.0, dxv, solved, cost);
+    rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, lambda, s.dx, s.solved, s.cost, lambda_w, running);
     if (rc == VIML_OK) fused = true;
     else if (rc != VIML_ERR_UNSUPPORTED) return rc;
   }
   if (!fused) {
-    rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, Sx, gx);
+    rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
     if (rc != VIML_OK) return rc;
   }
-  if (step) {
-    rc = VIML_OK;
-    if (!fused) {
-      rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, cost);
-      if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, opt ? opt->lambda : 0.0, Sx, gx, dxv, solved, cost);
-    }
-    if (rc == VIML_OK) rc = viml_launch_gn_update(ctx, a, X, d_extra, dxv, solved, o_poses, o_ex, o_dep, o_extra);
-    if (rc != VIML_OK) return rc;
-    LinearizeArgs a2 = a;
-    a2.poses = o_poses, a2.ex_pose = o_ex, a2.inv_depth = o_dep;
-    rc = viml_launch_prep(ctx, a2);
-    if (rc != VIML_OK) return rc;
-    if (vi) {   // f(x+): the IMU / prior residuals re-evaluated at x+ (same CSR structure), 1/2 |r|^2 without the linear model
-      InertialArgs vp = va;
-      vp.poses = o_poses, vp.ex_pose = o_ex, vp.extra = o_extra;
-      InertialCsr cp = csr;
-      cp.residual = res_plus, cp.jacobian = nullptr;
-      rc = viml_launch_inertial(ctx, vp, viml_inertial_out{}, cp, false);
-      DenseArgs dp = dn;
-      dp.residual = res_plus;
-      if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, nullptr, 1, cost);
-    } else {
-      rc = viml_launch_cost(ctx, a2, dn, dxv, solved, 1, cost);
-    }
-    if (rc != VIML_OK) return rc;
+  if (!step) return VIML_OK;
+  rc = VIML_OK;
+  if (!fused) {
+    rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
+    if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, lambda, s.Sx, s.gx, s.dx, s.solved, s.cost, lambda_w, running);
   }
+  if (rc == VIML_OK) rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running);
+  if (rc != VIML_OK) return rc;
+  LinearizeArgs a2 = a;
+  a2.poses = s.o_poses, a2.ex_pose = s.o_ex, a2.inv_depth = s.o_dep;
+  rc = viml_launch_prep(ctx, a2);
+  if (rc != VIML_OK) return rc;
+  if (s.vi) {   // f(x+): the IMU / prior residuals re-evaluated at x+ (same CSR structure), 1/2 |r|^2 without the linear model
+    InertialArgs vp = va;
+    vp.poses = s.o_poses, vp.ex_pose = s.o_ex, vp.extra = s.o_extra;
+    InertialCsr cp = s.csr;
+    cp.residual = s.res_plus, cp.jacobian = nullptr;
+    rc = viml_launch_inertial(ctx, vp, viml_inertial_out{}, cp, false);
+    DenseArgs dp = dn;
+    dp.residual = s.res_plus;
+    if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, nullptr, 1, s.cost, running);
+  } else {
+    rc = viml_launch_cost(ctx, a2, dn, s.dx, s.solved, 1, s.cost, running);
+  }
+  return rc;
+}
+
+// Checks shared by viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi: the batch, and with `vi` the inertial
+// factors and the extra state.
+int check_step_inputs(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
+                      uint32_t flags, const viml_inertial_factors* vi, const char* who) {
+  int rc = check_batch(ctx, in);
+  if (rc != VIML_OK) return rc;
+  const int P = in->poses_per_window, D = 6 * (P + 1);
+  if (vi) {
+    rc = check_inertial(ctx, vi, in->n_windows, P, (flags & VIML_PTRS_DEVICE) != 0);
+    if (rc != VIML_OK) return rc;
+    if (vi->extra_dim > 0 && !extra_state) {
+      ctx->err = std::string(who) + ": extra_dim > 0 needs extra_state";
+      return VIML_ERR_INVALID;
+    }
+  }
+  const int X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0;
+  const int64_t ND = dense && !vi ? dense->n_factors : 0;
+  if (X < 0 || ND < 0 || D + X > kMaxDx) return fail(ctx, VIML_ERR_INVALID, "dense factors: extra_dim out of range (D + extra_dim <= 232)");
+  return VIML_OK;
+}
+
+// viml_reduced_system / viml_gn_step / viml_gn_step_vi: one step (or the reduced system alone).
+int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
+        const viml_gn_options* opt, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags,
+        const viml_inertial_factors* vi = nullptr) {
+  if (vi) dense = nullptr;
+  int rc = check_step_inputs(ctx, in, dense, extra_state, flags, vi, "viml_gn_step_vi");
+  if (rc != VIML_OK) return rc;
+  const int W = in->n_windows, F = in->feats_per_window, X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0;
+  const bool step = gout != nullptr;
+  if (step && !(gout->poses && gout->ex_pose && (F == 0 || gout->inv_depth) && gout->cost && gout->solved))
+    return fail(ctx, VIML_ERR_INVALID, "viml_gn_step needs poses, ex_pose, inv_depth, cost and solved outputs");
+  if (step && X > 0 && !gout->extra) return fail(ctx, VIML_ERR_INVALID, "viml_gn_step: extra_dim > 0 needs the extra output");
+  if (!step && !(rout && rout->Sx && rout->gx)) return fail(ctx, VIML_ERR_INVALID, "viml_reduced_system needs Sx and gx");
+  if (W == 0) return VIML_OK;
+  VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
+  Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
+  StepPlan s;
+  rc = stage_step(ctx, st, in, dense, extra_state, rout, gout, flags, vi, &s);
+  if (rc == VIML_OK) rc = st.commit();
+  if (rc == VIML_OK) rc = expand_tables(ctx, s);
+  if (rc == VIML_OK) rc = enqueue_step(ctx, s, opt ? opt->lambda : 0.0, nullptr, nullptr);
+  if (rc != VIML_OK) return rc;
   return st.finish();
+}
+
+int check_solve_options(viml_ctx* ctx, const viml_solve_options* o) {
+  if (!o) return fail(ctx, VIML_ERR_INVALID, "viml_solve_vi: null options");
+  if (o->max_iterations <= 0 || o->max_consecutive_invalid < 0)
+    return fail(ctx, VIML_ERR_INVALID, "viml_solve_vi: max_iterations must be > 0 and max_consecutive_invalid >= 0");
+  if (!(std::isfinite(o->min_radius) && std::isfinite(o->initial_radius) && std::isfinite(o->max_radius) && o->min_radius > 0.0 &&
+        o->min_radius <= o->initial_radius && o->initial_radius <= o->max_radius))
+    return fail(ctx, VIML_ERR_INVALID, "viml_solve_vi: radii must be finite with 0 < min_radius <= initial_radius <= max_radius");
+  if (!(o->min_relative_decrease >= 0.0 && o->function_tolerance >= 0.0 && o->parameter_tolerance >= 0.0))
+    return fail(ctx, VIML_ERR_INVALID, "viml_solve_vi: min_relative_decrease and the tolerances must be >= 0");
+  return VIML_OK;
 }
 
 }  // namespace
@@ -449,6 +512,68 @@ int viml_gn_step_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inert
   if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
   if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
   return run(ctx, in, nullptr, extra_state, opt, nullptr, out, flags, vi);
+}
+
+int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
+                  const viml_solve_options* opt, const viml_solve_out* out, uint32_t flags) {
+  if (!ctx) return VIML_ERR_INVALID;
+  if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
+  if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
+  int rc = check_step_inputs(ctx, in, nullptr, extra_state, flags, vi, "viml_solve_vi");
+  if (rc == VIML_OK) rc = check_solve_options(ctx, opt);
+  if (rc != VIML_OK) return rc;
+  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, X = vi->extra_dim, M = opt->max_iterations;
+  if (!(out->poses && out->ex_pose && (F == 0 || out->inv_depth) && (X == 0 || out->extra) && out->status && out->iterations &&
+        out->accepted && out->cost))
+    return fail(ctx, VIML_ERR_INVALID, "viml_solve_vi needs poses, ex_pose, inv_depth (F > 0), extra (X > 0), status, iterations, "
+                                       "accepted and cost outputs");
+  if (W == 0) return VIML_OK;
+  VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
+  Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
+  StepPlan s;
+  const viml_gn_out scratch{};   // x+, dx, cost and solved of every round stay on the device
+  rc = stage_step(ctx, st, in, nullptr, extra_state, nullptr, &scratch, flags, vi, &s);
+  if (rc != VIML_OK) return rc;
+  SolveArgs sa{};
+  sa.opt = *opt;
+  sa.P = P, sa.F = F, sa.X = X, sa.Dx = s.Dx;
+  st.out((SolveState*)nullptr, (size_t)W, &sa.state);
+  st.out((int32_t*)nullptr, (size_t)W, &sa.running);
+  st.out((double*)nullptr, (size_t)W, &sa.lambda_w);
+  st.out((double*)nullptr, (size_t)W * P * 7, &sa.x_poses);
+  st.out((double*)nullptr, (size_t)W * 7, &sa.x_ex);
+  st.out((double*)nullptr, (size_t)W * F, &sa.x_dep);
+  st.out((double*)nullptr, (size_t)W * X, &sa.x_extra);
+  st.out(out->poses, (size_t)W * P * 7, &sa.out.poses);
+  st.out(out->ex_pose, (size_t)W * 7, &sa.out.ex_pose);
+  st.out(out->inv_depth, (size_t)W * F, &sa.out.inv_depth);
+  st.out(out->extra, (size_t)W * X, &sa.out.extra);
+  st.out(out->status, (size_t)W, &sa.out.status);
+  st.out(out->iterations, (size_t)W, &sa.out.iterations);
+  st.out(out->accepted, (size_t)W, &sa.out.accepted);
+  st.out(out->cost, (size_t)W * 2, &sa.out.cost);
+  st.out(out->radius, out->radius ? (size_t)W : 0, &sa.out.radius);
+  st.out(out->trace, out->trace ? (size_t)W * M * 4 : 0, &sa.out.trace);
+  rc = st.commit();
+  if (rc == VIML_OK) rc = expand_tables(ctx, s);
+  if (rc != VIML_OK) return rc;
+  // the rounds work on a copy of the initial state: the inputs stay untouched
+  const size_t n_pose = (size_t)W * P * 7, n_ex = (size_t)W * 7, n_dep = (size_t)W * F, n_extra = (size_t)W * X;
+  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_poses, s.a.poses, n_pose * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_ex, s.a.ex_pose, n_ex * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (n_dep) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_dep, s.a.inv_depth, n_dep * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (n_extra) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_extra, s.extra, n_extra * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  s.a.poses = sa.x_poses, s.a.ex_pose = sa.x_ex, s.a.inv_depth = sa.x_dep, s.extra = sa.x_extra;
+  sa.p_poses = s.o_poses, sa.p_ex = s.o_ex, sa.p_dep = s.o_dep, sa.p_extra = s.o_extra;
+  sa.dx = s.dx, sa.cost = s.cost, sa.solved = s.solved;
+  // round 0 runs every window at lambda = 1 / initial_radius; policy_kernel then starts each window's state from that step and
+  // hands the next round its running flags and lambdas
+  for (int r = 0; r < M && rc == VIML_OK; ++r) {
+    rc = enqueue_step(ctx, s, 1.0 / opt->initial_radius, r ? sa.lambda_w : nullptr, r ? sa.running : nullptr);
+    if (rc == VIML_OK) rc = viml_launch_solve_policy(ctx, W, sa, r);
+  }
+  if (rc != VIML_OK) return rc;
+  return st.finish();
 }
 
 int viml_inertial_evaluate(viml_ctx* ctx, const viml_window_batch* state, const double* extra_state, const viml_inertial_factors* vi,

@@ -105,14 +105,19 @@ constexpr int kFusedStage = 6656;   // doubles for a staged dense-factor Jacobia
 constexpr int kTile = 8;
 __device__ __forceinline__ int tile_at(int I, int J) { return (I * (I + 1) / 2 + J) * 64; }
 
+// lambda_w (nullable): a damping per window instead of `lambda`; running (nullable): a window with running[w] == 0 is skipped
+// (its CTA returns at once and writes nothing).
 template <bool FUSED>
 __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda, const double* __restrict__ Sx, const double* __restrict__ gx,
                                                           double* __restrict__ dx, int32_t* __restrict__ solved, double* __restrict__ cost,
-                                                          int D, DenseArgs dn, const double* __restrict__ S, const double* __restrict__ g) {
+                                                          int D, DenseArgs dn, const double* __restrict__ S, const double* __restrict__ g,
+                                                          const double* __restrict__ lambda_w, const int32_t* __restrict__ running) {
   extern __shared__ __align__(16) double sm[];
   __shared__ int s_ok;
   __shared__ double s_red[8], s_dinv[kTile];
   const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (running && !running[w]) return;
+  if (lambda_w) lambda = lambda_w[w];
   const int NB = (Dx + kTile - 1) / kTile, Dp = NB * kTile;
   double* __restrict__ L = sm;                                   // NB (NB + 1) / 2 tiles
   double* __restrict__ y = sm + (size_t)NB * (NB + 1) / 2 * 64;  // [Dp]
@@ -400,11 +405,14 @@ __device__ __forceinline__ void pose_plus(const double* __restrict__ x, const do
   o[3] = qx / n, o[4] = qy / n, o[5] = qz / n, o[6] = w / n;
 }
 
-// New state of every window: poses / extrinsic by Plus, landmarks by back-substitution, extra state by addition.
+// New state of every window: poses / extrinsic by Plus, landmarks by back-substitution, extra state by addition.  running
+// (nullable): windows with running[w] == 0 are skipped.
 __global__ void __launch_bounds__(128) update_kernel(LinearizeArgs A, int X, const double* __restrict__ extra_in, const double* __restrict__ dx,
                                                      const int32_t* __restrict__ solved, double* __restrict__ o_poses,
-                                                     double* __restrict__ o_ex, double* __restrict__ o_dep, double* __restrict__ o_extra) {
+                                                     double* __restrict__ o_ex, double* __restrict__ o_dep, double* __restrict__ o_extra,
+                                                     const int32_t* __restrict__ running) {
   const int w = blockIdx.x, tid = threadIdx.x, P = A.P, F = A.F, D = A.D, Dx = D + X;
+  if (running && !running[w]) return;
   const bool ok = solved[w] != 0;
   const double* __restrict__ d = dx + (size_t)w * Dx;
   for (int p = tid; p <= P; p += blockDim.x) {
@@ -437,11 +445,14 @@ __global__ void __launch_bounds__(128) update_kernel(LinearizeArgs A, int X, con
 
 // cost[3w + slot] = 1/2 sum rho(|r|^2) over the window's point and line factors at the state of A (pose cache ready)
 // + 1/2 sum |r_k + J_k dx|^2 over its dense-block factors (dx == nullptr, or a window the step did not solve: at the
-// linearisation point, so that cost[1] == cost[0] even when a Jacobian holds a NaN).
+// linearisation point, so that cost[1] == cost[0] even when a Jacobian holds a NaN).  running (nullable): windows with
+// running[w] == 0 are skipped.
 __global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn, const double* __restrict__ dx,
-                                                   const int32_t* __restrict__ solved, int slot, double* __restrict__ cost) {
+                                                   const int32_t* __restrict__ solved, int slot, double* __restrict__ cost,
+                                                   const int32_t* __restrict__ running) {
   __shared__ double s_red[4];
   const int w = blockIdx.x, tid = threadIdx.x, Dx = A.D + dn.X;
+  if (running && !running[w]) return;
   const bool moved = dx != nullptr && solved[w] != 0;
   const bool cauchy = (A.flags & VIML_LOSS_CAUCHY) != 0;
   LinearizeArgs R = A;
@@ -493,6 +504,124 @@ __global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn
     for (int k = 0; k < (int)blockDim.x / 32; ++k) t += s_red[k];
     cost[3 * (size_t)w + slot] = 0.5 * t;
   }
+}
+
+// ---- the trust-region policy of viml_solve_vi (viml.h) -------------------------------------------------------------------------
+// One CTA per window after each round's step.  A stopped window only writes a NaN trace row.  A running one reduces |dx| (the
+// reduced step and the landmark increments x+ - x) and |x|, then thread 0 applies the policy; the scalar arithmetic goes through
+// __d*_rn so that no multiply-add is fused, and an IEEE restatement (tests/solve_policy.py) reproduces the radius, the decisions and
+// the trace bit for bit.  The CTA then moves x+ into x on acceptance and, at the window's last step, x into the outputs.
+__global__ void __launch_bounds__(128) policy_kernel(SolveArgs s, int round) {
+  __shared__ double s_red[2][4];
+  __shared__ int s_accept, s_stop;
+  const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int P = s.P, F = s.F, X = s.X, Dx = s.Dx, M = s.opt.max_iterations;
+  const double nan = __longlong_as_double(0x7ff8000000000000LL);
+  double* __restrict__ trow = s.out.trace ? s.out.trace + ((size_t)w * M + round) * 4 : nullptr;
+  if (round > 0 && !s.running[w]) {
+    if (trow && tid < 4) trow[tid] = nan;
+    return;
+  }
+  double dd = 0.0, xx = 0.0;
+  for (int i = tid; i < Dx; i += 128) {
+    const double v = s.dx[(size_t)w * Dx + i];
+    dd += v * v;
+  }
+  for (int l = tid; l < F; l += 128) {
+    const double v = s.x_dep[(size_t)w * F + l], e = s.p_dep[(size_t)w * F + l] - v;
+    dd += e * e;
+    xx += v * v;
+  }
+  for (int i = tid; i < 7 * P + 7 + X; i += 128) {
+    const double v = i < 7 * P ? s.x_poses[(size_t)w * 7 * P + i] : i < 7 * P + 7 ? s.x_ex[(size_t)w * 7 + i - 7 * P]
+                                                                                     : s.x_extra[(size_t)w * X + i - 7 * P - 7];
+    xx += v * v;
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    dd += __shfl_xor_sync(0xffffffffu, dd, o);
+    xx += __shfl_xor_sync(0xffffffffu, xx, o);
+  }
+  if (lane == 0) s_red[0][warp] = dd, s_red[1][warp] = xx;
+  __syncthreads();
+  if (tid == 0) {
+    const viml_solve_options& o = s.opt;
+    SolveState st = s.state[w];
+    const double f = s.cost[3 * (size_t)w], fp = s.cost[3 * (size_t)w + 1], m = s.cost[3 * (size_t)w + 2];
+    int accept = 0, status = -1;
+    if (round == 0) {   // f(x0) is this round's f(x)
+      st.radius = o.initial_radius, st.decrease_factor = 2.0, st.f0 = f, st.f = f;
+      st.consecutive_invalid = st.iterations = st.accepted = 0;
+      if (!isfinite(f)) status = VIML_SOLVE_FAILURE;
+    }
+    if (status >= 0) {
+      if (trow) trow[0] = trow[1] = trow[2] = trow[3] = nan;
+    } else {
+      if (trow) trow[0] = f, trow[1] = fp, trow[2] = m, trow[3] = __ddiv_rn(1.0, st.radius);
+      st.f = f;
+      if (!s.solved[w] || !isfinite(fp) || !(m > 0.0)) {
+        st.consecutive_invalid += 1;
+        st.radius = __ddiv_rn(st.radius, st.decrease_factor);
+        st.decrease_factor = __dmul_rn(st.decrease_factor, 2.0);
+        if (st.consecutive_invalid > o.max_consecutive_invalid) status = VIML_SOLVE_FAILURE;
+      } else {
+        st.consecutive_invalid = 0;
+        const double dnorm = sqrt(s_red[0][0] + s_red[0][1] + s_red[0][2] + s_red[0][3]);
+        const double xnorm = sqrt(s_red[1][0] + s_red[1][1] + s_red[1][2] + s_red[1][3]);
+        if (dnorm <= __dmul_rn(o.parameter_tolerance, __dadd_rn(xnorm, o.parameter_tolerance))) {
+          status = VIML_SOLVE_PARAMETER_TOL;
+        } else if (fabs(__dsub_rn(f, fp)) <= __dmul_rn(o.function_tolerance, f)) {
+          status = VIML_SOLVE_FUNCTION_TOL;
+        } else {
+          const double rho = __ddiv_rn(__dsub_rn(f, fp), m);
+          if (rho > o.min_relative_decrease) {
+            accept = 1;
+            st.accepted += 1;
+            st.f = fp;
+            const double t = __dsub_rn(__dmul_rn(2.0, rho), 1.0);
+            const double c = __dsub_rn(1.0, __dmul_rn(__dmul_rn(t, t), t)), third = 1.0 / 3.0;
+            const double r = __ddiv_rn(st.radius, c > third ? c : third);
+            st.radius = r < o.max_radius ? r : o.max_radius;
+            st.decrease_factor = 2.0;
+          } else {
+            st.radius = __ddiv_rn(st.radius, st.decrease_factor);
+            st.decrease_factor = __dmul_rn(st.decrease_factor, 2.0);
+          }
+        }
+      }
+      st.iterations += 1;
+      if (status < 0) {
+        if (st.radius < o.min_radius) status = VIML_SOLVE_MIN_RADIUS;
+        else if (st.iterations == M) status = VIML_SOLVE_NO_CONVERGENCE;
+      }
+    }
+    st.status = status;
+    s.state[w] = st;
+    if (status >= 0) {
+      s.running[w] = 0;
+      s.out.status[w] = status, s.out.iterations[w] = st.iterations, s.out.accepted[w] = st.accepted;
+      s.out.cost[2 * (size_t)w] = st.f0, s.out.cost[2 * (size_t)w + 1] = st.f;
+      if (s.out.radius) s.out.radius[w] = st.radius;
+    } else {
+      s.running[w] = 1;
+      s.lambda_w[w] = __ddiv_rn(1.0, st.radius);
+    }
+    s_accept = accept, s_stop = status >= 0;
+  }
+  __syncthreads();
+  const bool acc = s_accept != 0, stop = s_stop != 0;
+  if (!acc && !stop) return;
+  auto move = [&](double* __restrict__ x, const double* __restrict__ xp, double* __restrict__ out, size_t base, int n) {
+    for (int i = tid; i < n; i += 128) {
+      const double v = acc ? xp[base + i] : x[base + i];
+      if (acc) x[base + i] = v;
+      if (stop) out[base + i] = v;
+    }
+  };
+  move(s.x_poses, s.p_poses, s.out.poses, (size_t)w * 7 * P, 7 * P);
+  move(s.x_ex, s.p_ex, s.out.ex_pose, (size_t)w * 7, 7);
+  if (F > 0) move(s.x_dep, s.p_dep, s.out.inv_depth, (size_t)w * F, F);
+  if (X > 0) move(s.x_extra, s.p_extra, s.out.extra, (size_t)w * X, X);
 }
 
 }  // namespace gn

@@ -678,11 +678,12 @@ constexpr size_t gn_solve_smem(int Dx) {
 static_assert(gn_solve_smem(kMaxDx) <= 220 * 1024, "the tiled Cholesky of the largest reduced system must fit in shared memory");
 
 int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const double* Sx, const double* gx, double* dx, int32_t* solved,
-                         double* cost) {
+                         double* cost, const double* lambda_w, const int32_t* running) {
   const size_t smem = gn_solve_smem(Dx);
   LaunchScope ls(ctx, K_GN);
   VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  gn::solve_tiled_kernel<false><<<W, 256, smem, ctx->stream>>>(Dx, lambda, Sx, gx, dx, solved, cost, 0, DenseArgs{}, nullptr, nullptr);
+  gn::solve_tiled_kernel<false><<<W, 256, smem, ctx->stream>>>(Dx, lambda, Sx, gx, dx, solved, cost, 0, DenseArgs{}, nullptr, nullptr,
+                                                                lambda_w, running);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
@@ -690,29 +691,37 @@ int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const doub
 // Reduced system + solve in one kernel (viml_gn_step when the caller does not ask for Sx / gx): returns VIML_ERR_UNSUPPORTED when
 // the system does not fit the fused kernel's shared memory, and the caller takes the two-kernel path.
 int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double lambda,
-                                 double* dx, int32_t* solved, double* cost) {
+                                 double* dx, int32_t* solved, double* cost, const double* lambda_w, const int32_t* running) {
   const int Dx = D + dn.X, NB = (Dx + 7) / 8;
   const size_t smem = ((size_t)NB * (NB + 1) / 2 * 64 + 3 * (size_t)NB * 8 + gn::kFusedStage) * sizeof(double);
   if (smem > 224 * 1024) return VIML_ERR_UNSUPPORTED;
   LaunchScope ls(ctx, K_GN);
   VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  gn::solve_tiled_kernel<true><<<W, 256, smem, ctx->stream>>>(Dx, lambda, nullptr, nullptr, dx, solved, cost, D, dn, S, g);
+  gn::solve_tiled_kernel<true><<<W, 256, smem, ctx->stream>>>(Dx, lambda, nullptr, nullptr, dx, solved, cost, D, dn, S, g, lambda_w,
+                                                               running);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
 
 int viml_launch_gn_update(viml_ctx* ctx, const LinearizeArgs& a, int X, const double* extra_in, const double* dx, const int32_t* solved,
-                          double* o_poses, double* o_ex, double* o_dep, double* o_extra) {
+                          double* o_poses, double* o_ex, double* o_dep, double* o_extra, const int32_t* running) {
   LaunchScope ls(ctx, K_GN);
-  gn::update_kernel<<<a.W, 128, 0, ctx->stream>>>(a, X, extra_in, dx, solved, o_poses, o_ex, o_dep, o_extra);
+  gn::update_kernel<<<a.W, 128, 0, ctx->stream>>>(a, X, extra_in, dx, solved, o_poses, o_ex, o_dep, o_extra, running);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
 
 int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, const int32_t* solved, int slot,
-                     double* cost) {
+                     double* cost, const int32_t* running) {
   LaunchScope ls(ctx, K_GN);
-  gn::cost_kernel<<<a.W, 128, 0, ctx->stream>>>(a, dn, dx, solved, slot, cost);
+  gn::cost_kernel<<<a.W, 128, 0, ctx->stream>>>(a, dn, dx, solved, slot, cost, running);
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
+int viml_launch_solve_policy(viml_ctx* ctx, int W, const SolveArgs& s, int round) {
+  LaunchScope ls(ctx, K_GN);
+  gn::policy_kernel<<<W, 128, 0, ctx->stream>>>(s, round);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
