@@ -65,7 +65,7 @@ extern "C" {
 #define VIML_ERR_INVALID (-1)  /* bad argument / inconsistent sizes                               */
 #define VIML_ERR_CUDA (-2)     /* CUDA runtime error (text in viml_last_error)                    */
 #define VIML_ERR_NO_DEVICE (-3)/* no usable sm_100 device: there is deliberately no CPU fallback  */
-#define VIML_ERR_NOMAP (-4)    /* viml_line_associate before viml_set_map                         */
+#define VIML_ERR_NOMAP (-4)    /* viml_line_associate or a line table before viml_set_map         */
 #define VIML_ERR_UNSUPPORTED (-5)
 
 /* ---- flags ---------------------------------------------------------------------------------- */
@@ -167,7 +167,14 @@ int viml_load_line_map(viml_ctx* ctx, const char* path, int64_t* n_lines);
  * the batch carries lf_map_index[k] (index into the map installed by viml_set_map) and lf_seg2d_f32[k] = {sx, sy, ex, ey}: 20 bytes
  * per line factor instead of 72.  The device forms the nine lf_geom values with the reference's operation order (no fused
  * multiply-add): identical results.  Needs a map (VIML_ERR_NOMAP otherwise); an index outside the map is VIML_ERR_INVALID on the
- * host-pointer path and is clamped on the device-pointer path.                                        */
+ * host-pointer path and is clamped on the device-pointer path.
+ *
+ * Every entry point that takes a batch checks it the same way.  Both flavours check the sizes, the null arrays and the map of a line
+ * table (VIML_ERR_NOMAP) before anything is launched.  With host pointers both window offsets must also be CSRs of their factor
+ * arrays and every pose, feature, line frame and map index must be in range, else VIML_ERR_INVALID; no kernel ever reads a bad index.
+ * The offsets are checked before anything is launched, and so are the indices, except in viml_linearize_batch on 512 windows or more:
+ * it checks them chunk by chunk of windows, so the outputs of the chunks before a bad one may already be written.  With device
+ * pointers the offsets and indices are the caller's to keep.                                                                        */
 typedef struct viml_window_batch {
   int32_t n_windows;         /* W                                                               */
   int32_t poses_per_window;  /* P  (WINDOW_SIZE+1 = 11; up to 255)                              */

@@ -154,6 +154,22 @@ struct LinearizeArgs {  // device pointers only
   uint32_t flags;
 };
 
+// How a viml_window_batch carries its observations and line factors (viml.h), decided once by check_window_batch.
+struct BatchForm {
+  bool obs_table, obs_f32;            // observations as the per-feature table (only when NP > 0), in float32
+  bool line_table;                    // line factors as (map index, 2D segment)
+  const void *feat_obs, *pf_obs_j;    // the arrays of the chosen table form
+  size_t obs_bytes;                   // bytes of one {x, y} of the table: 16 or 8
+};
+// viml_api.cu: what every entry point that takes a viml_window_batch checks.  Sizes, null arrays, the form, VIML_ERR_NOMAP for a line
+// table without a map; with host pointers (dev == false) also that both window offsets are CSRs of the factor arrays.
+int check_window_batch(viml_ctx* ctx, const viml_window_batch* in, bool dev, BatchForm* form);
+// Host pointers: the pose, feature, frame and map indices of point factors [pa, pb) and line factors [la, lb) (VIML_ERR_INVALID).
+int check_batch_indices(viml_ctx* ctx, const viml_window_batch* in, const BatchForm& form, int64_t pa, int64_t pb, int64_t la,
+                        int64_t lb);
+// The LinearizeArgs of the whole batch with the context's camera and loss constants; the pointers are left null.
+LinearizeArgs linearize_args(const viml_ctx* ctx, const viml_window_batch* in, uint32_t flags);
+
 // Largest reduced system a Gauss-Newton step takes, Dx = D + extra_dim (viml.h): its tiled Cholesky keeps the lower triangle in
 // shared memory (linearize_kernels.cu checks the size at compile time).
 constexpr int kMaxDx = 232;

@@ -61,18 +61,6 @@ struct Stager {
   }
 };
 
-int check_batch(viml_ctx* ctx, const viml_window_batch* in) {
-  if (!in) return fail(ctx, VIML_ERR_INVALID, "null window batch");
-  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window;
-  if (W < 0 || P < 1 || P > 255 || F < 0 || F > 65535 || in->n_point_factors < 0 || in->n_line_factors < 0)
-    return fail(ctx, VIML_ERR_INVALID, "window batch sizes out of range");
-  if (W > 0 && (!in->poses || !in->ex_pose || (F > 0 && !in->inv_depth) || !in->pf_window_offset ||
-                (in->n_point_factors > 0 && (!in->pf_idx || (!in->pf_obs && !(in->feat_obs && in->pf_obs_j) && !(in->feat_obs_f32 && in->pf_obs_j_f32)))) ||
-                (in->n_line_factors > 0 && (!in->lf_window_offset || !in->lf_frame || (!in->lf_geom && !(in->lf_map_index && in->lf_seg2d_f32))))))
-    return fail(ctx, VIML_ERR_INVALID, "null input array");
-  return VIML_OK;
-}
-
 // viml_inertial_factors: null checks always, index / size validation on the host-pointer path (the device path reads nothing back).
 int check_inertial(viml_ctx* ctx, const viml_inertial_factors* vi, int W, int P, bool dev) {
   if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
@@ -244,56 +232,45 @@ struct StepPlan {
   int32_t* solved;
   double *o_poses, *o_ex, *o_dep, *o_extra;
   // observation / line tables expanded on the device once (viml.h, viml_window_batch)
-  bool obs_table, obs_f32, line_table;
-  const double *fobs, *obsj;
-  const float *fobs32, *obsj32, *lseg;
+  BatchForm form;
+  const char *fobs, *obsj;
+  const float* lseg;
   const int32_t* lidx;
   double *obs, *geom;   // their expansions
 };
 
-// Checks what viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi share and stages their inputs, scratch and the
-// outputs of `rout` / `gout` (null fields: device scratch) into `st`.  The caller commits `st`, then calls expand_tables().
-int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
-               const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags, const viml_inertial_factors* vi, StepPlan* s) {
+// Stages the inputs of viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi (checked by check_step_inputs, which
+// gave `form`), their scratch and the outputs of `rout` / `gout` (null fields: device scratch) into `st`.  The caller commits `st`,
+// then calls expand_tables().
+int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const BatchForm& form, const viml_dense_factors* dense,
+               const double* extra_state, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags,
+               const viml_inertial_factors* vi, StepPlan* s) {
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
   const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
-  const bool dev = st.dev;
   *s = StepPlan{};
   s->W = W, s->X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, s->Dx = D + s->X;
   s->vi = vi != nullptr, s->want_sx = rout && (rout->Sx || rout->gx);
+  s->form = form;
   const int X = s->X, Dx = s->Dx;
   s->dn.X = X;
   int rc = stage_dense(ctx, st, dense, W, Dx, &s->dn);
   if (rc != VIML_OK) return rc;
-  LinearizeArgs& a = s->a;
-  a.W = W, a.P = P, a.F = F, a.D = D, a.NP = NP, a.NL = NL, a.pf_begin = 0, a.lf_begin = 0, a.NL_stride = NL;
-  a.sqrt_info = ctx->cfg.sqrt_info, a.cauchy_a = ctx->cfg.cauchy_a, a.inv_cauchy_a2 = 1.0 / (ctx->cfg.cauchy_a * ctx->cfg.cauchy_a);
-  a.fx = ctx->cfg.fx, a.fy = ctx->cfg.fy, a.cx = ctx->cfg.cx, a.cy = ctx->cfg.cy;
-  a.flags = (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR;
+  LinearizeArgs& a = s->a = linearize_args(ctx, in, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR);
   st.in(in->poses, (size_t)W * P * 7, &a.poses);
   st.in(in->ex_pose, (size_t)W * 7, &a.ex_pose);
   st.in(in->inv_depth, (size_t)W * F, &a.inv_depth);
   st.in(in->pf_window_offset, (size_t)W + 1, &a.pf_window_offset);
   st.in(in->pf_idx, (size_t)NP, &a.pf_idx);
-  s->obs_table = !in->pf_obs && NP > 0;   // observations as a per-feature table (viml.h): expanded on the device
-  s->obs_f32 = s->obs_table && !(in->feat_obs && in->pf_obs_j);
-  if (s->obs_f32) {
-    st.in(in->feat_obs_f32, (size_t)W * F * 2, &s->fobs32);
-    st.in(in->pf_obs_j_f32, (size_t)NP * 2, &s->obsj32);
-  } else if (s->obs_table) {
-    st.in(in->feat_obs, (size_t)W * F * 2, &s->fobs);
-    st.in(in->pf_obs_j, (size_t)NP * 2, &s->obsj);
+  if (form.obs_table) {
+    st.in((const char*)form.feat_obs, (size_t)W * F * form.obs_bytes, &s->fobs);
+    st.in((const char*)form.pf_obs_j, (size_t)NP * form.obs_bytes, &s->obsj);
   } else {
     st.in(in->pf_obs, (size_t)NP * 4, &a.pf_obs);
   }
   st.in(in->pf_pts_i_z, in->pf_pts_i_z ? (size_t)NP : 0, &a.pf_pts_i_z);
   st.in(in->lf_window_offset, NL > 0 ? (size_t)W + 1 : 0, &a.lf_window_offset);
   st.in(in->lf_frame, (size_t)NL, &a.lf_frame);
-  s->line_table = NL > 0 && !in->lf_geom;   // line factors as (map line, 2D segment): expanded on the device
-  if (s->line_table) {
-    if (!dev)
-      for (int64_t k = 0; k < NL; ++k)
-        if (in->lf_map_index[k] < 0 || in->lf_map_index[k] >= ctx->n_map) return fail(ctx, VIML_ERR_INVALID, "line factor: map index outside the map");
+  if (form.line_table) {
     st.in(in->lf_map_index, (size_t)NL, &s->lidx);
     st.in(in->lf_seg2d_f32, (size_t)NL * 4, &s->lseg);
   } else {
@@ -306,8 +283,8 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const vim
   }
   // scratch (host == nullptr) and outputs
   st.out((double*)nullptr, (size_t)W * (P * kPoseCache + kExCache), &a.cache);
-  if (s->obs_table) st.out((double*)nullptr, (size_t)NP * 4, &s->obs);
-  if (s->line_table) st.out((double*)nullptr, (size_t)NL * 9, &s->geom);
+  if (form.obs_table) st.out((double*)nullptr, (size_t)NP * 4, &s->obs);
+  if (form.line_table) st.out((double*)nullptr, (size_t)NL * 9, &s->geom);
   st.out((double*)nullptr, (size_t)W * D * D, &a.out.H_pp);
   st.out((double*)nullptr, (size_t)W * F * D, &a.out.H_lp);
   st.out((double*)nullptr, (size_t)W * F, &a.out.H_ll);
@@ -331,13 +308,12 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const vim
 
 // The observation and line tables of the batch, expanded into the per-factor arrays every step reads (after st.commit()).
 int expand_tables(viml_ctx* ctx, StepPlan& s) {
-  if (s.obs_table) {
+  if (s.form.obs_table) {
     s.a.pf_obs = s.obs;
-    const int rc = s.obs_f32 ? viml_launch_expand_obs(ctx, s.a, s.fobs32, s.obsj32, true)
-                             : viml_launch_expand_obs(ctx, s.a, s.fobs, s.obsj, false);
+    const int rc = viml_launch_expand_obs(ctx, s.a, s.fobs, s.obsj, s.form.obs_f32);
     if (rc != VIML_OK) return rc;
   }
-  if (s.line_table) {
+  if (s.form.line_table) {
     s.a.lf_geom = s.geom;
     return viml_launch_expand_lines(ctx, s.a, s.lidx, s.lseg);
   }
@@ -404,15 +380,18 @@ int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* 
   return rc;
 }
 
-// Checks shared by viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi: the batch, and with `vi` the inertial
-// factors and the extra state.
+// Checks shared by viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi: the batch (*form: how it carries its
+// observations and line factors), and with `vi` the inertial factors and the extra state.
 int check_step_inputs(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
-                      uint32_t flags, const viml_inertial_factors* vi, const char* who) {
-  int rc = check_batch(ctx, in);
+                      uint32_t flags, const viml_inertial_factors* vi, const char* who, BatchForm* form) {
+  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
+  int rc = check_window_batch(ctx, in, dev, form);
+  if (rc == VIML_OK && !dev && in->n_windows > 0)
+    rc = check_batch_indices(ctx, in, *form, 0, in->n_point_factors, 0, in->n_line_factors);
   if (rc != VIML_OK) return rc;
   const int P = in->poses_per_window, D = 6 * (P + 1);
   if (vi) {
-    rc = check_inertial(ctx, vi, in->n_windows, P, (flags & VIML_PTRS_DEVICE) != 0);
+    rc = check_inertial(ctx, vi, in->n_windows, P, dev);
     if (rc != VIML_OK) return rc;
     if (vi->extra_dim > 0 && !extra_state) {
       ctx->err = std::string(who) + ": extra_dim > 0 needs extra_state";
@@ -430,7 +409,8 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
         const viml_gn_options* opt, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags,
         const viml_inertial_factors* vi = nullptr) {
   if (vi) dense = nullptr;
-  int rc = check_step_inputs(ctx, in, dense, extra_state, flags, vi, "viml_gn_step_vi");
+  BatchForm form;
+  int rc = check_step_inputs(ctx, in, dense, extra_state, flags, vi, "viml_gn_step_vi", &form);
   if (rc != VIML_OK) return rc;
   const int W = in->n_windows, F = in->feats_per_window, X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0;
   const bool step = gout != nullptr;
@@ -442,7 +422,7 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
   Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
   StepPlan s;
-  rc = stage_step(ctx, st, in, dense, extra_state, rout, gout, flags, vi, &s);
+  rc = stage_step(ctx, st, in, form, dense, extra_state, rout, gout, flags, vi, &s);
   if (rc == VIML_OK) rc = st.commit();
   if (rc == VIML_OK) rc = expand_tables(ctx, s);
   if (rc == VIML_OK) rc = enqueue_step(ctx, s, opt ? opt->lambda : 0.0, nullptr, nullptr);
@@ -519,7 +499,8 @@ int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertia
   if (!ctx) return VIML_ERR_INVALID;
   if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
   if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
-  int rc = check_step_inputs(ctx, in, nullptr, extra_state, flags, vi, "viml_solve_vi");
+  BatchForm form;
+  int rc = check_step_inputs(ctx, in, nullptr, extra_state, flags, vi, "viml_solve_vi", &form);
   if (rc == VIML_OK) rc = check_solve_options(ctx, opt);
   if (rc != VIML_OK) return rc;
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, X = vi->extra_dim, M = opt->max_iterations;
@@ -532,7 +513,7 @@ int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertia
   Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
   StepPlan s;
   const viml_gn_out scratch{};   // x+, dx, cost and solved of every round stay on the device
-  rc = stage_step(ctx, st, in, nullptr, extra_state, nullptr, &scratch, flags, vi, &s);
+  rc = stage_step(ctx, st, in, form, nullptr, extra_state, nullptr, &scratch, flags, vi, &s);
   if (rc != VIML_OK) return rc;
   SolveArgs sa{};
   sa.opt = *opt;

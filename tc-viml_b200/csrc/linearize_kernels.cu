@@ -48,7 +48,7 @@ __global__ void expand_obs_kernel(LinearizeArgs a, const T2* __restrict__ feat_o
   for (int k = k0 + threadIdx.x; k < k1; k += blockDim.x) {
     const uint32_t feat = a.pf_idx[k] >> 16;
     const T2 pj = pf_obs_j[k];
-    double pix = 0.0, piy = 0.0;   // a bad index is dropped later, by the kernels
+    double pix = 0.0, piy = 0.0;   // never read out of range; valid indices are the caller's to keep (viml.h, viml_window_batch)
     if (feat < (uint32_t)a.F) pix = (double)fo[feat].x, piy = (double)fo[feat].y;
     dst[k] = make_double4(pix, piy, (double)pj.x, (double)pj.y);
   }

@@ -6,7 +6,6 @@
 #include <cstdlib>
 #include <algorithm>
 #include <cstring>
-#include <ctime>
 #include <numeric>
 #include <vector>
 
@@ -316,33 +315,87 @@ int viml_set_map(viml_ctx* ctx, const double* lines, int64_t n) {
   return VIML_OK;
 }
 
+}  // extern "C"
+
 // ---- linearisation -----------------------------------------------------------------------------
-int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_linearize_out* out, uint32_t flags) {
-  if (!ctx) return VIML_ERR_INVALID;
-  if (!in || !out) return fail(ctx, VIML_ERR_INVALID, "null batch or output struct");
+int check_window_batch(viml_ctx* ctx, const viml_window_batch* in, bool dev, BatchForm* form) {
+  *form = BatchForm{};
+  if (!in) return fail(ctx, VIML_ERR_INVALID, "null window batch");
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window;
   const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
   if (W < 0 || P < 1 || P > 255 || F < 0 || F > 65535 || NP < 0 || NL < 0)
     return fail(ctx, VIML_ERR_INVALID, "window batch sizes out of range");
+  if (W == 0) return VIML_OK;
+  const bool f64_table = in->feat_obs && in->pf_obs_j, f32_table = in->feat_obs_f32 && in->pf_obs_j_f32;
+  form->obs_table = NP > 0 && !in->pf_obs && (f64_table || f32_table);
+  form->obs_f32 = form->obs_table && !f64_table;
+  form->feat_obs = !form->obs_table ? nullptr : form->obs_f32 ? (const void*)in->feat_obs_f32 : (const void*)in->feat_obs;
+  form->pf_obs_j = !form->obs_table ? nullptr : form->obs_f32 ? (const void*)in->pf_obs_j_f32 : (const void*)in->pf_obs_j;
+  form->obs_bytes = form->obs_f32 ? 8 : 16;
+  form->line_table = NL > 0 && !in->lf_geom && in->lf_map_index && in->lf_seg2d_f32;
+  if (!in->poses || !in->ex_pose || (F > 0 && !in->inv_depth) || !in->pf_window_offset ||
+      (NP > 0 && (!in->pf_idx || (!in->pf_obs && !form->obs_table))) ||
+      (NL > 0 && (!in->lf_window_offset || !in->lf_frame || (!in->lf_geom && !form->line_table))))
+    return fail(ctx, VIML_ERR_INVALID, "null input array");
+  if (form->line_table && (!ctx->map_set || ctx->n_map <= 0))
+    return fail(ctx, VIML_ERR_NOMAP, "line factors given by map index need a map (viml_set_map)");
+  if (dev) return VIML_OK;   // device pointers cannot be read here: their offsets and indices are the caller's to keep (viml.h)
+  const int32_t* po = in->pf_window_offset;
+  bool ok = po[0] == 0 && po[W] == NP;
+  for (int w = 0; w < W && ok; ++w) ok = po[w] <= po[w + 1];
+  if (NL > 0) {
+    const int32_t* lo = in->lf_window_offset;
+    ok = ok && lo[0] == 0 && lo[W] == NL;
+    for (int w = 0; w < W && ok; ++w) ok = lo[w] <= lo[w + 1];
+  }
+  if (!ok) return fail(ctx, VIML_ERR_INVALID, "window offsets are not a CSR of the factor arrays (offset[0] == 0, non-decreasing, offset[W] == n_factors)");
+  return VIML_OK;
+}
+
+int check_batch_indices(viml_ctx* ctx, const viml_window_batch* in, const BatchForm& form, int64_t pa, int64_t pb, int64_t la,
+                        int64_t lb) {
+  uint32_t bad = 0;
+  const uint32_t uP = (uint32_t)in->poses_per_window, uF = (uint32_t)in->feats_per_window;
+  for (int64_t k = pa; k < pb; ++k) {
+    const uint32_t ix = in->pf_idx[k];
+    bad |= (uint32_t)((ix & 0xffu) >= uP) | (uint32_t)(((ix >> 8) & 0xffu) >= uP) | (uint32_t)((ix >> 16) >= uF);
+  }
+  for (int64_t k = la; k < lb; ++k) bad |= (uint32_t)((uint32_t)in->lf_frame[k] >= uP);
+  if (form.line_table)
+    for (int64_t k = la; k < lb; ++k) bad |= (uint32_t)((uint64_t)(int64_t)in->lf_map_index[k] >= (uint64_t)ctx->n_map);
+  if (bad) return fail(ctx, VIML_ERR_INVALID, "factor index out of range (pose index >= poses_per_window, feature >= feats_per_window, line frame >= poses_per_window or map index outside the map)");
+  return VIML_OK;
+}
+
+LinearizeArgs linearize_args(const viml_ctx* ctx, const viml_window_batch* in, uint32_t flags) {
+  LinearizeArgs a{};
+  a.W = in->n_windows, a.P = in->poses_per_window, a.F = in->feats_per_window, a.D = 6 * (a.P + 1);
+  a.NP = in->n_point_factors, a.NL = in->n_line_factors;
+  a.pf_begin = 0, a.lf_begin = 0, a.NL_stride = a.NL;
+  a.sqrt_info = ctx->cfg.sqrt_info, a.cauchy_a = ctx->cfg.cauchy_a;
+  a.inv_cauchy_a2 = 1.0 / (ctx->cfg.cauchy_a * ctx->cfg.cauchy_a);
+  a.fx = ctx->cfg.fx, a.fy = ctx->cfg.fy, a.cx = ctx->cfg.cx, a.cy = ctx->cfg.cy;
+  a.flags = flags;
+  return a;
+}
+
+extern "C" {
+
+int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_linearize_out* out, uint32_t flags) {
+  if (!ctx) return VIML_ERR_INVALID;
+  if (!in || !out) return fail(ctx, VIML_ERR_INVALID, "null batch or output struct");
+  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
+  BatchForm form;
+  int rc = check_window_batch(ctx, in, dev, &form);
+  if (rc != VIML_OK) return rc;
   if (!(flags & (VIML_OUT_RESIDUAL_JACOBIAN | VIML_OUT_HB | VIML_OUT_SCHUR)))
     return fail(ctx, VIML_ERR_INVALID, "no output mode requested");
+  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
+  const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
   if (W == 0) return VIML_OK;
-  const bool obs_f32 = !in->pf_obs && !(in->feat_obs && in->pf_obs_j) && in->feat_obs_f32 && in->pf_obs_j_f32;
-  const bool obs_table = !in->pf_obs && ((in->feat_obs && in->pf_obs_j) || obs_f32);   // observations as a per-feature table
-  const void* h_fobs = obs_f32 ? (const void*)in->feat_obs_f32 : (const void*)in->feat_obs;
-  const void* h_obsj = obs_f32 ? (const void*)in->pf_obs_j_f32 : (const void*)in->pf_obs_j;
-  const size_t ob = obs_f32 ? 8 : 16;   // bytes of one {x, y}
-  const bool line_table = NL > 0 && !in->lf_geom && in->lf_map_index && in->lf_seg2d_f32;   // line factors as (map line, 2D segment)
-  if (!in->poses || !in->ex_pose || (F > 0 && !in->inv_depth) || !in->pf_window_offset ||
-      (NP > 0 && (!in->pf_idx || (!in->pf_obs && !obs_table))) ||
-      (NL > 0 && (!in->lf_window_offset || !in->lf_frame || (!in->lf_geom && !line_table))))
-    return fail(ctx, VIML_ERR_INVALID, "null input array");
-  if (line_table && (!ctx->map_set || ctx->n_map <= 0))
-    return fail(ctx, VIML_ERR_NOMAP, "line factors given by map index need a map (viml_set_map)");
-  const int D = 6 * (P + 1);
-  timespec ts_begin;
-  clock_gettime(CLOCK_MONOTONIC, &ts_begin);
-  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
+  const bool obs_table = form.obs_table, obs_f32 = form.obs_f32, line_table = form.line_table;
+  const void *h_fobs = form.feat_obs, *h_obsj = form.pf_obs_j;
+  const size_t ob = form.obs_bytes;
   const bool wantA = (flags & VIML_OUT_RESIDUAL_JACOBIAN) != 0;
   const bool wantHB = (flags & VIML_OUT_HB) != 0, wantS = (flags & VIML_OUT_SCHUR) != 0;
   if (wantHB && !(out->H_pp && out->H_lp && out->H_ll && out->b_p && out->b_l))
@@ -351,13 +404,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
 
-  LinearizeArgs a{};
-  a.W = W, a.P = P, a.F = F, a.D = D, a.NP = NP, a.NL = NL;
-  a.pf_begin = 0, a.lf_begin = 0, a.NL_stride = NL;
-  a.sqrt_info = ctx->cfg.sqrt_info, a.cauchy_a = ctx->cfg.cauchy_a;
-  a.inv_cauchy_a2 = 1.0 / (ctx->cfg.cauchy_a * ctx->cfg.cauchy_a);
-  a.fx = ctx->cfg.fx, a.fy = ctx->cfg.fy, a.cx = ctx->cfg.cx, a.cy = ctx->cfg.cy;
-  a.flags = flags;
+  LinearizeArgs a = linearize_args(ctx, in, flags);
 
   const size_t n_pose = (size_t)W * P * 7, n_ex = (size_t)W * 7, n_dep = (size_t)W * F;
   const size_t szHpp = (size_t)W * D * D, szHlp = (size_t)W * F * D, szF = (size_t)W * F, szD = (size_t)W * D;
@@ -377,16 +424,16 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     a.pf_pts_i_z = in->pf_pts_i_z;
     a.lf_window_offset = in->lf_window_offset, a.lf_frame = in->lf_frame, a.lf_geom = in->lf_geom;
     a.out = *out;
-    if ((obs_table && NP > 0) || line_table) {
+    if (obs_table || line_table) {
       VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(DeviceArena::padded((size_t)NP * 32) + DeviceArena::padded((size_t)NL * 72)));
-      if (obs_table && NP > 0) {
+      if (obs_table) {
         a.pf_obs = ctx->in_arena.take<double>((size_t)NP * 4);
-        const int rc = viml_launch_expand_obs(ctx, a, h_fobs, h_obsj, obs_f32);
+        rc = viml_launch_expand_obs(ctx, a, h_fobs, h_obsj, obs_f32);
         if (rc != VIML_OK) return rc;
       }
       if (line_table) {
         a.lf_geom = ctx->in_arena.take<double>((size_t)NL * 9);
-        const int rc = viml_launch_expand_lines(ctx, a, in->lf_map_index, in->lf_seg2d_f32);
+        rc = viml_launch_expand_lines(ctx, a, in->lf_map_index, in->lf_seg2d_f32);
         if (rc != VIML_OK) return rc;
       }
     }
@@ -402,33 +449,9 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     return viml_launch_linearize(ctx, a);
   }
 
-  // host pointers: the packed indices and CSR offsets are validated before anything is launched (device pointers cannot
-  // be read here; on that path plan_kernel routes windows with bad indices to the generic kernel, which drops them)
-  {
-    const int32_t* po = in->pf_window_offset;
-    bool ok = po[0] == 0 && po[W] == NP;
-    for (int w = 0; w < W && ok; ++w) ok = po[w] <= po[w + 1];
-    if (NL > 0) {
-      const int32_t* lo = in->lf_window_offset;
-      ok = ok && lo[0] == 0 && lo[W] == NL;
-      for (int w = 0; w < W && ok; ++w) ok = lo[w] <= lo[w + 1];
-    }
-    if (!ok) return fail(ctx, VIML_ERR_INVALID, "window offsets are not a CSR of the factor arrays (offset[0] == 0, non-decreasing, offset[W] == n_factors)");
-  }
-  // packed indices: checked chunk by chunk inside the pipeline below (the host runs ahead of the asynchronous copies and
+  // host pointers: check_window_batch has checked the offsets; the packed indices are checked before any kernel reads them, all
+  // at once on the pinned path and chunk by chunk inside the pipeline (the host runs ahead of the asynchronous copies and
   // kernels, so the ~1 ms scan of a 2.3 M-factor batch hides behind the transfers of the previous chunk)
-  auto indices_ok = [&](int64_t pa, int64_t pb, int64_t la, int64_t lb) {
-    uint32_t bad = 0;
-    const uint32_t uP = (uint32_t)P, uF = (uint32_t)F;
-    for (int64_t k = pa; k < pb; ++k) {
-      const uint32_t ix = in->pf_idx[k];
-      bad |= (uint32_t)((ix & 0xffu) >= uP) | (uint32_t)(((ix >> 8) & 0xffu) >= uP) | (uint32_t)((ix >> 16) >= uF);
-    }
-    for (int64_t k = la; k < lb; ++k) bad |= (uint32_t)((uint32_t)in->lf_frame[k] >= uP);
-    if (line_table)
-      for (int64_t k = la; k < lb; ++k) bad |= (uint32_t)((uint64_t)(int64_t)in->lf_map_index[k] >= (uint64_t)ctx->n_map);
-    return bad == 0;
-  };
   // ---- host pointers: chunked pipeline  H2D(c+1) | kernels(c) | D2H(c-1)  on three streams ----
   // Device buffers hold the whole batch at the same absolute positions as the host arrays; a chunk is a range of
   // windows, its kernels run on a "view" (pointers advanced to the first window of the chunk, factor ranges
@@ -494,7 +517,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
   // 5-10 us of driver and DMA set-up whatever its size (more from pageable memory), and this call has ~10 input and up to 14
   // output arrays: the inputs are gathered into ONE pinned block laid out like the device arena and go up in one copy, the
   // outputs come back in one copy and are handed out from the pinned block.
-  if (W < 512 && ctx->in_arena.used + ctx->out_arena.used <= ((size_t)4 << 20) && !getenv("VIML_NO_STAGING")) {
+  if (W < 512 && ctx->in_arena.used + ctx->out_arena.used <= ((size_t)4 << 20)) {
     auto grow = [&](char** buf, size_t* cap, size_t need) -> cudaError_t {
       if (need <= *cap) return cudaSuccess;
       if (*buf) cudaFreeHost(*buf);
@@ -505,8 +528,8 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     };
     VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_in, &ctx->h_stage_in_cap, ctx->in_arena.used));
     VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_out, &ctx->h_stage_out_cap, ctx->out_arena.used));
-    if (!indices_ok(0, NP, 0, NL))
-      return fail(ctx, VIML_ERR_INVALID, "factor index out of range (pose index >= poses_per_window, feature >= feats_per_window, line frame >= poses_per_window or map index outside the map)");
+    rc = check_batch_indices(ctx, in, form, 0, NP, 0, NL);
+    if (rc != VIML_OK) return rc;
     char* const ibase = ctx->in_arena.base;
     auto put = [&](const void* dptr, const void* src, size_t bytes) {
       if (bytes) memcpy(ctx->h_stage_in + ((const char*)dptr - ibase), src, bytes);
@@ -522,7 +545,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
       else put(d_geom, in->lf_geom, (size_t)NL * 72);
     }
     VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ibase, ctx->h_stage_in, ctx->in_arena.used, cudaMemcpyHostToDevice, st));
-    int rc = obs_table ? viml_launch_expand_obs(ctx, a, d_fobs, d_obsj, obs_f32) : VIML_OK;
+    rc = obs_table ? viml_launch_expand_obs(ctx, a, d_fobs, d_obsj, obs_f32) : VIML_OK;
     if (rc == VIML_OK && line_table) rc = viml_launch_expand_lines(ctx, a, d_lidx, d_lseg);
     if (rc == VIML_OK) rc = viml_launch_linearize(ctx, a);
     if (rc != VIML_OK) return rc;
@@ -543,32 +566,12 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
   }
 
   cudaStream_t s_in = ctx->copy_stream, s_out = ctx->copy_stream2;
-  cudaEvent_t tv0 = nullptr;
-  if (getenv("VIML_E2E_TIMING")) {
-    cudaEventCreate(&tv0);
-    cudaEventRecord(tv0, s_in);
-  }
   // offsets first (tiny, needed by every chunk); the previous call's work on `st` is already complete (synchronous API)
   VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_poff, in->pf_window_offset, (size_t)(W + 1) * 4, cudaMemcpyHostToDevice, s_in));
   if (NL > 0) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_loff, in->lf_window_offset, (size_t)(W + 1) * 4, cudaMemcpyHostToDevice, s_in));
-  int nchunk = W >= 512 ? 4 : 1;   // measured on the 4096-window batch with the float32 table (75 MB up, 88 MB down): 2, 3, 4, 5, 6, 8, 12, 16 chunks -> 2.96, 2.81, 2.67, 2.75, 2.70, 2.79, 2.93, 2.96 ms
-  if (const char* e = getenv("VIML_CHUNKS")) nchunk = std::max(1, std::min(W, atoi(e)));   // tuning hook
-  std::vector<int> wt(nchunk, 1);       // relative chunk sizes
-  if (const char* e = getenv("VIML_CHUNK_WEIGHTS")) {   // tuning hook: e.g. "1,2,4,4,5" (also sets the chunk count)
-    std::vector<int> v;
-    for (const char* q = e; *q;) {
-      v.push_back(std::max(1, atoi(q)));
-      while (*q && *q != ',') ++q;
-      if (*q == ',') ++q;
-    }
-    if (!v.empty() && (int)v.size() <= W) wt = v, nchunk = (int)v.size();
-  }
-  std::vector<int> wb(nchunk + 1, 0);
-  {
-    int64_t tot = 0, run = 0;
-    for (int x : wt) tot += x;
-    for (int c = 0; c < nchunk; ++c) run += wt[c], wb[c + 1] = (int)((int64_t)W * run / tot);
-  }
+  const int nchunk = W >= 512 ? 4 : 1;   // measured on the 4096-window batch with the float32 table (75 MB up, 88 MB down): 2, 3, 4, 5, 6, 8, 12, 16 chunks -> 2.96, 2.81, 2.67, 2.75, 2.70, 2.79, 2.93, 2.96 ms
+  std::vector<int> wb(nchunk + 1);
+  for (int c = 0; c <= nchunk; ++c) wb[c] = (int)((int64_t)W * c / nchunk);
   // small per-window arrays: whole batch, one copy each
   VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_poses, in->poses, n_pose * 8, cudaMemcpyHostToDevice, s_in));
   VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_ex, in->ex_pose, n_ex * 8, cudaMemcpyHostToDevice, s_in));
@@ -579,7 +582,6 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     cudaEventCreateWithFlags(&ev_in[c], cudaEventDisableTiming);
     cudaEventCreateWithFlags(&ev_k[c], cudaEventDisableTiming);
   }
-  int rc = VIML_OK;
   auto h2d = [&](void* d, const void* h, size_t bytes) {
     if (bytes) cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s_in);
   };
@@ -613,10 +615,8 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     const int w0 = wb[c], w1 = wb[c + 1], Wc = w1 - w0;
     const int64_t pa = in->pf_window_offset[w0], pb = in->pf_window_offset[w1];
     const int64_t la = NL > 0 ? in->lf_window_offset[w0] : 0, lb = NL > 0 ? in->lf_window_offset[w1] : 0;
-    if (!indices_ok(pa, pb, la, lb)) {   // bad indices never reach a kernel: this chunk and the following ones are not launched
-      rc = fail(ctx, VIML_ERR_INVALID, "factor index out of range (pose index >= poses_per_window, feature >= feats_per_window, line frame >= poses_per_window or map index outside the map)");
-      break;
-    }
+    rc = check_batch_indices(ctx, in, form, pa, pb, la, lb);
+    if (rc != VIML_OK) break;   // bad indices never reach a kernel: this chunk and the following ones are not launched
     cudaStreamWaitEvent(st, ev_in[c], 0);
     // view of windows [w0, w1)
     LinearizeArgs v = a;
@@ -641,27 +641,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
         if (cnt) cudaMemcpyAsync(sl.host + off, *sl.dev + off, cnt * 8, cudaMemcpyDeviceToHost, s_out);
       }
   }
-  const bool e2e_timing = getenv("VIML_E2E_TIMING") != nullptr;
-  timespec ts_q;
-  cudaEvent_t tv[3] = {nullptr, nullptr, nullptr};
-  if (e2e_timing) {
-    clock_gettime(CLOCK_MONOTONIC, &ts_q);
-    for (auto& e : tv) cudaEventCreate(&e);
-    cudaEventRecord(tv[0], s_in), cudaEventRecord(tv[1], st), cudaEventRecord(tv[2], s_out);
-  }
   cudaError_t e1 = cudaStreamSynchronize(s_out), e2 = cudaStreamSynchronize(st), e3 = cudaStreamSynchronize(s_in);
-  if (e2e_timing) {   // diagnosis: how long the host took to queue the pipeline vs how long the device needed to drain it
-    timespec ts_d;
-    clock_gettime(CLOCK_MONOTONIC, &ts_d);
-    float a = 0, b = 0, c2 = 0;
-    cudaEventElapsedTime(&a, tv0, tv[0]), cudaEventElapsedTime(&b, tv0, tv[1]), cudaEventElapsedTime(&c2, tv0, tv[2]);
-    fprintf(stderr, "[viml e2e] device: uploads done %.3f ms, kernels done %.3f ms, downloads done %.3f ms after the first upload was queued\n", a, b, c2);
-    for (auto& e : tv) cudaEventDestroy(e);
-    cudaEventDestroy(tv0);
-    fprintf(stderr, "[viml e2e] queued after %.3f ms, drained after %.3f ms (%d chunks)\n",
-            (ts_q.tv_sec - ts_begin.tv_sec) * 1e3 + (ts_q.tv_nsec - ts_begin.tv_nsec) * 1e-6,
-            (ts_d.tv_sec - ts_begin.tv_sec) * 1e3 + (ts_d.tv_nsec - ts_begin.tv_nsec) * 1e-6, nchunk);
-  }
   for (int c = 0; c < nchunk; ++c) cudaEventDestroy(ev_in[c]), cudaEventDestroy(ev_k[c]);
   if (rc != VIML_OK) return rc;
   VIML_TRY_CUDA(ctx, e1);
@@ -781,8 +761,7 @@ int viml_line_associate(viml_ctx* ctx, const viml_assoc_query* q, const viml_ass
   // back on the second copy stream while chunk c + 1 computes.
   VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(4 * pad((size_t)Pq * 56) + pad(nq * 32) + pad((size_t)Pq * 4)));
   cudaStream_t cs = ctx->copy_stream, ds = ctx->copy_stream2;
-  int C = Pq >= 512 ? 4 : 1;   // measured on the cfg-3 sweep: 2, 4, 6, 8, 12, 16 chunks -> 2.32, 2.19, 2.30, 2.36, 2.79, 2.76 ms
-  if (const char* e = getenv("VIML_ASSOC_CHUNKS")) C = std::max(1, std::min(Pq, atoi(e)));   // tuning hook
+  const int C = Pq >= 512 ? 4 : 1;   // measured on the cfg-3 sweep: 2, 4, 6, 8, 12, 16 chunks -> 2.32, 2.19, 2.30, 2.36, 2.79, 2.76 ms
   auto up = [&](const void* src, size_t bytes) -> void* {
     char* d = ctx->in_arena.take<char>(bytes);
     if (bytes) cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, cs);
