@@ -91,4 +91,15 @@ with pkg.Context(cfg) as c:
     r["gn_step_device_ms"] = wall(step_dev)
     r["gn_step_vi_device_ms"] = wall(step_vi_dev)
     res["step_1024"] = r
+
+    # small host-pointer calls (a live sliding window): latency-bound, one copy each way
+    rng = np.random.default_rng(3)
+    for w in (1, 12):
+        b = synth.make_windows(w, seed=9)
+        vi, extra = synth.make_inertial_factors(b, seed=5)
+        M = rng.standard_normal((w, 98, 90))
+        A, bm = np.einsum("kij,kil->kjl", M, M), rng.standard_normal((w, 90))
+        res[f"host_{w}"] = {"gn_step_vi_ms": wall(lambda: c.gn_step_vi(b, vi, extra, abi.LOSS_CAUCHY, lam=lam), 50),
+                            "solve_vi_10_rounds_ms": wall(lambda: c.solve_vi(b, vi, extra, abi.LOSS_CAUCHY, max_iterations=10), 50),
+                            "marginalize_90_15_ms": wall(lambda: c.marginalize(A, bm, 15), 50)}
 print(json.dumps(res, indent=1))

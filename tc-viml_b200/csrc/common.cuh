@@ -2,8 +2,10 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstdint>
 #include <cstdio>
+#include <cstring>
 #include <string>
 #include <utility>
 #include <vector>
@@ -80,8 +82,8 @@ struct viml_ctx {
   int32_t* d_fov_slot_count = nullptr; // [VIML_FOV_SLOTS]
   int64_t fov_words = 0;
   unsigned long long* d_assoc_stats = nullptr;  // {gate tests, gated pairs, overlap-scored, distance-scored} of the last association call
-  DeviceArena in_arena, out_arena, scratch, scratch2, scratch3, gn_in, gn_out, s_full;
-  // pinned staging of the small-batch host path (one H2D, one D2H per call)
+  DeviceArena in_arena, out_arena, scratch, scratch2, scratch3, s_full;
+  // pinned blocks of Stager's one-copy path (one H2D, one D2H per call)
   char *h_stage_in = nullptr, *h_stage_out = nullptr;
   size_t h_stage_in_cap = 0, h_stage_out_cap = 0;
   void* nccl_lib = nullptr;
@@ -90,6 +92,103 @@ struct viml_ctx {
   bool force_generic = false;  // tests: route everything through the generic atomic kernels
   bool prof = false;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events[VIML_NUM_KERNELS];
+};
+
+inline int fail(viml_ctx* ctx, int code, const char* msg) {
+  if (ctx) ctx->err = msg;
+  return code;
+}
+
+// Host <-> device staging for the synchronous host-pointer flavour of an entry point: in() slots are placed in ctx->in_arena and
+// copied up by commit(), out() slots in ctx->out_arena and copied back by finish(), which synchronises.  An out() with a null host
+// pointer is device scratch.  With host pointers a slot whose count is 0 is null.  With VIML_PTRS_DEVICE the caller's pointers pass
+// through unchanged and only scratch is placed.
+// A host call whose staged bytes total at most kOneCopyBytes goes up in one copy and comes back in one: every cudaMemcpyAsync
+// costs 5-10 us of driver and DMA set-up whatever its size (more from pageable memory), and a step stages some 30 arrays.  The
+// inputs are gathered into the pinned ctx->h_stage_in laid out like in_arena; the device range that holds every output comes back
+// into ctx->h_stage_out and is handed out from there.
+struct Stager {
+  static constexpr size_t kOneCopyBytes = size_t(4) << 20;
+  viml_ctx* ctx;
+  bool dev;
+  struct In { const void* host; size_t bytes; const void** slot; };
+  struct Out { void* host; size_t bytes; void** slot; };
+  std::vector<In> ins;
+  std::vector<Out> outs;
+  Stager(viml_ctx* c, bool d) : ctx(c), dev(d) {   // room for the arrays of any call: no reallocation while staging
+    ins.reserve(32);
+    outs.reserve(32);
+  }
+  template <class T>
+  void in(const T* host, size_t count, const T** slot) {
+    *slot = dev ? host : nullptr;
+    if (!dev && host && count) ins.push_back({host, count * sizeof(T), reinterpret_cast<const void**>(slot)});
+  }
+  template <class T>
+  void out(T* host, size_t count, T** slot) {
+    *slot = dev ? host : nullptr;
+    if ((!dev || !host) && count) outs.push_back({dev ? nullptr : host, count * sizeof(T), reinterpret_cast<void**>(slot)});
+  }
+  size_t in_bytes() const {
+    size_t b = 0;
+    for (auto& e : ins) b += DeviceArena::padded(e.bytes);
+    return b;
+  }
+  size_t out_bytes() const {
+    size_t b = 0;
+    for (auto& e : outs) b += DeviceArena::padded(e.bytes);
+    return b;
+  }
+  bool one_copy() const { return !dev && in_bytes() + out_bytes() <= kOneCopyBytes; }
+  // a pinned block of the one-copy path: grown, never shrunk
+  static cudaError_t grow(char** buf, size_t* cap, size_t need) {
+    if (need <= *cap) return cudaSuccess;
+    if (*buf) cudaFreeHost(*buf);
+    *buf = nullptr, *cap = 0;
+    const cudaError_t e = cudaHostAlloc((void**)buf, need + need / 2 + 4096, cudaHostAllocDefault);
+    if (e == cudaSuccess) *cap = need + need / 2 + 4096;
+    return e;
+  }
+  int commit() {
+    const size_t ib = in_bytes(), ob = out_bytes();
+    const bool one = one_copy();
+    VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(ib));
+    VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(ob));
+    if (one) {
+      VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_in, &ctx->h_stage_in_cap, ib));
+      VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_out, &ctx->h_stage_out_cap, ob));
+    }
+    for (auto& e : ins) {
+      char* d = ctx->in_arena.take<char>(e.bytes);
+      if (one) memcpy(ctx->h_stage_in + (d - ctx->in_arena.base), e.host, e.bytes);
+      else VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d, e.host, e.bytes, cudaMemcpyHostToDevice, ctx->stream));
+      *e.slot = d;
+    }
+    if (one && ib) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ctx->in_arena.base, ctx->h_stage_in, ib, cudaMemcpyHostToDevice, ctx->stream));
+    for (auto& e : outs) *e.slot = ctx->out_arena.take<char>(e.bytes);
+    return VIML_OK;
+  }
+  int finish() {
+    if (dev) return VIML_OK;
+    if (one_copy()) {
+      char *lo = nullptr, *hi = nullptr;
+      for (auto& e : outs)
+        if (e.host) {
+          char* b = (char*)*e.slot;
+          lo = lo ? std::min(lo, b) : b, hi = hi ? std::max(hi, b + e.bytes) : b + e.bytes;
+        }
+      if (lo) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ctx->h_stage_out, lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, ctx->stream));
+      VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+      for (auto& e : outs)
+        if (e.host) memcpy(e.host, ctx->h_stage_out + ((char*)*e.slot - lo), e.bytes);
+    } else {
+      for (auto& e : outs)
+        if (e.host) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(e.host, *e.slot, e.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+      VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    VIML_TRY_CUDA(ctx, cudaGetLastError());
+    return VIML_OK;
+  }
 };
 
 enum KernelId {
@@ -169,6 +268,22 @@ int check_batch_indices(viml_ctx* ctx, const viml_window_batch* in, const BatchF
                         int64_t lb);
 // The LinearizeArgs of the whole batch with the context's camera and loss constants; the pointers are left null.
 LinearizeArgs linearize_args(const viml_ctx* ctx, const viml_window_batch* in, uint32_t flags);
+// A viml_window_batch staged for the device: its arrays in `a` (outputs left to the caller), and the observation / line tables
+// with the scratch they are expanded into.
+struct StagedBatch {
+  LinearizeArgs a;
+  BatchForm form;
+  const char *fobs, *obsj;
+  const float* lseg;
+  const int32_t* lidx;
+  double *obs, *geom;   // their expansions
+};
+// Stages the batch (checked by check_window_batch, which gave `form`) into `st`: the inputs of linearize_args(ctx, in, flags), the
+// table sources, the expansion targets and the pose cache.  The Stager keeps the addresses of *b's fields; after st.commit() the
+// caller calls expand_tables().
+void stage_batch(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const BatchForm& form, uint32_t flags, StagedBatch* b);
+// The observation and line tables of the batch, expanded into the per-factor arrays every kernel reads.
+int expand_tables(viml_ctx* ctx, StagedBatch& b);
 
 // Largest reduced system a Gauss-Newton step takes, Dx = D + extra_dim (viml.h): its tiled Cholesky keeps the lower triangle in
 // shared memory (linearize_kernels.cu checks the size at compile time).

@@ -13,54 +13,6 @@
 
 namespace {
 
-int fail(viml_ctx* ctx, int code, const char* msg) {
-  if (ctx) ctx->err = msg;
-  return code;
-}
-
-// Host <-> device staging for the synchronous host-pointer flavour of an entry point: inputs are copied into one arena,
-// outputs live in another and are copied back by finish().  With VIML_PTRS_DEVICE the caller's pointers pass through.
-struct Stager {
-  viml_ctx* ctx;
-  bool dev;
-  struct In { const void* host; size_t bytes; const void** slot; };
-  struct Out { void* host; size_t bytes; void** slot; };
-  std::vector<In> ins;
-  std::vector<Out> outs;
-  template <class T>
-  void in(const T* host, size_t count, const T** slot) {
-    *slot = host;
-    if (!dev && host && count) ins.push_back({host, count * sizeof(T), reinterpret_cast<const void**>(slot)});
-  }
-  // an output (or scratch when host == nullptr / device mode without a caller buffer)
-  template <class T>
-  void out(T* host, size_t count, T** slot) {
-    *slot = host;
-    if ((!dev || !host) && count) outs.push_back({dev ? nullptr : host, count * sizeof(T), reinterpret_cast<void**>(slot)});
-  }
-  int commit() {
-    size_t ib = 0, ob = 0;
-    for (auto& e : ins) ib += DeviceArena::padded(e.bytes);
-    for (auto& e : outs) ob += DeviceArena::padded(e.bytes);
-    VIML_TRY_CUDA(ctx, ctx->gn_in.reserve(ib));
-    VIML_TRY_CUDA(ctx, ctx->gn_out.reserve(ob));
-    for (auto& e : ins) {
-      char* d = ctx->gn_in.take<char>(e.bytes);
-      VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d, e.host, e.bytes, cudaMemcpyHostToDevice, ctx->stream));
-      *e.slot = d;
-    }
-    for (auto& e : outs) *e.slot = ctx->gn_out.take<char>(e.bytes);
-    return VIML_OK;
-  }
-  int finish() {
-    if (dev) return VIML_OK;
-    for (auto& e : outs)
-      if (e.host) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(e.host, *e.slot, e.bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    return VIML_OK;
-  }
-};
-
 // viml_inertial_factors: null checks always, index / size validation on the host-pointer path (the device path reads nothing back).
 int check_inertial(viml_ctx* ctx, const viml_inertial_factors* vi, int W, int P, bool dev) {
   if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
@@ -218,11 +170,11 @@ int stage_dense(viml_ctx* ctx, Stager& st, const viml_dense_factors* dense, int 
 }
 
 // Everything one Gauss-Newton step enqueues (device pointers), staged once: viml_gn_step / viml_gn_step_vi enqueue one step,
-// viml_solve_vi one per round.  The state the step starts from is a.poses, a.ex_pose, a.inv_depth and extra; x+ goes to o_*.
+// viml_solve_vi one per round.  The state the step starts from is b.a.poses, b.a.ex_pose, b.a.inv_depth and extra; x+ goes to o_*.
 struct StepPlan {
   int W, X, Dx;
   bool vi, want_sx;   // the dense-block factors are the IMU / prior factors; the caller asked for Sx or gx
-  LinearizeArgs a;
+  StagedBatch b;      // the window batch and its observation / line tables
   DenseArgs dn;
   InertialArgs va;
   InertialCsr csr;
@@ -231,12 +183,6 @@ struct StepPlan {
   double *Sx, *gx, *dx, *cost;
   int32_t* solved;
   double *o_poses, *o_ex, *o_dep, *o_extra;
-  // observation / line tables expanded on the device once (viml.h, viml_window_batch)
-  BatchForm form;
-  const char *fobs, *obsj;
-  const float* lseg;
-  const int32_t* lidx;
-  double *obs, *geom;   // their expansions
 };
 
 // Stages the inputs of viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi (checked by check_step_inputs, which
@@ -246,45 +192,21 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
                const double* extra_state, const viml_reduced_out* rout, const viml_gn_out* gout, uint32_t flags,
                const viml_inertial_factors* vi, StepPlan* s) {
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
-  const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
   *s = StepPlan{};
   s->W = W, s->X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, s->Dx = D + s->X;
   s->vi = vi != nullptr, s->want_sx = rout && (rout->Sx || rout->gx);
-  s->form = form;
   const int X = s->X, Dx = s->Dx;
   s->dn.X = X;
   int rc = stage_dense(ctx, st, dense, W, Dx, &s->dn);
   if (rc != VIML_OK) return rc;
-  LinearizeArgs& a = s->a = linearize_args(ctx, in, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR);
-  st.in(in->poses, (size_t)W * P * 7, &a.poses);
-  st.in(in->ex_pose, (size_t)W * 7, &a.ex_pose);
-  st.in(in->inv_depth, (size_t)W * F, &a.inv_depth);
-  st.in(in->pf_window_offset, (size_t)W + 1, &a.pf_window_offset);
-  st.in(in->pf_idx, (size_t)NP, &a.pf_idx);
-  if (form.obs_table) {
-    st.in((const char*)form.feat_obs, (size_t)W * F * form.obs_bytes, &s->fobs);
-    st.in((const char*)form.pf_obs_j, (size_t)NP * form.obs_bytes, &s->obsj);
-  } else {
-    st.in(in->pf_obs, (size_t)NP * 4, &a.pf_obs);
-  }
-  st.in(in->pf_pts_i_z, in->pf_pts_i_z ? (size_t)NP : 0, &a.pf_pts_i_z);
-  st.in(in->lf_window_offset, NL > 0 ? (size_t)W + 1 : 0, &a.lf_window_offset);
-  st.in(in->lf_frame, (size_t)NL, &a.lf_frame);
-  if (form.line_table) {
-    st.in(in->lf_map_index, (size_t)NL, &s->lidx);
-    st.in(in->lf_seg2d_f32, (size_t)NL * 4, &s->lseg);
-  } else {
-    st.in(in->lf_geom, (size_t)NL * 9, &a.lf_geom);
-  }
+  stage_batch(ctx, st, in, form, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR, &s->b);
+  LinearizeArgs& a = s->b.a;
   st.in(extra_state, extra_state ? (size_t)W * X : 0, &s->extra);
   if (vi) {
     stage_inertial(st, vi, W, P, &s->va);
     stage_inertial_csr(st, s->va, &s->csr, &s->res_plus);
   }
   // scratch (host == nullptr) and outputs
-  st.out((double*)nullptr, (size_t)W * (P * kPoseCache + kExCache), &a.cache);
-  if (form.obs_table) st.out((double*)nullptr, (size_t)NP * 4, &s->obs);
-  if (form.line_table) st.out((double*)nullptr, (size_t)NL * 9, &s->geom);
   st.out((double*)nullptr, (size_t)W * D * D, &a.out.H_pp);
   st.out((double*)nullptr, (size_t)W * F * D, &a.out.H_lp);
   st.out((double*)nullptr, (size_t)W * F, &a.out.H_ll);
@@ -306,26 +228,12 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
   return VIML_OK;
 }
 
-// The observation and line tables of the batch, expanded into the per-factor arrays every step reads (after st.commit()).
-int expand_tables(viml_ctx* ctx, StepPlan& s) {
-  if (s.form.obs_table) {
-    s.a.pf_obs = s.obs;
-    const int rc = viml_launch_expand_obs(ctx, s.a, s.fobs, s.obsj, s.form.obs_f32);
-    if (rc != VIML_OK) return rc;
-  }
-  if (s.form.line_table) {
-    s.a.lf_geom = s.geom;
-    return viml_launch_expand_lines(ctx, s.a, s.lidx, s.lseg);
-  }
-  return VIML_OK;
-}
-
-// One step at the state of s.a / s.extra: the reduced system (Sx, gx when the caller asked for them) and, with s.cost set, the
+// One step at the state of s.b.a / s.extra: the reduced system (Sx, gx when the caller asked for them) and, with s.cost set, the
 // solve, the update into s.o_* and the costs.  lambda_w / running: see viml_launch_gn_reduced_solve (nullptr: `lambda`, every window).
 // With s.vi the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at
 // x+ (cost[1], exactly); s.dn is then replaced by their CSR.
 int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* lambda_w, const int32_t* running) {
-  const LinearizeArgs& a = s.a;
+  const LinearizeArgs& a = s.b.a;
   const int W = s.W, D = a.D, X = s.X, Dx = s.Dx;
   const bool step = s.cost != nullptr;
   int rc = viml_launch_linearize(ctx, a);
@@ -424,7 +332,7 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   StepPlan s;
   rc = stage_step(ctx, st, in, form, dense, extra_state, rout, gout, flags, vi, &s);
   if (rc == VIML_OK) rc = st.commit();
-  if (rc == VIML_OK) rc = expand_tables(ctx, s);
+  if (rc == VIML_OK) rc = expand_tables(ctx, s.b);
   if (rc == VIML_OK) rc = enqueue_step(ctx, s, opt ? opt->lambda : 0.0, nullptr, nullptr);
   if (rc != VIML_OK) return rc;
   return st.finish();
@@ -536,15 +444,15 @@ int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertia
   st.out(out->radius, out->radius ? (size_t)W : 0, &sa.out.radius);
   st.out(out->trace, out->trace ? (size_t)W * M * 4 : 0, &sa.out.trace);
   rc = st.commit();
-  if (rc == VIML_OK) rc = expand_tables(ctx, s);
+  if (rc == VIML_OK) rc = expand_tables(ctx, s.b);
   if (rc != VIML_OK) return rc;
   // the rounds work on a copy of the initial state: the inputs stay untouched
   const size_t n_pose = (size_t)W * P * 7, n_ex = (size_t)W * 7, n_dep = (size_t)W * F, n_extra = (size_t)W * X;
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_poses, s.a.poses, n_pose * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_ex, s.a.ex_pose, n_ex * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-  if (n_dep) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_dep, s.a.inv_depth, n_dep * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_poses, s.b.a.poses, n_pose * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_ex, s.b.a.ex_pose, n_ex * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (n_dep) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_dep, s.b.a.inv_depth, n_dep * 8, cudaMemcpyDeviceToDevice, ctx->stream));
   if (n_extra) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(sa.x_extra, s.extra, n_extra * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-  s.a.poses = sa.x_poses, s.a.ex_pose = sa.x_ex, s.a.inv_depth = sa.x_dep, s.extra = sa.x_extra;
+  s.b.a.poses = sa.x_poses, s.b.a.ex_pose = sa.x_ex, s.b.a.inv_depth = sa.x_dep, s.extra = sa.x_extra;
   sa.p_poses = s.o_poses, sa.p_ex = s.o_ex, sa.p_dep = s.o_dep, sa.p_extra = s.o_extra;
   sa.dx = s.dx, sa.cost = s.cost, sa.solved = s.solved;
   // round 0 runs every window at lambda = 1 / initial_radius; policy_kernel then starts each window's state from that step and

@@ -34,11 +34,6 @@ double cos_threshold(double angle_th) {
   return r;
 }
 
-int fail(viml_ctx* ctx, int code, const char* msg) {
-  if (ctx) ctx->err = msg;
-  return code;
-}
-
 }  // namespace
 
 static void drop_prof_events(viml_ctx* ctx) {
@@ -99,8 +94,6 @@ void viml_destroy(viml_ctx* ctx) {
   ctx->scratch.release();
   ctx->scratch2.release();
   ctx->scratch3.release();
-  ctx->gn_in.release();
-  ctx->gn_out.release();
   ctx->s_full.release();
   if (ctx->d_map) cudaFree(ctx->d_map);
   if (ctx->d_map_sorted) cudaFree(ctx->d_map_sorted);
@@ -379,6 +372,50 @@ LinearizeArgs linearize_args(const viml_ctx* ctx, const viml_window_batch* in, u
   return a;
 }
 
+void stage_batch(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const BatchForm& form, uint32_t flags, StagedBatch* b) {
+  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window;
+  const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
+  *b = StagedBatch{};
+  b->form = form;
+  LinearizeArgs& a = b->a = linearize_args(ctx, in, flags);
+  st.in(in->poses, (size_t)W * P * 7, &a.poses);
+  st.in(in->ex_pose, (size_t)W * 7, &a.ex_pose);
+  st.in(in->inv_depth, (size_t)W * F, &a.inv_depth);
+  st.in(in->pf_window_offset, (size_t)W + 1, &a.pf_window_offset);
+  st.in(in->pf_idx, (size_t)NP, &a.pf_idx);
+  if (form.obs_table) {
+    st.in((const char*)form.feat_obs, (size_t)W * F * form.obs_bytes, &b->fobs);
+    st.in((const char*)form.pf_obs_j, (size_t)NP * form.obs_bytes, &b->obsj);
+  } else {
+    st.in(in->pf_obs, (size_t)NP * 4, &a.pf_obs);
+  }
+  st.in(in->pf_pts_i_z, in->pf_pts_i_z ? (size_t)NP : 0, &a.pf_pts_i_z);
+  st.in(in->lf_window_offset, NL > 0 ? (size_t)W + 1 : 0, &a.lf_window_offset);
+  st.in(in->lf_frame, (size_t)NL, &a.lf_frame);
+  if (form.line_table) {
+    st.in(in->lf_map_index, (size_t)NL, &b->lidx);
+    st.in(in->lf_seg2d_f32, (size_t)NL * 4, &b->lseg);
+  } else {
+    st.in(in->lf_geom, (size_t)NL * 9, &a.lf_geom);
+  }
+  st.out((double*)nullptr, (size_t)W * (P * kPoseCache + kExCache), &a.cache);
+  if (form.obs_table) st.out((double*)nullptr, (size_t)NP * 4, &b->obs);
+  if (form.line_table) st.out((double*)nullptr, (size_t)NL * 9, &b->geom);
+}
+
+int expand_tables(viml_ctx* ctx, StagedBatch& b) {
+  if (b.form.obs_table) {
+    b.a.pf_obs = b.obs;
+    const int rc = viml_launch_expand_obs(ctx, b.a, b.fobs, b.obsj, b.form.obs_f32);
+    if (rc != VIML_OK) return rc;
+  }
+  if (b.form.line_table) {
+    b.a.lf_geom = b.geom;
+    return viml_launch_expand_lines(ctx, b.a, b.lidx, b.lseg);
+  }
+  return VIML_OK;
+}
+
 extern "C" {
 
 int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_linearize_out* out, uint32_t flags) {
@@ -393,69 +430,62 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
   const int64_t NP = in->n_point_factors, NL = in->n_line_factors;
   if (W == 0) return VIML_OK;
-  const bool obs_table = form.obs_table, obs_f32 = form.obs_f32, line_table = form.line_table;
-  const void *h_fobs = form.feat_obs, *h_obsj = form.pf_obs_j;
-  const size_t ob = form.obs_bytes;
   const bool wantA = (flags & VIML_OUT_RESIDUAL_JACOBIAN) != 0;
   const bool wantHB = (flags & VIML_OUT_HB) != 0, wantS = (flags & VIML_OUT_SCHUR) != 0;
   if (wantHB && !(out->H_pp && out->H_lp && out->H_ll && out->b_p && out->b_l))
     return fail(ctx, VIML_ERR_INVALID, "VIML_OUT_HB needs H_pp, H_lp, H_ll, b_p and b_l");
   if (wantS && !(out->S && out->g)) return fail(ctx, VIML_ERR_INVALID, "VIML_OUT_SCHUR needs S and g");
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
-
-  LinearizeArgs a = linearize_args(ctx, in, flags);
-
-  const size_t n_pose = (size_t)W * P * 7, n_ex = (size_t)W * 7, n_dep = (size_t)W * F;
-  const size_t szHpp = (size_t)W * D * D, szHlp = (size_t)W * F * D, szF = (size_t)W * F, szD = (size_t)W * D;
-  // scratch: pose cache (+ H blocks when only the Schur complement is wanted)
-  size_t scratch_bytes = DeviceArena::padded((size_t)W * (P * kPoseCache + kExCache) * sizeof(double)) +
-                         DeviceArena::padded((size_t)W * sizeof(int));
-  const bool scratchH = wantS && (!wantHB || !dev);
-  if (scratchH && dev)
-    scratch_bytes += DeviceArena::padded(szHpp * 8) + DeviceArena::padded(szHlp * 8) + 2 * DeviceArena::padded(szF * 8) +
-                     DeviceArena::padded(szD * 8);
-  VIML_TRY_CUDA(ctx, ctx->scratch.reserve(scratch_bytes));
-  a.cache = ctx->scratch.take<double>((size_t)W * (P * kPoseCache + kExCache));
-
-  if (dev) {
-    a.poses = in->poses, a.ex_pose = in->ex_pose, a.inv_depth = in->inv_depth;
-    a.pf_window_offset = in->pf_window_offset, a.pf_idx = in->pf_idx, a.pf_obs = in->pf_obs;
-    a.pf_pts_i_z = in->pf_pts_i_z;
-    a.lf_window_offset = in->lf_window_offset, a.lf_frame = in->lf_frame, a.lf_geom = in->lf_geom;
-    a.out = *out;
-    if (obs_table || line_table) {
-      VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(DeviceArena::padded((size_t)NP * 32) + DeviceArena::padded((size_t)NL * 72)));
-      if (obs_table) {
-        a.pf_obs = ctx->in_arena.take<double>((size_t)NP * 4);
-        rc = viml_launch_expand_obs(ctx, a, h_fobs, h_obsj, obs_f32);
-        if (rc != VIML_OK) return rc;
-      }
-      if (line_table) {
-        a.lf_geom = ctx->in_arena.take<double>((size_t)NL * 9);
-        rc = viml_launch_expand_lines(ctx, a, in->lf_map_index, in->lf_seg2d_f32);
-        if (rc != VIML_OK) return rc;
-      }
-    }
-    if (!wantA) a.out.pf_residual = a.out.pf_jac_pose_i = a.out.pf_jac_pose_j = a.out.pf_jac_ex = a.out.pf_jac_feat =
-                    a.out.lf_residual = a.out.lf_jac_pose = nullptr;
-    if (wantS && !wantHB) {
-      a.out.H_pp = ctx->scratch.take<double>(szHpp);
-      a.out.H_lp = ctx->scratch.take<double>(szHlp);
-      a.out.H_ll = ctx->scratch.take<double>(szF);
-      a.out.b_l = ctx->scratch.take<double>(szF);
-      a.out.b_p = ctx->scratch.take<double>(szD);
-    }
-    return viml_launch_linearize(ctx, a);
+  Stager st{ctx, dev};
+  StagedBatch b;
+  stage_batch(ctx, st, in, form, flags, &b);
+  viml_linearize_out& o = b.a.out;
+  if (wantA) {
+    auto a_out = [&](double* host, size_t count, double** slot) { st.out(host, host ? count : 0, slot); };
+    a_out(out->pf_residual, (size_t)NP * 2, &o.pf_residual);
+    a_out(out->pf_jac_pose_i, (size_t)NP * 14, &o.pf_jac_pose_i);
+    a_out(out->pf_jac_pose_j, (size_t)NP * 14, &o.pf_jac_pose_j);
+    a_out(out->pf_jac_ex, (size_t)NP * 14, &o.pf_jac_ex);
+    a_out(out->pf_jac_feat, (size_t)NP * 2, &o.pf_jac_feat);
+    a_out(out->lf_residual, (size_t)NL * 2, &o.lf_residual);
+    a_out(out->lf_jac_pose, (size_t)NL * 14, &o.lf_jac_pose);
+  }
+  if (wantHB || wantS) {   // with VIML_OUT_SCHUR alone the H blocks are scratch
+    st.out(wantHB ? out->H_pp : nullptr, (size_t)W * D * D, &o.H_pp);
+    st.out(wantHB ? out->H_lp : nullptr, (size_t)W * F * D, &o.H_lp);
+    st.out(wantHB ? out->H_ll : nullptr, (size_t)W * F, &o.H_ll);
+    st.out(wantHB ? out->b_p : nullptr, (size_t)W * D, &o.b_p);
+    st.out(wantHB ? out->b_l : nullptr, (size_t)W * F, &o.b_l);
+  }
+  if (wantS) {
+    st.out(out->S, (size_t)W * ((flags & VIML_S_PACKED) ? D * (D + 1) / 2 : D * D), &o.S);
+    st.out(out->g, (size_t)W * D, &o.g);
+  }
+  if (dev || (W < 512 && st.one_copy())) {
+    // host pointers: check_window_batch has checked the offsets, the packed indices are checked before any kernel reads them
+    if (!dev) rc = check_batch_indices(ctx, in, form, 0, NP, 0, NL);
+    if (rc == VIML_OK) rc = st.commit();
+    if (rc == VIML_OK) rc = expand_tables(ctx, b);
+    if (rc == VIML_OK) rc = viml_launch_linearize(ctx, b.a);
+    if (rc != VIML_OK) return rc;
+    return st.finish();
   }
 
-  // host pointers: check_window_batch has checked the offsets; the packed indices are checked before any kernel reads them, all
-  // at once on the pinned path and chunk by chunk inside the pipeline (the host runs ahead of the asynchronous copies and
-  // kernels, so the ~1 ms scan of a 2.3 M-factor batch hides behind the transfers of the previous chunk)
-  // ---- host pointers: chunked pipeline  H2D(c+1) | kernels(c) | D2H(c-1)  on three streams ----
-  // Device buffers hold the whole batch at the same absolute positions as the host arrays; a chunk is a range of
-  // windows, its kernels run on a "view" (pointers advanced to the first window of the chunk, factor ranges
-  // absolute).  PCIe is full duplex, so with pinned host memory the call approaches max(H2D, D2H) time.
+  // ---- host pointers, W >= 512 or more than Stager::kOneCopyBytes: chunked pipeline
+  // H2D(c+1) | kernels(c) | D2H(c-1) on three streams.  Device buffers hold the whole batch at the same absolute positions as the
+  // host arrays; a chunk is a range of windows, its kernels run on a "view" (pointers advanced to the first window of the chunk,
+  // factor ranges absolute).  PCIe is full duplex, so with pinned host memory the call approaches max(H2D, D2H) time.
+  // check_window_batch has checked the offsets; the packed indices are checked chunk by chunk before the chunk's kernels (the host
+  // runs ahead of the asynchronous copies and kernels, so the ~1 ms scan of a 2.3 M-factor batch hides behind the transfers of the
+  // previous chunk).
+  const bool obs_table = form.obs_table, obs_f32 = form.obs_f32, line_table = form.line_table;
+  const void *h_fobs = form.feat_obs, *h_obsj = form.pf_obs_j;
+  const size_t ob = form.obs_bytes;
+  cudaStream_t s_k = ctx->stream;
+  LinearizeArgs a = linearize_args(ctx, in, flags);
+  const size_t n_pose = (size_t)W * P * 7, n_ex = (size_t)W * 7, n_dep = (size_t)W * F;
+  VIML_TRY_CUDA(ctx, ctx->scratch.reserve(DeviceArena::padded((size_t)W * (P * kPoseCache + kExCache) * sizeof(double))));
+  a.cache = ctx->scratch.take<double>((size_t)W * (P * kPoseCache + kExCache));
   auto pad = [](size_t b) { return DeviceArena::padded(b); };
   size_t in_bytes = pad(n_pose * 8) + pad(n_ex * 8) + pad(n_dep * 8) + 2 * pad((size_t)(W + 1) * 4);
   in_bytes += pad((size_t)NP * 4) + pad((size_t)NP * 32) + pad((size_t)NP * 8);
@@ -513,60 +543,12 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
   VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(out_bytes));
   for (auto& sl : slots) *sl.dev = ctx->out_arena.take<double>(sl.per_window * W + sl.per_pf * NP + sl.per_lf * NL);
 
-  // ---- small batches (a live sliding window: BASELINE configs[0]): latency, not bandwidth.  Every cudaMemcpyAsync costs
-  // 5-10 us of driver and DMA set-up whatever its size (more from pageable memory), and this call has ~10 input and up to 14
-  // output arrays: the inputs are gathered into ONE pinned block laid out like the device arena and go up in one copy, the
-  // outputs come back in one copy and are handed out from the pinned block.
-  if (W < 512 && ctx->in_arena.used + ctx->out_arena.used <= ((size_t)4 << 20)) {
-    auto grow = [&](char** buf, size_t* cap, size_t need) -> cudaError_t {
-      if (need <= *cap) return cudaSuccess;
-      if (*buf) cudaFreeHost(*buf);
-      *buf = nullptr, *cap = 0;
-      const cudaError_t e = cudaHostAlloc((void**)buf, need + need / 2 + 4096, cudaHostAllocDefault);
-      if (e == cudaSuccess) *cap = need + need / 2 + 4096;
-      return e;
-    };
-    VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_in, &ctx->h_stage_in_cap, ctx->in_arena.used));
-    VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_out, &ctx->h_stage_out_cap, ctx->out_arena.used));
-    rc = check_batch_indices(ctx, in, form, 0, NP, 0, NL);
-    if (rc != VIML_OK) return rc;
-    char* const ibase = ctx->in_arena.base;
-    auto put = [&](const void* dptr, const void* src, size_t bytes) {
-      if (bytes) memcpy(ctx->h_stage_in + ((const char*)dptr - ibase), src, bytes);
-    };
-    put(d_poses, in->poses, n_pose * 8), put(d_ex, in->ex_pose, n_ex * 8), put(d_dep, in->inv_depth, n_dep * 8);
-    put(d_poff, in->pf_window_offset, (size_t)(W + 1) * 4), put(d_idx, in->pf_idx, (size_t)NP * 4);
-    if (obs_table) put(d_obsj, h_obsj, (size_t)NP * ob), put(d_fobs, h_fobs, n_dep * ob);
-    else put(d_obs, in->pf_obs, (size_t)NP * 32);
-    if (d_z) put(d_z, in->pf_pts_i_z, (size_t)NP * 8);
-    if (NL > 0) {
-      put(d_loff, in->lf_window_offset, (size_t)(W + 1) * 4), put(d_frame, in->lf_frame, (size_t)NL * 4);
-      if (line_table) put(d_lidx, in->lf_map_index, (size_t)NL * 4), put(d_lseg, in->lf_seg2d_f32, (size_t)NL * 16);
-      else put(d_geom, in->lf_geom, (size_t)NL * 72);
-    }
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ibase, ctx->h_stage_in, ctx->in_arena.used, cudaMemcpyHostToDevice, st));
-    rc = obs_table ? viml_launch_expand_obs(ctx, a, d_fobs, d_obsj, obs_f32) : VIML_OK;
-    if (rc == VIML_OK && line_table) rc = viml_launch_expand_lines(ctx, a, d_lidx, d_lseg);
-    if (rc == VIML_OK) rc = viml_launch_linearize(ctx, a);
-    if (rc != VIML_OK) return rc;
-    // the device range that holds every slot the caller wants
-    char *lo = nullptr, *hi = nullptr;
-    for (auto& sl : slots)
-      if (sl.host) {
-        char* b = (char*)*sl.dev;
-        char* e = b + (sl.per_window * W + sl.per_pf * NP + sl.per_lf * NL) * 8;
-        lo = lo ? std::min(lo, b) : b, hi = hi ? std::max(hi, e) : e;
-      }
-    if (lo) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ctx->h_stage_out, lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, st));
-    VIML_TRY_CUDA(ctx, cudaStreamSynchronize(st));
-    for (auto& sl : slots)
-      if (sl.host) memcpy(sl.host, ctx->h_stage_out + ((char*)*sl.dev - lo), (sl.per_window * W + sl.per_pf * NP + sl.per_lf * NL) * 8);
-    VIML_TRY_CUDA(ctx, cudaGetLastError());
-    return VIML_OK;
-  }
-
   cudaStream_t s_in = ctx->copy_stream, s_out = ctx->copy_stream2;
-  // offsets first (tiny, needed by every chunk); the previous call's work on `st` is already complete (synchronous API)
+  // the uploads wait for the work already queued on the context stream: it may still read in_arena (viml_fov_update returns
+  // without synchronising when it is not asked for the count)
+  VIML_TRY_CUDA(ctx, cudaEventRecord(ctx->ev_a, s_k));
+  VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(s_in, ctx->ev_a, 0));
+  // offsets first (tiny, needed by every chunk)
   VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_poff, in->pf_window_offset, (size_t)(W + 1) * 4, cudaMemcpyHostToDevice, s_in));
   if (NL > 0) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_loff, in->lf_window_offset, (size_t)(W + 1) * 4, cudaMemcpyHostToDevice, s_in));
   const int nchunk = W >= 512 ? 4 : 1;   // measured on the 4096-window batch with the float32 table (75 MB up, 88 MB down): 2, 3, 4, 5, 6, 8, 12, 16 chunks -> 2.96, 2.81, 2.67, 2.75, 2.70, 2.79, 2.93, 2.96 ms
@@ -617,7 +599,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     const int64_t la = NL > 0 ? in->lf_window_offset[w0] : 0, lb = NL > 0 ? in->lf_window_offset[w1] : 0;
     rc = check_batch_indices(ctx, in, form, pa, pb, la, lb);
     if (rc != VIML_OK) break;   // bad indices never reach a kernel: this chunk and the following ones are not launched
-    cudaStreamWaitEvent(st, ev_in[c], 0);
+    cudaStreamWaitEvent(s_k, ev_in[c], 0);
     // view of windows [w0, w1)
     LinearizeArgs v = a;
     v.W = Wc, v.NP = pb - pa, v.NL = lb - la, v.pf_begin = pa, v.lf_begin = la;
@@ -632,7 +614,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     if (Wc > 0 && obs_table) rc = viml_launch_expand_obs(ctx, v, d_fobs + (size_t)w0 * F * ob, d_obsj, obs_f32);
     if (Wc > 0 && rc == VIML_OK && line_table) rc = viml_launch_expand_lines(ctx, v, d_lidx, d_lseg);
     if (Wc > 0 && rc == VIML_OK) rc = viml_launch_linearize(ctx, v);
-    cudaEventRecord(ev_k[c], st);
+    cudaEventRecord(ev_k[c], s_k);
     cudaStreamWaitEvent(s_out, ev_k[c], 0);
     for (auto& sl : slots)
       if (sl.host) {
@@ -641,7 +623,7 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
         if (cnt) cudaMemcpyAsync(sl.host + off, *sl.dev + off, cnt * 8, cudaMemcpyDeviceToHost, s_out);
       }
   }
-  cudaError_t e1 = cudaStreamSynchronize(s_out), e2 = cudaStreamSynchronize(st), e3 = cudaStreamSynchronize(s_in);
+  cudaError_t e1 = cudaStreamSynchronize(s_out), e2 = cudaStreamSynchronize(s_k), e3 = cudaStreamSynchronize(s_in);
   for (int c = 0; c < nchunk; ++c) cudaEventDestroy(ev_in[c]), cudaEventDestroy(ev_k[c]);
   if (rc != VIML_OK) return rc;
   VIML_TRY_CUDA(ctx, e1);
@@ -660,33 +642,21 @@ int viml_marginalize_batch(viml_ctx* ctx, const viml_marg_batch* in, const viml_
     return fail(ctx, VIML_ERR_INVALID, "marg batch sizes out of range (pos <= 256, n >= 1)");
   if (K == 0) return VIML_OK;
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
-  if (flags & VIML_PTRS_DEVICE)
-    return viml_launch_marginalize(ctx, K, pos, m, in->eps, in->A, in->b, out->A_schur, out->b_schur,
-                                   out->linearized_jacobians, out->linearized_residuals);
   const size_t szA = (size_t)K * pos * pos, szb = (size_t)K * pos, szS = (size_t)K * n * n, szs = (size_t)K * n;
-  auto pad = [](size_t b) { return DeviceArena::padded(b); };
-  VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(pad(szA * 8) + pad(szb * 8)));
-  double* dA = ctx->in_arena.take<double>(szA);
-  double* db = ctx->in_arena.take<double>(szb);
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(dA, in->A, szA * 8, cudaMemcpyHostToDevice, st));
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(db, in->b, szb * 8, cudaMemcpyHostToDevice, st));
-  VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(2 * pad(szS * 8) + 2 * pad(szs * 8)));
-  double* dS = ctx->out_arena.take<double>(szS);
-  double* ds = ctx->out_arena.take<double>(szs);
-  double* dJ = ctx->out_arena.take<double>(szS);
-  double* dr = ctx->out_arena.take<double>(szs);
-  const bool lin = out->linearized_jacobians || out->linearized_residuals;
-  int rc = viml_launch_marginalize(ctx, K, pos, m, in->eps, dA, db, dS, ds, lin ? dJ : nullptr, lin ? dr : nullptr);
+  Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
+  const double *dA = nullptr, *db = nullptr;
+  double *dS = nullptr, *ds = nullptr, *dJ = nullptr, *dr = nullptr;
+  st.in(in->A, szA, &dA);
+  st.in(in->b, szb, &db);
+  // an output the caller did not ask for is null: the kernel skips it
+  st.out(out->A_schur, out->A_schur ? szS : 0, &dS);
+  st.out(out->b_schur, out->b_schur ? szs : 0, &ds);
+  st.out(out->linearized_jacobians, out->linearized_jacobians ? szS : 0, &dJ);
+  st.out(out->linearized_residuals, out->linearized_residuals ? szs : 0, &dr);
+  int rc = st.commit();
+  if (rc == VIML_OK) rc = viml_launch_marginalize(ctx, K, pos, m, in->eps, dA, db, dS, ds, dJ, dr);
   if (rc != VIML_OK) return rc;
-  if (out->A_schur) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(out->A_schur, dS, szS * 8, cudaMemcpyDeviceToHost, st));
-  if (out->b_schur) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(out->b_schur, ds, szs * 8, cudaMemcpyDeviceToHost, st));
-  if (out->linearized_jacobians)
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(out->linearized_jacobians, dJ, szS * 8, cudaMemcpyDeviceToHost, st));
-  if (out->linearized_residuals)
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(out->linearized_residuals, dr, szs * 8, cudaMemcpyDeviceToHost, st));
-  VIML_TRY_CUDA(ctx, cudaStreamSynchronize(st));
-  return VIML_OK;
+  return st.finish();
 }
 
 // ---- association -----------------------------------------------------------------------------------
@@ -925,43 +895,40 @@ int viml_track_gate(viml_ctx* ctx, int32_t n_tracks, const int32_t* track_offset
   if (!ctx->map_set) return fail(ctx, VIML_ERR_NOMAP, "viml_track_gate before viml_set_map");
   if (n_tracks == 0) return VIML_OK;
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
-  if (flags & VIML_PTRS_DEVICE) return viml_launch_track_gate(ctx, n_tracks, track_offset, line_index, credible_line, credible_matching);
-  const int64_t nobs = track_offset[n_tracks];
-  if (nobs < 0 || (nobs > 0 && (!line_index || !credible_line))) return fail(ctx, VIML_ERR_INVALID, "viml_track_gate: null observation arrays");
-  auto pad = [](size_t b) { return DeviceArena::padded(b); };
-  VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(pad((size_t)(n_tracks + 1) * 4) + pad((size_t)nobs * 4 + 4)));
-  VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(pad((size_t)nobs + 1) + pad((size_t)n_tracks)));
-  int32_t* doff = ctx->in_arena.take<int32_t>((size_t)n_tracks + 1);
-  int32_t* didx = ctx->in_arena.take<int32_t>((size_t)nobs + 1);
-  uint8_t* dcl = ctx->out_arena.take<uint8_t>((size_t)nobs + 1);
-  uint8_t* dcm = ctx->out_arena.take<uint8_t>((size_t)n_tracks);
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(doff, track_offset, (size_t)(n_tracks + 1) * 4, cudaMemcpyHostToDevice, st));
-  if (nobs) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(didx, line_index, (size_t)nobs * 4, cudaMemcpyHostToDevice, st));
-  const int rc = viml_launch_track_gate(ctx, n_tracks, doff, didx, dcl, dcm);
+  Stager st{ctx, (flags & VIML_PTRS_DEVICE) != 0};
+  int64_t nobs = 0;   // device pointers pass through: the observation count is not needed
+  if (!st.dev) {
+    nobs = track_offset[n_tracks];
+    if (nobs < 0 || (nobs > 0 && (!line_index || !credible_line))) return fail(ctx, VIML_ERR_INVALID, "viml_track_gate: null observation arrays");
+  }
+  const int32_t *doff = nullptr, *didx = nullptr;
+  uint8_t *dcl = nullptr, *dcm = nullptr;
+  st.in(track_offset, (size_t)n_tracks + 1, &doff);
+  st.in(line_index, (size_t)nobs, &didx);
+  st.out(credible_line, (size_t)nobs, &dcl);
+  st.out(credible_matching, (size_t)n_tracks, &dcm);
+  int rc = st.commit();
+  if (rc == VIML_OK) rc = viml_launch_track_gate(ctx, n_tracks, doff, didx, dcl, dcm);
   if (rc != VIML_OK) return rc;
-  if (nobs) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(credible_line, dcl, (size_t)nobs, cudaMemcpyDeviceToHost, st));
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(credible_matching, dcm, (size_t)n_tracks, cudaMemcpyDeviceToHost, st));
-  VIML_TRY_CUDA(ctx, cudaStreamSynchronize(st));
-  return VIML_OK;
+  return st.finish();
 }
 
 int viml_selftest_division(viml_ctx* ctx, const double* a, const double* b, int64_t n, int64_t* mismatches) {
   if (!ctx) return VIML_ERR_INVALID;
   if (n < 0 || (n > 0 && (!a || !b)) || !mismatches) return fail(ctx, VIML_ERR_INVALID, "bad division self-test arguments");
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
-  VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(2 * DeviceArena::padded((size_t)n * 8) + 256));
-  double* da = ctx->in_arena.take<double>((size_t)n);
-  double* db = ctx->in_arena.take<double>((size_t)n);
-  unsigned long long* dm = ctx->in_arena.take<unsigned long long>(1);
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(da, a, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(db, b, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-  VIML_TRY_CUDA(ctx, cudaMemsetAsync(dm, 0, 8, ctx->stream));
-  const int rc = viml_launch_divcheck(ctx, da, db, n, dm);
+  Stager st{ctx, false};
+  const double *da = nullptr, *db = nullptr;
+  unsigned long long h = 0, *dm = nullptr;
+  st.in(a, (size_t)n, &da);
+  st.in(b, (size_t)n, &db);
+  st.out(&h, 1, &dm);
+  int rc = st.commit();
   if (rc != VIML_OK) return rc;
-  unsigned long long h = 0;
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(&h, dm, 8, cudaMemcpyDeviceToHost, ctx->stream));
-  VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  VIML_TRY_CUDA(ctx, cudaMemsetAsync(dm, 0, 8, ctx->stream));
+  rc = viml_launch_divcheck(ctx, da, db, n, dm);
+  if (rc == VIML_OK) rc = st.finish();
+  if (rc != VIML_OK) return rc;
   *mismatches = (int64_t)h;
   return VIML_OK;
 }
