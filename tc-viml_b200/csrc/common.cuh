@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
@@ -99,20 +100,31 @@ inline int fail(viml_ctx* ctx, int code, const char* msg) {
   return code;
 }
 
-// Host <-> device staging for the synchronous host-pointer flavour of an entry point: in() slots are placed in ctx->in_arena and
-// copied up by commit(), out() slots in ctx->out_arena and copied back by finish(), which synchronises.  An out() with a null host
-// pointer is device scratch.  With host pointers a slot whose count is 0 is null.  With VIML_PTRS_DEVICE the caller's pointers pass
-// through unchanged and only scratch is placed.
-// A host call whose staged bytes total at most kOneCopyBytes goes up in one copy and comes back in one: every cudaMemcpyAsync
-// costs 5-10 us of driver and DMA set-up whatever its size (more from pageable memory), and a step stages some 30 arrays.  The
-// inputs are gathered into the pinned ctx->h_stage_in laid out like in_arena; the device range that holds every output comes back
-// into ctx->h_stage_out and is handed out from there.
+// Host <-> device staging of an entry point: where a host call's arrays live on the device, and how they get there and back.
+// in() slots are placed in ctx->in_arena and copied up, out() slots in ctx->out_arena and copied back.  An out() with a null host
+// pointer is device scratch; an inout() is an out() whose device slot first receives the caller's buffer (entries the kernels do
+// not write keep the caller's content).  With host pointers a slot whose count is 0 is null.  With VIML_PTRS_DEVICE the caller's
+// pointers pass through unchanged and only scratch is placed.
+// Host pointers are copied in one of three modes:
+//  - one copy: commit() / finish() of a call whose staged bytes total at most kOneCopyBytes.  Every cudaMemcpyAsync costs 5-10 us
+//    of driver and DMA set-up whatever its size (more from pageable memory), and a step stages some 30 arrays, so the inputs are
+//    gathered into the pinned ctx->h_stage_in laid out like in_arena (one H2D), and the device range that holds every output comes
+//    back into ctx->h_stage_out (one D2H) and is handed out from there.
+//  - per array: commit() / finish() of a larger call, one copy per array on the context stream.
+//  - chunked: run_chunked(), a pipeline of chunks over three streams for the large calls whose work splits into independent units
+//    (windows, poses).  A slot given a Split goes up / comes back chunk by chunk; the other slots are whole.
+// commit() and finish() synchronise nothing but the context stream at the end of finish(); run_chunked() returns synchronised.
 struct Stager {
   static constexpr size_t kOneCopyBytes = size_t(4) << 20;
+  // Positions on the unit axes of a chunked run (up to three: the linearisation's windows, point factors and line factors).
+  using Units = std::array<int64_t, 3>;
+  // How a slot splits into chunks: `per` elements for each unit of axis `axis`, in each of `planes` planes of an SoA array
+  // ([planes][n] with n = count / planes: a chunk is one 2D copy of its range of every plane).  axis < 0: whole.
+  struct Split { int axis = -1; size_t per = 0; int planes = 1; };
   viml_ctx* ctx;
   bool dev;
-  struct In { const void* host; size_t bytes; const void** slot; };
-  struct Out { void* host; size_t bytes; void** slot; };
+  struct In { const void* host; size_t bytes; const void** slot; Split sp; char* d; };   // sp.per in bytes; d: the placed slot
+  struct Out { void* host; size_t bytes; void** slot; Split sp; bool inout; char* d; };
   std::vector<In> ins;
   std::vector<Out> outs;
   Stager(viml_ctx* c, bool d) : ctx(c), dev(d) {   // room for the arrays of any call: no reallocation while staging
@@ -120,14 +132,19 @@ struct Stager {
     outs.reserve(32);
   }
   template <class T>
-  void in(const T* host, size_t count, const T** slot) {
+  void in(const T* host, size_t count, const T** slot, Split sp = {}) {
     *slot = dev ? host : nullptr;
-    if (!dev && host && count) ins.push_back({host, count * sizeof(T), reinterpret_cast<const void**>(slot)});
+    sp.per *= sizeof(T);
+    if (!dev && host && count) ins.push_back({host, count * sizeof(T), reinterpret_cast<const void**>(slot), sp, nullptr});
   }
   template <class T>
-  void out(T* host, size_t count, T** slot) {
+  void inout(T* host, size_t count, T** slot, Split sp = {}) { out(host, count, slot, sp, true); }
+  template <class T>
+  void out(T* host, size_t count, T** slot, Split sp = {}, bool inout = false) {
     *slot = dev ? host : nullptr;
-    if ((!dev || !host) && count) outs.push_back({dev ? nullptr : host, count * sizeof(T), reinterpret_cast<void**>(slot)});
+    sp.per *= sizeof(T);
+    if ((!dev || !host) && count)
+      outs.push_back({dev ? nullptr : host, count * sizeof(T), reinterpret_cast<void**>(slot), sp, inout && !dev && host, nullptr});
   }
   size_t in_bytes() const {
     size_t b = 0;
@@ -149,23 +166,40 @@ struct Stager {
     if (e == cudaSuccess) *cap = need + need / 2 + 4096;
     return e;
   }
+  // places every slot in the arenas
+  int place() {
+    VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(in_bytes()));
+    VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(out_bytes()));
+    for (auto& e : ins) *e.slot = e.d = ctx->in_arena.take<char>(e.bytes);
+    for (auto& e : outs) *e.slot = e.d = ctx->out_arena.take<char>(e.bytes);
+    return VIML_OK;
+  }
+  // Copies the units [lo, hi) of a slot of `bytes` (all of it when it is whole): one copy, or one 2D copy of its planes.
+  static cudaError_t copy(void* dst, const void* src, size_t bytes, const Split& s, const Units& lo, const Units& hi,
+                          cudaMemcpyKind kind, cudaStream_t st) {
+    const size_t off = s.axis < 0 ? 0 : s.per * (size_t)lo[s.axis];
+    const size_t n = s.axis < 0 ? bytes / s.planes : s.per * (size_t)(hi[s.axis] - lo[s.axis]);
+    if (!n) return cudaSuccess;
+    if (s.planes == 1) return cudaMemcpyAsync((char*)dst + off, (const char*)src + off, n, kind, st);
+    const size_t pitch = bytes / s.planes;
+    return cudaMemcpy2DAsync((char*)dst + off, pitch, (const char*)src + off, pitch, n, s.planes, kind, st);
+  }
+  // One copy or per array: places the slots and queues the uploads on the context stream, in-out slots after the inputs.
   int commit() {
     const size_t ib = in_bytes(), ob = out_bytes();
     const bool one = one_copy();
-    VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(ib));
-    VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(ob));
+    const int rc = place();
+    if (rc != VIML_OK) return rc;
     if (one) {
       VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_in, &ctx->h_stage_in_cap, ib));
       VIML_TRY_CUDA(ctx, grow(&ctx->h_stage_out, &ctx->h_stage_out_cap, ob));
+      for (auto& e : ins) memcpy(ctx->h_stage_in + (e.d - ctx->in_arena.base), e.host, e.bytes);
+      if (ib) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ctx->in_arena.base, ctx->h_stage_in, ib, cudaMemcpyHostToDevice, ctx->stream));
+    } else {
+      for (auto& e : ins) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(e.d, e.host, e.bytes, cudaMemcpyHostToDevice, ctx->stream));
     }
-    for (auto& e : ins) {
-      char* d = ctx->in_arena.take<char>(e.bytes);
-      if (one) memcpy(ctx->h_stage_in + (d - ctx->in_arena.base), e.host, e.bytes);
-      else VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d, e.host, e.bytes, cudaMemcpyHostToDevice, ctx->stream));
-      *e.slot = d;
-    }
-    if (one && ib) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(ctx->in_arena.base, ctx->h_stage_in, ib, cudaMemcpyHostToDevice, ctx->stream));
-    for (auto& e : outs) *e.slot = ctx->out_arena.take<char>(e.bytes);
+    for (auto& e : outs)
+      if (e.inout) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(e.d, e.host, e.bytes, cudaMemcpyHostToDevice, ctx->stream));
     return VIML_OK;
   }
   int finish() {
@@ -186,6 +220,73 @@ struct Stager {
         if (e.host) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(e.host, *e.slot, e.bytes, cudaMemcpyDeviceToHost, ctx->stream));
       VIML_TRY_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     }
+    VIML_TRY_CUDA(ctx, cudaGetLastError());
+    return VIML_OK;
+  }
+  // Chunked (host pointers only): H2D(c + 1) | kernels(c) | D2H(c - 1) on copy_stream, the context stream and copy_stream2.  PCIe
+  // is full duplex, so with pinned host memory a call approaches max(H2D, D2H) time.  `n` units make C chunks, chunk c the units
+  // [n c / C, n (c + 1) / C); at(u) gives the position of unit boundary u on every axis.
+  //  1. copy_stream waits for the context stream: work queued there may still read the arenas.
+  //  2. Whole inputs and in-out uploads go up; the context stream waits for them.
+  //  3. Every chunk's inputs go up, each chunk followed by its event.
+  //  4. step() runs: work over all units, which may synchronise the host (the uploads of step 3 overlap it).
+  //  5. Per chunk: the context stream waits for its event, chunk(lo, hi) builds its view and launches, and copy_stream2 brings back
+  //     the chunk's range of every host-backed output (whole outputs after the last chunk).
+  // The three streams are synchronised and the events destroyed on every exit; the first error is returned.  An error of chunk()
+  // launches no later chunk; the outputs of the chunks before it may already be written.
+  template <class At, class Step, class Chunk>
+  int run_chunked(int n, At at, Step step, Chunk chunk) {
+    // measured on the 4096-window linearisation with the float32 table (75 MB up, 88 MB down): 2, 3, 4, 5, 6, 8, 12, 16 chunks ->
+    // 2.96, 2.81, 2.67, 2.75, 2.70, 2.79, 2.93, 2.96 ms; on the cfg-3 association sweep: 2, 4, 6, 8, 12, 16 -> 2.32, 2.19, 2.30,
+    // 2.36, 2.79, 2.76 ms
+    const int C = n >= 512 ? 4 : 1;
+    std::vector<Units> b(C + 1);
+    for (int c = 0; c <= C; ++c) b[c] = at((int)((int64_t)n * c / C));
+    std::vector<cudaEvent_t> ev;   // the C upload events, then one per launched chunk
+    auto event = [&](cudaStream_t s) {
+      cudaEvent_t e;
+      cudaError_t r = cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
+      if (r == cudaSuccess) ev.push_back(e), r = cudaEventRecord(e, s);
+      return r;
+    };
+    auto run = [&]() -> int {
+      cudaStream_t s_k = ctx->stream, s_in = ctx->copy_stream, s_out = ctx->copy_stream2;
+      int rc = place();
+      if (rc != VIML_OK) return rc;
+      VIML_TRY_CUDA(ctx, cudaEventRecord(ctx->ev_a, s_k));
+      VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(s_in, ctx->ev_a, 0));
+      for (auto& e : ins)
+        if (e.sp.axis < 0) VIML_TRY_CUDA(ctx, copy(e.d, e.host, e.bytes, e.sp, b[0], b[C], cudaMemcpyHostToDevice, s_in));
+      for (auto& e : outs)
+        if (e.inout) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(e.d, e.host, e.bytes, cudaMemcpyHostToDevice, s_in));
+      VIML_TRY_CUDA(ctx, cudaEventRecord(ctx->ev_b, s_in));
+      VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(s_k, ctx->ev_b, 0));
+      for (int c = 0; c < C; ++c) {
+        for (auto& e : ins)
+          if (e.sp.axis >= 0) VIML_TRY_CUDA(ctx, copy(e.d, e.host, e.bytes, e.sp, b[c], b[c + 1], cudaMemcpyHostToDevice, s_in));
+        VIML_TRY_CUDA(ctx, event(s_in));
+      }
+      rc = step();
+      for (int c = 0; c < C && rc == VIML_OK; ++c) {
+        VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(s_k, ev[c], 0));
+        rc = chunk(b[c], b[c + 1]);
+        if (rc != VIML_OK) break;
+        VIML_TRY_CUDA(ctx, event(s_k));
+        VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(s_out, ev.back(), 0));
+        for (auto& e : outs)
+          if (e.host && (e.sp.axis >= 0 || c == C - 1))
+            VIML_TRY_CUDA(ctx, copy(e.host, e.d, e.bytes, e.sp, b[c], b[c + 1], cudaMemcpyDeviceToHost, s_out));
+      }
+      return rc;
+    };
+    const int rc = run();
+    const cudaError_t e1 = cudaStreamSynchronize(ctx->copy_stream2), e2 = cudaStreamSynchronize(ctx->stream),
+                      e3 = cudaStreamSynchronize(ctx->copy_stream);
+    for (cudaEvent_t e : ev) cudaEventDestroy(e);
+    if (rc != VIML_OK) return rc;
+    VIML_TRY_CUDA(ctx, e1);
+    VIML_TRY_CUDA(ctx, e2);
+    VIML_TRY_CUDA(ctx, e3);
     VIML_TRY_CUDA(ctx, cudaGetLastError());
     return VIML_OK;
   }
@@ -278,9 +379,12 @@ struct StagedBatch {
   const int32_t* lidx;
   double *obs, *geom;   // their expansions
 };
+// The unit axes of a window batch in a chunked run: windows, point factors, line factors.
+constexpr int kAxWindow = 0, kAxPf = 1, kAxLf = 2;
 // Stages the batch (checked by check_window_batch, which gave `form`) into `st`: the inputs of linearize_args(ctx, in, flags), the
-// table sources, the expansion targets and the pose cache.  The Stager keeps the addresses of *b's fields; after st.commit() the
-// caller calls expand_tables().
+// table sources, the expansion targets and the pose cache.  The per-factor inputs and the per-window observation table are split
+// by factor / window; the rest is whole.  The Stager keeps the addresses of *b's fields; after st.commit() the caller calls
+// expand_tables().
 void stage_batch(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const BatchForm& form, uint32_t flags, StagedBatch* b);
 // The observation and line tables of the batch, expanded into the per-factor arrays every kernel reads.
 int expand_tables(viml_ctx* ctx, StagedBatch& b);

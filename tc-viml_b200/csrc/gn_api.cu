@@ -491,14 +491,10 @@ int viml_inertial_evaluate(viml_ctx* ctx, const viml_window_batch* state, const 
   st.out(out->imu_jac_sb_i, out->imu_jac_sb_i ? NI * 135 : 0, &o.imu_jac_sb_i);
   st.out(out->imu_jac_pose_j, out->imu_jac_pose_j ? NI * 105 : 0, &o.imu_jac_pose_j);
   st.out(out->imu_jac_sb_j, out->imu_jac_sb_j ? NI * 135 : 0, &o.imu_jac_sb_j);
-  st.out(out->prior_residual, out->prior_residual ? (size_t)W * v.n_max : 0, &o.prior_residual);
+  // in-out: rows past n_w keep the caller's content
+  st.inout(out->prior_residual, out->prior_residual ? (size_t)W * v.n_max : 0, &o.prior_residual);
   rc = st.commit();
-  if (rc != VIML_OK) return rc;
-  // host flavour: the staged prior residuals start as a copy of the caller's buffer, so that rows past n_w keep its content
-  if (!dev && out->prior_residual)
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(o.prior_residual, out->prior_residual, (size_t)W * v.n_max * sizeof(double), cudaMemcpyHostToDevice,
-                                       ctx->stream));
-  rc = viml_launch_inertial(ctx, v, o, InertialCsr{}, false);
+  if (rc == VIML_OK) rc = viml_launch_inertial(ctx, v, o, InertialCsr{}, false);
   if (rc != VIML_OK) return rc;
   return st.finish();
 }

@@ -382,21 +382,21 @@ void stage_batch(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const B
   st.in(in->ex_pose, (size_t)W * 7, &a.ex_pose);
   st.in(in->inv_depth, (size_t)W * F, &a.inv_depth);
   st.in(in->pf_window_offset, (size_t)W + 1, &a.pf_window_offset);
-  st.in(in->pf_idx, (size_t)NP, &a.pf_idx);
+  st.in(in->pf_idx, (size_t)NP, &a.pf_idx, {kAxPf, 1});
   if (form.obs_table) {
-    st.in((const char*)form.feat_obs, (size_t)W * F * form.obs_bytes, &b->fobs);
-    st.in((const char*)form.pf_obs_j, (size_t)NP * form.obs_bytes, &b->obsj);
+    st.in((const char*)form.feat_obs, (size_t)W * F * form.obs_bytes, &b->fobs, {kAxWindow, (size_t)F * form.obs_bytes});
+    st.in((const char*)form.pf_obs_j, (size_t)NP * form.obs_bytes, &b->obsj, {kAxPf, form.obs_bytes});
   } else {
-    st.in(in->pf_obs, (size_t)NP * 4, &a.pf_obs);
+    st.in(in->pf_obs, (size_t)NP * 4, &a.pf_obs, {kAxPf, 4});
   }
-  st.in(in->pf_pts_i_z, in->pf_pts_i_z ? (size_t)NP : 0, &a.pf_pts_i_z);
+  st.in(in->pf_pts_i_z, in->pf_pts_i_z ? (size_t)NP : 0, &a.pf_pts_i_z, {kAxPf, 1});
   st.in(in->lf_window_offset, NL > 0 ? (size_t)W + 1 : 0, &a.lf_window_offset);
   st.in(in->lf_frame, (size_t)NL, &a.lf_frame);
   if (form.line_table) {
-    st.in(in->lf_map_index, (size_t)NL, &b->lidx);
-    st.in(in->lf_seg2d_f32, (size_t)NL * 4, &b->lseg);
+    st.in(in->lf_map_index, (size_t)NL, &b->lidx, {kAxLf, 1});
+    st.in(in->lf_seg2d_f32, (size_t)NL * 4, &b->lseg, {kAxLf, 4});
   } else {
-    st.in(in->lf_geom, (size_t)NL * 9, &a.lf_geom);
+    st.in(in->lf_geom, (size_t)NL * 9, &a.lf_geom, {kAxLf, 1, 9});   // [9][NL]
   }
   st.out((double*)nullptr, (size_t)W * (P * kPoseCache + kExCache), &a.cache);
   if (form.obs_table) st.out((double*)nullptr, (size_t)NP * 4, &b->obs);
@@ -441,25 +441,30 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
   stage_batch(ctx, st, in, form, flags, &b);
   viml_linearize_out& o = b.a.out;
   if (wantA) {
-    auto a_out = [&](double* host, size_t count, double** slot) { st.out(host, host ? count : 0, slot); };
-    a_out(out->pf_residual, (size_t)NP * 2, &o.pf_residual);
-    a_out(out->pf_jac_pose_i, (size_t)NP * 14, &o.pf_jac_pose_i);
-    a_out(out->pf_jac_pose_j, (size_t)NP * 14, &o.pf_jac_pose_j);
-    a_out(out->pf_jac_ex, (size_t)NP * 14, &o.pf_jac_ex);
-    a_out(out->pf_jac_feat, (size_t)NP * 2, &o.pf_jac_feat);
-    a_out(out->lf_residual, (size_t)NL * 2, &o.lf_residual);
-    a_out(out->lf_jac_pose, (size_t)NL * 14, &o.lf_jac_pose);
+    auto a_out = [&](double* host, size_t per, int axis, double** slot) {
+      st.out(host, host ? per * (size_t)(axis == kAxPf ? NP : NL) : 0, slot, {axis, per});
+    };
+    a_out(out->pf_residual, 2, kAxPf, &o.pf_residual);
+    a_out(out->pf_jac_pose_i, 14, kAxPf, &o.pf_jac_pose_i);
+    a_out(out->pf_jac_pose_j, 14, kAxPf, &o.pf_jac_pose_j);
+    a_out(out->pf_jac_ex, 14, kAxPf, &o.pf_jac_ex);
+    a_out(out->pf_jac_feat, 2, kAxPf, &o.pf_jac_feat);
+    a_out(out->lf_residual, 2, kAxLf, &o.lf_residual);
+    a_out(out->lf_jac_pose, 14, kAxLf, &o.lf_jac_pose);
   }
+  // the per-window outputs, elements per window: H_pp, H_lp, H_ll, b_p, b_l, S, g
+  const size_t n_pp = (size_t)D * D, n_lp = (size_t)F * D, n_S = (flags & VIML_S_PACKED) ? (size_t)D * (D + 1) / 2 : n_pp;
+  auto w_out = [&](double* host, size_t per, double** slot) { st.out(host, (size_t)W * per, slot, {kAxWindow, per}); };
   if (wantHB || wantS) {   // with VIML_OUT_SCHUR alone the H blocks are scratch
-    st.out(wantHB ? out->H_pp : nullptr, (size_t)W * D * D, &o.H_pp);
-    st.out(wantHB ? out->H_lp : nullptr, (size_t)W * F * D, &o.H_lp);
-    st.out(wantHB ? out->H_ll : nullptr, (size_t)W * F, &o.H_ll);
-    st.out(wantHB ? out->b_p : nullptr, (size_t)W * D, &o.b_p);
-    st.out(wantHB ? out->b_l : nullptr, (size_t)W * F, &o.b_l);
+    w_out(wantHB ? out->H_pp : nullptr, n_pp, &o.H_pp);
+    w_out(wantHB ? out->H_lp : nullptr, n_lp, &o.H_lp);
+    w_out(wantHB ? out->H_ll : nullptr, F, &o.H_ll);
+    w_out(wantHB ? out->b_p : nullptr, D, &o.b_p);
+    w_out(wantHB ? out->b_l : nullptr, F, &o.b_l);
   }
   if (wantS) {
-    st.out(out->S, (size_t)W * ((flags & VIML_S_PACKED) ? D * (D + 1) / 2 : D * D), &o.S);
-    st.out(out->g, (size_t)W * D, &o.g);
+    w_out(out->S, n_S, &o.S);
+    w_out(out->g, D, &o.g);
   }
   if (dev || (W < 512 && st.one_copy())) {
     // host pointers: check_window_batch has checked the offsets, the packed indices are checked before any kernel reads them
@@ -470,167 +475,31 @@ int viml_linearize_batch(viml_ctx* ctx, const viml_window_batch* in, const viml_
     if (rc != VIML_OK) return rc;
     return st.finish();
   }
-
-  // ---- host pointers, W >= 512 or more than Stager::kOneCopyBytes: chunked pipeline
-  // H2D(c+1) | kernels(c) | D2H(c-1) on three streams.  Device buffers hold the whole batch at the same absolute positions as the
-  // host arrays; a chunk is a range of windows, its kernels run on a "view" (pointers advanced to the first window of the chunk,
-  // factor ranges absolute).  PCIe is full duplex, so with pinned host memory the call approaches max(H2D, D2H) time.
+  // Host pointers, W >= 512 or more than Stager::kOneCopyBytes: chunks of windows.  A chunk's kernels run on a view of the batch
+  // (per-window pointers advanced to its first window, per-factor arrays absolute: they are indexed by the global factor id).
   // check_window_batch has checked the offsets; the packed indices are checked chunk by chunk before the chunk's kernels (the host
-  // runs ahead of the asynchronous copies and kernels, so the ~1 ms scan of a 2.3 M-factor batch hides behind the transfers of the
-  // previous chunk).
-  const bool obs_table = form.obs_table, obs_f32 = form.obs_f32, line_table = form.line_table;
-  const void *h_fobs = form.feat_obs, *h_obsj = form.pf_obs_j;
-  const size_t ob = form.obs_bytes;
-  cudaStream_t s_k = ctx->stream;
-  LinearizeArgs a = linearize_args(ctx, in, flags);
-  const size_t n_pose = (size_t)W * P * 7, n_ex = (size_t)W * 7, n_dep = (size_t)W * F;
-  VIML_TRY_CUDA(ctx, ctx->scratch.reserve(DeviceArena::padded((size_t)W * (P * kPoseCache + kExCache) * sizeof(double))));
-  a.cache = ctx->scratch.take<double>((size_t)W * (P * kPoseCache + kExCache));
-  auto pad = [](size_t b) { return DeviceArena::padded(b); };
-  size_t in_bytes = pad(n_pose * 8) + pad(n_ex * 8) + pad(n_dep * 8) + 2 * pad((size_t)(W + 1) * 4);
-  in_bytes += pad((size_t)NP * 4) + pad((size_t)NP * 32) + pad((size_t)NP * 8);
-  in_bytes += pad((size_t)NL * 4) + pad((size_t)NL * 72);
-  if (obs_table) in_bytes += pad((size_t)NP * ob) + pad(n_dep * ob);
-  if (line_table) in_bytes += pad((size_t)NL * 4) + pad((size_t)NL * 16);
-  VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(in_bytes));
-  double* d_poses = ctx->in_arena.take<double>(n_pose);
-  double* d_ex = ctx->in_arena.take<double>(n_ex);
-  double* d_dep = ctx->in_arena.take<double>(n_dep);
-  int32_t* d_poff = ctx->in_arena.take<int32_t>((size_t)W + 1);
-  uint32_t* d_idx = ctx->in_arena.take<uint32_t>((size_t)NP);
-  double* d_obs = ctx->in_arena.take<double>((size_t)NP * 4);
-  double* d_z = in->pf_pts_i_z ? ctx->in_arena.take<double>((size_t)NP) : nullptr;
-  int32_t* d_loff = NL > 0 ? ctx->in_arena.take<int32_t>((size_t)W + 1) : nullptr;
-  int32_t* d_frame = NL > 0 ? ctx->in_arena.take<int32_t>((size_t)NL) : nullptr;
-  double* d_geom = NL > 0 ? ctx->in_arena.take<double>((size_t)NL * 9) : nullptr;
-  char* d_obsj = obs_table ? ctx->in_arena.take<char>((size_t)NP * ob) : nullptr;
-  char* d_fobs = obs_table ? ctx->in_arena.take<char>(n_dep * ob) : nullptr;
-  int32_t* d_lidx = line_table ? ctx->in_arena.take<int32_t>((size_t)NL) : nullptr;
-  float* d_lseg = line_table ? ctx->in_arena.take<float>((size_t)NL * 4) : nullptr;
-  a.poses = d_poses, a.ex_pose = d_ex, a.inv_depth = d_dep, a.pf_window_offset = d_poff, a.pf_idx = d_idx;
-  a.pf_obs = d_obs, a.pf_pts_i_z = d_z, a.lf_window_offset = d_loff, a.lf_frame = d_frame, a.lf_geom = d_geom;
-
-  struct Slot { double** dev; double* host; size_t per_window, per_pf, per_lf; };
-  std::vector<Slot> slots;
-  size_t out_bytes = 0;
-  auto want = [&](double** dslot, double* host, size_t per_window, size_t per_pf, size_t per_lf, bool force) {
-    if (host || force) {
-      slots.push_back({dslot, host, per_window, per_pf, per_lf});
-      out_bytes += pad((per_window * W + per_pf * NP + per_lf * NL) * 8);
-    }
+  // runs ahead of the asynchronous copies and kernels, so the ~1 ms scan of a 2.3 M-factor batch hides behind the transfers).
+  auto at = [&](int w) -> Stager::Units { return {w, in->pf_window_offset[w], NL > 0 ? in->lf_window_offset[w] : 0}; };
+  auto chunk = [&](const Stager::Units& lo, const Stager::Units& hi) {
+    const int w0 = (int)lo[kAxWindow];
+    int rc = check_batch_indices(ctx, in, form, lo[kAxPf], hi[kAxPf], lo[kAxLf], hi[kAxLf]);
+    if (rc != VIML_OK) return rc;   // bad indices never reach a kernel: this chunk and the following ones are not launched
+    StagedBatch v = b;
+    LinearizeArgs& va = v.a;
+    va.W = (int)hi[kAxWindow] - w0, va.NP = hi[kAxPf] - lo[kAxPf], va.NL = hi[kAxLf] - lo[kAxLf];
+    va.pf_begin = lo[kAxPf], va.lf_begin = lo[kAxLf];
+    va.poses += (size_t)w0 * P * 7, va.ex_pose += (size_t)w0 * 7, va.inv_depth += (size_t)w0 * F, va.pf_window_offset += w0;
+    if (NL > 0) va.lf_window_offset += w0;
+    va.cache += (size_t)w0 * (P * kPoseCache + kExCache);
+    if (v.fobs) v.fobs += (size_t)w0 * F * form.obs_bytes;
+    auto advance = [&](double*& p, size_t per) { if (p) p += (size_t)w0 * per; };
+    viml_linearize_out& vo = va.out;
+    advance(vo.H_pp, n_pp), advance(vo.H_lp, n_lp), advance(vo.H_ll, F), advance(vo.b_p, D), advance(vo.b_l, F);
+    advance(vo.S, n_S), advance(vo.g, D);
+    rc = expand_tables(ctx, v);
+    return rc != VIML_OK ? rc : viml_launch_linearize(ctx, v.a);
   };
-  const bool needH = wantHB || wantS;
-  if (wantA) {
-    want(&a.out.pf_residual, out->pf_residual, 0, 2, 0, false);
-    want(&a.out.pf_jac_pose_i, out->pf_jac_pose_i, 0, 14, 0, false);
-    want(&a.out.pf_jac_pose_j, out->pf_jac_pose_j, 0, 14, 0, false);
-    want(&a.out.pf_jac_ex, out->pf_jac_ex, 0, 14, 0, false);
-    want(&a.out.pf_jac_feat, out->pf_jac_feat, 0, 2, 0, false);
-    want(&a.out.lf_residual, out->lf_residual, 0, 0, 2, false);
-    want(&a.out.lf_jac_pose, out->lf_jac_pose, 0, 0, 14, false);
-  }
-  if (needH) {
-    want(&a.out.H_pp, wantHB ? out->H_pp : nullptr, (size_t)D * D, 0, 0, true);
-    want(&a.out.H_lp, wantHB ? out->H_lp : nullptr, (size_t)F * D, 0, 0, true);
-    want(&a.out.H_ll, wantHB ? out->H_ll : nullptr, (size_t)F, 0, 0, true);
-    want(&a.out.b_p, wantHB ? out->b_p : nullptr, (size_t)D, 0, 0, true);
-    want(&a.out.b_l, wantHB ? out->b_l : nullptr, (size_t)F, 0, 0, true);
-  }
-  if (wantS) {
-    want(&a.out.S, out->S, (flags & VIML_S_PACKED) ? (size_t)D * (D + 1) / 2 : (size_t)D * D, 0, 0, true);
-    want(&a.out.g, out->g, (size_t)D, 0, 0, true);
-  }
-  VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(out_bytes));
-  for (auto& sl : slots) *sl.dev = ctx->out_arena.take<double>(sl.per_window * W + sl.per_pf * NP + sl.per_lf * NL);
-
-  cudaStream_t s_in = ctx->copy_stream, s_out = ctx->copy_stream2;
-  // the uploads wait for the work already queued on the context stream: it may still read in_arena (viml_fov_update returns
-  // without synchronising when it is not asked for the count)
-  VIML_TRY_CUDA(ctx, cudaEventRecord(ctx->ev_a, s_k));
-  VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(s_in, ctx->ev_a, 0));
-  // offsets first (tiny, needed by every chunk)
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_poff, in->pf_window_offset, (size_t)(W + 1) * 4, cudaMemcpyHostToDevice, s_in));
-  if (NL > 0) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_loff, in->lf_window_offset, (size_t)(W + 1) * 4, cudaMemcpyHostToDevice, s_in));
-  const int nchunk = W >= 512 ? 4 : 1;   // measured on the 4096-window batch with the float32 table (75 MB up, 88 MB down): 2, 3, 4, 5, 6, 8, 12, 16 chunks -> 2.96, 2.81, 2.67, 2.75, 2.70, 2.79, 2.93, 2.96 ms
-  std::vector<int> wb(nchunk + 1);
-  for (int c = 0; c <= nchunk; ++c) wb[c] = (int)((int64_t)W * c / nchunk);
-  // small per-window arrays: whole batch, one copy each
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_poses, in->poses, n_pose * 8, cudaMemcpyHostToDevice, s_in));
-  VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_ex, in->ex_pose, n_ex * 8, cudaMemcpyHostToDevice, s_in));
-  if (n_dep) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_dep, in->inv_depth, n_dep * 8, cudaMemcpyHostToDevice, s_in));
-  if (NL > 0) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(d_frame, in->lf_frame, (size_t)NL * 4, cudaMemcpyHostToDevice, s_in));
-  std::vector<cudaEvent_t> ev_in(nchunk), ev_k(nchunk);
-  for (int c = 0; c < nchunk; ++c) {
-    cudaEventCreateWithFlags(&ev_in[c], cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&ev_k[c], cudaEventDisableTiming);
-  }
-  auto h2d = [&](void* d, const void* h, size_t bytes) {
-    if (bytes) cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, s_in);
-  };
-  // every upload is queued first (the copies depend on nothing but the caller's arrays), so the upload stream runs at link
-  // speed while the host validates the indices of chunk c and launches its kernels
-  for (int c = 0; c < nchunk; ++c) {
-    const int w0 = wb[c], w1 = wb[c + 1];
-    const int64_t pa = in->pf_window_offset[w0], pb = in->pf_window_offset[w1];
-    const int64_t la = NL > 0 ? in->lf_window_offset[w0] : 0, lb = NL > 0 ? in->lf_window_offset[w1] : 0;
-    // per chunk only the three large arrays (observations, packed indices, line geometry as ONE strided copy of its nine
-    // planes); the small per-window arrays went up for the whole batch before the loop — every copy costs ~10-20 us of
-    // DMA set-up however small it is, and 17 copies per chunk kept the upload stream busy for 6 ms on 125 MB
-    h2d(d_idx + pa, in->pf_idx + pa, (size_t)(pb - pa) * 4);
-    if (obs_table) {
-      h2d(d_obsj + ob * pa, (const char*)h_obsj + ob * pa, (size_t)(pb - pa) * ob);
-      h2d(d_fobs + (size_t)w0 * F * ob, (const char*)h_fobs + (size_t)w0 * F * ob, (size_t)(w1 - w0) * F * ob);
-    } else {
-      h2d(d_obs + 4 * pa, in->pf_obs + 4 * pa, (size_t)(pb - pa) * 32);
-    }
-    if (d_z) h2d(d_z + pa, in->pf_pts_i_z + pa, (size_t)(pb - pa) * 8);
-    if (lb > la && line_table) {
-      h2d(d_lidx + la, in->lf_map_index + la, (size_t)(lb - la) * 4);
-      h2d(d_lseg + 4 * la, in->lf_seg2d_f32 + 4 * la, (size_t)(lb - la) * 16);
-    } else if (lb > la) {
-      cudaMemcpy2DAsync(d_geom + la, (size_t)NL * 8, in->lf_geom + la, (size_t)NL * 8, (size_t)(lb - la) * 8, 9,
-                        cudaMemcpyHostToDevice, s_in);
-    }
-    cudaEventRecord(ev_in[c], s_in);
-  }
-  for (int c = 0; c < nchunk && rc == VIML_OK; ++c) {
-    const int w0 = wb[c], w1 = wb[c + 1], Wc = w1 - w0;
-    const int64_t pa = in->pf_window_offset[w0], pb = in->pf_window_offset[w1];
-    const int64_t la = NL > 0 ? in->lf_window_offset[w0] : 0, lb = NL > 0 ? in->lf_window_offset[w1] : 0;
-    rc = check_batch_indices(ctx, in, form, pa, pb, la, lb);
-    if (rc != VIML_OK) break;   // bad indices never reach a kernel: this chunk and the following ones are not launched
-    cudaStreamWaitEvent(s_k, ev_in[c], 0);
-    // view of windows [w0, w1)
-    LinearizeArgs v = a;
-    v.W = Wc, v.NP = pb - pa, v.NL = lb - la, v.pf_begin = pa, v.lf_begin = la;
-    v.poses = a.poses + (size_t)w0 * P * 7, v.ex_pose = a.ex_pose + (size_t)w0 * 7, v.inv_depth = a.inv_depth + (size_t)w0 * F;
-    v.pf_window_offset = a.pf_window_offset + w0;
-    if (NL > 0) v.lf_window_offset = a.lf_window_offset + w0;
-    v.cache = a.cache + (size_t)w0 * (P * kPoseCache + kExCache);
-    for (auto& sl : slots) {
-      double** vd = (double**)((char*)&v.out + ((char*)sl.dev - (char*)&a.out));
-      *vd = *sl.dev + sl.per_window * w0;   // per-factor arrays stay absolute (indexed by the global factor id)
-    }
-    if (Wc > 0 && obs_table) rc = viml_launch_expand_obs(ctx, v, d_fobs + (size_t)w0 * F * ob, d_obsj, obs_f32);
-    if (Wc > 0 && rc == VIML_OK && line_table) rc = viml_launch_expand_lines(ctx, v, d_lidx, d_lseg);
-    if (Wc > 0 && rc == VIML_OK) rc = viml_launch_linearize(ctx, v);
-    cudaEventRecord(ev_k[c], s_k);
-    cudaStreamWaitEvent(s_out, ev_k[c], 0);
-    for (auto& sl : slots)
-      if (sl.host) {
-        const size_t off = sl.per_window * w0 + sl.per_pf * pa + sl.per_lf * la;
-        const size_t cnt = sl.per_window * Wc + sl.per_pf * (pb - pa) + sl.per_lf * (lb - la);
-        if (cnt) cudaMemcpyAsync(sl.host + off, *sl.dev + off, cnt * 8, cudaMemcpyDeviceToHost, s_out);
-      }
-  }
-  cudaError_t e1 = cudaStreamSynchronize(s_out), e2 = cudaStreamSynchronize(s_k), e3 = cudaStreamSynchronize(s_in);
-  for (int c = 0; c < nchunk; ++c) cudaEventDestroy(ev_in[c]), cudaEventDestroy(ev_k[c]);
-  if (rc != VIML_OK) return rc;
-  VIML_TRY_CUDA(ctx, e1);
-  VIML_TRY_CUDA(ctx, e2);
-  VIML_TRY_CUDA(ctx, e3);
-  VIML_TRY_CUDA(ctx, cudaGetLastError());
-  return VIML_OK;
+  return st.run_chunked(W, at, [] { return VIML_OK; }, chunk);
 }
 
 // ---- dense marginalisation -----------------------------------------------------------------------
@@ -705,91 +574,50 @@ int viml_line_associate(viml_ctx* ctx, const viml_assoc_query* q, const viml_ass
   a.stats = ctx->d_assoc_stats;
   a.map_sorted = ctx->d_map_sorted, a.map_orig = ctx->d_map_orig, a.tile_sphere = ctx->d_tile_sphere, a.group_sphere = ctx->d_group_sphere, a.n_tiles = ctx->n_tiles;
   a.fov_capacity = out->fov_index ? out->fov_capacity : 0;
-  auto pad = [](size_t b) { return DeviceArena::padded(b); };
-  const size_t nq = (size_t)Pq * L;
-  if (dev) {
-    size_t sb = 0;
-    if (!out->fov_mask) sb += pad((size_t)Pq * words * 4);
-    if (!out->fov_count) sb += pad((size_t)Pq * 4);
-    VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(sb));
-    a.match_poses = q->match_poses ? q->match_poses : q->cull_poses;
-    a.cull_poses = q->cull_poses ? q->cull_poses : a.match_poses;
-    a.ex_pose = q->ex_pose, a.lines2d = q->lines2d, a.n_lines2d = q->n_lines2d;
-    a.cull_ex_pose = q->cull_ex_pose ? q->cull_ex_pose : q->ex_pose;
-    a.match_index = out->match_index, a.err = out->err, a.projected = out->projected;
-    a.fov_index = out->fov_index;
-    a.fov_mask = out->fov_mask ? out->fov_mask : ctx->out_arena.take<uint32_t>((size_t)Pq * words);
-    a.fov_count = out->fov_count ? out->fov_count : ctx->out_arena.take<int32_t>(Pq);
+  const size_t nq = (size_t)Pq * L, cap = a.fov_capacity;
+  // Every output is per pose; the kernels always write match_index, err, projected, fov_count and fov_mask (scratch where the
+  // caller did not ask).  Host pointers: entries past fov_count keep the caller's fov_index, and ragged queries past n_lines2d keep
+  // the caller's match_index, err and projected.
+  Stager s{ctx, dev};
+  auto per_pose = [](size_t n) { return Stager::Split{0, n}; };
+  s.in(q->cull_poses ? q->cull_poses : q->match_poses, (size_t)Pq * 7, &a.cull_poses);
+  s.in(q->match_poses, (size_t)Pq * 7, &a.match_poses);
+  s.in(q->ex_pose, (size_t)Pq * 7, &a.ex_pose);
+  s.in(q->cull_ex_pose, (size_t)Pq * 7, &a.cull_ex_pose);
+  s.in(q->n_lines2d, (size_t)Pq, &a.n_lines2d);
+  s.in(q->lines2d, nq * 4, &a.lines2d, per_pose((size_t)L * 4));
+  const bool ragged = out->match_index && q->n_lines2d;   // in-out
+  s.out(out->match_index, nq, &a.match_index, per_pose(L), ragged);
+  s.out(out->err, nq * 3, &a.err, per_pose((size_t)L * 3), ragged);
+  s.out(out->projected, nq * 4, &a.projected, per_pose((size_t)L * 4), ragged);
+  s.out(out->fov_count, (size_t)Pq, &a.fov_count, per_pose(1));
+  s.inout(out->fov_index, (size_t)Pq * cap, &a.fov_index, per_pose(cap));
+  s.out(out->fov_mask, (size_t)Pq * words, &a.fov_mask, per_pose((size_t)words));
+  // once the slots are placed: the poses the query did not give separately, and the cached lists
+  auto prepare = [&]() -> int {
+    if (!q->match_poses) a.match_poses = a.cull_poses;
+    if (!q->cull_ex_pose) a.cull_ex_pose = a.ex_pose;
     if (cached) {
       if (words) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.fov_mask, cmask, (size_t)Pq * words * 4, cudaMemcpyDeviceToDevice, st));
       VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.fov_count, ccount, (size_t)Pq * 4, cudaMemcpyDeviceToDevice, st));
     }
-    return viml_launch_associate(ctx, a);
-  }
-  // Host buffers: poses are independent, so a large query is run as a pipeline of pose chunks -- all uploads are queued
-  // on the copy stream up front (one event per chunk), chunk c's kernels wait for its upload only, and its results go
-  // back on the second copy stream while chunk c + 1 computes.
-  VIML_TRY_CUDA(ctx, ctx->in_arena.reserve(4 * pad((size_t)Pq * 56) + pad(nq * 32) + pad((size_t)Pq * 4)));
-  cudaStream_t cs = ctx->copy_stream, ds = ctx->copy_stream2;
-  const int C = Pq >= 512 ? 4 : 1;   // measured on the cfg-3 sweep: 2, 4, 6, 8, 12, 16 chunks -> 2.32, 2.19, 2.30, 2.36, 2.79, 2.76 ms
-  auto up = [&](const void* src, size_t bytes) -> void* {
-    char* d = ctx->in_arena.take<char>(bytes);
-    if (bytes) cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, cs);
-    return d;
+    return VIML_OK;
   };
-  VIML_TRY_CUDA(ctx, cudaEventRecord(ctx->ev_a, st));   // the copy stream starts after whatever the caller queued before
-  VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(cs, ctx->ev_a, 0));
-  a.cull_poses = (const double*)up(q->cull_poses ? q->cull_poses : q->match_poses, (size_t)Pq * 56);
-  a.match_poses = q->match_poses ? (const double*)up(q->match_poses, (size_t)Pq * 56) : a.cull_poses;
-  a.ex_pose = (const double*)up(q->ex_pose, (size_t)Pq * 56);
-  a.cull_ex_pose = q->cull_ex_pose ? (const double*)up(q->cull_ex_pose, (size_t)Pq * 56) : a.ex_pose;
-  a.n_lines2d = q->n_lines2d ? (const int32_t*)up(q->n_lines2d, (size_t)Pq * 4) : nullptr;
-  double* d_l2d = ctx->in_arena.take<double>(nq * 4);
-  a.lines2d = d_l2d;
-  const size_t cap = a.fov_capacity;
-  VIML_TRY_CUDA(ctx, ctx->out_arena.reserve(pad(nq * 4) + pad(nq * 12) + pad(nq * 32) + pad((size_t)Pq * 4) +
-                                            pad((size_t)Pq * cap * 4) + pad((size_t)Pq * words * 4)));
-  a.match_index = ctx->out_arena.take<int32_t>(nq);
-  a.err = ctx->out_arena.take<float>(nq * 3);
-  a.projected = ctx->out_arena.take<double>(nq * 4);
-  a.fov_count = ctx->out_arena.take<int32_t>(Pq);
-  a.fov_index = cap ? ctx->out_arena.take<int32_t>((size_t)Pq * cap) : nullptr;
-  a.fov_mask = ctx->out_arena.take<uint32_t>((size_t)Pq * words);
-  if (cached) {
-    if (words) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.fov_mask, cmask, (size_t)Pq * words * 4, cudaMemcpyDeviceToDevice, st));
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.fov_count, ccount, (size_t)Pq * 4, cudaMemcpyDeviceToDevice, st));
+  if (dev) {
+    int rc = s.commit();
+    if (rc == VIML_OK) rc = prepare();
+    return rc != VIML_OK ? rc : viml_launch_associate(ctx, a);
   }
-  if (out->fov_index && cap)  // entries past fov_count keep the caller's content
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.fov_index, out->fov_index, (size_t)Pq * cap * 4, cudaMemcpyHostToDevice, cs));
-  if (out->match_index && q->n_lines2d) {  // ragged queries past n_lines2d keep the caller's content
-    VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.match_index, out->match_index, nq * 4, cudaMemcpyHostToDevice, cs));
-    if (out->err) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.err, out->err, nq * 12, cudaMemcpyHostToDevice, cs));
-    if (out->projected) VIML_TRY_CUDA(ctx, cudaMemcpyAsync(a.projected, out->projected, nq * 32, cudaMemcpyHostToDevice, cs));
-  }
-  // phase 1 (camera poses, FoV cull, list offsets) runs once for all poses as soon as the small arrays are up — it does not need
-  // the detected lines, whose upload it overlaps — and holds the call's only synchronisation; phase 2 then runs chunk by chunk
-  VIML_TRY_CUDA(ctx, cudaEventRecord(ctx->ev_b, cs));
-  VIML_TRY_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev_b, 0));
-  std::vector<cudaEvent_t> ev_in(C), ev_k(C);
-  auto chunk = [&](int c, int& p0, int& p1) { p0 = (int)((int64_t)Pq * c / C), p1 = (int)((int64_t)Pq * (c + 1) / C); };
-  for (int c = 0; c < C; ++c) {
-    int p0, p1;
-    chunk(c, p0, p1);
-    cudaEventCreateWithFlags(&ev_in[c], cudaEventDisableTiming);
-    cudaEventCreateWithFlags(&ev_k[c], cudaEventDisableTiming);
-    const size_t o = (size_t)p0 * L * 4, n = (size_t)(p1 - p0) * L * 4;
-    if (n) cudaMemcpyAsync(d_l2d + o, q->lines2d + o, n * 8, cudaMemcpyHostToDevice, cs);
-    cudaEventRecord(ev_in[c], cs);
-  }
+  // Host pointers: poses are independent, so the query runs in chunks of poses.  Phase 1 (camera poses, FoV cull, list offsets)
+  // runs once for all poses as soon as the small arrays are up -- it does not need the detected lines, whose upload it overlaps --
+  // and holds the call's only synchronisation; phase 2 (list fill, projection, match) then runs chunk by chunk.
   AssocPlan plan;
-  int rc = viml_assoc_phase1(ctx, a, &plan);
-  auto down = [&](void* host, const void* d, size_t bytes) {
-    if (host && bytes) cudaMemcpyAsync(host, d, bytes, cudaMemcpyDeviceToHost, ds);
+  auto phase1 = [&] {
+    const int rc = prepare();
+    return rc != VIML_OK ? rc : viml_assoc_phase1(ctx, a, &plan);
   };
-  for (int c = 0; c < C && rc == VIML_OK; ++c) {
-    int p0, p1;
-    chunk(c, p0, p1);
-    cudaStreamWaitEvent(st, ev_in[c], 0);
+  auto chunk = [&](const Stager::Units& lo, const Stager::Units& hi) {
+    const int p0 = (int)lo[0], p1 = (int)hi[0];
     AssocArgs v = a;   // view of poses [p0, p1)
     v.Pq = p1 - p0;
     v.cull_poses = a.cull_poses + (size_t)p0 * 7, v.match_poses = a.match_poses + (size_t)p0 * 7;
@@ -798,25 +626,9 @@ int viml_line_associate(viml_ctx* ctx, const viml_assoc_query* q, const viml_ass
     v.match_index = a.match_index + (size_t)p0 * L, v.err = a.err + (size_t)p0 * L * 3, v.projected = a.projected + (size_t)p0 * L * 4;
     v.fov_count = a.fov_count + p0, v.fov_index = a.fov_index ? a.fov_index + (size_t)p0 * cap : nullptr;
     v.fov_mask = a.fov_mask + (size_t)p0 * words;
-    if (v.Pq > 0) rc = viml_assoc_phase2(ctx, v, plan, p0, p1);
-    cudaEventRecord(ev_k[c], st);
-    cudaStreamWaitEvent(ds, ev_k[c], 0);
-    const size_t np = (size_t)(p1 - p0), nqc = np * L;
-    down(out->match_index ? out->match_index + (size_t)p0 * L : nullptr, v.match_index, nqc * 4);
-    down(out->err ? out->err + (size_t)p0 * L * 3 : nullptr, v.err, nqc * 12);
-    down(out->projected ? out->projected + (size_t)p0 * L * 4 : nullptr, v.projected, nqc * 32);
-    down(out->fov_count ? out->fov_count + p0 : nullptr, v.fov_count, np * 4);
-    down(out->fov_index ? out->fov_index + (size_t)p0 * cap : nullptr, v.fov_index, np * cap * 4);
-    down(out->fov_mask ? out->fov_mask + (size_t)p0 * words : nullptr, v.fov_mask, np * words * 4);
-  }
-  cudaError_t e1 = cudaStreamSynchronize(ds), e2 = cudaStreamSynchronize(st), e3 = cudaStreamSynchronize(cs);
-  for (int c = 0; c < C; ++c) cudaEventDestroy(ev_in[c]), cudaEventDestroy(ev_k[c]);
-  if (rc != VIML_OK) return rc;
-  VIML_TRY_CUDA(ctx, e1);
-  VIML_TRY_CUDA(ctx, e2);
-  VIML_TRY_CUDA(ctx, e3);
-  VIML_TRY_CUDA(ctx, cudaGetLastError());
-  return VIML_OK;
+    return viml_assoc_phase2(ctx, v, plan, p0, p1);
+  };
+  return s.run_chunked(Pq, [](int p) { return Stager::Units{p, 0, 0}; }, phase1, chunk);
 }
 
 // ---- FoV cache ---------------------------------------------------------------------------------------
