@@ -390,8 +390,25 @@ void stage_batch(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const B
 int expand_tables(viml_ctx* ctx, StagedBatch& b);
 
 // Largest reduced system a Gauss-Newton step takes, Dx = D + extra_dim (viml.h): its tiled Cholesky keeps the lower triangle in
-// shared memory (linearize_kernels.cu checks the size at compile time).
+// shared memory.
 constexpr int kMaxDx = 232;
+// Dynamic shared memory (bytes) of the tiled Cholesky solves of a Dx x Dx system (gn_kernels.cuh): the lower triangle of 8 x 8
+// tiles and the right-hand side; the fused kernel, which builds the system in place, also keeps g, the undamped diagonal and a
+// stage of kFusedStage doubles for a dense-factor Jacobian and residual (a 76 x 75 prior: 6460).
+constexpr int kFusedStage = 6656;
+constexpr size_t kSolveSmemMax = 224 * 1024;   // of the 227 KB a block may opt in to, beside the kernels' static shared memory
+constexpr size_t gn_solve_smem(int Dx) {
+  const size_t NB = (Dx + 7) / 8;
+  return (NB * (NB + 1) / 2 * 64 + NB * 8) * sizeof(double);
+}
+constexpr size_t gn_fused_solve_smem(int Dx) {
+  return gn_solve_smem(Dx) + (2 * (size_t)((Dx + 7) / 8) * 8 + kFusedStage) * sizeof(double);
+}
+// A Gauss-Newton step whose caller does not ask for Sx / gx builds and solves the system in the fused kernel where it fits,
+// Dx <= 200; above, reduced_kernel writes Sx / gx and the unfused kernel solves it.
+constexpr bool gn_fused_takes(int Dx) { return gn_fused_solve_smem(Dx) <= kSolveSmemMax; }
+static_assert(gn_solve_smem(kMaxDx) <= kSolveSmemMax, "the unfused tiled Cholesky must take the largest reduced system");
+static_assert(gn_fused_takes(200) && !gn_fused_takes(201), "the fused kernel takes Dx <= 200 (DESIGN.md 4.4)");
 
 struct DenseArgs {  // device pointers only; viml_dense_factors
   int X;          // extra tangent columns behind the D pose / extrinsic columns
@@ -451,7 +468,8 @@ int viml_launch_expand_obs(viml_ctx* ctx, const LinearizeArgs& a, const void* fe
 int viml_launch_expand_lines(viml_ctx* ctx, const LinearizeArgs& a, const int32_t* lf_map_index, const float* lf_seg2d);
 int viml_launch_reduced(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double* Sx, double* gx);
 // lambda_w (nullable): a damping per window instead of `lambda`; running (nullable): only windows with running[w] != 0 are solved,
-// updated and costed (the others are left untouched).
+// updated and costed (the others are left untouched).  viml_launch_gn_reduced_solve builds and solves the system in one kernel
+// (Dx = D + dn.X with gn_fused_takes(Dx)); viml_launch_gn_solve solves the Sx / gx of viml_launch_reduced.
 int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double lambda,
                                  double* dx, int32_t* solved, double* cost, const double* lambda_w = nullptr,
                                  const int32_t* running = nullptr);

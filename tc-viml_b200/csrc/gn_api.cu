@@ -173,7 +173,8 @@ int stage_dense(viml_ctx* ctx, Stager& st, const viml_dense_factors* dense, int 
 // viml_solve_vi one per round.  The state the step starts from is b.a.poses, b.a.ex_pose, b.a.inv_depth and extra; x+ goes to o_*.
 struct StepPlan {
   int W, X, Dx;
-  bool vi, want_sx;   // the dense-block factors are the IMU / prior factors; the caller asked for Sx or gx
+  bool vi;            // the dense-block factors are the IMU / prior factors
+  bool fused;         // a step that builds and solves the reduced system in one kernel: Sx / gx are neither wanted nor staged
   StagedBatch b;      // the window batch and its observation / line tables
   DenseArgs dn;
   InertialArgs va;
@@ -194,8 +195,8 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
   *s = StepPlan{};
   s->W = W, s->X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, s->Dx = D + s->X;
-  s->vi = vi != nullptr, s->want_sx = rout && (rout->Sx || rout->gx);
   const int X = s->X, Dx = s->Dx;
+  s->vi = vi != nullptr, s->fused = gout && !(rout && (rout->Sx || rout->gx)) && gn_fused_takes(Dx);
   s->dn.X = X;
   int rc = stage_dense(ctx, st, dense, W, Dx, &s->dn);
   if (rc != VIML_OK) return rc;
@@ -214,8 +215,10 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
   st.out((double*)nullptr, (size_t)W * F, &a.out.b_l);
   st.out((double*)nullptr, (size_t)W * D * D, &a.out.S);
   st.out((double*)nullptr, (size_t)W * D, &a.out.g);
-  st.out(rout ? rout->Sx : nullptr, (size_t)W * Dx * Dx, &s->Sx);
-  st.out(rout ? rout->gx : nullptr, (size_t)W * Dx, &s->gx);
+  if (!s->fused) {
+    st.out(rout ? rout->Sx : nullptr, (size_t)W * Dx * Dx, &s->Sx);
+    st.out(rout ? rout->gx : nullptr, (size_t)W * Dx, &s->gx);
+  }
   if (gout) {
     st.out(gout->dx, (size_t)W * Dx, &s->dx);
     st.out(gout->cost, (size_t)W * 3, &s->cost);
@@ -228,8 +231,9 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
   return VIML_OK;
 }
 
-// One step at the state of s.b.a / s.extra: the reduced system (Sx, gx when the caller asked for them) and, with s.cost set, the
-// solve, the update into s.o_* and the costs.  lambda_w / running: see viml_launch_gn_reduced_solve (nullptr: `lambda`, every window).
+// One step at the state of s.b.a / s.extra: without s.cost the reduced system Sx, gx alone; with it the cost at x, the solve (the
+// system built in the solve kernel when s.fused), the update into s.o_* and the cost at x+.  lambda_w / running: see
+// viml_launch_gn_reduced_solve (nullptr: `lambda`, every window).
 // With s.vi the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at
 // x+ (cost[1], exactly); s.dn is then replaced by their CSR.
 int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* lambda_w, const int32_t* running) {
@@ -248,23 +252,13 @@ int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* 
     dn.window_offset = s.csr.window_offset, dn.row_offset = s.csr.row_offset, dn.col_offset = s.csr.col_offset;
     dn.jac_offset = s.csr.jac_offset, dn.col_index = s.csr.col_index, dn.residual = s.csr.residual, dn.jacobian = s.csr.jacobian;
   }
-  // a step that does not have to hand Sx / gx to the caller builds and solves the reduced system in one kernel
-  bool fused = false;
-  if (step && !s.want_sx) {
-    rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
-    if (rc != VIML_OK) return rc;
+  if (!step) return viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
+  rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
+  if (rc != VIML_OK) return rc;
+  if (s.fused) {
     rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, lambda, s.dx, s.solved, s.cost, lambda_w, running);
-    if (rc == VIML_OK) fused = true;
-    else if (rc != VIML_ERR_UNSUPPORTED) return rc;
-  }
-  if (!fused) {
+  } else {
     rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
-    if (rc != VIML_OK) return rc;
-  }
-  if (!step) return VIML_OK;
-  rc = VIML_OK;
-  if (!fused) {
-    rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
     if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, lambda, s.Sx, s.gx, s.dx, s.solved, s.cost, lambda_w, running);
   }
   if (rc == VIML_OK) rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running);

@@ -10,35 +10,38 @@
 
 namespace gn {
 
-// Sx = embed(S) + sum_k J_k^T J_k,  gx = embed(g) + sum_k J_k^T r_k.  One CTA per window; the window's dense factors are
-// added one after the other (two factors may share columns).  A factor's Jacobian (n x c, row-major) is staged in shared memory
-// with a row stride of c_pad + 4 doubles (conflict-free fragment loads) and J^T J is formed as 8 x 8 tiles on the FP64 tensor pipe:
-// the upper-triangle tiles dealt round-robin to the warps, ceil(n / 4) DMMA steps each, scattered through the factor's column map
-// with their mirrors.  A factor that does not fit the staging area (cap doubles) takes the entry-by-entry loop.
-constexpr int kReducedStage = 12288;   // doubles of dynamic shared memory (96 KB): a 76 x 75 prior needs 76 x 84
+// Factor k of a DenseArgs: n rows x c columns, its Jacobian (row-major), residual and tangent columns.
+struct DenseFactor {
+  int n, c;
+  const double* J;
+  const double* r;
+  const int32_t* ci;
+};
+__device__ __forceinline__ DenseFactor dense_factor(const DenseArgs& dn, int k) {
+  return {(int)(dn.row_offset[k + 1] - dn.row_offset[k]), (int)(dn.col_offset[k + 1] - dn.col_offset[k]), dn.jacobian + dn.jac_offset[k],
+          dn.residual + dn.row_offset[k], dn.col_index + dn.col_offset[k]};
+}
 
-__global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const double* __restrict__ S, const double* __restrict__ g,
-                                                      double* __restrict__ Sx, double* __restrict__ gx) {
-  extern __shared__ __align__(16) double sJ[];
-  const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, Dx = D + dn.X;
-  double* __restrict__ A = Sx + (size_t)w * Dx * Dx;
-  double* __restrict__ b = gx + (size_t)w * Dx;
-  const double* __restrict__ Sw = S + (size_t)w * D * D;
-  for (int e = tid; e < Dx * Dx; e += blockDim.x) {
-    const int r = e / Dx, c = e - r * Dx;
-    A[e] = (r < D && c < D) ? Sw[r * D + c] : 0.0;
-  }
-  for (int e = tid; e < Dx; e += blockDim.x) b[e] = e < D ? g[(size_t)w * D + e] : 0.0;
+// Adds J_k^T J_k and J_k^T r_k of window w's dense-block factors, one factor after the other (two factors may share columns), by a
+// CTA of 256 threads.  A factor's Jacobian is staged in sJ with a row stride of c_pad + 4 doubles (conflict-free fragment loads) and
+// J^T J is formed as 8 x 8 tiles on the FP64 tensor pipe: the upper-triangle tiles dealt round-robin to the warps, ceil(n / 4) DMMA
+// steps each.  A factor that does not fit the stage (cap doubles) takes the entry-by-entry loop, which counts as one diagonal tile.
+// add(i, j, v, diag) adds entry (i, j) = (ci[a], ci[b]) of J^T J, the tile of column a at or left of b's, diag for a diagonal tile;
+// LOWER: a diagonal tile hands over only its a >= b half.  J^T r is added into b.  kq = lane & 3, mq = lane >> 2: the thread's
+// place in a DMMA fragment (the fused kernel has them at hand for its factorisation).
+template <bool LOWER, class Add>
+__device__ __forceinline__ void add_dense_factors(const DenseArgs& dn, int w, int cap, double* __restrict__ sJ, double* __restrict__ b,
+                                                  int kq, int mq, Add add) {
   if (dn.ND == 0) return;
-  __syncthreads();
-  const int kq = lane & 3, mq = lane >> 2;
+  const int tid = threadIdx.x, warp = tid >> 5;
   for (int k = dn.window_offset[w]; k < dn.window_offset[w + 1]; ++k) {
-    const int n = (int)(dn.row_offset[k + 1] - dn.row_offset[k]), c = (int)(dn.col_offset[k + 1] - dn.col_offset[k]);
-    const double* __restrict__ J = dn.jacobian + dn.jac_offset[k];
-    const double* __restrict__ r = dn.residual + dn.row_offset[k];
-    const int32_t* __restrict__ ci = dn.col_index + dn.col_offset[k];
+    const DenseFactor f = dense_factor(dn, k);
+    const int n = f.n, c = f.c;
+    const double* __restrict__ J = f.J;
+    const double* __restrict__ r = f.r;
+    const int32_t* __restrict__ ci = f.ci;
     const int np = (n + 3) & ~3, cp = (c + 7) & ~7, ld = cp + 4;
-    if (np * ld + np <= kReducedStage) {
+    if (np * ld + np <= cap) {
       double* __restrict__ sr = sJ + np * ld;   // the residual behind the Jacobian
       for (int e = tid; e < np * ld; e += 256) {
         const int q = e / ld, a = e - q * ld;
@@ -57,15 +60,8 @@ __global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const
         for (int s4 = 0; s4 < np; s4 += 4) stream::dmma(c0, c1, pa[s4 * ld], pb[s4 * ld]);
         const int a = 8 * ta + mq, bb = 8 * tb + 2 * kq;
         if (a < c) {
-          const size_t ra = (size_t)ci[a] * Dx;
-          if (bb < c) {
-            A[ra + ci[bb]] += c0;
-            if (ta != tb) A[(size_t)ci[bb] * Dx + ci[a]] += c0;
-          }
-          if (bb + 1 < c) {
-            A[ra + ci[bb + 1]] += c1;
-            if (ta != tb) A[(size_t)ci[bb + 1] * Dx + ci[a]] += c1;
-          }
+          if (bb < c && (!LOWER || ta != tb || a >= bb)) add(ci[a], ci[bb], c0, ta == tb);
+          if (bb + 1 < c && (!LOWER || ta != tb || a >= bb + 1)) add(ci[a], ci[bb + 1], c1, ta == tb);
         }
       }
       for (int a = tid; a < c; a += 256) {
@@ -74,13 +70,14 @@ __global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const
         b[ci[a]] += v;
       }
     } else {
-      for (int e = tid; e < c * c; e += blockDim.x) {
+      for (int e = tid; e < c * c; e += 256) {
         const int a = e / c, bb = e - a * c;
+        if (LOWER && a < bb) continue;
         double v = 0.0;
         for (int q = 0; q < n; ++q) v = fma(J[(size_t)q * c + a], J[(size_t)q * c + bb], v);
-        A[(size_t)ci[a] * Dx + ci[bb]] += v;
+        add(ci[a], ci[bb], v, true);
       }
-      for (int a = tid; a < c; a += blockDim.x) {
+      for (int a = tid; a < c; a += 256) {
         double v = 0.0;
         for (int q = 0; q < n; ++q) v = fma(J[(size_t)q * c + a], r[q], v);
         b[ci[a]] += v;
@@ -88,6 +85,29 @@ __global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const
     }
     __syncthreads();
   }
+}
+
+// Sx = embed(S) + sum_k J_k^T J_k,  gx = embed(g) + sum_k J_k^T r_k.  One CTA per window; an entry of an off-diagonal tile is added
+// with its mirror.
+constexpr int kReducedStage = 12288;   // doubles of dynamic shared memory (96 KB): a 76 x 75 prior needs 76 x 84
+
+__global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const double* __restrict__ S, const double* __restrict__ g,
+                                                      double* __restrict__ Sx, double* __restrict__ gx) {
+  extern __shared__ __align__(16) double sJ[];
+  const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, Dx = D + dn.X;
+  double* __restrict__ A = Sx + (size_t)w * Dx * Dx;
+  double* __restrict__ b = gx + (size_t)w * Dx;
+  const double* __restrict__ Sw = S + (size_t)w * D * D;
+  for (int e = tid; e < Dx * Dx; e += blockDim.x) {
+    const int r = e / Dx, c = e - r * Dx;
+    A[e] = (r < D && c < D) ? Sw[r * D + c] : 0.0;
+  }
+  for (int e = tid; e < Dx; e += blockDim.x) b[e] = e < D ? g[(size_t)w * D + e] : 0.0;
+  __syncthreads();
+  add_dense_factors<false>(dn, w, kReducedStage, sJ, b, lane & 3, lane >> 2, [=](int i, int j, double v, bool diag) {
+    A[(size_t)i * Dx + j] += v;
+    if (!diag) A[(size_t)j * Dx + i] += v;
+  });
 }
 
 // ---- tiled Cholesky solve ---------------------------------------------------------------------------------------------------------
@@ -98,10 +118,11 @@ __global__ void __launch_bounds__(256) reduced_kernel(int D, DenseArgs dn, const
 // round-robin to warps 1..7 while warp 0 updates and factors the next diagonal tile (look-ahead).  22 tile columns and ~44 barriers
 // for Dx = 171, and the O(n^3) part runs on the FP64 tensor pipe.  Forward / backward substitution tile by tile.
 // solved[w] = 0 when a pivot is not positive (dx = 0 then).  cost[3w + 2] = -gx.dx - 1/2 dx.Sx.dx (undamped model).
-// FUSED: the matrix is not read from Sx but built in place — embed(S) plus the window's dense-block factors (J^T J as DMMA tiles
-// from a staged Jacobian, like reduced_kernel) — so that Sx never makes its 234 KB round trip through HBM; the model decrease then
-// uses A x = -g:  x^T Sx x = -g.x - lambda sum d_i x_i^2  with d the undamped diagonal.
-constexpr int kFusedStage = 6656;   // doubles for a staged dense-factor Jacobian + residual in the fused kernel (a 76 x 75 prior: 6460)
+// FUSED: the matrix is not read from Sx but built in place — embed(S) plus the window's dense-block factors through
+// add_dense_factors, like reduced_kernel, with a stage of kFusedStage doubles — so that Sx never makes its 234 KB round trip through
+// HBM; the model decrease then uses A x = -g:  x^T Sx x = -g.x - lambda sum d_i x_i^2  with d the undamped diagonal.  A step takes
+// the fused kernel where its shared memory fits (gn_fused_takes in common.cuh: Dx <= 200) and the caller does not want Sx / gx;
+// otherwise reduced_kernel writes Sx / gx and the unfused kernel solves them.
 constexpr int kTile = 8;
 __device__ __forceinline__ int tile_at(int I, int J) { return (I * (I + 1) / 2 + J) * 64; }
 
@@ -148,62 +169,12 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
     }
     for (int e = tid; e < Dp; e += 256) gv[e] = e < D ? g[(size_t)w * D + e] : 0.0;
     __syncthreads();
-    for (int k = dn.ND ? dn.window_offset[w] : 0; k < (dn.ND ? dn.window_offset[w + 1] : 0); ++k) {
-      const int n = (int)(dn.row_offset[k + 1] - dn.row_offset[k]), c = (int)(dn.col_offset[k + 1] - dn.col_offset[k]);
-      const double* __restrict__ J = dn.jacobian + dn.jac_offset[k];
-      const double* __restrict__ r = dn.residual + dn.row_offset[k];
-      const int32_t* __restrict__ ci = dn.col_index + dn.col_offset[k];
-      const int np = (n + 3) & ~3, cp = (c + 7) & ~7, ld = cp + 4;
-      auto lower = [&](int gi, int gj) -> double& {
-        const int hi = max(gi, gj), lo = min(gi, gj);
-        return L[tile_at(hi >> 3, lo >> 3) + (hi & 7) * 8 + (lo & 7)];
-      };
-      if (np * ld + np <= kFusedStage) {
-        double* __restrict__ sr = sJ + np * ld;
-        for (int e = tid; e < np * ld; e += 256) {
-          const int q = e / ld, a = e - q * ld;
-          sJ[e] = (q < n && a < c) ? J[(size_t)q * c + a] : 0.0;
-        }
-        for (int q = tid; q < np; q += 256) sr[q] = q < n ? r[q] : 0.0;
-        __syncthreads();
-        const int nt = cp >> 3, ntile = nt * (nt + 1) / 2;
-        for (int t = warp; t < ntile; t += 8) {
-          int rem = t, ta = 0;
-          while (rem >= nt - ta) rem -= nt - ta, ++ta;
-          const int tb = ta + rem;
-          double c0 = 0.0, c1 = 0.0;
-          const double* __restrict__ pa = sJ + kq * ld + 8 * ta + mq;
-          const double* __restrict__ pb = sJ + kq * ld + 8 * tb + mq;
-          for (int s4 = 0; s4 < np; s4 += 4) stream::dmma(c0, c1, pa[s4 * ld], pb[s4 * ld]);
-          // entry (a, b) and its mirror land on the same lower-triangle slot: off-diagonal tiles add once, a diagonal tile
-          // (which holds both) adds the a >= b half
-          const int a = 8 * ta + mq, bb = 8 * tb + 2 * kq;
-          if (a < c) {
-            if (bb < c && (ta != tb || a >= bb)) lower(ci[a], ci[bb]) += c0;
-            if (bb + 1 < c && (ta != tb || a >= bb + 1)) lower(ci[a], ci[bb + 1]) += c1;
-          }
-        }
-        for (int a = tid; a < c; a += 256) {
-          double v = 0.0;
-          for (int q = 0; q < n; ++q) v = fma(sJ[q * ld + a], sr[q], v);
-          gv[ci[a]] += v;
-        }
-      } else {
-        for (int e = tid; e < c * c; e += 256) {
-          const int a = e / c, bb = e - a * c;
-          if (a < bb) continue;
-          double v = 0.0;
-          for (int q = 0; q < n; ++q) v = fma(J[(size_t)q * c + a], J[(size_t)q * c + bb], v);
-          lower(ci[a], ci[bb]) += v;
-        }
-        for (int a = tid; a < c; a += 256) {
-          double v = 0.0;
-          for (int q = 0; q < n; ++q) v = fma(J[(size_t)q * c + a], r[q], v);
-          gv[ci[a]] += v;
-        }
-      }
-      __syncthreads();
-    }
+    // entry (i, j) and its mirror land on the same lower-triangle slot: off-diagonal tiles add once, a diagonal tile (which holds
+    // both) the a >= b half
+    add_dense_factors<true>(dn, w, kFusedStage, sJ, gv, kq, mq, [=](int i, int j, double v, bool) {
+      const int hi = max(i, j), lo = min(i, j);
+      L[tile_at(hi >> 3, lo >> 3) + (hi & 7) * 8 + (lo & 7)] += v;
+    });
     for (int i = tid; i < Dp; i += 256) {
       double& d = L[tile_at(i >> 3, i >> 3) + (i & 7) * 8 + (i & 7)];
       dv[i] = d;
@@ -484,14 +455,11 @@ __global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn
     }
   if (dn.ND > 0)
     for (int k = dn.window_offset[w]; k < dn.window_offset[w + 1]; ++k) {
-      const int n = (int)(dn.row_offset[k + 1] - dn.row_offset[k]), c = (int)(dn.col_offset[k + 1] - dn.col_offset[k]);
-      const double* __restrict__ J = dn.jacobian + dn.jac_offset[k];
-      const double* __restrict__ r = dn.residual + dn.row_offset[k];
-      const int32_t* __restrict__ ci = dn.col_index + dn.col_offset[k];
-      for (int q = tid; q < n; q += blockDim.x) {
-        double v = r[q];
+      const DenseFactor f = dense_factor(dn, k);
+      for (int q = tid; q < f.n; q += blockDim.x) {
+        double v = f.r[q];
         if (moved)
-          for (int a = 0; a < c; ++a) v = fma(J[(size_t)q * c + a], dx[(size_t)w * Dx + ci[a]], v);
+          for (int a = 0; a < f.c; ++a) v = fma(f.J[(size_t)q * f.c + a], dx[(size_t)w * Dx + f.ci[a]], v);
         acc += v * v;
       }
     }

@@ -670,13 +670,6 @@ int viml_launch_reduced(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const 
   return VIML_OK;
 }
 
-// Shared memory of solve_tiled_kernel<false> for a Dx x Dx system: the lower triangle of 8 x 8 tiles and the right-hand side.
-constexpr size_t gn_solve_smem(int Dx) {
-  const size_t NB = (Dx + 7) / 8;
-  return (NB * (NB + 1) / 2 * 64 + NB * 8) * sizeof(double);
-}
-static_assert(gn_solve_smem(kMaxDx) <= 220 * 1024, "the tiled Cholesky of the largest reduced system must fit in shared memory");
-
 int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const double* Sx, const double* gx, double* dx, int32_t* solved,
                          double* cost, const double* lambda_w, const int32_t* running) {
   const size_t smem = gn_solve_smem(Dx);
@@ -688,13 +681,10 @@ int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const doub
   return VIML_OK;
 }
 
-// Reduced system + solve in one kernel (viml_gn_step when the caller does not ask for Sx / gx): returns VIML_ERR_UNSUPPORTED when
-// the system does not fit the fused kernel's shared memory, and the caller takes the two-kernel path.
 int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double lambda,
                                  double* dx, int32_t* solved, double* cost, const double* lambda_w, const int32_t* running) {
-  const int Dx = D + dn.X, NB = (Dx + 7) / 8;
-  const size_t smem = ((size_t)NB * (NB + 1) / 2 * 64 + 3 * (size_t)NB * 8 + gn::kFusedStage) * sizeof(double);
-  if (smem > 224 * 1024) return VIML_ERR_UNSUPPORTED;
+  const int Dx = D + dn.X;
+  const size_t smem = gn_fused_solve_smem(Dx);
   LaunchScope ls(ctx, K_GN);
   VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   gn::solve_tiled_kernel<true><<<W, 256, smem, ctx->stream>>>(Dx, lambda, nullptr, nullptr, dx, solved, cost, D, dn, S, g, lambda_w,

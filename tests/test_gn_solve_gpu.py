@@ -26,7 +26,7 @@ import scipy.linalg
 U = 2.0 ** -53
 LD = np.longdouble
 U_LD = float(np.finfo(LD).eps) / 2   # unit roundoff of the extended type the reference computes in
-FUSED_STAGE, REDUCED_STAGE = 6656, 12288   # gn::kFusedStage, gn::kReducedStage (doubles)
+FUSED_STAGE, REDUCED_STAGE = 6656, 12288   # kFusedStage (common.cuh), gn::kReducedStage (doubles)
 MAX_DX = 232
 
 
