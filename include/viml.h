@@ -29,7 +29,8 @@
  *   viml_gn_step_vi        <- viml_gn_step over the window's whole problem: the IMU and prior factors evaluated on the device at
  *                             x (system) and at x+ (cost[1] = f(x+))
  *   viml_solve_vi          <- ceres::Solve of the window's whole problem  estimator.cpp:1888-1905 (TrustRegionMinimizer with
- *                             LevenbergMarquardtStrategy; every step is viml_gn_step_vi's; deviations at the declaration)
+ *                             LevenbergMarquardtStrategy, every step viml_gn_step_vi's; with VIML_SOLVE_DOGLEG the reference's
+ *                             DoglegStrategy, trust_region_strategy_type = DOGLEG; deviations at the declaration)
  *   viml_fov_update / viml_fov_slide / VIML_FOV_CACHED
  *                          <- the per-slot FoV lists the estimator keeps between frames: UpdateLinesInFoV at frame entry
  *                             (estimator.cpp:342) and their shifts in slideWindowWithLinesFoV (estimator.cpp:2148, :2160, :2218)
@@ -76,6 +77,7 @@ extern "C" {
 #define VIML_S_PACKED 0x20u              /* with VIML_OUT_SCHUR: S is written as its upper triangle, [W][D(D+1)/2], row r holds
                                             columns r..D-1 (entry (r,c) at r*D - r(r-1)/2 + c - r): half the bytes back to the host */
 #define VIML_PTRS_DEVICE 0x100u          /* in/out pointers are device pointers; call is asynchronous  */
+#define VIML_SOLVE_DOGLEG 0x400u         /* viml_solve_vi: the dogleg strategy instead of Levenberg-Marquardt (other calls ignore it) */
 
 typedef struct viml_ctx viml_ctx;
 
@@ -389,13 +391,35 @@ int viml_gn_step_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inert
  * A stopped window's state, counters and outputs never change again.  The policy arithmetic is plain IEEE binary64 without fused
  * multiply-adds, so a scalar restatement reproduces it bit for bit.
  * Deviations from Ceres' Solve as the reference configures it:
- *   - the strategy is LEVENBERG_MARQUARDT; the reference asks for DOGLEG, which needs the full-space gradient and the Cauchy point;
+ *   - the strategy is LEVENBERG_MARQUARDT; the reference asks for DOGLEG, which VIML_SOLVE_DOGLEG selects (below);
  *   - the damping is viml_gn_step's lambda diag(Sx) on the landmark-reduced system (Ceres damps J^T J before the elimination and
  *     clamps the diagonal to [1e-6, 1e32]);
  *   - no gradient tolerance (the full-problem gradient is not formed) and no max_solver_time.
  * Input validation is viml_gn_step_vi's, plus the options below and the required outputs.  W == 0 returns VIML_OK.  With
  * VIML_PTRS_DEVICE the call neither synchronises nor reads anything back: all max_iterations rounds are enqueued on the context
- * stream, and rounds after every window has stopped do only the ungated work (linearisation, Schur step, IMU / prior evaluation).  */
+ * stream, and rounds after every window has stopped do only the ungated work (linearisation, Schur step, IMU / prior evaluation).
+ *
+ * VIML_SOLVE_DOGLEG: the same trust-region loop (order of the tests, tolerances, |dx|, |x|, counters, statuses) with Ceres'
+ * DoglegStrategy (traditional dogleg) and its default Jacobi scaling, restated from Ceres' documented behaviour (not pinned against
+ * its source).  initial_radius, max_radius and min_radius are the dogleg radius.  Over the N = D + X + F columns of the window's
+ * whole problem, H = the loss-corrected visual J^T J plus the IMU / prior J^T J at x, g = J^T r; a landmark with H_ll <= 1e-8 takes
+ * no part (every entry below is 0 for it).  s_i = 1 / (1 + sqrt(H_ii(x0))) once per solve; per window radius = initial_radius,
+ * mu = 1e-8, reuse = false.  A round that does not reuse forms:
+ *   d_i = sqrt(min(max(s_i^2 H_ii, 1e-6), 1e32)), gamma_i = s_i g_i / d_i, w_i = s_i gamma_i / d_i, alpha = |gamma|^2 / w^T H w
+ *   (0 when both are 0), and the Gauss-Newton step (H + mu diag(d^2 / s^2)) dgn = -g through the Schur step (landmark columns
+ *   damped before the elimination, the reduced columns on the reduced system's diagonal, the landmarks back-substituted with the
+ *   damped H_ll); n = d dgn / s.  It is invalid when mu >= 1 or the Cholesky fails.
+ * Every running round takes the step at the current radius: |n| <= radius: dgn; else alpha |gamma| >= radius:
+ *   -(radius / |gamma|) w; else Ceres' interpolation -alpha (1 - beta) w + beta dgn with beta on the boundary.  The model decrease is
+ *   -(g.step + step^T H step / 2), formed from the stored scalars.  The strategy's updates:
+ *   invalid: consecutive_invalid += 1, mu *= 10, the radius stays; the next round forms a new step;
+ *   accepted: rho < 1/4: radius /= 2; rho > 3/4: radius = min(max_radius, max(radius, 3 |step|_D)); mu = max(1e-8, 2 mu / 10);
+ *   rejected: radius /= 2, and the next round reuses the Gauss-Newton step and the Cauchy point (no new factorisation).
+ * trace column 3 is the radius the step was formed at; `radius` is the final radius.  Deviations from Ceres' DoglegStrategy:
+ *   - each round tries one mu; Ceres retries the factorisation inside the iteration up to its largest mu, here a failed
+ *     factorisation is an invalid step;
+ *   - the landmark eps rule above; the radius is capped at max_radius;
+ *   - no gradient tolerance and no max_solver_time, as for Levenberg-Marquardt.  */
 typedef struct viml_solve_options {
   int32_t max_iterations;           /* > 0; every computed step counts, accepted or not   (ceres: max_num_iterations, 50)         */
   int32_t max_consecutive_invalid;  /* >= 0                                                (max_num_consecutive_invalid_steps, 5)  */
@@ -423,8 +447,8 @@ typedef struct viml_solve_out {
   int32_t* accepted;    /* [W] steps accepted        */
   double* cost;         /* [W][2] f(x0), f(final state) */
   double* radius;       /* [W] final radius, or NULL */
-  double* trace;        /* [W][max_iterations][4] or NULL: f(x), f(x+), model decrease, lambda of every step; NaN rows after
-                           the window stopped */
+  double* trace;        /* [W][max_iterations][4] or NULL: f(x), f(x+), model decrease, lambda of every step (VIML_SOLVE_DOGLEG:
+                           the radius); NaN rows after the window stopped */
 } viml_solve_out;
 
 int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,

@@ -11,8 +11,8 @@ import os
 import numpy as np
 
 from . import _abi, build, parity, shard, synth  # noqa: F401
-from ._abi import (LOSS_CAUCHY, OUT_HB, OUT_RESIDUAL_JACOBIAN, OUT_SCHUR, PTRS_DEVICE, S_PACKED, Batch,  # noqa: F401
-                   make_config)
+from ._abi import (LOSS_CAUCHY, OUT_HB, OUT_RESIDUAL_JACOBIAN, OUT_SCHUR, PTRS_DEVICE, S_PACKED, SOLVE_DOGLEG,  # noqa: F401
+                   Batch, make_config)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VIML_LIB_PATH") or os.path.join(_HERE, "libviml_b200.so")   # override: A/B runs of kernel variants

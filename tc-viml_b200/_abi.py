@@ -21,6 +21,7 @@ LOSS_CAUCHY = 0x10
 S_PACKED = 0x20
 PTRS_DEVICE = 0x100
 FOV_CACHED = 0x200
+SOLVE_DOGLEG = 0x400
 FOV_SLOTS = 11
 BLOCK_POSE, BLOCK_EX, BLOCK_EXTRA = 0, 1, 2
 PRIOR_X0_STRIDE = 9

@@ -470,13 +470,17 @@ int viml_launch_reduced(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const 
 // lambda_w (nullable): a damping per window instead of `lambda`; running (nullable): only windows with running[w] != 0 are solved,
 // updated and costed (the others are left untouched).  viml_launch_gn_reduced_solve builds and solves the system in one kernel
 // (Dx = D + dn.X with gn_fused_takes(Dx)); viml_launch_gn_solve solves the Sx / gx of viml_launch_reduced.
+// damp (nullable): an additive damping per reduced column [W][Dx] instead of lambda diag(Sx).
 int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double lambda,
                                  double* dx, int32_t* solved, double* cost, const double* lambda_w = nullptr,
-                                 const int32_t* running = nullptr);
+                                 const int32_t* running = nullptr, const double* damp = nullptr);
 int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const double* Sx, const double* gx, double* dx, int32_t* solved,
-                         double* cost, const double* lambda_w = nullptr, const int32_t* running = nullptr);
+                         double* cost, const double* lambda_w = nullptr, const int32_t* running = nullptr,
+                         const double* damp = nullptr);
+// dl (nullable): the landmark increments [W][F], used instead of the back-substitution.
 int viml_launch_gn_update(viml_ctx* ctx, const LinearizeArgs& a, int X, const double* extra_in, const double* dx, const int32_t* solved,
-                          double* o_poses, double* o_ex, double* o_dep, double* o_extra, const int32_t* running = nullptr);
+                          double* o_poses, double* o_ex, double* o_dep, double* o_extra, const int32_t* running = nullptr,
+                          const double* dl = nullptr);
 int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const double* dx, const int32_t* solved, int slot,
                      double* cost, const int32_t* running = nullptr);
 
@@ -485,6 +489,25 @@ struct SolveState {
   double radius, decrease_factor;
   double f0, f;                 // f(x0), f at the current state x
   int32_t consecutive_invalid, iterations, accepted, status;
+  double mu;                    // VIML_SOLVE_DOGLEG: the Gauss-Newton step's damping
+  int32_t reuse;                // VIML_SOLVE_DOGLEG: the next step reuses the stored Gauss-Newton step and Cauchy point
+};
+// VIML_SOLVE_DOGLEG: what a window keeps between rounds (device pointers; N = Dx + F columns: poses / extrinsic, extra state, inverse
+// depths).  scal per window: |gamma|^2, n.n, gamma.n, w^T H w, w^T H dgn, dgn^T H dgn, valid (1 / 0), the chosen step's D-space norm.
+constexpr int kDoglegScal = 8;
+constexpr double kDoglegMinMu = 1e-8, kDoglegMaxMu = 1.0;
+struct DoglegArgs {
+  int Dx, F;
+  double* s;        // [W][N] Jacobi scaling, from H at x0
+  double* d;        // [W][N] sqrt(clamp(s^2 H_ii, 1e-6, 1e32)) at the point of the stored step
+  double* gamma;    // [W][N] s g / d
+  double* w;        // [W][N] s gamma / d  (the Cauchy direction in unscaled columns)
+  double* gn;       // [W][N] the Gauss-Newton step
+  double* hll;      // [W][F] undamped H_ll
+  double* damp;     // [W][Dx] mu d^2 / s^2 on the reduced columns
+  double* dl;       // [W][F] the landmark part of the chosen step
+  double* scal;     // [W][kDoglegScal]
+  int32_t* fresh;   // [W] running and not reusing: the round forms a new Gauss-Newton step
 };
 struct SolveArgs {  // device pointers only
   viml_solve_options opt;
@@ -498,9 +521,22 @@ struct SolveArgs {  // device pointers only
   const double* cost;           // [W][3]  this round's f(x), f(x+), model decrease
   const int32_t* solved;        // [W]
   viml_solve_out out;           // device pointers (radius, trace nullable)
+  const double* dogleg;         // [W][kDoglegScal] DoglegArgs::scal with VIML_SOLVE_DOGLEG, else null (Levenberg-Marquardt)
+  int32_t* fresh;               // DoglegArgs::fresh, written for the next round (VIML_SOLVE_DOGLEG)
 };
 // One CTA per window: applies the policy of viml.h to this round's step (round 0 also starts the state from the options).
 int viml_launch_solve_policy(viml_ctx* ctx, int W, const SolveArgs& s, int round);
+// VIML_SOLVE_DOGLEG, one CTA per window (round 0: every window, radius = initial_radius, mu = kDoglegMinMu; later rounds read the state):
+// dogleg_prepare (fresh windows, after the assembly at x, before the Schur step) forms s (round 0), d, gamma, w, w^T H w and the
+// damping, which it adds to a.out.H_ll; dogleg_finish (fresh windows, after the solve) back-substitutes the landmarks with the damped
+// H_ll and stores the Gauss-Newton step and its scalars; dogleg_step (running windows) writes the step at the current radius into dx /
+// g.dl, its model decrease into cost[3w + 2] and its validity into solved.
+int viml_launch_dogleg_prepare(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const DoglegArgs& g, const SolveState* state,
+                               int round);
+int viml_launch_dogleg_finish(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const DoglegArgs& g, const SolveState* state,
+                              int round, const double* dx, const int32_t* solved);
+int viml_launch_dogleg_step(viml_ctx* ctx, int W, const DoglegArgs& g, const SolveState* state, double initial_radius, int round,
+                            const int32_t* running, double* dx, double* cost, int32_t* solved);
 // schur_kernels.cu
 int viml_launch_schur(viml_ctx* ctx, int W, int F, int D, const double* H_pp, const double* H_lp, const double* H_ll,
                       const double* b_p, const double* b_l, double* S, double* g, double eps);

@@ -231,16 +231,35 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
   return VIML_OK;
 }
 
+// One dogleg round of viml_solve_vi (VIML_SOLVE_DOGLEG): the per-window storage, the trust-region state it reads and the round.
+struct DoglegRound {
+  const DoglegArgs* g;
+  const SolveState* state;
+  double initial_radius;
+  int round;
+};
+
 // One step at the state of s.b.a / s.extra: without s.cost the reduced system Sx, gx alone; with it the cost at x, the solve (the
 // system built in the solve kernel when s.fused), the update into s.o_* and the cost at x+.  lambda_w / running: see
 // viml_launch_gn_reduced_solve (nullptr: `lambda`, every window).
+// dg (nullable): the step is the dogleg step of viml.h instead.  The round linearises without the Schur step, forms the damping
+// (dogleg_prepare) and runs the Schur step itself on the damped H_ll; the solve and dogleg_finish run where dg->g->fresh is set
+// (round 0: every window), dogleg_step and everything after it where `running` is.
 // With s.vi the dense-block factors are the window's prior and IMU factors, evaluated on the device at x (system, cost[0]) and at
 // x+ (cost[1], exactly); s.dn is then replaced by their CSR.
-int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* lambda_w, const int32_t* running) {
+int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* lambda_w, const int32_t* running,
+                 const DoglegRound* dg = nullptr) {
   const LinearizeArgs& a = s.b.a;
   const int W = s.W, D = a.D, X = s.X, Dx = s.Dx;
   const bool step = s.cost != nullptr;
-  int rc = viml_launch_linearize(ctx, a);
+  int rc;
+  if (dg) {
+    LinearizeArgs al = a;
+    al.flags &= ~VIML_OUT_SCHUR;
+    rc = viml_launch_linearize(ctx, al);
+  } else {
+    rc = viml_launch_linearize(ctx, a);
+  }
   if (rc != VIML_OK) return rc;
   DenseArgs dn = s.dn;
   InertialArgs va = s.va;
@@ -255,13 +274,31 @@ int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* 
   if (!step) return viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
   rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
   if (rc != VIML_OK) return rc;
-  if (s.fused) {
+  if (dg) {
+    const DoglegArgs& g = *dg->g;
+    const int32_t* fresh = dg->round ? g.fresh : nullptr;
+    rc = viml_launch_dogleg_prepare(ctx, a, dn, g, dg->state, dg->round);
+    if (rc != VIML_OK) return rc;
+    // MarginalizationInfo::eps, as in viml_launch_linearize
+    rc = viml_launch_schur(ctx, W, a.F, D, a.out.H_pp, a.out.H_lp, a.out.H_ll, a.out.b_p, a.out.b_l, a.out.S, a.out.g, 1e-8);
+    if (rc == VIML_OK && s.fused) {
+      rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, 0.0, s.dx, s.solved, s.cost, nullptr, fresh, g.damp);
+    } else if (rc == VIML_OK) {
+      rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
+      if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, 0.0, s.Sx, s.gx, s.dx, s.solved, s.cost, nullptr, fresh, g.damp);
+    }
+    if (rc == VIML_OK) rc = viml_launch_dogleg_finish(ctx, a, dn, g, dg->state, dg->round, s.dx, s.solved);
+    if (rc == VIML_OK) rc = viml_launch_dogleg_step(ctx, W, g, dg->state, dg->initial_radius, dg->round, running, s.dx, s.cost, s.solved);
+    if (rc == VIML_OK)
+      rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running, g.dl);
+  } else if (s.fused) {
     rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, lambda, s.dx, s.solved, s.cost, lambda_w, running);
   } else {
     rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
     if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, lambda, s.Sx, s.gx, s.dx, s.solved, s.cost, lambda_w, running);
   }
-  if (rc == VIML_OK) rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running);
+  if (rc == VIML_OK && !dg)
+    rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running);
   if (rc != VIML_OK) return rc;
   LinearizeArgs a2 = a;
   a2.poses = s.o_poses, a2.ex_pose = s.o_ex, a2.inv_depth = s.o_dep;
@@ -437,6 +474,18 @@ int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertia
   st.out(out->cost, (size_t)W * 2, &sa.out.cost);
   st.out(out->radius, out->radius ? (size_t)W : 0, &sa.out.radius);
   st.out(out->trace, out->trace ? (size_t)W * M * 4 : 0, &sa.out.trace);
+  const bool dogleg = (flags & VIML_SOLVE_DOGLEG) != 0;
+  DoglegArgs g{};
+  if (dogleg) {
+    const size_t N = (size_t)s.Dx + F;
+    g.Dx = s.Dx, g.F = F;
+    for (double** p : {&g.s, &g.d, &g.gamma, &g.w, &g.gn}) st.out((double*)nullptr, (size_t)W * N, p);
+    st.out((double*)nullptr, (size_t)W * F, &g.hll);
+    st.out((double*)nullptr, (size_t)W * F, &g.dl);
+    st.out((double*)nullptr, (size_t)W * s.Dx, &g.damp);
+    st.out((double*)nullptr, (size_t)W * kDoglegScal, &g.scal);
+    st.out((int32_t*)nullptr, (size_t)W, &g.fresh);
+  }
   rc = st.commit();
   if (rc == VIML_OK) rc = expand_tables(ctx, s.b);
   if (rc != VIML_OK) return rc;
@@ -449,10 +498,13 @@ int viml_solve_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertia
   s.b.a.poses = sa.x_poses, s.b.a.ex_pose = sa.x_ex, s.b.a.inv_depth = sa.x_dep, s.extra = sa.x_extra;
   sa.p_poses = s.o_poses, sa.p_ex = s.o_ex, sa.p_dep = s.o_dep, sa.p_extra = s.o_extra;
   sa.dx = s.dx, sa.cost = s.cost, sa.solved = s.solved;
+  if (dogleg) sa.dogleg = g.scal, sa.fresh = g.fresh;
   // round 0 runs every window at lambda = 1 / initial_radius; policy_kernel then starts each window's state from that step and
   // hands the next round its running flags and lambdas
+  // (dogleg: round 0 forms every window's step at initial_radius and mu = 1e-8)
   for (int r = 0; r < M && rc == VIML_OK; ++r) {
-    rc = enqueue_step(ctx, s, 1.0 / opt->initial_radius, r ? sa.lambda_w : nullptr, r ? sa.running : nullptr);
+    const DoglegRound dg{&g, sa.state, opt->initial_radius, r};
+    rc = enqueue_step(ctx, s, 1.0 / opt->initial_radius, r ? sa.lambda_w : nullptr, r ? sa.running : nullptr, dogleg ? &dg : nullptr);
     if (rc == VIML_OK) rc = viml_launch_solve_policy(ctx, W, sa, r);
   }
   if (rc != VIML_OK) return rc;

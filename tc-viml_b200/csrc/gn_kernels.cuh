@@ -127,18 +127,21 @@ constexpr int kTile = 8;
 __device__ __forceinline__ int tile_at(int I, int J) { return (I * (I + 1) / 2 + J) * 64; }
 
 // lambda_w (nullable): a damping per window instead of `lambda`; running (nullable): a window with running[w] == 0 is skipped
-// (its CTA returns at once and writes nothing).
+// (its CTA returns at once and writes nothing); damp (nullable): (Sx + diag(damp_w)) dx = -gx, an additive damping per column
+// instead of lambda diag(Sx).
 template <bool FUSED>
 __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda, const double* __restrict__ Sx, const double* __restrict__ gx,
                                                           double* __restrict__ dx, int32_t* __restrict__ solved, double* __restrict__ cost,
                                                           int D, DenseArgs dn, const double* __restrict__ S, const double* __restrict__ g,
-                                                          const double* __restrict__ lambda_w, const int32_t* __restrict__ running) {
+                                                          const double* __restrict__ lambda_w, const int32_t* __restrict__ running,
+                                                          const double* __restrict__ damp) {
   extern __shared__ __align__(16) double sm[];
   __shared__ int s_ok;
   __shared__ double s_red[8], s_dinv[kTile];
   const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   if (running && !running[w]) return;
   if (lambda_w) lambda = lambda_w[w];
+  const double* __restrict__ dmp = damp ? damp + (size_t)w * Dx : nullptr;
   const int NB = (Dx + kTile - 1) / kTile, Dp = NB * kTile;
   double* __restrict__ L = sm;                                   // NB (NB + 1) / 2 tiles
   double* __restrict__ y = sm + (size_t)NB * (NB + 1) / 2 * 64;  // [Dp]
@@ -178,7 +181,10 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
     for (int i = tid; i < Dp; i += 256) {
       double& d = L[tile_at(i >> 3, i >> 3) + (i & 7) * 8 + (i & 7)];
       dv[i] = d;
-      if (i < Dx) d *= 1.0 + lambda;
+      if (i < Dx) {
+        if (dmp) d += dmp[i];
+        else d *= 1.0 + lambda;
+      }
       y[i] = -gv[i];
     }
   } else {
@@ -194,7 +200,8 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
           const int e = e0 + u * 256;
           if (e >= Dx * Dx) break;
           const int i = e / Dx, j = e - i * Dx;
-          if (pass == 0 && j <= i) L[tile_at(i >> 3, j >> 3) + (i & 7) * 8 + (j & 7)] = (i == j) ? v[u] * (1.0 + lambda) : 0.5 * v[u];
+          if (pass == 0 && j <= i)
+            L[tile_at(i >> 3, j >> 3) + (i & 7) * 8 + (j & 7)] = (i == j) ? (dmp ? v[u] + dmp[i] : v[u] * (1.0 + lambda)) : 0.5 * v[u];
           if (pass == 1 && j > i) L[tile_at(j >> 3, i >> 3) + (j & 7) * 8 + (i & 7)] += 0.5 * v[u];
         }
       }
@@ -331,10 +338,10 @@ __global__ void __launch_bounds__(256) solve_tiled_kernel(int Dx, double lambda,
   // model decrease with the undamped Sx: -g.x - x.Sx x / 2 (exactly 0 for a window that was not solved, even when its system
   // holds a NaN or an infinity)
   double part = 0.0;
-  if (FUSED) {   // (Sx + lambda diag d) x = -g  =>  x.Sx x = -g.x - lambda sum d_i x_i^2
+  if (FUSED) {   // (Sx + lambda diag d) x = -g  =>  x.Sx x = -g.x - lambda sum d_i x_i^2  (damp_i in place of lambda d_i)
     for (int i = tid; i < Dx; i += 256) {
       const double xi = ok ? y[i] : 0.0;
-      if (ok) part += -0.5 * gv[i] * xi + 0.5 * lambda * dv[i] * xi * xi;
+      if (ok) part += -0.5 * gv[i] * xi + 0.5 * (dmp ? dmp[i] : lambda * dv[i]) * xi * xi;
       dx[(size_t)w * Dx + i] = xi;
     }
   } else {       // a warp per row of Sx (coalesced), lanes over the columns
@@ -376,12 +383,12 @@ __device__ __forceinline__ void pose_plus(const double* __restrict__ x, const do
   o[3] = qx / n, o[4] = qy / n, o[5] = qz / n, o[6] = w / n;
 }
 
-// New state of every window: poses / extrinsic by Plus, landmarks by back-substitution, extra state by addition.  running
-// (nullable): windows with running[w] == 0 are skipped.
+// New state of every window: poses / extrinsic by Plus, landmarks by back-substitution (or by the increments dl_in when given),
+// extra state by addition.  running (nullable): windows with running[w] == 0 are skipped.
 __global__ void __launch_bounds__(128) update_kernel(LinearizeArgs A, int X, const double* __restrict__ extra_in, const double* __restrict__ dx,
                                                      const int32_t* __restrict__ solved, double* __restrict__ o_poses,
                                                      double* __restrict__ o_ex, double* __restrict__ o_dep, double* __restrict__ o_extra,
-                                                     const int32_t* __restrict__ running) {
+                                                     const int32_t* __restrict__ running, const double* __restrict__ dl_in) {
   const int w = blockIdx.x, tid = threadIdx.x, P = A.P, F = A.F, D = A.D, Dx = D + X;
   if (running && !running[w]) return;
   const bool ok = solved[w] != 0;
@@ -398,8 +405,10 @@ __global__ void __launch_bounds__(128) update_kernel(LinearizeArgs A, int X, con
   for (int l = tid; l < F; l += blockDim.x) {
     const double lam = A.inv_depth[(size_t)w * F + l];
     double dl = 0.0;
-    const double hll = A.out.H_ll[(size_t)w * F + l];
-    if (ok && hll > 1e-8) {
+    const double hll = dl_in ? 0.0 : A.out.H_ll[(size_t)w * F + l];
+    if (ok && dl_in) {
+      dl = dl_in[(size_t)w * F + l];
+    } else if (ok && hll > 1e-8) {
       const double* __restrict__ row = A.out.H_lp + ((size_t)w * F + l) * D;
       double s = A.out.b_l[(size_t)w * F + l];
       for (int c = 0; c < D; ++c) s = fma(row[c], d[c], s);
@@ -474,11 +483,258 @@ __global__ void __launch_bounds__(128) cost_kernel(LinearizeArgs A, DenseArgs dn
   }
 }
 
+// ---- the dogleg strategy of viml_solve_vi (VIML_SOLVE_DOGLEG, viml.h) -----------------------------------------------------------
+// The full problem has N = Dx + F columns; H is the loss-corrected visual J^T J (H_pp, H_lp, diagonal H_ll) plus the dense-block
+// factors' J^T J, g = J^T r.  A landmark with H_ll <= 1e-8 takes no part (the Schur step's eps rule): its entries are 0 throughout.
+// Every reduction below has a fixed order (per thread, then the warp's shuffle tree, then the warps in order), so a window's result
+// depends on nothing but its own inputs.
+constexpr double kDoglegEps = 1e-8;
+
+// The sum over the CTA of one value per thread (NW warps), in a fixed order; every thread gets it.
+template <int NW>
+__device__ __forceinline__ double cta_sum(double v, double* s_red) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  __syncthreads();
+  if (lane == 0) s_red[warp] = v;
+  __syncthreads();
+  double t = 0.0;
+#pragma unroll
+  for (int k = 0; k < NW; ++k) t += s_red[k];
+  return t;
+}
+
+__device__ __forceinline__ double dogleg_d(double s, double h) {   // Ceres' D-space diagonal of the scaled column
+  return sqrt(fmin(fmax(s * s * h, 1e-6), 1e32));
+}
+
+// Kernel A, fresh windows, after the assembly and the inertial evaluation at x and before the Schur step: diag(H), g, s (round 0),
+// d, gamma, w, |gamma|^2, w^T H w, the damping of the reduced columns, and the damping of the landmark columns added to H_ll (whose
+// undamped values are kept in g.hll).
+__global__ void __launch_bounds__(256) dogleg_prepare_kernel(LinearizeArgs A, DenseArgs dn, DoglegArgs G, const SolveState* __restrict__ state,
+                                                             int round) {
+  __shared__ double s_h[kMaxDx], s_g[kMaxDx], s_w[kMaxDx], s_red[8];
+  const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (round > 0 && !G.fresh[w]) return;
+  const int D = A.D, F = A.F, Dx = G.Dx, N = Dx + F;
+  const double mu = round > 0 ? state[w].mu : kDoglegMinMu;
+  const double* __restrict__ Hpp = A.out.H_pp + (size_t)w * D * D;
+  const double* __restrict__ Hlp = A.out.H_lp + (size_t)w * F * D;
+  double* __restrict__ Hll = A.out.H_ll + (size_t)w * F;
+  const double* __restrict__ bl = A.out.b_l + (size_t)w * F;
+  double *sw = G.s + (size_t)w * N, *dw = G.d + (size_t)w * N, *gw = G.gamma + (size_t)w * N, *ww = G.w + (size_t)w * N;
+  for (int i = tid; i < Dx; i += 256) {
+    s_h[i] = i < D ? Hpp[(size_t)i * D + i] : 0.0;
+    s_g[i] = i < D ? A.out.b_p[(size_t)w * D + i] : 0.0;
+  }
+  __syncthreads();
+  if (dn.ND > 0)   // one factor after the other; inside a factor every column is a different one
+    for (int k = dn.window_offset[w]; k < dn.window_offset[w + 1]; ++k) {
+      const DenseFactor f = dense_factor(dn, k);
+      for (int a = tid; a < f.c; a += 256) {
+        double hh = 0.0, gg = 0.0;
+        for (int q = 0; q < f.n; ++q) {
+          const double j = f.J[(size_t)q * f.c + a];
+          hh = fma(j, j, hh);
+          gg = fma(j, f.r[q], gg);
+        }
+        s_h[f.ci[a]] += hh;
+        s_g[f.ci[a]] += gg;
+      }
+      __syncthreads();
+    }
+  double gg = 0.0, whw = 0.0;
+  for (int i = tid; i < Dx; i += 256) {
+    const double h = s_h[i];
+    if (round == 0) sw[i] = 1.0 / (1.0 + sqrt(h));
+    const double si = sw[i], di = dogleg_d(si, h);
+    const double gam = si * s_g[i] / di, wi = si * gam / di;
+    dw[i] = di, gw[i] = gam, ww[i] = wi, s_w[i] = wi;
+    G.damp[(size_t)w * Dx + i] = mu * (di * di) / (si * si);
+    gg += gam * gam;
+  }
+  for (int l = tid; l < F; l += 256) {
+    const double h = Hll[l];
+    G.hll[(size_t)w * F + l] = h;
+    if (round == 0) sw[Dx + l] = 1.0 / (1.0 + sqrt(h));
+    double di = 0.0, gam = 0.0, wl = 0.0;
+    if (h > kDoglegEps) {
+      const double si = sw[Dx + l];
+      di = dogleg_d(si, h);
+      gam = si * bl[l] / di, wl = si * gam / di;
+      Hll[l] = h + mu * (di * di) / (si * si);
+      gg += gam * gam;
+      whw += h * wl * wl;
+    }
+    dw[Dx + l] = di, gw[Dx + l] = gam, ww[Dx + l] = wl;
+  }
+  __syncthreads();
+  for (int i = warp; i < D; i += 8) {   // w_p^T H_pp w_p: a warp per row
+    double t = 0.0;
+    for (int c = lane; c < D; c += 32) t = fma(Hpp[(size_t)i * D + c], s_w[c], t);
+    whw += t * s_w[i];
+  }
+  for (int l = warp; l < F; l += 8) {   // 2 w_l (H_lp w_p)_l
+    const double wl = ww[Dx + l];
+    if (wl == 0.0) continue;
+    double t = 0.0;
+    for (int c = lane; c < D; c += 32) t = fma(Hlp[(size_t)l * D + c], s_w[c], t);
+    whw += 2.0 * wl * t;
+  }
+  if (dn.ND > 0)   // |J_k w|^2
+    for (int k = dn.window_offset[w]; k < dn.window_offset[w + 1]; ++k) {
+      const DenseFactor f = dense_factor(dn, k);
+      for (int q = tid; q < f.n; q += 256) {
+        double v = 0.0;
+        for (int a = 0; a < f.c; ++a) v = fma(f.J[(size_t)q * f.c + a], s_w[f.ci[a]], v);
+        whw += v * v;
+      }
+    }
+  gg = cta_sum<8>(gg, s_red);
+  whw = cta_sum<8>(whw, s_red);
+  if (tid == 0) G.scal[(size_t)w * kDoglegScal + 0] = gg, G.scal[(size_t)w * kDoglegScal + 3] = whw;
+}
+
+// Kernel B, fresh windows, after the solve of the damped reduced system (dx): the landmarks back-substituted with the damped H_ll
+// (still in A.out.H_ll), the Gauss-Newton step dgn stored, n = d dgn / s, and n.n, gamma.n, w^T H dgn, dgn^T H dgn, valid.
+__global__ void __launch_bounds__(256) dogleg_finish_kernel(LinearizeArgs A, DenseArgs dn, DoglegArgs G, const SolveState* __restrict__ state,
+                                                            int round, const double* __restrict__ dx, const int32_t* __restrict__ solved) {
+  __shared__ double s_d[kMaxDx], s_w[kMaxDx], s_red[8];
+  const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (round > 0 && !G.fresh[w]) return;
+  const int D = A.D, F = A.F, Dx = G.Dx, N = Dx + F;
+  const double mu = round > 0 ? state[w].mu : kDoglegMinMu;
+  const double* __restrict__ Hpp = A.out.H_pp + (size_t)w * D * D;
+  const double* __restrict__ Hlp = A.out.H_lp + (size_t)w * F * D;
+  const double* __restrict__ Hd = A.out.H_ll + (size_t)w * F;
+  const double* __restrict__ bl = A.out.b_l + (size_t)w * F;
+  const double* __restrict__ h0 = G.hll + (size_t)w * F;
+  const double *sw = G.s + (size_t)w * N, *dw = G.d + (size_t)w * N, *gw = G.gamma + (size_t)w * N, *ww = G.w + (size_t)w * N;
+  double* __restrict__ gn = G.gn + (size_t)w * N;
+  double nn = 0.0, gnn = 0.0, whd = 0.0, dhd = 0.0;
+  for (int i = tid; i < Dx; i += 256) {
+    const double v = dx[(size_t)w * Dx + i];
+    s_d[i] = v, s_w[i] = ww[i], gn[i] = v;
+    const double n = dw[i] * v / sw[i];
+    nn += n * n;
+    gnn += gw[i] * n;
+  }
+  __syncthreads();
+  for (int i = warp; i < D; i += 8) {   // (H_pp dgn_p)_i against w_i and dgn_i
+    double t = 0.0;
+    for (int c = lane; c < D; c += 32) t = fma(Hpp[(size_t)i * D + c], s_d[c], t);
+    whd += s_w[i] * t, dhd += s_d[i] * t;   // the lanes' partial sums
+  }
+  for (int l = warp; l < F; l += 8) {
+    double td = 0.0, tw = 0.0;
+    for (int c = lane; c < D; c += 32) {
+      const double h = Hlp[(size_t)l * D + c];
+      td = fma(h, s_d[c], td);
+      tw = fma(h, s_w[c], tw);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) td += __shfl_xor_sync(0xffffffffu, td, o), tw += __shfl_xor_sync(0xffffffffu, tw, o);
+    if (lane == 0) {
+      const double h = h0[l];
+      double v = 0.0;
+      if (h > kDoglegEps) {
+        v = -(bl[l] + td) / Hd[l];
+        const double wl = ww[Dx + l], n = dw[Dx + l] * v / sw[Dx + l];
+        nn += n * n;
+        gnn += gw[Dx + l] * n;
+        whd += wl * td + v * tw + h * wl * v;
+        dhd += 2.0 * v * td + h * v * v;
+      }
+      gn[Dx + l] = v;
+    }
+  }
+  if (dn.ND > 0)   // (J_k w) . (J_k dgn) and |J_k dgn|^2
+    for (int k = dn.window_offset[w]; k < dn.window_offset[w + 1]; ++k) {
+      const DenseFactor f = dense_factor(dn, k);
+      for (int q = tid; q < f.n; q += 256) {
+        double jw = 0.0, jd = 0.0;
+        for (int a = 0; a < f.c; ++a) {
+          const double j = f.J[(size_t)q * f.c + a];
+          jw = fma(j, s_w[f.ci[a]], jw);
+          jd = fma(j, s_d[f.ci[a]], jd);
+        }
+        whd += jw * jd;
+        dhd += jd * jd;
+      }
+    }
+  nn = cta_sum<8>(nn, s_red);
+  gnn = cta_sum<8>(gnn, s_red);
+  whd = cta_sum<8>(whd, s_red);
+  dhd = cta_sum<8>(dhd, s_red);
+  if (tid == 0) {
+    double* sc = G.scal + (size_t)w * kDoglegScal;
+    sc[1] = nn, sc[2] = gnn, sc[4] = whd, sc[5] = dhd;
+    sc[6] = (solved[w] && mu < kDoglegMaxMu) ? 1.0 : 0.0;
+  }
+}
+
+// Kernel C, running windows: Ceres' traditional dogleg step at the current radius from the stored scalars (scalar __d*_rn arithmetic,
+// restated by tests/dogleg_policy.py), as a w + b dgn: its reduced part into dx, its landmark part into G.dl, its model decrease
+// -(g.step + step^T H step / 2) into cost[3w + 2], its D-space norm into scal[7] and its validity into solved.
+__global__ void __launch_bounds__(128) dogleg_step_kernel(DoglegArgs G, const SolveState* __restrict__ state, double initial_radius, int round,
+                                                          const int32_t* __restrict__ running, double* __restrict__ dx,
+                                                          double* __restrict__ cost, int32_t* __restrict__ solved) {
+  __shared__ double s_ab[2];
+  const int w = blockIdx.x, tid = threadIdx.x, Dx = G.Dx, F = G.F, N = Dx + F;
+  if (running && !running[w]) return;
+  double* __restrict__ sc = G.scal + (size_t)w * kDoglegScal;
+  if (tid == 0) {
+    const double radius = round > 0 ? state[w].radius : initial_radius;
+    const double gg = sc[0], nn = sc[1], gnn = sc[2], whw = sc[3], whd = sc[4], dhd = sc[5];
+    const bool valid = sc[6] != 0.0;
+    double a = 0.0, b = 0.0, norm = 0.0, m = 0.0;
+    if (valid) {
+      const double gnorm = sqrt(gg), nnorm = sqrt(nn);
+      const double alpha = (gg == 0.0 && whw == 0.0) ? 0.0 : __ddiv_rn(gg, whw);
+      if (nnorm <= radius) {                               // 1. the Gauss-Newton step
+        b = 1.0, norm = nnorm;
+      } else if (__dmul_rn(alpha, gnorm) >= radius) {     // 2. along the gradient to the boundary
+        a = -__ddiv_rn(radius, gnorm), norm = radius;
+      } else {                                             // 3. from the Cauchy point towards the Gauss-Newton step
+        const double ag = __dmul_rn(alpha, gnorm), a2 = __dmul_rn(ag, ag);
+        const double ba = -__dmul_rn(alpha, gnn);
+        const double c = __dsub_rn(ba, a2);
+        const double bma = __dadd_rn(__dsub_rn(a2, __dmul_rn(2.0, ba)), nn);
+        const double r2a = __dsub_rn(__dmul_rn(radius, radius), a2);
+        const double dd = sqrt(__dadd_rn(__dmul_rn(c, c), __dmul_rn(bma, r2a)));
+        const double beta = c <= 0.0 ? __ddiv_rn(__dsub_rn(dd, c), bma) : __ddiv_rn(r2a, __dadd_rn(dd, c));
+        a = -__dmul_rn(alpha, __dsub_rn(1.0, beta)), b = beta;
+        norm = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(__dmul_rn(a, a), gg), __dmul_rn(__dmul_rn(2.0, __dmul_rn(a, b)), gnn)),
+                              __dmul_rn(__dmul_rn(b, b), nn)));
+      }
+      const double lin = __dadd_rn(__dmul_rn(a, gg), __dmul_rn(b, gnn));
+      const double quad = __dadd_rn(__dadd_rn(__dmul_rn(__dmul_rn(a, a), whw), __dmul_rn(__dmul_rn(2.0, __dmul_rn(a, b)), whd)),
+                                    __dmul_rn(__dmul_rn(b, b), dhd));
+      m = -__dadd_rn(lin, __dmul_rn(0.5, quad));
+    }
+    sc[7] = norm;
+    cost[3 * (size_t)w + 2] = m;
+    solved[w] = valid ? 1 : 0;
+    s_ab[0] = valid ? a : 0.0, s_ab[1] = valid ? b : 0.0;
+  }
+  __syncthreads();
+  const double a = s_ab[0], b = s_ab[1];
+  const bool any = a != 0.0 || b != 0.0;
+  const double *ww = G.w + (size_t)w * N, *gn = G.gn + (size_t)w * N;
+  for (int i = tid; i < N; i += 128) {
+    const double v = any ? __dadd_rn(__dmul_rn(a, ww[i]), __dmul_rn(b, gn[i])) : 0.0;
+    if (i < Dx) dx[(size_t)w * Dx + i] = v;
+    else G.dl[(size_t)w * F + i - Dx] = v;
+  }
+}
+
 // ---- the trust-region policy of viml_solve_vi (viml.h) -------------------------------------------------------------------------
 // One CTA per window after each round's step.  A stopped window only writes a NaN trace row.  A running one reduces |dx| (the
 // reduced step and the landmark increments x+ - x) and |x|, then thread 0 applies the policy; the scalar arithmetic goes through
 // __d*_rn so that no multiply-add is fused, and an IEEE restatement (tests/solve_policy.py) reproduces the radius, the decisions and
 // the trace bit for bit.  The CTA then moves x+ into x on acceptance and, at the window's last step, x into the outputs.
+// s.dogleg != null: the strategy updates are the dogleg's (viml.h, VIML_SOLVE_DOGLEG; tests/dogleg_policy.py restates them).
 __global__ void __launch_bounds__(128) policy_kernel(SolveArgs s, int round) {
   __shared__ double s_red[2][4];
   __shared__ int s_accept, s_stop;
@@ -514,23 +770,30 @@ __global__ void __launch_bounds__(128) policy_kernel(SolveArgs s, int round) {
   __syncthreads();
   if (tid == 0) {
     const viml_solve_options& o = s.opt;
+    const bool dogleg = s.dogleg != nullptr;
     SolveState st = s.state[w];
     const double f = s.cost[3 * (size_t)w], fp = s.cost[3 * (size_t)w + 1], m = s.cost[3 * (size_t)w + 2];
     int accept = 0, status = -1;
     if (round == 0) {   // f(x0) is this round's f(x)
       st.radius = o.initial_radius, st.decrease_factor = 2.0, st.f0 = f, st.f = f;
       st.consecutive_invalid = st.iterations = st.accepted = 0;
+      st.mu = kDoglegMinMu, st.reuse = 0;
       if (!isfinite(f)) status = VIML_SOLVE_FAILURE;
     }
     if (status >= 0) {
       if (trow) trow[0] = trow[1] = trow[2] = trow[3] = nan;
     } else {
-      if (trow) trow[0] = f, trow[1] = fp, trow[2] = m, trow[3] = __ddiv_rn(1.0, st.radius);
+      if (trow) trow[0] = f, trow[1] = fp, trow[2] = m, trow[3] = dogleg ? st.radius : __ddiv_rn(1.0, st.radius);
       st.f = f;
       if (!s.solved[w] || !isfinite(fp) || !(m > 0.0)) {
         st.consecutive_invalid += 1;
-        st.radius = __ddiv_rn(st.radius, st.decrease_factor);
-        st.decrease_factor = __dmul_rn(st.decrease_factor, 2.0);
+        if (dogleg) {   // the radius stays; a new Gauss-Newton step with ten times the damping
+          st.mu = __dmul_rn(st.mu, 10.0);
+          st.reuse = 0;
+        } else {
+          st.radius = __ddiv_rn(st.radius, st.decrease_factor);
+          st.decrease_factor = __dmul_rn(st.decrease_factor, 2.0);
+        }
         if (st.consecutive_invalid > o.max_consecutive_invalid) status = VIML_SOLVE_FAILURE;
       } else {
         st.consecutive_invalid = 0;
@@ -546,11 +809,27 @@ __global__ void __launch_bounds__(128) policy_kernel(SolveArgs s, int round) {
             accept = 1;
             st.accepted += 1;
             st.f = fp;
-            const double t = __dsub_rn(__dmul_rn(2.0, rho), 1.0);
-            const double c = __dsub_rn(1.0, __dmul_rn(__dmul_rn(t, t), t)), third = 1.0 / 3.0;
-            const double r = __ddiv_rn(st.radius, c > third ? c : third);
-            st.radius = r < o.max_radius ? r : o.max_radius;
-            st.decrease_factor = 2.0;
+            if (dogleg) {
+              if (rho < 0.25) {
+                st.radius = __dmul_rn(st.radius, 0.5);
+              } else if (rho > 0.75) {
+                const double r3 = __dmul_rn(3.0, s.dogleg[(size_t)w * kDoglegScal + 7]);
+                const double r = st.radius > r3 ? st.radius : r3;
+                st.radius = r < o.max_radius ? r : o.max_radius;
+              }
+              const double mu = __ddiv_rn(__dmul_rn(2.0, st.mu), 10.0);
+              st.mu = mu > kDoglegMinMu ? mu : kDoglegMinMu;
+              st.reuse = 0;
+            } else {
+              const double t = __dsub_rn(__dmul_rn(2.0, rho), 1.0);
+              const double c = __dsub_rn(1.0, __dmul_rn(__dmul_rn(t, t), t)), third = 1.0 / 3.0;
+              const double r = __ddiv_rn(st.radius, c > third ? c : third);
+              st.radius = r < o.max_radius ? r : o.max_radius;
+              st.decrease_factor = 2.0;
+            }
+          } else if (dogleg) {   // the next round reuses the Gauss-Newton step and the Cauchy point at half the radius
+            st.radius = __dmul_rn(st.radius, 0.5);
+            st.reuse = 1;
           } else {
             st.radius = __ddiv_rn(st.radius, st.decrease_factor);
             st.decrease_factor = __dmul_rn(st.decrease_factor, 2.0);
@@ -567,12 +846,14 @@ __global__ void __launch_bounds__(128) policy_kernel(SolveArgs s, int round) {
     s.state[w] = st;
     if (status >= 0) {
       s.running[w] = 0;
+      if (dogleg) s.fresh[w] = 0;
       s.out.status[w] = status, s.out.iterations[w] = st.iterations, s.out.accepted[w] = st.accepted;
       s.out.cost[2 * (size_t)w] = st.f0, s.out.cost[2 * (size_t)w + 1] = st.f;
       if (s.out.radius) s.out.radius[w] = st.radius;
     } else {
       s.running[w] = 1;
-      s.lambda_w[w] = __ddiv_rn(1.0, st.radius);
+      if (dogleg) s.fresh[w] = !st.reuse;
+      else s.lambda_w[w] = __ddiv_rn(1.0, st.radius);
     }
     s_accept = accept, s_stop = status >= 0;
   }

@@ -671,32 +671,33 @@ int viml_launch_reduced(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const 
 }
 
 int viml_launch_gn_solve(viml_ctx* ctx, int W, int Dx, double lambda, const double* Sx, const double* gx, double* dx, int32_t* solved,
-                         double* cost, const double* lambda_w, const int32_t* running) {
+                         double* cost, const double* lambda_w, const int32_t* running, const double* damp) {
   const size_t smem = gn_solve_smem(Dx);
   LaunchScope ls(ctx, K_GN);
   VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   gn::solve_tiled_kernel<false><<<W, 256, smem, ctx->stream>>>(Dx, lambda, Sx, gx, dx, solved, cost, 0, DenseArgs{}, nullptr, nullptr,
-                                                                lambda_w, running);
+                                                                lambda_w, running, damp);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
 
 int viml_launch_gn_reduced_solve(viml_ctx* ctx, int W, int D, const DenseArgs& dn, const double* S, const double* g, double lambda,
-                                 double* dx, int32_t* solved, double* cost, const double* lambda_w, const int32_t* running) {
+                                 double* dx, int32_t* solved, double* cost, const double* lambda_w, const int32_t* running,
+                                 const double* damp) {
   const int Dx = D + dn.X;
   const size_t smem = gn_fused_solve_smem(Dx);
   LaunchScope ls(ctx, K_GN);
   VIML_TRY_CUDA(ctx, cudaFuncSetAttribute(gn::solve_tiled_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   gn::solve_tiled_kernel<true><<<W, 256, smem, ctx->stream>>>(Dx, lambda, nullptr, nullptr, dx, solved, cost, D, dn, S, g, lambda_w,
-                                                               running);
+                                                               running, damp);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
 
 int viml_launch_gn_update(viml_ctx* ctx, const LinearizeArgs& a, int X, const double* extra_in, const double* dx, const int32_t* solved,
-                          double* o_poses, double* o_ex, double* o_dep, double* o_extra, const int32_t* running) {
+                          double* o_poses, double* o_ex, double* o_dep, double* o_extra, const int32_t* running, const double* dl) {
   LaunchScope ls(ctx, K_GN);
-  gn::update_kernel<<<a.W, 128, 0, ctx->stream>>>(a, X, extra_in, dx, solved, o_poses, o_ex, o_dep, o_extra, running);
+  gn::update_kernel<<<a.W, 128, 0, ctx->stream>>>(a, X, extra_in, dx, solved, o_poses, o_ex, o_dep, o_extra, running, dl);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
@@ -712,6 +713,30 @@ int viml_launch_cost(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn,
 int viml_launch_solve_policy(viml_ctx* ctx, int W, const SolveArgs& s, int round) {
   LaunchScope ls(ctx, K_GN);
   gn::policy_kernel<<<W, 128, 0, ctx->stream>>>(s, round);
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
+int viml_launch_dogleg_prepare(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const DoglegArgs& g, const SolveState* state,
+                               int round) {
+  LaunchScope ls(ctx, K_GN);
+  gn::dogleg_prepare_kernel<<<a.W, 256, 0, ctx->stream>>>(a, dn, g, state, round);
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
+int viml_launch_dogleg_finish(viml_ctx* ctx, const LinearizeArgs& a, const DenseArgs& dn, const DoglegArgs& g, const SolveState* state,
+                              int round, const double* dx, const int32_t* solved) {
+  LaunchScope ls(ctx, K_GN);
+  gn::dogleg_finish_kernel<<<a.W, 256, 0, ctx->stream>>>(a, dn, g, state, round, dx, solved);
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
+int viml_launch_dogleg_step(viml_ctx* ctx, int W, const DoglegArgs& g, const SolveState* state, double initial_radius, int round,
+                            const int32_t* running, double* dx, double* cost, int32_t* solved) {
+  LaunchScope ls(ctx, K_GN);
+  gn::dogleg_step_kernel<<<W, 128, 0, ctx->stream>>>(g, state, initial_radius, round, running, dx, cost, solved);
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
 }
