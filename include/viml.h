@@ -11,6 +11,8 @@
  *                             ThreadsConstructA (J^T J, J^T r)  vins_estimator/src/factor/marginalization_factor.cpp:141-172
  *                             landmark part of MarginalizationInfo::marginalize  marginalization_factor.cpp:267-282
  *   viml_marginalize_batch <- MarginalizationInfo::marginalize  marginalization_factor.cpp:174-299 (dense prior part)
+ *   viml_marginalize_vi    <- the marginalisation of OptimizationWithLine  estimator.cpp:1911-2113 (MARGIN_OLD, MARGIN_SECOND_NEW):
+ *                             the next prior of every window, in viml_inertial_factors' prior layout
  *   viml_line_associate    <- Estimator::UpdateLinesInFoV       vins_estimator/src/estimator.cpp:385-447
  *                             Estimator::LineCorrespondenceInFrame  estimator.cpp:671-885
  *                             (+ CalAngleDist :601-613, CalEulerDist :615-669, Line2D fm.cpp:4-15,:46-71)
@@ -479,6 +481,54 @@ typedef struct viml_marg_out {
 
 int viml_marginalize_batch(viml_ctx* ctx, const viml_marg_batch* in, const viml_marg_out* out,
                            uint32_t flags);
+
+/* ---- the next prior of every window, marginalised on the device ------------------------------------------------------------
+ * The marginalisation of Estimator::OptimizationWithLine after its solve (estimator.cpp:1911-2113): per window the residual blocks
+ * that touch the outgoing frame are linearised at the given state, the outgoing blocks are marginalised with
+ * MarginalizationInfo::marginalize's numerics (marginalization_factor.cpp:264-293, eps = 1e-8) and the result is written as the prior
+ * fields of the next frame's viml_inertial_factors.  `in`, `vi` and `extra_state` are viml_solve_vi's inputs with the state set to
+ * the linearisation point (normally viml_solve_out's final state); margin[w] is the window's MarginalizationFlag.
+ *
+ * VIML_MARGIN_OLD (estimator.cpp:1911-2046), residual blocks of window w:
+ *   - the prior, if prior_n[w] > 0; pose 0 and the speed-bias of pose 0 are dropped if it holds them;
+ *   - the IMU factors whose pose i is 0 and whose sum_dt (imu_preint[k][0]) is below 10.0; pose 0 and speed-bias 0 dropped;
+ *   - every point factor with i == 0 (VIML_LOSS_CAUCHY: with the loss correction); pose 0 and its feature dropped.  The features
+ *     are eliminated first by the Schur step of viml_linearize_batch (H_ll <= 1e-8 skipped), then pose 0 and speed-bias 0 by the
+ *     eigen pseudo-inverse.  Line factors and point factors with i != 0 take no part.
+ *   Kept: every other block these factors touch, slid like addr_shift: pose p -> slot p-1, the speed-bias of pose p -> that of
+ *   p-1, the extrinsic stays.
+ * VIML_MARGIN_SECOND_NEW (estimator.cpp:2047-2113): if the prior holds pose P-2, the prior alone is marginalised with that pose
+ *   dropped, and pose P-1 (and its speed-bias) moves to slot P-2.  Otherwise the output is the input prior, copied unchanged, as
+ *   the reference keeps last_marginalization_info.
+ * Output (the prior fields of viml_inertial_factors, same meaning and strides): prior_n[w] = n, the leading n x n of
+ * prior_jacobian and n of prior_residual (linearized_jacobians / linearized_residuals), prior_n_blocks and prior_block rows
+ * {kind, index after the slide, size, first column}, prior_x0 rows = the kept blocks' values at the given state (entries past
+ * `size` are 0).  prior_n[w] = 0 when nothing is kept.  Entries past n / n_blocks keep the caller's content.
+ * Deviation: the kept blocks are ordered poses ascending (after the slide), then the extrinsic, then extra blocks by ascending
+ * offset; the reference iterates an unordered_map keyed by heap addresses.
+ * Preconditions (the host-pointer flavour checks them and returns VIML_ERR_INVALID): those of viml_solve_vi's batch and inertial
+ * factors; margin[w] is 0 or 1 and P >= 2; the speed-bias of pose p sits at extra offset 9p (para_SpeedBias), so imu_sb[k] ==
+ * {9i, 9j} and every extra block of the prior is a 9-block at such an offset; with VIML_MARGIN_SECOND_NEW the prior does not hold
+ * the speed-bias of pose P-2 (the reference asserts it); no feature has factors with both i == 0 and i != 0; every window's kept
+ * dimension fits out->prior_n_max and its block count out->prior_max_blocks.  The device flavour reads nothing back, clamps
+ * indices, writes prior_n[w] = 0 for a window whose result does not fit, and leaves the rest to the caller.  The outputs must not
+ * overlap the inputs (double-buffer across frames).  W == 0 returns VIML_OK.  Flags: VIML_PTRS_DEVICE, VIML_LOSS_CAUCHY. */
+#define VIML_MARGIN_OLD 0          /* estimator.h MarginalizationFlag values */
+#define VIML_MARGIN_SECOND_NEW 1
+
+typedef struct viml_prior_out {    /* the prior fields of viml_inertial_factors, same meaning and strides */
+  int32_t prior_n_max;
+  int32_t prior_max_blocks;
+  int32_t* prior_n;                /* [W]                                   */
+  double* prior_jacobian;          /* [W][n_max][n_max]                     */
+  double* prior_residual;          /* [W][n_max]                            */
+  int32_t* prior_n_blocks;         /* [W]                                   */
+  int32_t* prior_block;            /* [W][max_blocks][4]                    */
+  double* prior_x0;                /* [W][max_blocks][VIML_PRIOR_X0_STRIDE] */
+} viml_prior_out;
+
+int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
+                        const int32_t* margin /* [W] */, const viml_prior_out* out, uint32_t flags);
 
 /* ---- 2D-3D line association --------------------------------------------------------------------
  * For every pose p: (1) FoV cull of the whole map with cull_poses[p] (UpdateLinesInFoV; the reference

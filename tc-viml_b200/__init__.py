@@ -11,7 +11,7 @@ import os
 import numpy as np
 
 from . import _abi, build, parity, shard, synth  # noqa: F401
-from ._abi import (LOSS_CAUCHY, OUT_HB, OUT_RESIDUAL_JACOBIAN, OUT_SCHUR, PTRS_DEVICE, S_PACKED, SOLVE_DOGLEG,  # noqa: F401
+from ._abi import (LOSS_CAUCHY, MARGIN_OLD, MARGIN_SECOND_NEW, OUT_HB, OUT_RESIDUAL_JACOBIAN, OUT_SCHUR, PTRS_DEVICE, S_PACKED, SOLVE_DOGLEG,  # noqa: F401
                    Batch, make_config)
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -27,7 +27,7 @@ ABI_SYMBOLS = (
     "viml_marginalize_batch", "viml_line_associate", "viml_assoc_stats", "viml_allreduce_hb",
     "viml_load_line_map", "viml_reduced_system", "viml_reduced_from_schur", "viml_gn_step",
     "viml_fov_update", "viml_fov_slide", "viml_track_gate", "viml_triangulate_batch",
-    "viml_inertial_evaluate", "viml_gn_step_vi", "viml_solve_vi",
+    "viml_inertial_evaluate", "viml_gn_step_vi", "viml_solve_vi", "viml_marginalize_vi",
 )
 
 
@@ -92,6 +92,8 @@ def load_library():
                                     C.POINTER(_abi.GnOptions), C.POINTER(_abi.GnOut), C.c_uint32]
     lib.viml_solve_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.InertialFactors), C.c_void_p,
                                   C.POINTER(_abi.SolveOptions), C.POINTER(_abi.SolveOut), C.c_uint32]
+    lib.viml_marginalize_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.InertialFactors), C.c_void_p,
+                                        C.c_void_p, C.POINTER(_abi.PriorOut), C.c_uint32]
     _LIB = lib
     return lib
 
@@ -331,6 +333,29 @@ class Context:
         o.extra = _abi.ptr(res["extra"]) if X > 0 else None
         self._check(self.lib.viml_solve_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), C.byref(opt), C.byref(o),
                                            flags & ~PTRS_DEVICE))
+        return res
+
+    def marginalize_vi(self, batch, vi, extra, margin, flags, n_max=None, max_blocks=None, obs_table=False):
+        """viml_marginalize_vi with host buffers at the state of batch / extra: the next prior of every window (margin[w] =
+        MARGIN_OLD or MARGIN_SECOND_NEW) as a dict of the prior fields of Inertial (prior_n [W], prior_jacobian [W, n_max, n_max],
+        prior_residual [W, n_max], prior_n_blocks [W], prior_block [W, max_blocks, 4], prior_x0 [W, max_blocks, 9]).  n_max defaults
+        to vi's, max_blocks to 2 P + 1 (every block a window can keep); entries past n / n_blocks are NaN / -1."""
+        W, P = batch.W, batch.P
+        n_max = vi.n_max if n_max is None else int(n_max)
+        mb = 2 * P + 1 if max_blocks is None else int(max_blocks)
+        res = {"prior_n": np.full(W, -1, dtype=np.int32), "prior_jacobian": np.full((W, n_max, n_max), np.nan),
+               "prior_residual": np.full((W, n_max), np.nan), "prior_n_blocks": np.full(W, -1, dtype=np.int32),
+               "prior_block": np.full((W, mb, 4), -1, dtype=np.int32), "prior_x0": np.full((W, mb, _abi.PRIOR_X0_STRIDE), np.nan)}
+        s, _keep = self._batch_struct(batch, obs_table)
+        v = vi.struct()
+        ex = None if extra is None else np.ascontiguousarray(extra, dtype=np.float64)
+        mg = np.ascontiguousarray(margin, dtype=np.int32)
+        o = _abi.PriorOut()
+        o.prior_n_max, o.prior_max_blocks = n_max, mb
+        for k in _abi.PRIOR_OUT_FIELDS:
+            setattr(o, k, _abi.ptr(res[k]))
+        self._check(self.lib.viml_marginalize_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), _abi.ptr(mg), C.byref(o),
+                                                 flags & ~PTRS_DEVICE))
         return res
 
     def linearize(self, batch, flags, out=None, obs_table=False, line_table=False):

@@ -25,6 +25,7 @@ SOLVE_DOGLEG = 0x400
 FOV_SLOTS = 11
 BLOCK_POSE, BLOCK_EX, BLOCK_EXTRA = 0, 1, 2
 PRIOR_X0_STRIDE = 9
+MARGIN_OLD, MARGIN_SECOND_NEW = 0, 1
 SOLVE_NO_CONVERGENCE, SOLVE_FUNCTION_TOL, SOLVE_PARAMETER_TOL, SOLVE_MIN_RADIUS, SOLVE_FAILURE = 0, 1, 2, 3, 4
 
 c_double_p = C.POINTER(C.c_double)
@@ -180,6 +181,15 @@ INERTIAL_OUT_FIELDS = ("imu_residual", "imu_jac_pose_i", "imu_jac_sb_i", "imu_ja
 
 class InertialOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in INERTIAL_OUT_FIELDS]
+
+
+PRIOR_OUT_FIELDS = ("prior_n", "prior_jacobian", "prior_residual", "prior_n_blocks", "prior_block", "prior_x0")
+
+
+class PriorOut(C.Structure):
+    """viml_prior_out — where viml_marginalize_vi writes the next prior (the prior fields of viml_inertial_factors)."""
+
+    _fields_ = [("prior_n_max", C.c_int32), ("prior_max_blocks", C.c_int32)] + [(n, C.c_void_p) for n in PRIOR_OUT_FIELDS]
 
 
 class Inertial:

@@ -459,6 +459,33 @@ struct InertialCsr {
 // the Ceres layouts.
 int viml_launch_inertial(viml_ctx* ctx, const InertialArgs& v, const viml_inertial_out& out, const InertialCsr& csr, bool offsets);
 
+// viml_marginalize_vi (marg_kernels.cu): the selection of every window's factors, the gather of its dense problem and the output prior's
+// block list.  Device pointers only.
+struct MargViArgs {
+  int W, P, D, X;
+  int pm;                        // stride of the gathered problems: A [W][pm][pm], b [W][pm]
+  const int32_t* margin;         // [W] VIML_MARGIN_*
+  InertialArgs v;                // the IMU factors and the prior, at the state of v.poses / v.ex_pose / v.extra
+  InertialCsr csr;               // their evaluation at that state (the unselected IMU factors are zeroed there)
+  const int32_t* pf_window_offset;   // the batch's point factors (pf_obs expanded)
+  const uint32_t* pf_idx;
+  const double* pf_obs;
+  const double* pf_pts_i_z;      // nullable
+  int32_t* cnt;                  // [W] selected point factors per window
+  int32_t* sel_offset;           // [W+1] the selected point factors: a CSR over the windows ...
+  uint32_t* sel_idx;             // ... of at most NP factors
+  double* sel_obs;
+  double* sel_z;                 // null when pf_pts_i_z is
+  const double *Sx, *gx;         // [W][Dx][Dx], [W][Dx] of the selected factors
+  double *A, *b;
+  int2* sizes;                   // [W] {pos, m} of the gathered problem ({0, 0}: nothing to marginalise)
+  viml_prior_out out;
+};
+// count + select (before the linearisation of the selected factors; after the IMU / prior evaluation into csr), gather (after the
+// reduced system).
+int viml_launch_marg_select(viml_ctx* ctx, const MargViArgs& g);
+int viml_launch_marg_gather(viml_ctx* ctx, const MargViArgs& g);
+
 // linearize_kernels.cu
 int viml_launch_linearize(viml_ctx* ctx, const LinearizeArgs& a);
 int viml_launch_prep(viml_ctx* ctx, const LinearizeArgs& a);   // pose cache of the state in `a` only
@@ -541,9 +568,12 @@ int viml_launch_dogleg_step(viml_ctx* ctx, int W, const DoglegArgs& g, const Sol
 int viml_launch_schur(viml_ctx* ctx, int W, int F, int D, const double* H_pp, const double* H_lp, const double* H_ll,
                       const double* b_p, const double* b_l, double* S, double* g, double eps);
 double viml_dmma_peak_tflops(viml_ctx* ctx);
-// marg_kernels.cu
+// marg_kernels.cu.  sizes == nullptr: K problems of pos x pos with m marginalised, outputs [K][n][n] / [K][n].  sizes [K] = {pos_k, m_k}
+// (pos_k - m_k <= 0: skipped): problem k in the leading part of a pos x pos slot, m_k <= m_max, its outputs in the leading n_k x n_k of
+// an n_max x n_max slot (n_k <= n_max).
 int viml_launch_marginalize(viml_ctx* ctx, int K, int pos, int m, double eps, const double* A, const double* b,
-                            double* A_schur, double* b_schur, double* lin_jac, double* lin_res);
+                            double* A_schur, double* b_schur, double* lin_jac, double* lin_res, const int2* sizes = nullptr,
+                            int m_max = 0, int n_max = 0);
 
 struct AssocArgs {  // device pointers only
   int Pq, L;

@@ -381,9 +381,163 @@ int check_solve_options(viml_ctx* ctx, const viml_solve_options* o) {
   return VIML_OK;
 }
 
+// viml_marginalize_vi's preconditions on host pointers (viml.h), after check_step_inputs.  The kept dimension and block count of every
+// window follow marg_gather_kernel's selection.
+int check_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const int32_t* margin,
+                         const viml_prior_out* out) {
+  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window;
+  for (int w = 0; w < W; ++w)
+    if (margin[w] != VIML_MARGIN_OLD && margin[w] != VIML_MARGIN_SECOND_NEW) return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: margin[w] must be 0 or 1");
+  for (int64_t k = 0; k < vi->n_imu; ++k)
+    if (vi->imu_sb[2 * k] != 9 * vi->imu_pose[2 * k] || vi->imu_sb[2 * k + 1] != 9 * vi->imu_pose[2 * k + 1])
+      return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: the speed-bias of pose p must sit at extra offset 9p (imu_sb == {9i, 9j})");
+  const int NS = 2 * P + 1;
+  std::vector<uint8_t> touch(NS), feat(F);
+  for (int w = 0; w < W; ++w) {
+    const bool old = margin[w] == VIML_MARGIN_OLD;
+    const int n_in = vi->prior_n_max > 0 ? vi->prior_n[w] : 0, nb_in = n_in > 0 ? vi->prior_n_blocks[w] : 0;
+    std::fill(touch.begin(), touch.end(), 0);
+    bool has = false;
+    for (int b = 0; b < nb_in; ++b) {
+      const int32_t* blk = vi->prior_block + ((size_t)w * vi->prior_max_blocks + b) * 4;
+      int s = P;
+      if (blk[0] == VIML_BLOCK_POSE) {
+        s = blk[1];
+      } else if (blk[0] == VIML_BLOCK_EXTRA) {
+        if (blk[2] != 9 || blk[1] % 9 != 0 || blk[1] / 9 >= P)
+          return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: an extra block of the prior must be the 9-block of a speed-bias (offset 9p, p < P)");
+        s = P + 1 + blk[1] / 9;
+        if (!old && blk[1] / 9 == P - 2)
+          return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: MARGIN_SECOND_NEW with the speed-bias of pose P-2 in the prior");
+      }
+      has = has || s == P - 2;
+      touch[s] = 1;
+    }
+    std::fill(feat.begin(), feat.end(), 0);
+    for (int64_t k = in->pf_window_offset[w]; k < in->pf_window_offset[w + 1]; ++k) {
+      const uint32_t ix = in->pf_idx[k];
+      const int i = ix & 0xffu, j = (ix >> 8) & 0xffu, f = ix >> 16;
+      feat[f] |= i == 0 ? 1 : 2;
+      if (feat[f] == 3) return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: a feature has factors with both i == 0 and i != 0");
+      if (old && i == 0) touch[0] = touch[j] = touch[P] = 1;
+    }
+    int n = 0, nb = 0;
+    if (!old && !has) {
+      n = n_in, nb = nb_in;
+    } else {
+      if (old && vi->n_imu > 0)
+        for (int64_t f = vi->imu_window_offset[w]; f < vi->imu_window_offset[w + 1]; ++f)
+          if (vi->imu_pose[2 * f] == 0 && vi->imu_preint[f * 17] < 10.0) {
+            const int j = vi->imu_pose[2 * f + 1];
+            touch[0] = touch[j] = touch[P + 1] = touch[P + 1 + j] = 1;
+          }
+      const int dp = old ? 0 : P - 2, ds = old ? P + 1 : -1;
+      for (int s = 0; s < NS; ++s)
+        if (touch[s] && s != dp && s != ds) n += s <= P ? 6 : 9, ++nb;
+    }
+    if (n > out->prior_n_max || nb > out->prior_max_blocks)
+      return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: a window's kept dimension or block count exceeds the output's prior_n_max / prior_max_blocks");
+  }
+  return VIML_OK;
+}
+
 }  // namespace
 
 extern "C" {
+
+int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
+                        const int32_t* margin, const viml_prior_out* out, uint32_t flags) {
+  if (!ctx) return VIML_ERR_INVALID;
+  if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
+  if (!vi) return fail(ctx, VIML_ERR_INVALID, "null inertial factors");
+  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
+  BatchForm form;
+  int rc = check_step_inputs(ctx, in, nullptr, extra_state, flags, vi, "viml_marginalize_vi", &form);
+  if (rc != VIML_OK) return rc;
+  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1), X = vi->extra_dim, Dx = D + X;
+  const int64_t NP = in->n_point_factors;
+  if (P < 2) return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: needs P >= 2");
+  if (W == 0) return VIML_OK;
+  const int n_max = out->prior_n_max, mb = out->prior_max_blocks;
+  if (!margin || n_max < 0 || mb < 0 || !out->prior_n || !out->prior_n_blocks ||
+      (n_max > 0 && (!out->prior_jacobian || !out->prior_residual)) || (mb > 0 && (!out->prior_block || !out->prior_x0)))
+    return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: null margin or output array, or negative output sizes");
+  if (!dev) {
+    rc = check_marginalize_vi(ctx, in, vi, margin, out);
+    if (rc != VIML_OK) return rc;
+  }
+  VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
+  Stager st{ctx, dev};
+  viml_window_batch pts = *in;   // line factors take no part (est.cpp:1911-2046 adds none)
+  pts.n_line_factors = 0;
+  BatchForm pform = form;
+  pform.line_table = false;
+  StagedBatch b;
+  stage_batch(ctx, st, &pts, pform, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR, &b);
+  LinearizeArgs& a = b.a;
+  MargViArgs g{};
+  g.W = W, g.P = P, g.D = D, g.X = X;
+  g.pm = std::min(Dx, 15 + n_max);   // m <= 15: pose 0 and speed-bias 0
+  const double* extra = nullptr;
+  st.in(extra_state, extra_state ? (size_t)W * X : 0, &extra);
+  st.in(margin, (size_t)W, &g.margin);
+  stage_inertial(st, vi, W, P, &g.v);
+  double* res_plus = nullptr;
+  stage_inertial_csr(st, g.v, &g.csr, &res_plus);
+  st.out((int32_t*)nullptr, (size_t)W, &g.cnt);
+  st.out((int32_t*)nullptr, (size_t)W + 1, &g.sel_offset);
+  st.out((uint32_t*)nullptr, (size_t)NP, &g.sel_idx);
+  st.out((double*)nullptr, (size_t)NP * 4, &g.sel_obs);
+  if (in->pf_pts_i_z) st.out((double*)nullptr, (size_t)NP, &g.sel_z);
+  st.out((double*)nullptr, (size_t)W * D * D, &a.out.H_pp);
+  st.out((double*)nullptr, (size_t)W * F * D, &a.out.H_lp);
+  st.out((double*)nullptr, (size_t)W * F, &a.out.H_ll);
+  st.out((double*)nullptr, (size_t)W * D, &a.out.b_p);
+  st.out((double*)nullptr, (size_t)W * F, &a.out.b_l);
+  st.out((double*)nullptr, (size_t)W * D * D, &a.out.S);
+  st.out((double*)nullptr, (size_t)W * D, &a.out.g);
+  double *Sx = nullptr, *gx = nullptr;
+  st.out((double*)nullptr, (size_t)W * Dx * Dx, &Sx);
+  st.out((double*)nullptr, (size_t)W * Dx, &gx);
+  st.out((double*)nullptr, (size_t)W * g.pm * g.pm, &g.A);
+  st.out((double*)nullptr, (size_t)W * g.pm, &g.b);
+  st.out((int2*)nullptr, (size_t)W, &g.sizes);
+  // entries past n / n_blocks keep the caller's content
+  g.out.prior_n_max = n_max, g.out.prior_max_blocks = mb;
+  st.out(out->prior_n, (size_t)W, &g.out.prior_n);
+  st.out(out->prior_n_blocks, (size_t)W, &g.out.prior_n_blocks);
+  st.inout(out->prior_jacobian, (size_t)W * n_max * n_max, &g.out.prior_jacobian);
+  st.inout(out->prior_residual, (size_t)W * n_max, &g.out.prior_residual);
+  st.inout(out->prior_block, (size_t)W * mb * 4, &g.out.prior_block);
+  st.inout(out->prior_x0, (size_t)W * mb * VIML_PRIOR_X0_STRIDE, &g.out.prior_x0);
+  rc = st.commit();
+  if (rc == VIML_OK) rc = expand_tables(ctx, b);
+  if (rc != VIML_OK) return rc;
+  // the IMU factors and the prior at x, into the dense-factor CSR
+  g.v.poses = a.poses, g.v.ex_pose = a.ex_pose, g.v.extra = extra;
+  rc = viml_launch_inertial(ctx, g.v, viml_inertial_out{}, g.csr, true);
+  if (rc != VIML_OK) return rc;
+  g.pf_window_offset = a.pf_window_offset, g.pf_idx = a.pf_idx, g.pf_obs = a.pf_obs, g.pf_pts_i_z = a.pf_pts_i_z;
+  rc = viml_launch_marg_select(ctx, g);
+  if (rc != VIML_OK) return rc;
+  // the selected point factors: S, g of the window with their features eliminated (NP is an upper bound of their number)
+  a.pf_window_offset = g.sel_offset, a.pf_idx = g.sel_idx, a.pf_obs = g.sel_obs, a.pf_pts_i_z = g.sel_z;
+  rc = viml_launch_linearize(ctx, a);
+  if (rc != VIML_OK) return rc;
+  DenseArgs dn{};
+  dn.X = X, dn.ND = (int64_t)W + g.v.NI;   // an upper bound: the kernels read ND only as "any dense factors"
+  dn.window_offset = g.csr.window_offset, dn.row_offset = g.csr.row_offset, dn.col_offset = g.csr.col_offset;
+  dn.jac_offset = g.csr.jac_offset, dn.col_index = g.csr.col_index, dn.residual = g.csr.residual, dn.jacobian = g.csr.jacobian;
+  rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, Sx, gx);
+  if (rc != VIML_OK) return rc;
+  g.Sx = Sx, g.gx = gx;
+  rc = viml_launch_marg_gather(ctx, g);
+  if (rc == VIML_OK && n_max > 0)   // MarginalizationInfo::eps (marginalization_factor.h:70)
+    rc = viml_launch_marginalize(ctx, W, g.pm, 0, 1e-8, g.A, g.b, nullptr, nullptr, g.out.prior_jacobian, g.out.prior_residual, g.sizes,
+                                 15, n_max);
+  if (rc != VIML_OK) return rc;
+  return st.finish();
+}
 
 int viml_reduced_system(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const viml_reduced_out* out,
                         uint32_t flags) {

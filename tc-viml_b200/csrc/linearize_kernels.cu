@@ -456,7 +456,8 @@ template <bool MODE_A, bool MODE_B>
 __global__ void __launch_bounds__(128, MODE_B ? 2 : VIML_POINTS_MINB) points_kernel(LinearizeArgs A) {
   __shared__ double2 stage[MODE_A ? 4 * 7 * 32 : 1];
   const int64_t k_raw = A.pf_begin + blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-  const int64_t k_end = A.pf_begin + A.NP;
+  // the CSR's end: equal to pf_begin + NP for a whole batch or a chunk of one; viml_marginalize_vi passes NP as an upper bound
+  const int64_t k_end = min(A.pf_begin + A.NP, (int64_t)A.pf_window_offset[A.W]);
   const int lane = threadIdx.x & 31;
   const int64_t k_warp = k_raw - lane;
   if (k_warp >= k_end) return;                       // whole warp out of range

@@ -109,26 +109,32 @@ __device__ void ascending_rank(const double* __restrict__ a, int n, int* rank) {
   __syncthreads();
 }
 
-__global__ void __launch_bounds__(kMargThreads) marg_kernel(int K, int pos, int m, double eps,
+// sizes == nullptr: every problem is pos x pos with m0 marginalised, outputs [K][n][n] / [K][n] (ld = n = pos - m0).  Otherwise
+// problem k is sizes[k] = {pos_k, m_k} (pos_k - m_k <= 0: skipped) in the leading part of a pos x pos slot of A / b, and its outputs
+// fill the leading n_k x n_k of an ld x ld slot (per_cta sized for the largest m_k and n_k).
+__global__ void __launch_bounds__(kMargThreads) marg_kernel(int K, int pos, int m0, double eps,
                                                             const double* __restrict__ A, const double* __restrict__ b,
                                                             double* __restrict__ A_schur, double* __restrict__ b_schur,
                                                             double* __restrict__ lin_jac, double* __restrict__ lin_res,
-                                                            double* __restrict__ scratch, size_t per_cta) {
+                                                            double* __restrict__ scratch, size_t per_cta,
+                                                            const int2* __restrict__ sizes, int ld) {
   __shared__ double red[65];
   __shared__ int pq[256];
   __shared__ double cs[256];
   __shared__ int rank[256];
   __shared__ double lam[256];
-  const int n = pos - m, tid = threadIdx.x, nt = blockDim.x;
+  const int tid = threadIdx.x, nt = blockDim.x;
   double* ws = scratch + (size_t)blockIdx.x * per_cta;
-  double* Wm = ws;                          // m*m   work / eigenvalues on the diagonal
-  double* Vm = Wm + (size_t)m * m;          // m*m
-  double* Inv = Vm + (size_t)m * m;         // m*m
-  double* T = Inv + (size_t)m * m;          // n*m
-  double* Wn = T + (size_t)n * m;           // n*n
-  double* Vn = Wn + (size_t)n * n;          // n*n
-  double* br = Vn + (size_t)n * n;          // n
   for (int k = blockIdx.x; k < K; k += gridDim.x) {
+    const int m = sizes ? sizes[k].y : m0, n = (sizes ? sizes[k].x : pos) - m;
+    if (n <= 0) continue;                     // CTA-uniform
+    double* Wm = ws;                          // m*m   work / eigenvalues on the diagonal
+    double* Vm = Wm + (size_t)m * m;          // m*m
+    double* Inv = Vm + (size_t)m * m;         // m*m
+    double* T = Inv + (size_t)m * m;          // n*m
+    double* Wn = T + (size_t)n * m;           // n*n
+    double* Vn = Wn + (size_t)n * n;          // n*n
+    double* br = Vn + (size_t)n * n;          // n
     const double* Ak = A + (size_t)k * pos * pos;
     const double* bk = b + (size_t)k * pos;
     __syncthreads();
@@ -166,14 +172,14 @@ __global__ void __launch_bounds__(kMargThreads) marg_kernel(int K, int pos, int 
         for (int j = 0; j < m; ++j) s += T[r * m + j] * Ak[(size_t)j * pos + m + c];
         const double val = Ak[(size_t)(m + r) * pos + m + c] - s;
         Wn[e] = val;
-        if (A_schur) A_schur[(size_t)k * n * n + e] = val;
+        if (A_schur) A_schur[(size_t)k * ld * ld + (size_t)r * ld + c] = val;
       } else {
         const int r = e - n * n;
         double s = 0.0;
         for (int j = 0; j < m; ++j) s += T[r * m + j] * bk[j];
         const double val = bk[m + r] - s;
         br[r] = val;
-        if (b_schur) b_schur[(size_t)k * n + r] = val;
+        if (b_schur) b_schur[(size_t)k * ld + r] = val;
       }
     }
     __syncthreads();
@@ -195,7 +201,7 @@ __global__ void __launch_bounds__(kMargThreads) marg_kernel(int K, int pos, int 
         if (!lin_jac) continue;
         const int kk = e / n, c = e % n;  // source eigenpair kk -> output row rank[kk]
         const double S = lam[kk] > eps ? lam[kk] : 0.0;                                    // :285
-        lin_jac[(size_t)k * n * n + (size_t)rank[kk] * n + c] = sqrt(S) * Vn[c * n + kk];  // :292
+        lin_jac[(size_t)k * ld * ld + (size_t)rank[kk] * ld + c] = sqrt(S) * Vn[c * n + kk];  // :292
       } else {
         if (!lin_res) continue;
         const int kk = e - n * n;
@@ -203,25 +209,231 @@ __global__ void __launch_bounds__(kMargThreads) marg_kernel(int K, int pos, int 
         const double sq = sqrt(Sinv);
         double s = 0.0;
         for (int c = 0; c < n; ++c) s += (sq * Vn[c * n + kk]) * br[c];                     // :293
-        lin_res[(size_t)k * n + rank[kk]] = s;
+        lin_res[(size_t)k * ld + rank[kk]] = s;
       }
     }
   }
 }
 
+// ---- viml_marginalize_vi: which factors and blocks of each window take part, and the dense problem they give -------------------
+// Block slots of a window: pose p -> p, the extrinsic -> P, the speed-bias of pose q (extra offset 9q) -> P + 1 + q.
+__device__ __forceinline__ bool imu_selected(const InertialArgs& v, int64_t f, bool old) {   // est.cpp:1916-1930
+  return old && min(max(v.imu_pose[2 * f], 0), v.P - 1) == 0 && v.imu_preint[f * 17] < 10.0;
+}
+
+// Point factors with i == 0 of every MARGIN_OLD window (est.cpp:1933-1966).
+__global__ void __launch_bounds__(128) marg_count_kernel(MargViArgs g) {
+  __shared__ int s_cnt;
+  const int w = blockIdx.x, tid = threadIdx.x;
+  if (tid == 0) s_cnt = 0;
+  __syncthreads();
+  if (g.margin[w] == VIML_MARGIN_OLD) {
+    int c = 0;
+    for (int64_t k = g.pf_window_offset[w] + tid; k < g.pf_window_offset[w + 1]; k += blockDim.x) c += (g.pf_idx[k] & 0xffu) == 0;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+    if ((tid & 31) == 0) atomicAdd(&s_cnt, c);
+  }
+  __syncthreads();
+  if (tid == 0) g.cnt[w] = s_cnt;
+}
+
+// One CTA per window: the window's selected point factors, in input order, into the CSR sel_* (the window's offset is the sum of the
+// counts before it), and the IMU factors that take no part zeroed in the dense-factor CSR (their J^T J and J^T r add exact zeros).
+__global__ void __launch_bounds__(128) marg_select_kernel(MargViArgs g) {
+  __shared__ int s_part[4];
+  __shared__ int s_base;
+  const int w = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int c = 0;
+  for (int u = tid; u < w; u += blockDim.x) c += g.cnt[u];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+  if (lane == 0) s_part[warp] = c;
+  __syncthreads();
+  if (tid == 0) {
+    s_base = s_part[0] + s_part[1] + s_part[2] + s_part[3];
+    g.sel_offset[w] = s_base;
+    if (w == g.W - 1) g.sel_offset[g.W] = s_base + g.cnt[w];
+  }
+  __syncthreads();
+  const bool old = g.margin[w] == VIML_MARGIN_OLD;
+  int at = s_base;
+  if (old) {
+    for (int64_t k0 = g.pf_window_offset[w]; k0 < g.pf_window_offset[w + 1]; k0 += blockDim.x) {
+      const int64_t k = k0 + tid;
+      const bool sel = k < g.pf_window_offset[w + 1] && (g.pf_idx[k] & 0xffu) == 0;
+      const unsigned mask = __ballot_sync(0xffffffffu, sel);
+      __syncthreads();   // s_part of the previous chunk has been read
+      if (lane == 0) s_part[warp] = __popc(mask);
+      __syncthreads();
+      int before = 0, total = 0;
+      for (int u = 0; u < 4; ++u) before += u < warp ? s_part[u] : 0, total += s_part[u];
+      if (sel) {
+        const int64_t d = at + before + __popc(mask & ((1u << lane) - 1u));
+        g.sel_idx[d] = g.pf_idx[k];
+        reinterpret_cast<double4*>(g.sel_obs)[d] = reinterpret_cast<const double4*>(g.pf_obs)[k];
+        if (g.sel_z) g.sel_z[d] = g.pf_pts_i_z[k];
+      }
+      at += total;
+    }
+  }
+  const InertialArgs& v = g.v;
+  if (v.NI == 0) return;
+  const bool prior = v.n_max > 0 && v.prior_n[w] > 0;   // imu_kernel's CSR slot of factor f
+  for (int64_t f = v.imu_window_offset[w]; f < v.imu_window_offset[w + 1]; ++f) {
+    if (imu_selected(v, f, old)) continue;
+    const int kf = g.csr.window_offset[w] + (prior ? 1 : 0) + (int)(f - v.imu_window_offset[w]);
+    for (int e = tid; e < 15; e += blockDim.x) g.csr.residual[g.csr.row_offset[kf] + e] = 0.0;
+    for (int e = tid; e < 450; e += blockDim.x) g.csr.jacobian[g.csr.jac_offset[kf] + e] = 0.0;
+  }
+}
+
+// One CTA per window: the blocks the selected factors touch, their columns in A = [marginalised | kept] gathered from Sx / gx, the
+// problem size {pos, m}, and the output prior's n, block list and x0 (marg_kernel writes its Jacobian and residual).  A MARGIN_SECOND_NEW
+// window whose prior does not hold pose P-2 gets its input prior copied.
+__global__ void __launch_bounds__(256) marg_gather_kernel(MargViArgs g) {
+  __shared__ int s_touch[2 * 255 + 1];
+  __shared__ int s_col[kMaxDx];          // tangent column of each row of A
+  __shared__ int s_blk[2 * 255 + 1][3];  // kept block: slot, output index, first column
+  __shared__ int s_has, s_pos, s_m, s_nb;
+  const InertialArgs& v = g.v;
+  const viml_prior_out& o = g.out;
+  const int w = blockIdx.x, tid = threadIdx.x, nt = blockDim.x, P = g.P, D = g.D, X = g.X, Dx = D + X, NS = 2 * P + 1;
+  const int QS = min(P, X / 9);           // speed-bias slots inside the extra state
+  const bool old = g.margin[w] == VIML_MARGIN_OLD;
+  const int n_in = v.n_max > 0 ? min(max(v.prior_n[w], 0), v.n_max) : 0;
+  const int nb_in = n_in > 0 ? min(max(v.prior_n_blocks[w], 0), v.max_blocks) : 0;
+  auto prior_slot = [&](int b) {          // -1: an extra block outside the speed-bias slots
+    const int32_t* blk = v.prior_block + ((size_t)w * v.max_blocks + b) * 4;
+    if (blk[0] == VIML_BLOCK_POSE) return min(max(blk[1], 0), P - 1);
+    if (blk[0] == VIML_BLOCK_EX) return P;
+    return QS > 0 ? P + 1 + min(max(blk[1] / 9, 0), QS - 1) : -1;
+  };
+  for (int s = tid; s < NS; s += nt) s_touch[s] = 0;
+  if (tid == 0) s_has = 0;
+  __syncthreads();
+  for (int b = tid; b < nb_in; b += nt)
+    if (prior_slot(b) == P - 2) s_has = 1;
+  __syncthreads();
+  double* pj = o.prior_jacobian + (size_t)w * o.prior_n_max * o.prior_n_max;
+  double* pr = o.prior_residual + (size_t)w * o.prior_n_max;
+  int32_t* pb = o.prior_block + (size_t)w * o.prior_max_blocks * 4;
+  double* px = o.prior_x0 + (size_t)w * o.prior_max_blocks * VIML_PRIOR_X0_STRIDE;
+  if (!old && !s_has) {   // est.cpp:2047-2049: last_marginalization_info is kept
+    const bool fits = n_in <= o.prior_n_max && nb_in <= o.prior_max_blocks;
+    if (tid == 0) {
+      o.prior_n[w] = fits ? n_in : 0, o.prior_n_blocks[w] = fits ? nb_in : 0;
+      g.sizes[w] = make_int2(0, 0);
+    }
+    if (!fits) return;
+    const double* J = v.prior_jacobian + (size_t)w * v.n_max * v.n_max;
+    for (int e = tid; e < n_in * n_in; e += nt) pj[(size_t)(e / n_in) * o.prior_n_max + e % n_in] = J[(size_t)(e / n_in) * v.n_max + e % n_in];
+    for (int e = tid; e < n_in; e += nt) pr[e] = v.prior_residual[(size_t)w * v.n_max + e];
+    for (int e = tid; e < nb_in * 4; e += nt) pb[e] = v.prior_block[(size_t)w * v.max_blocks * 4 + e];
+    for (int e = tid; e < nb_in * VIML_PRIOR_X0_STRIDE; e += nt) px[e] = v.prior_x0[(size_t)w * v.max_blocks * VIML_PRIOR_X0_STRIDE + e];
+    return;
+  }
+  for (int b = tid; b < nb_in; b += nt) {
+    const int s = prior_slot(b);
+    if (s >= 0) s_touch[s] = 1;
+  }
+  if (old) {
+    for (int64_t k = g.sel_offset[w] + tid; k < g.sel_offset[w + 1]; k += nt) {   // pose 0, pose j, extrinsic
+      s_touch[0] = 1, s_touch[P] = 1;
+      s_touch[min(max((int)((g.sel_idx[k] >> 8) & 0xffu), 0), P - 1)] = 1;
+    }
+    if (v.NI > 0 && QS > 0)
+      for (int64_t f = v.imu_window_offset[w] + tid; f < v.imu_window_offset[w + 1]; f += nt) {
+        if (!imu_selected(v, f, true)) continue;
+        s_touch[0] = 1;
+        s_touch[min(max(v.imu_pose[2 * f + 1], 0), P - 1)] = 1;
+        s_touch[P + 1 + min(max(v.imu_sb[2 * f] / 9, 0), QS - 1)] = 1;
+        s_touch[P + 1 + min(max(v.imu_sb[2 * f + 1] / 9, 0), QS - 1)] = 1;
+      }
+  }
+  __syncthreads();
+  if (tid == 0) {
+    // marginalised: MARGIN_OLD pose 0 then speed-bias 0 (est.cpp:1922, :1950); MARGIN_SECOND_NEW pose P-2 (:2064)
+    const int dp = old ? 0 : P - 2, ds = old ? P + 1 : -1;
+    int pos = 0, nb = 0;
+    if (s_touch[dp])
+      for (int t = 0; t < 6; ++t) s_col[pos++] = 6 * dp + t;
+    if (ds >= 0 && s_touch[ds])
+      for (int t = 0; t < 9; ++t) s_col[pos++] = D + t;
+    const int m = pos;
+    for (int s = 0; s < NS; ++s) {   // kept, in output order: poses ascending, the extrinsic, speed-biases ascending
+      if (!s_touch[s] || s == dp || s == ds) continue;
+      const int local = s <= P ? 6 : 9, t0 = s < P ? 6 * s : s == P ? 6 * P : D + 9 * (s - P - 1);
+      const int q = s < P ? s : s - P - 1;   // addr_shift (est.cpp:2030-2040, :2098-2108)
+      const int slid = old ? q - 1 : q == P - 1 ? P - 2 : q;
+      s_blk[nb][0] = s, s_blk[nb][1] = s == P ? 0 : s < P ? slid : 9 * slid, s_blk[nb][2] = pos - m;
+      ++nb;
+      for (int t = 0; t < local; ++t) s_col[pos++] = t0 + t;
+    }
+    const bool fits = pos - m <= o.prior_n_max && nb <= o.prior_max_blocks && pos <= g.pm;
+    s_pos = fits && pos > m ? pos : 0, s_m = m, s_nb = fits && pos > m ? nb : 0;
+    o.prior_n[w] = s_pos ? pos - m : 0, o.prior_n_blocks[w] = s_nb;
+    g.sizes[w] = make_int2(s_pos, m);
+  }
+  __syncthreads();
+  const int pos = s_pos, nb = s_nb;
+  for (int e = tid; e < nb * 4; e += nt) {
+    const int b = e >> 2, c = e & 3, s = s_blk[b][0];
+    pb[e] = c == 0 ? (s < P ? VIML_BLOCK_POSE : s == P ? VIML_BLOCK_EX : VIML_BLOCK_EXTRA) : c == 1 ? s_blk[b][1] : c == 2 ? (s <= P ? 7 : 9)
+                                                                                                                   : s_blk[b][2];
+  }
+  for (int e = tid; e < nb * VIML_PRIOR_X0_STRIDE; e += nt) {   // keep_block_data: the values at the linearisation point
+    const int b = e / VIML_PRIOR_X0_STRIDE, t = e % VIML_PRIOR_X0_STRIDE, s = s_blk[b][0];
+    const double* x = s < P ? v.poses + ((size_t)w * P + s) * 7 : s == P ? v.ex_pose + (size_t)w * 7 : v.extra + (size_t)w * X + 9 * (s - P - 1);
+    px[e] = t < (s <= P ? 7 : 9) ? x[t] : 0.0;
+  }
+  const double* Sx = g.Sx + (size_t)w * Dx * Dx;
+  double* A = g.A + (size_t)w * g.pm * g.pm;
+  for (int e = tid; e < pos * pos; e += nt) {
+    const int r = e / pos, c = e - r * pos;
+    A[(size_t)r * g.pm + c] = Sx[(size_t)s_col[r] * Dx + s_col[c]];
+  }
+  for (int r = tid; r < pos; r += nt) g.b[(size_t)w * g.pm + r] = g.gx[(size_t)w * Dx + s_col[r]];
+}
+
 }  // namespace
 
+int viml_launch_marg_select(viml_ctx* ctx, const MargViArgs& g) {
+  {
+    LaunchScope ls(ctx, K_MARG);
+    marg_count_kernel<<<g.W, 128, 0, ctx->stream>>>(g);
+  }
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  {
+    LaunchScope ls(ctx, K_MARG);
+    marg_select_kernel<<<g.W, 128, 0, ctx->stream>>>(g);
+  }
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
+int viml_launch_marg_gather(viml_ctx* ctx, const MargViArgs& g) {
+  {
+    LaunchScope ls(ctx, K_MARG);
+    marg_gather_kernel<<<g.W, 256, 0, ctx->stream>>>(g);
+  }
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
 int viml_launch_marginalize(viml_ctx* ctx, int K, int pos, int m, double eps, const double* A, const double* b,
-                            double* A_schur, double* b_schur, double* lin_jac, double* lin_res) {
-  const int n = pos - m;
-  const size_t per_cta = (size_t)3 * m * m + (size_t)n * m + (size_t)2 * n * n + n + 32;
+                            double* A_schur, double* b_schur, double* lin_jac, double* lin_res, const int2* sizes, int m_max,
+                            int n_max) {
+  // sized: n_k <= pos bounds the work matrices, n_max is the output's leading dimension
+  const int mm = sizes ? m_max : m, n = sizes ? std::min(n_max, pos) : pos - m, ld = sizes ? n_max : pos - m;
+  const size_t per_cta = (size_t)3 * mm * mm + (size_t)n * mm + (size_t)2 * n * n + n + 32;
   const int grid = K < 2 * ctx->sm_count ? K : 2 * ctx->sm_count;
   VIML_TRY_CUDA(ctx, ctx->scratch.reserve(per_cta * grid * sizeof(double) + 256));
   double* scratch = ctx->scratch.take<double>(per_cta * grid);
   {
     LaunchScope ls(ctx, K_MARG);
     marg_kernel<<<grid, kMargThreads, 0, ctx->stream>>>(K, pos, m, eps, A, b, A_schur, b_schur, lin_jac, lin_res,
-                                                        scratch, per_cta);
+                                                        scratch, per_cta, sizes, ld);
   }
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
