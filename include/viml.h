@@ -13,6 +13,8 @@
  *   viml_marginalize_batch <- MarginalizationInfo::marginalize  marginalization_factor.cpp:174-299 (dense prior part)
  *   viml_marginalize_vi    <- the marginalisation of OptimizationWithLine  estimator.cpp:1911-2113 (MARGIN_OLD, MARGIN_SECOND_NEW):
  *                             the next prior of every window, in viml_inertial_factors' prior layout
+ *   viml_slide_vi          <- Estimator::slideWindow (estimator.cpp:2121-2218) with FeatureManager::removeBackShiftDepth /
+ *                             removeFront: the next frame's poses, speed-biases and re-anchored inverse depths
  *   viml_line_associate    <- Estimator::UpdateLinesInFoV       vins_estimator/src/estimator.cpp:385-447
  *                             Estimator::LineCorrespondenceInFrame  estimator.cpp:671-885
  *                             (+ CalAngleDist :601-613, CalEulerDist :615-669, Line2D fm.cpp:4-15,:46-71)
@@ -529,6 +531,45 @@ typedef struct viml_prior_out {    /* the prior fields of viml_inertial_factors,
 
 int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const double* extra_state,
                         const int32_t* margin /* [W] */, const viml_prior_out* out, uint32_t flags);
+
+/* ---- the window slide after the marginalisation, on the device ----------------------------------------------------------------
+ * Estimator::slideWindow (est.cpp:2121-2218) and FeatureManager::removeBackShiftDepth / removeFront for a batch of windows: the
+ * parameter blocks of the next frame's window, from the state the marginalisation linearised at (normally viml_solve_out's final
+ * state).  `in`, `extra_state` and `margin` are viml_marginalize_vi's; extra_dim is X.  Per window w:
+ * VIML_MARGIN_OLD (slideWindow with frame_count == WINDOW_SIZE, slideWindowOld with shift_depth):
+ *   - pose p moves to slot p-1 for p >= 1 and the newest slot keeps the old newest pose (Ps[WINDOW_SIZE] = Ps[WINDOW_SIZE-1] after
+ *     the swap loop); the speed-bias 9-block at extra offset 9p moves the same way; extra values past 9P and the extrinsic are
+ *     copied unchanged;
+ *   - every feature f with at least two point factors whose i == 0 is re-anchored in the camera of the old pose 1, with
+ *     removeBackShiftDepth's statements: d = 1 / inv_depth[f]; uv_i = (pts_i.x, pts_i.y, pts_i.z) of its first such factor
+ *     (pts_i.z = pf_pts_i_z or 1; any of the observation forms); R0 = R(q_0) R(q_ex), P0 = p_0 + R(q_0) t_ex from the OLD pose 0,
+ *     R1, P1 likewise from the OLD pose 1; w = R0 (uv_i d) + P0; pts_j = R1^T (w - P1); inv_depth[f] = 1 / pts_j.z if pts_j.z > 0,
+ *     else 1 / init_depth (a NaN takes the else branch, as the reference's comparison does);
+ *   - a feature anchored at 0 with exactly one factor is erased by the reference: its slot keeps its input value (the caller's to
+ *     reuse); every other inverse depth is copied bit for bit.
+ * VIML_MARGIN_SECOND_NEW (slideWindow's second-new branch, removeFront): pose and speed-bias P-1 move to slot P-2, P-1 keeps its
+ *   value; the inverse depths and the extrinsic are copied unchanged (removeFront moves no depth).  Merging the pre-integrations
+ *   stays with the host, like all IMU pre-integration.
+ * Line factors take no part.  Rotations come from the normalised quaternion (Eigen's normalized().toRotationMatrix(), the norm
+ * summed x, y, z, w left to right), for the extrinsic too; matrix products are summed left to right; all arithmetic is IEEE
+ * binary64 without fused multiply-adds, so a scalar restatement reproduces it bit for bit.
+ * Deviations, restated from the named functions and not pinned against compiled reference code: the state stays in parameter-block
+ * form, so double2vector / vector2double are not replayed — no yaw re-gauge (the depth transform is invariant under its rigid
+ * transform, which could change it by rounding only), no quaternion -> matrix -> quaternion round trip, and inverse depths that are
+ * not re-anchored are not passed through 1 / (1 / x).
+ * Preconditions (the host-pointer flavour checks them and returns VIML_ERR_INVALID): those of viml_marginalize_vi's batch; margin[w]
+ * is 0 or 1; P >= 2; X >= 9P; init_depth finite and > 0; no feature has factors with both i == 0 and i != 0.  P, X and init_depth are
+ * checked in both flavours; the device flavour reads nothing back, clamps feature indices and leaves the rest to the caller.  The
+ * outputs must not overlap the inputs (double-buffer across frames).  W == 0 returns VIML_OK.  Flags: VIML_PTRS_DEVICE.        */
+typedef struct viml_slide_out {
+  double* poses;      /* [W][P][7]                      */
+  double* ex_pose;    /* [W][7]                         */
+  double* inv_depth;  /* [W][F]  (required when F > 0)  */
+  double* extra;      /* [W][X]  (required when X > 0)  */
+} viml_slide_out;
+
+int viml_slide_vi(viml_ctx* ctx, const viml_window_batch* in, const double* extra_state, int32_t extra_dim,
+                  const int32_t* margin /* [W] */, double init_depth, const viml_slide_out* out, uint32_t flags);
 
 /* ---- 2D-3D line association --------------------------------------------------------------------
  * For every pose p: (1) FoV cull of the whole map with cull_poses[p] (UpdateLinesInFoV; the reference

@@ -27,7 +27,7 @@ ABI_SYMBOLS = (
     "viml_marginalize_batch", "viml_line_associate", "viml_assoc_stats", "viml_allreduce_hb",
     "viml_load_line_map", "viml_reduced_system", "viml_reduced_from_schur", "viml_gn_step",
     "viml_fov_update", "viml_fov_slide", "viml_track_gate", "viml_triangulate_batch",
-    "viml_inertial_evaluate", "viml_gn_step_vi", "viml_solve_vi", "viml_marginalize_vi",
+    "viml_inertial_evaluate", "viml_gn_step_vi", "viml_solve_vi", "viml_marginalize_vi", "viml_slide_vi",
 )
 
 
@@ -94,6 +94,8 @@ def load_library():
                                   C.POINTER(_abi.SolveOptions), C.POINTER(_abi.SolveOut), C.c_uint32]
     lib.viml_marginalize_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.POINTER(_abi.InertialFactors), C.c_void_p,
                                         C.c_void_p, C.POINTER(_abi.PriorOut), C.c_uint32]
+    lib.viml_slide_vi.argtypes = [C.c_void_p, C.POINTER(_abi.WindowBatch), C.c_void_p, C.c_int32, C.c_void_p, C.c_double,
+                                  C.POINTER(_abi.SlideOut), C.c_uint32]
     _LIB = lib
     return lib
 
@@ -356,6 +358,22 @@ class Context:
             setattr(o, k, _abi.ptr(res[k]))
         self._check(self.lib.viml_marginalize_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), _abi.ptr(mg), C.byref(o),
                                                  flags & ~PTRS_DEVICE))
+        return res
+
+    def slide_vi(self, batch, extra, margin, flags, init_depth=5.0, obs_table=False):
+        """viml_slide_vi with host buffers: the next frame's state of every window (margin[w] = MARGIN_OLD or MARGIN_SECOND_NEW) as
+        a dict(poses [W, P, 7], ex_pose [W, 7], inv_depth [W, F], extra [W, X])."""
+        ex = np.ascontiguousarray(extra, dtype=np.float64)
+        W, X = batch.W, ex.shape[1] if ex.ndim == 2 else 0
+        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
+               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan)}
+        s, _keep = self._batch_struct(batch, obs_table)
+        mg = np.ascontiguousarray(margin, dtype=np.int32)
+        o = _abi.SlideOut()
+        for k in _abi.SLIDE_OUT_FIELDS:
+            setattr(o, k, _abi.ptr(res[k]) if res[k].size else None)
+        self._check(self.lib.viml_slide_vi(self.h, C.byref(s), _abi.ptr(ex), X, _abi.ptr(mg), float(init_depth), C.byref(o),
+                                           flags & ~PTRS_DEVICE))
         return res
 
     def linearize(self, batch, flags, out=None, obs_table=False, line_table=False):

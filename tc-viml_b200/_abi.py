@@ -192,6 +192,15 @@ class PriorOut(C.Structure):
     _fields_ = [("prior_n_max", C.c_int32), ("prior_max_blocks", C.c_int32)] + [(n, C.c_void_p) for n in PRIOR_OUT_FIELDS]
 
 
+SLIDE_OUT_FIELDS = ("poses", "ex_pose", "inv_depth", "extra")
+
+
+class SlideOut(C.Structure):
+    """viml_slide_out — the next frame's parameter blocks written by viml_slide_vi."""
+
+    _fields_ = [(n, C.c_void_p) for n in SLIDE_OUT_FIELDS]
+
+
 class Inertial:
     """Host-side container of one viml_inertial_factors (numpy arrays, shapes as in viml.h).
 

@@ -486,6 +486,20 @@ struct MargViArgs {
 int viml_launch_marg_select(viml_ctx* ctx, const MargViArgs& g);
 int viml_launch_marg_gather(viml_ctx* ctx, const MargViArgs& g);
 
+// viml_slide_vi (marg_kernels.cu): the next frame's state of every window.  Device pointers only.
+struct SlideArgs {
+  int W, P, F, X;
+  double init_depth;
+  const int32_t* margin;            // [W] VIML_MARGIN_*
+  const double *poses, *ex_pose, *inv_depth, *extra;   // the state at the linearisation point
+  const int32_t* pf_window_offset;  // the batch's point factors (pf_obs expanded)
+  const uint32_t* pf_idx;
+  const double* pf_obs;
+  const double* pf_pts_i_z;         // nullable
+  viml_slide_out out;
+};
+int viml_launch_slide(viml_ctx* ctx, const SlideArgs& s);
+
 // linearize_kernels.cu
 int viml_launch_linearize(viml_ctx* ctx, const LinearizeArgs& a);
 int viml_launch_prep(viml_ctx* ctx, const LinearizeArgs& a);   // pose cache of the state in `a` only

@@ -381,18 +381,44 @@ int check_solve_options(viml_ctx* ctx, const viml_solve_options* o) {
   return VIML_OK;
 }
 
+// The host-pointer preconditions viml_marginalize_vi and viml_slide_vi share (viml.h), after the batch's indices are checked: every
+// margin[w] is 0 or 1, and no feature has point factors with both i == 0 and i != 0 (the outgoing frame anchors all of a feature's
+// factors or none).
+int check_margin_and_anchors(viml_ctx* ctx, const viml_window_batch* in, const int32_t* margin, const char* who) {
+  const int W = in->n_windows, F = in->feats_per_window;
+  for (int w = 0; w < W; ++w)
+    if (margin[w] != VIML_MARGIN_OLD && margin[w] != VIML_MARGIN_SECOND_NEW) {
+      ctx->err = std::string(who) + ": margin[w] must be 0 or 1";
+      return VIML_ERR_INVALID;
+    }
+  std::vector<uint8_t> feat(F);
+  for (int w = 0; w < W; ++w) {
+    std::fill(feat.begin(), feat.end(), 0);
+    for (int64_t k = in->pf_window_offset[w]; k < in->pf_window_offset[w + 1]; ++k) {
+      const uint32_t ix = in->pf_idx[k];
+      const int f = ix >> 16;
+      feat[f] |= (ix & 0xffu) == 0 ? 1 : 2;
+      if (feat[f] == 3) {
+        ctx->err = std::string(who) + ": a feature has factors with both i == 0 and i != 0";
+        return VIML_ERR_INVALID;
+      }
+    }
+  }
+  return VIML_OK;
+}
+
 // viml_marginalize_vi's preconditions on host pointers (viml.h), after check_step_inputs.  The kept dimension and block count of every
 // window follow marg_gather_kernel's selection.
 int check_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_inertial_factors* vi, const int32_t* margin,
                          const viml_prior_out* out) {
-  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window;
-  for (int w = 0; w < W; ++w)
-    if (margin[w] != VIML_MARGIN_OLD && margin[w] != VIML_MARGIN_SECOND_NEW) return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: margin[w] must be 0 or 1");
+  const int W = in->n_windows, P = in->poses_per_window;
+  int rc = check_margin_and_anchors(ctx, in, margin, "viml_marginalize_vi");
+  if (rc != VIML_OK) return rc;
   for (int64_t k = 0; k < vi->n_imu; ++k)
     if (vi->imu_sb[2 * k] != 9 * vi->imu_pose[2 * k] || vi->imu_sb[2 * k + 1] != 9 * vi->imu_pose[2 * k + 1])
       return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: the speed-bias of pose p must sit at extra offset 9p (imu_sb == {9i, 9j})");
   const int NS = 2 * P + 1;
-  std::vector<uint8_t> touch(NS), feat(F);
+  std::vector<uint8_t> touch(NS);
   for (int w = 0; w < W; ++w) {
     const bool old = margin[w] == VIML_MARGIN_OLD;
     const int n_in = vi->prior_n_max > 0 ? vi->prior_n[w] : 0, nb_in = n_in > 0 ? vi->prior_n_blocks[w] : 0;
@@ -413,13 +439,9 @@ int check_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_
       has = has || s == P - 2;
       touch[s] = 1;
     }
-    std::fill(feat.begin(), feat.end(), 0);
-    for (int64_t k = in->pf_window_offset[w]; k < in->pf_window_offset[w + 1]; ++k) {
+    for (int64_t k = in->pf_window_offset[w]; old && k < in->pf_window_offset[w + 1]; ++k) {
       const uint32_t ix = in->pf_idx[k];
-      const int i = ix & 0xffu, j = (ix >> 8) & 0xffu, f = ix >> 16;
-      feat[f] |= i == 0 ? 1 : 2;
-      if (feat[f] == 3) return fail(ctx, VIML_ERR_INVALID, "viml_marginalize_vi: a feature has factors with both i == 0 and i != 0");
-      if (old && i == 0) touch[0] = touch[j] = touch[P] = 1;
+      if ((ix & 0xffu) == 0) touch[0] = touch[(ix >> 8) & 0xffu] = touch[P] = 1;
     }
     int n = 0, nb = 0;
     if (!old && !has) {
@@ -535,6 +557,53 @@ int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_i
   if (rc == VIML_OK && n_max > 0)   // MarginalizationInfo::eps (marginalization_factor.h:70)
     rc = viml_launch_marginalize(ctx, W, g.pm, 0, 1e-8, g.A, g.b, nullptr, nullptr, g.out.prior_jacobian, g.out.prior_residual, g.sizes,
                                  15, n_max);
+  if (rc != VIML_OK) return rc;
+  return st.finish();
+}
+
+int viml_slide_vi(viml_ctx* ctx, const viml_window_batch* in, const double* extra_state, int32_t extra_dim, const int32_t* margin,
+                  double init_depth, const viml_slide_out* out, uint32_t flags) {
+  if (!ctx) return VIML_ERR_INVALID;
+  if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
+  const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
+  BatchForm form;
+  int rc = check_window_batch(ctx, in, dev, &form);
+  if (rc == VIML_OK && !dev && in->n_windows > 0) rc = check_batch_indices(ctx, in, form, 0, in->n_point_factors, 0, in->n_line_factors);
+  if (rc != VIML_OK) return rc;
+  const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, X = extra_dim;
+  if (P < 2) return fail(ctx, VIML_ERR_INVALID, "viml_slide_vi: needs P >= 2");
+  if (X < 9 * P) return fail(ctx, VIML_ERR_INVALID, "viml_slide_vi: extra_dim must hold the P speed-bias blocks (X >= 9P)");
+  if (!(std::isfinite(init_depth) && init_depth > 0.0)) return fail(ctx, VIML_ERR_INVALID, "viml_slide_vi: init_depth must be finite and > 0");
+  if (W == 0) return VIML_OK;
+  if (!margin || !extra_state || !out->poses || !out->ex_pose || (F > 0 && !out->inv_depth) || !out->extra)
+    return fail(ctx, VIML_ERR_INVALID, "viml_slide_vi: null margin, extra_state or output array");
+  if (!dev) {
+    rc = check_margin_and_anchors(ctx, in, margin, "viml_slide_vi");
+    if (rc != VIML_OK) return rc;
+  }
+  VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
+  Stager st{ctx, dev};
+  viml_window_batch pts = *in;   // line factors take no part
+  pts.n_line_factors = 0;
+  BatchForm pform = form;
+  pform.line_table = false;
+  StagedBatch b;
+  stage_batch(ctx, st, &pts, pform, 0, &b);
+  SlideArgs s{};
+  s.W = W, s.P = P, s.F = F, s.X = X, s.init_depth = init_depth;
+  st.in(margin, (size_t)W, &s.margin);
+  st.in(extra_state, (size_t)W * X, &s.extra);
+  st.out(out->poses, (size_t)W * P * 7, &s.out.poses);
+  st.out(out->ex_pose, (size_t)W * 7, &s.out.ex_pose);
+  st.out(out->inv_depth, (size_t)W * F, &s.out.inv_depth);
+  st.out(out->extra, (size_t)W * X, &s.out.extra);
+  rc = st.commit();
+  if (rc == VIML_OK) rc = expand_tables(ctx, b);
+  if (rc != VIML_OK) return rc;
+  const LinearizeArgs& a = b.a;
+  s.poses = a.poses, s.ex_pose = a.ex_pose, s.inv_depth = a.inv_depth;
+  s.pf_window_offset = a.pf_window_offset, s.pf_idx = a.pf_idx, s.pf_obs = a.pf_obs, s.pf_pts_i_z = a.pf_pts_i_z;
+  rc = viml_launch_slide(ctx, s);
   if (rc != VIML_OK) return rc;
   return st.finish();
 }

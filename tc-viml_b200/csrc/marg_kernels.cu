@@ -7,6 +7,8 @@
 // The eigen-decomposition is a parallel two-sided cyclic Jacobi (round-robin pair ordering, n/2 disjoint
 // rotations per round); eigen pairs are sorted ascending like Eigen.  Work matrices live in a per-CTA slice
 // of device scratch (L1/L2 resident: <= 6 * 256^2 doubles).
+// Also the per-window kernels of viml_marginalize_vi (selection, gather) and of viml_slide_vi (the state slide and the depth
+// re-anchoring that follow the marginalisation).
 #include "common.cuh"
 
 namespace {
@@ -396,6 +398,107 @@ __global__ void __launch_bounds__(256) marg_gather_kernel(MargViArgs g) {
   for (int r = tid; r < pos; r += nt) g.b[(size_t)w * g.pm + r] = g.gx[(size_t)w * Dx + s_col[r]];
 }
 
+// ---- viml_slide_vi: the window slide (est.cpp:2121-2218) and removeBackShiftDepth, plain IEEE binary64 without fused multiply-adds --
+constexpr int kSlideThreads = 256;
+constexpr int kSlideChunk = 4096;   // features counted per pass over the window's point factors (F <= 65535: up to 16 passes)
+
+__device__ __forceinline__ double dot3_rn(double a0, double a1, double a2, double b0, double b1, double b2) {
+  return __dadd_rn(__dadd_rn(__dmul_rn(a0, b0), __dmul_rn(a1, b1)), __dmul_rn(a2, b2));
+}
+
+// normalized(q).toRotationMatrix() of a [p, q] block, Eigen's order (double2vector forms Rs so)
+__device__ void slide_rot(const double* p7, double* R) {
+  const double qx = p7[3], qy = p7[4], qz = p7[5], qw = p7[6];
+  const double n = __dsqrt_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(qx, qx), __dmul_rn(qy, qy)), __dmul_rn(qz, qz)), __dmul_rn(qw, qw)));
+  const double w = __ddiv_rn(qw, n), x = __ddiv_rn(qx, n), y = __ddiv_rn(qy, n), z = __ddiv_rn(qz, n);
+  const double tx = __dmul_rn(2.0, x), ty = __dmul_rn(2.0, y), tz = __dmul_rn(2.0, z);
+  const double twx = __dmul_rn(tx, w), twy = __dmul_rn(ty, w), twz = __dmul_rn(tz, w);
+  const double txx = __dmul_rn(tx, x), txy = __dmul_rn(ty, x), txz = __dmul_rn(tz, x);
+  const double tyy = __dmul_rn(ty, y), tyz = __dmul_rn(tz, y), tzz = __dmul_rn(tz, z);
+  R[0] = __dsub_rn(1.0, __dadd_rn(tyy, tzz)), R[1] = __dsub_rn(txy, twz), R[2] = __dadd_rn(txz, twy);
+  R[3] = __dadd_rn(txy, twz), R[4] = __dsub_rn(1.0, __dadd_rn(txx, tzz)), R[5] = __dsub_rn(tyz, twx);
+  R[6] = __dsub_rn(txz, twy), R[7] = __dadd_rn(tyz, twx), R[8] = __dsub_rn(1.0, __dadd_rn(txx, tyy));
+}
+
+// The camera of a pose: R = R(q) R(q_ex) (cam[0..8], row-major), P = p + R(q) t_ex (cam[9..11])
+__device__ void slide_camera(const double* pose, const double* ex, double* cam) {
+  double Rb[9], Re[9];
+  slide_rot(pose, Rb);
+  slide_rot(ex, Re);
+  for (int r = 0; r < 3; ++r) {
+    for (int c = 0; c < 3; ++c) cam[3 * r + c] = dot3_rn(Rb[3 * r], Rb[3 * r + 1], Rb[3 * r + 2], Re[c], Re[3 + c], Re[6 + c]);
+    cam[9 + r] = __dadd_rn(pose[r], dot3_rn(Rb[3 * r], Rb[3 * r + 1], Rb[3 * r + 2], ex[0], ex[1], ex[2]));
+  }
+}
+
+// removeBackShiftDepth for one feature: the inverse depth of the point seen from camera c0 along (ux, uy, uz) at 1 / inv, in camera c1
+__device__ double slide_reanchor(double inv, double ux, double uy, double uz, const double* c0, const double* c1, double init_depth) {
+  const double d = __ddiv_rn(1.0, inv);
+  const double a0 = __dmul_rn(ux, d), a1 = __dmul_rn(uy, d), a2 = __dmul_rn(uz, d);
+  double v[3];
+  for (int r = 0; r < 3; ++r)   // w - P1, w = R0 (uv_i d) + P0
+    v[r] = __dsub_rn(__dadd_rn(dot3_rn(c0[3 * r], c0[3 * r + 1], c0[3 * r + 2], a0, a1, a2), c0[9 + r]), c1[9 + r]);
+  const double zj = dot3_rn(c1[2], c1[5], c1[8], v[0], v[1], v[2]);   // row 2 of R1^T
+  return zj > 0.0 ? __ddiv_rn(1.0, zj) : __ddiv_rn(1.0, init_depth);
+}
+
+// One CTA per window: the state copied with the slide (coalesced over the window's P*7 + 7 + X + F values), then for MARGIN_OLD the
+// anchor-0 factors counted per feature (a shared-memory counter and the first factor of each feature in a chunk of kSlideChunk
+// features), and every feature with two or more re-anchored by one thread from its first factor.
+__global__ void __launch_bounds__(kSlideThreads) slide_kernel(SlideArgs s) {
+  __shared__ int s_cnt[kSlideChunk];
+  __shared__ int s_first[kSlideChunk];
+  __shared__ double s_cam[24];   // the cameras of the old poses 0 and 1
+  const int w = blockIdx.x, tid = threadIdx.x, nt = blockDim.x, P = s.P, F = s.F, X = s.X;
+  const bool old = s.margin[w] == VIML_MARGIN_OLD;
+  const double* pin = s.poses + (size_t)w * P * 7;
+  const double* ein = s.ex_pose + (size_t)w * 7;
+  const double* xin = s.extra + (size_t)w * X;
+  const double* din = s.inv_depth + (size_t)w * F;
+  double* dout = s.out.inv_depth + (size_t)w * F;
+  const int np = 7 * P, n = np + 7 + X + F;
+  auto from = [&](int q) { return old ? min(q + 1, P - 1) : q == P - 2 ? P - 1 : q; };   // the slot that moves into slot q
+  for (int e = tid; e < n; e += nt) {
+    if (e < np) {
+      const int p = e / 7;
+      s.out.poses[(size_t)w * np + e] = pin[7 * from(p) + e - 7 * p];
+    } else if (e < np + 7) {
+      s.out.ex_pose[(size_t)w * 7 + e - np] = ein[e - np];
+    } else if (e < np + 7 + X) {
+      const int x = e - np - 7, q = x / 9;
+      s.out.extra[(size_t)w * X + x] = xin[q < P ? 9 * from(q) + x - 9 * q : x];
+    } else {
+      dout[e - np - 7 - X] = din[e - np - 7 - X];
+    }
+  }
+  if (!old) return;   // CTA-uniform
+  if (tid == 0) slide_camera(pin, ein, s_cam);
+  if (tid == 32) slide_camera(pin + 7, ein, s_cam + 12);
+  const int k0 = s.pf_window_offset[w], k1 = s.pf_window_offset[w + 1];
+  for (int f0 = 0; f0 < F; f0 += kSlideChunk) {
+    const int nf = min(kSlideChunk, F - f0);
+    for (int f = tid; f < nf; f += nt) s_cnt[f] = 0, s_first[f] = 0x7fffffff;
+    __syncthreads();   // orders the copy of the depths above before their re-anchored values below, and publishes s_cam
+    for (int k = k0 + tid; k < k1; k += nt) {
+      const uint32_t ix = s.pf_idx[k];
+      const int f = (int)(ix >> 16) - f0;
+      if ((ix & 0xffu) == 0 && f >= 0 && f < nf) {
+        atomicAdd(&s_cnt[f], 1);
+        atomicMin(&s_first[f], k);
+      }
+    }
+    __syncthreads();
+    for (int f = tid; f < nf; f += nt) {
+      if (s_cnt[f] < 2) continue;   // one anchor-0 factor: the reference erases the feature
+      const int k = s_first[f];
+      const double* ob = s.pf_obs + (size_t)4 * k;
+      const double z = s.pf_pts_i_z ? s.pf_pts_i_z[k] : 1.0;
+      dout[f0 + f] = slide_reanchor(din[f0 + f], ob[0], ob[1], z, s_cam, s_cam + 12, s.init_depth);
+    }
+    __syncthreads();   // s_cnt / s_first are read before the next chunk resets them
+  }
+}
+
 }  // namespace
 
 int viml_launch_marg_select(viml_ctx* ctx, const MargViArgs& g) {
@@ -416,6 +519,15 @@ int viml_launch_marg_gather(viml_ctx* ctx, const MargViArgs& g) {
   {
     LaunchScope ls(ctx, K_MARG);
     marg_gather_kernel<<<g.W, 256, 0, ctx->stream>>>(g);
+  }
+  VIML_TRY_CUDA(ctx, cudaGetLastError());
+  return VIML_OK;
+}
+
+int viml_launch_slide(viml_ctx* ctx, const SlideArgs& s) {
+  {
+    LaunchScope ls(ctx, K_MARG);
+    slide_kernel<<<s.W, kSlideThreads, 0, ctx->stream>>>(s);
   }
   VIML_TRY_CUDA(ctx, cudaGetLastError());
   return VIML_OK;
