@@ -245,15 +245,19 @@ class Context:
                                                  flags & ~PTRS_DEVICE))
         return Sx, gx
 
-    def gn_step(self, batch, dense, extra, flags, lam=0.0, obs_table=False, line_table=False):
-        """viml_gn_step with host buffers: dict(poses, ex_pose, inv_depth, extra, dx, cost, solved)."""
-        X = dense.X if dense is not None else 0
+    @staticmethod
+    def _state_out(batch, X):
+        """NaN-filled host outputs of the window state: dict(poses, ex_pose, inv_depth, extra [W, X])."""
+        return {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
+                "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((batch.W, X), np.nan)}
+
+    def _gn_step(self, fn, batch, factors, X, extra, flags, lam, obs_table, line_table):
+        """fn = viml_gn_step (factors: the dense factors or None) or viml_gn_step_vi (the inertial factors) with host buffers."""
         W, Dx = batch.W, batch.D + X
-        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
-               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan),
-               "dx": np.full((W, Dx), np.nan), "cost": np.full((W, 3), np.nan), "solved": np.full(W, -1, dtype=np.int32)}
+        res = {**self._state_out(batch, X), "dx": np.full((W, Dx), np.nan), "cost": np.full((W, 3), np.nan),
+               "solved": np.full(W, -1, dtype=np.int32)}
         s, _keep = self._batch_struct(batch, obs_table, line_table)
-        d = dense.struct() if dense is not None else None
+        f = factors.struct() if factors is not None else None
         ex = None if extra is None else np.ascontiguousarray(extra, dtype=np.float64)
         opt = _abi.GnOptions()
         opt.lambda_ = float(lam)
@@ -261,9 +265,14 @@ class Context:
         for k in ("poses", "ex_pose", "inv_depth", "dx", "cost", "solved"):
             setattr(o, k, _abi.ptr(res[k]))
         o.extra = _abi.ptr(res["extra"]) if X > 0 else None
-        self._check(self.lib.viml_gn_step(self.h, C.byref(s), C.byref(d) if d is not None else None, _abi.ptr(ex), C.byref(opt),
-                                          C.byref(o), flags & ~PTRS_DEVICE))
+        self._check(fn(self.h, C.byref(s), C.byref(f) if f is not None else None, _abi.ptr(ex), C.byref(opt), C.byref(o),
+                       flags & ~PTRS_DEVICE))
         return res
+
+    def gn_step(self, batch, dense, extra, flags, lam=0.0, obs_table=False, line_table=False):
+        """viml_gn_step with host buffers: dict(poses, ex_pose, inv_depth, extra, dx, cost, solved)."""
+        X = dense.X if dense is not None else 0
+        return self._gn_step(self.lib.viml_gn_step, batch, dense, X, extra, flags, lam, obs_table, line_table)
 
     def inertial_evaluate(self, batch, extra, vi):
         """viml_inertial_evaluate with host buffers at the state (batch.poses, batch.ex_pose, extra [W, X]): dict of the
@@ -284,23 +293,7 @@ class Context:
 
     def gn_step_vi(self, batch, vi, extra, flags, lam=0.0, obs_table=False, line_table=False):
         """viml_gn_step_vi with host buffers: dict(poses, ex_pose, inv_depth, extra, dx, cost, solved)."""
-        X = vi.X
-        W, Dx = batch.W, batch.D + X
-        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
-               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan),
-               "dx": np.full((W, Dx), np.nan), "cost": np.full((W, 3), np.nan), "solved": np.full(W, -1, dtype=np.int32)}
-        s, _keep = self._batch_struct(batch, obs_table, line_table)
-        v = vi.struct()
-        ex = None if extra is None else np.ascontiguousarray(extra, dtype=np.float64)
-        opt = _abi.GnOptions()
-        opt.lambda_ = float(lam)
-        o = _abi.GnOut()
-        for k in ("poses", "ex_pose", "inv_depth", "dx", "cost", "solved"):
-            setattr(o, k, _abi.ptr(res[k]))
-        o.extra = _abi.ptr(res["extra"]) if X > 0 else None
-        self._check(self.lib.viml_gn_step_vi(self.h, C.byref(s), C.byref(v), _abi.ptr(ex), C.byref(opt), C.byref(o),
-                                             flags & ~PTRS_DEVICE))
-        return res
+        return self._gn_step(self.lib.viml_gn_step_vi, batch, vi, vi.X, extra, flags, lam, obs_table, line_table)
 
     @staticmethod
     def solve_options(max_iterations=50, max_consecutive_invalid=5, initial_radius=1e4, max_radius=1e16, min_radius=1e-32,
@@ -319,9 +312,7 @@ class Context:
         """viml_solve_vi with host buffers: dict(poses, ex_pose, inv_depth, extra, status, iterations, accepted, cost [W,2],
         radius [W], trace [W,max_iterations,4])."""
         X, W = vi.X, batch.W
-        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
-               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan),
-               "status": np.full(W, -1, dtype=np.int32), "iterations": np.full(W, -1, dtype=np.int32),
+        res = {**self._state_out(batch, X), "status": np.full(W, -1, dtype=np.int32), "iterations": np.full(W, -1, dtype=np.int32),
                "accepted": np.full(W, -1, dtype=np.int32), "cost": np.full((W, 2), np.nan), "radius": np.full(W, np.nan),
                "trace": np.full((W, max(int(max_iterations), 0), 4), -1.0)}
         s, _keep = self._batch_struct(batch, obs_table, line_table)
@@ -364,9 +355,8 @@ class Context:
         """viml_slide_vi with host buffers: the next frame's state of every window (margin[w] = MARGIN_OLD or MARGIN_SECOND_NEW) as
         a dict(poses [W, P, 7], ex_pose [W, 7], inv_depth [W, F], extra [W, X])."""
         ex = np.ascontiguousarray(extra, dtype=np.float64)
-        W, X = batch.W, ex.shape[1] if ex.ndim == 2 else 0
-        res = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
-               "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan)}
+        X = ex.shape[1] if ex.ndim == 2 else 0
+        res = self._state_out(batch, X)
         s, _keep = self._batch_struct(batch, obs_table)
         mg = np.ascontiguousarray(margin, dtype=np.int32)
         o = _abi.SlideOut()

@@ -169,6 +169,43 @@ int stage_dense(viml_ctx* ctx, Stager& st, const viml_dense_factors* dense, int 
   return VIML_OK;
 }
 
+// The extra tangent columns of a step: the inertial factors' when given, else the dense factors'.
+int step_extra_dim(const viml_dense_factors* dense, const viml_inertial_factors* vi) {
+  return vi ? vi->extra_dim : dense ? dense->extra_dim : 0;
+}
+
+// Device scratch of the H/b blocks and the Schur step of W windows (VIML_OUT_HB | VIML_OUT_SCHUR) into *o.
+void stage_hb_scratch(Stager& st, int W, int D, int F, viml_linearize_out* o) {
+  st.out((double*)nullptr, (size_t)W * D * D, &o->H_pp);
+  st.out((double*)nullptr, (size_t)W * F * D, &o->H_lp);
+  st.out((double*)nullptr, (size_t)W * F, &o->H_ll);
+  st.out((double*)nullptr, (size_t)W * D, &o->b_p);
+  st.out((double*)nullptr, (size_t)W * F, &o->b_l);
+  st.out((double*)nullptr, (size_t)W * D * D, &o->S);
+  st.out((double*)nullptr, (size_t)W * D, &o->g);
+}
+
+// The batch without its line factors (form: check_window_batch's): the marginalisation and the slide read the point factors only.
+void stage_point_batch(viml_ctx* ctx, Stager& st, const viml_window_batch* in, BatchForm form, uint32_t flags, StagedBatch* b) {
+  viml_window_batch pts = *in;
+  pts.n_line_factors = 0;
+  form.line_table = false;
+  stage_batch(ctx, st, &pts, form, flags, b);
+}
+
+// The dense-block factors every kernel reads, over the CSR `c` of the IMU / prior factors of `v`.  ND = W + NI is an upper bound:
+// the kernels read ND only as "any dense factors".
+DenseArgs dense_view(const InertialArgs& v, const InertialCsr& c) {
+  return DenseArgs{v.X, (int64_t)v.W + v.NI, c.window_offset, c.row_offset, c.col_offset, c.jac_offset, c.col_index, c.residual, c.jacobian};
+}
+
+// Evaluates the IMU / prior factors of `v` at (poses, ex_pose, extra), kept in `v`, into `csr`; csr.jacobian null: residuals only.
+int enqueue_inertial_at(viml_ctx* ctx, InertialArgs& v, const double* poses, const double* ex_pose, const double* extra,
+                        const InertialCsr& csr) {
+  v.poses = poses, v.ex_pose = ex_pose, v.extra = extra;
+  return viml_launch_inertial(ctx, v, viml_inertial_out{}, csr, csr.jacobian != nullptr);
+}
+
 // Everything one Gauss-Newton step enqueues (device pointers), staged once: viml_gn_step / viml_gn_step_vi enqueue one step,
 // viml_solve_vi one per round.  The state the step starts from is b.a.poses, b.a.ex_pose, b.a.inv_depth and extra; x+ goes to o_*.
 struct StepPlan {
@@ -194,27 +231,20 @@ int stage_step(viml_ctx* ctx, Stager& st, const viml_window_batch* in, const Bat
                const viml_inertial_factors* vi, StepPlan* s) {
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, D = 6 * (P + 1);
   *s = StepPlan{};
-  s->W = W, s->X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0, s->Dx = D + s->X;
+  s->W = W, s->X = step_extra_dim(dense, vi), s->Dx = D + s->X;
   const int X = s->X, Dx = s->Dx;
   s->vi = vi != nullptr, s->fused = gout && !(rout && (rout->Sx || rout->gx)) && gn_fused_takes(Dx);
   s->dn.X = X;
   int rc = stage_dense(ctx, st, dense, W, Dx, &s->dn);
   if (rc != VIML_OK) return rc;
   stage_batch(ctx, st, in, form, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR, &s->b);
-  LinearizeArgs& a = s->b.a;
   st.in(extra_state, extra_state ? (size_t)W * X : 0, &s->extra);
   if (vi) {
     stage_inertial(st, vi, W, P, &s->va);
     stage_inertial_csr(st, s->va, &s->csr, &s->res_plus);
   }
   // scratch (host == nullptr) and outputs
-  st.out((double*)nullptr, (size_t)W * D * D, &a.out.H_pp);
-  st.out((double*)nullptr, (size_t)W * F * D, &a.out.H_lp);
-  st.out((double*)nullptr, (size_t)W * F, &a.out.H_ll);
-  st.out((double*)nullptr, (size_t)W * D, &a.out.b_p);
-  st.out((double*)nullptr, (size_t)W * F, &a.out.b_l);
-  st.out((double*)nullptr, (size_t)W * D * D, &a.out.S);
-  st.out((double*)nullptr, (size_t)W * D, &a.out.g);
+  stage_hb_scratch(st, W, D, F, &s->b.a.out);
   if (!s->fused) {
     st.out(rout ? rout->Sx : nullptr, (size_t)W * Dx * Dx, &s->Sx);
     st.out(rout ? rout->gx : nullptr, (size_t)W * Dx, &s->gx);
@@ -239,6 +269,17 @@ struct DoglegRound {
   int round;
 };
 
+// The solve of a step: the system built and solved in one kernel where s.fused, else reduced_kernel into s.Sx / s.gx and the
+// unfused solve.  lambda, lambda_w, gate (the windows solved), damp: see viml_launch_gn_reduced_solve.
+int enqueue_solve(viml_ctx* ctx, const StepPlan& s, const DenseArgs& dn, double lambda, const double* lambda_w, const int32_t* gate,
+                  const double* damp) {
+  const LinearizeArgs& a = s.b.a;
+  if (s.fused) return viml_launch_gn_reduced_solve(ctx, s.W, a.D, dn, a.out.S, a.out.g, lambda, s.dx, s.solved, s.cost, lambda_w, gate, damp);
+  const int rc = viml_launch_reduced(ctx, s.W, a.D, dn, a.out.S, a.out.g, s.Sx, s.gx);
+  if (rc != VIML_OK) return rc;
+  return viml_launch_gn_solve(ctx, s.W, s.Dx, lambda, s.Sx, s.gx, s.dx, s.solved, s.cost, lambda_w, gate, damp);
+}
+
 // One step at the state of s.b.a / s.extra: without s.cost the reduced system Sx, gx alone; with it the cost at x, the solve (the
 // system built in the solve kernel when s.fused), the update into s.o_* and the cost at x+.  lambda_w / running: see
 // viml_launch_gn_reduced_solve (nullptr: `lambda`, every window).
@@ -250,83 +291,61 @@ struct DoglegRound {
 int enqueue_step(viml_ctx* ctx, const StepPlan& s, double lambda, const double* lambda_w, const int32_t* running,
                  const DoglegRound* dg = nullptr) {
   const LinearizeArgs& a = s.b.a;
-  const int W = s.W, D = a.D, X = s.X, Dx = s.Dx;
-  const bool step = s.cost != nullptr;
-  int rc;
-  if (dg) {
-    LinearizeArgs al = a;
-    al.flags &= ~VIML_OUT_SCHUR;
-    rc = viml_launch_linearize(ctx, al);
-  } else {
-    rc = viml_launch_linearize(ctx, a);
-  }
-  if (rc != VIML_OK) return rc;
-  DenseArgs dn = s.dn;
+  const int W = s.W, D = a.D;
+  const DoglegArgs* g = dg ? dg->g : nullptr;
+  LinearizeArgs al = a;
+  if (dg) al.flags &= ~VIML_OUT_SCHUR;
+  int rc = viml_launch_linearize(ctx, al);
   InertialArgs va = s.va;
-  if (s.vi) {   // the dense-block factors at x, in the CSR every kernel below reads
-    va.poses = a.poses, va.ex_pose = a.ex_pose, va.extra = s.extra;
-    rc = viml_launch_inertial(ctx, va, viml_inertial_out{}, s.csr, true);
-    if (rc != VIML_OK) return rc;
-    dn.ND = (int64_t)W + va.NI;   // an upper bound: the kernels read ND only as "any dense factors"
-    dn.window_offset = s.csr.window_offset, dn.row_offset = s.csr.row_offset, dn.col_offset = s.csr.col_offset;
-    dn.jac_offset = s.csr.jac_offset, dn.col_index = s.csr.col_index, dn.residual = s.csr.residual, dn.jacobian = s.csr.jacobian;
-  }
-  if (!step) return viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
-  rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
+  if (rc == VIML_OK && s.vi) rc = enqueue_inertial_at(ctx, va, a.poses, a.ex_pose, s.extra, s.csr);
   if (rc != VIML_OK) return rc;
-  if (dg) {
-    const DoglegArgs& g = *dg->g;
-    const int32_t* fresh = dg->round ? g.fresh : nullptr;
-    rc = viml_launch_dogleg_prepare(ctx, a, dn, g, dg->state, dg->round);
-    if (rc != VIML_OK) return rc;
+  const DenseArgs dn = s.vi ? dense_view(va, s.csr) : s.dn;
+  if (!s.cost) return viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
+  rc = viml_launch_cost(ctx, a, dn, nullptr, nullptr, 0, s.cost, running);
+  const int32_t* gate = running;
+  const double* damp = nullptr;
+  if (rc == VIML_OK && g) {   // the dogleg's damping array instead of lambda diag(Sx); a new Gauss-Newton step where fresh is set
+    rc = viml_launch_dogleg_prepare(ctx, a, dn, *g, dg->state, dg->round);
     // MarginalizationInfo::eps, as in viml_launch_linearize
-    rc = viml_launch_schur(ctx, W, a.F, D, a.out.H_pp, a.out.H_lp, a.out.H_ll, a.out.b_p, a.out.b_l, a.out.S, a.out.g, 1e-8);
-    if (rc == VIML_OK && s.fused) {
-      rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, 0.0, s.dx, s.solved, s.cost, nullptr, fresh, g.damp);
-    } else if (rc == VIML_OK) {
-      rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
-      if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, 0.0, s.Sx, s.gx, s.dx, s.solved, s.cost, nullptr, fresh, g.damp);
-    }
-    if (rc == VIML_OK) rc = viml_launch_dogleg_finish(ctx, a, dn, g, dg->state, dg->round, s.dx, s.solved);
-    if (rc == VIML_OK) rc = viml_launch_dogleg_step(ctx, W, g, dg->state, dg->initial_radius, dg->round, running, s.dx, s.cost, s.solved);
     if (rc == VIML_OK)
-      rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running, g.dl);
-  } else if (s.fused) {
-    rc = viml_launch_gn_reduced_solve(ctx, W, D, dn, a.out.S, a.out.g, lambda, s.dx, s.solved, s.cost, lambda_w, running);
-  } else {
-    rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, s.Sx, s.gx);
-    if (rc == VIML_OK) rc = viml_launch_gn_solve(ctx, W, Dx, lambda, s.Sx, s.gx, s.dx, s.solved, s.cost, lambda_w, running);
+      rc = viml_launch_schur(ctx, W, a.F, D, a.out.H_pp, a.out.H_lp, a.out.H_ll, a.out.b_p, a.out.b_l, a.out.S, a.out.g, 1e-8);
+    lambda = 0.0, lambda_w = nullptr, gate = dg->round ? g->fresh : nullptr, damp = g->damp;
   }
-  if (rc == VIML_OK && !dg)
-    rc = viml_launch_gn_update(ctx, a, X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running);
+  if (rc == VIML_OK) rc = enqueue_solve(ctx, s, dn, lambda, lambda_w, gate, damp);
+  if (rc == VIML_OK && g) rc = viml_launch_dogleg_finish(ctx, a, dn, *g, dg->state, dg->round, s.dx, s.solved);
+  if (rc == VIML_OK && g)
+    rc = viml_launch_dogleg_step(ctx, W, *g, dg->state, dg->initial_radius, dg->round, running, s.dx, s.cost, s.solved);
+  if (rc == VIML_OK)
+    rc = viml_launch_gn_update(ctx, a, s.X, s.extra, s.dx, s.solved, s.o_poses, s.o_ex, s.o_dep, s.o_extra, running, g ? g->dl : nullptr);
   if (rc != VIML_OK) return rc;
   LinearizeArgs a2 = a;
   a2.poses = s.o_poses, a2.ex_pose = s.o_ex, a2.inv_depth = s.o_dep;
   rc = viml_launch_prep(ctx, a2);
   if (rc != VIML_OK) return rc;
-  if (s.vi) {   // f(x+): the IMU / prior residuals re-evaluated at x+ (same CSR structure), 1/2 |r|^2 without the linear model
-    InertialArgs vp = va;
-    vp.poses = s.o_poses, vp.ex_pose = s.o_ex, vp.extra = s.o_extra;
-    InertialCsr cp = s.csr;
-    cp.residual = s.res_plus, cp.jacobian = nullptr;
-    rc = viml_launch_inertial(ctx, vp, viml_inertial_out{}, cp, false);
-    DenseArgs dp = dn;
-    dp.residual = s.res_plus;
-    if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, nullptr, 1, s.cost, running);
-  } else {
-    rc = viml_launch_cost(ctx, a2, dn, s.dx, s.solved, 1, s.cost, running);
-  }
+  if (!s.vi) return viml_launch_cost(ctx, a2, dn, s.dx, s.solved, 1, s.cost, running);
+  // f(x+): the IMU / prior residuals re-evaluated at x+ (same CSR structure), 1/2 |r|^2 without the linear model
+  InertialCsr cp = s.csr;
+  cp.residual = s.res_plus, cp.jacobian = nullptr;
+  rc = enqueue_inertial_at(ctx, va, s.o_poses, s.o_ex, s.o_extra, cp);
+  DenseArgs dp = dn;
+  dp.residual = s.res_plus;
+  if (rc == VIML_OK) rc = viml_launch_cost(ctx, a2, dp, nullptr, nullptr, 1, s.cost, running);
   return rc;
 }
 
-// Checks shared by viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi: the batch (*form: how it carries its
-// observations and line factors), and with `vi` the inertial factors and the extra state.
+// The window batch (*form: how it carries its observations and line factors), with host pointers its indices too.
+int check_batch(viml_ctx* ctx, const viml_window_batch* in, bool dev, BatchForm* form) {
+  const int rc = check_window_batch(ctx, in, dev, form);
+  if (rc != VIML_OK || dev || in->n_windows == 0) return rc;
+  return check_batch_indices(ctx, in, *form, 0, in->n_point_factors, 0, in->n_line_factors);
+}
+
+// Checks shared by viml_reduced_system / viml_gn_step / viml_gn_step_vi / viml_solve_vi / viml_marginalize_vi: the batch, and with
+// `vi` the inertial factors and the extra state.
 int check_step_inputs(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* dense, const double* extra_state,
                       uint32_t flags, const viml_inertial_factors* vi, const char* who, BatchForm* form) {
   const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
-  int rc = check_window_batch(ctx, in, dev, form);
-  if (rc == VIML_OK && !dev && in->n_windows > 0)
-    rc = check_batch_indices(ctx, in, *form, 0, in->n_point_factors, 0, in->n_line_factors);
+  int rc = check_batch(ctx, in, dev, form);
   if (rc != VIML_OK) return rc;
   const int P = in->poses_per_window, D = 6 * (P + 1);
   if (vi) {
@@ -337,7 +356,7 @@ int check_step_inputs(viml_ctx* ctx, const viml_window_batch* in, const viml_den
       return VIML_ERR_INVALID;
     }
   }
-  const int X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0;
+  const int X = step_extra_dim(dense, vi);
   const int64_t ND = dense && !vi ? dense->n_factors : 0;
   if (X < 0 || ND < 0 || D + X > kMaxDx) return fail(ctx, VIML_ERR_INVALID, "dense factors: extra_dim out of range (D + extra_dim <= 232)");
   return VIML_OK;
@@ -351,7 +370,7 @@ int run(viml_ctx* ctx, const viml_window_batch* in, const viml_dense_factors* de
   BatchForm form;
   int rc = check_step_inputs(ctx, in, dense, extra_state, flags, vi, "viml_gn_step_vi", &form);
   if (rc != VIML_OK) return rc;
-  const int W = in->n_windows, F = in->feats_per_window, X = vi ? vi->extra_dim : dense ? dense->extra_dim : 0;
+  const int W = in->n_windows, F = in->feats_per_window, X = step_extra_dim(dense, vi);
   const bool step = gout != nullptr;
   if (step && !(gout->poses && gout->ex_pose && (F == 0 || gout->inv_depth) && gout->cost && gout->solved))
     return fail(ctx, VIML_ERR_INVALID, "viml_gn_step needs poses, ex_pose, inv_depth, cost and solved outputs");
@@ -490,12 +509,8 @@ int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_i
   }
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
   Stager st{ctx, dev};
-  viml_window_batch pts = *in;   // line factors take no part (est.cpp:1911-2046 adds none)
-  pts.n_line_factors = 0;
-  BatchForm pform = form;
-  pform.line_table = false;
-  StagedBatch b;
-  stage_batch(ctx, st, &pts, pform, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR, &b);
+  StagedBatch b;   // line factors take no part (est.cpp:1911-2046 adds none)
+  stage_point_batch(ctx, st, in, form, (flags & VIML_LOSS_CAUCHY) | VIML_OUT_HB | VIML_OUT_SCHUR, &b);
   LinearizeArgs& a = b.a;
   MargViArgs g{};
   g.W = W, g.P = P, g.D = D, g.X = X;
@@ -511,13 +526,7 @@ int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_i
   st.out((uint32_t*)nullptr, (size_t)NP, &g.sel_idx);
   st.out((double*)nullptr, (size_t)NP * 4, &g.sel_obs);
   if (in->pf_pts_i_z) st.out((double*)nullptr, (size_t)NP, &g.sel_z);
-  st.out((double*)nullptr, (size_t)W * D * D, &a.out.H_pp);
-  st.out((double*)nullptr, (size_t)W * F * D, &a.out.H_lp);
-  st.out((double*)nullptr, (size_t)W * F, &a.out.H_ll);
-  st.out((double*)nullptr, (size_t)W * D, &a.out.b_p);
-  st.out((double*)nullptr, (size_t)W * F, &a.out.b_l);
-  st.out((double*)nullptr, (size_t)W * D * D, &a.out.S);
-  st.out((double*)nullptr, (size_t)W * D, &a.out.g);
+  stage_hb_scratch(st, W, D, F, &a.out);
   double *Sx = nullptr, *gx = nullptr;
   st.out((double*)nullptr, (size_t)W * Dx * Dx, &Sx);
   st.out((double*)nullptr, (size_t)W * Dx, &gx);
@@ -536,8 +545,7 @@ int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_i
   if (rc == VIML_OK) rc = expand_tables(ctx, b);
   if (rc != VIML_OK) return rc;
   // the IMU factors and the prior at x, into the dense-factor CSR
-  g.v.poses = a.poses, g.v.ex_pose = a.ex_pose, g.v.extra = extra;
-  rc = viml_launch_inertial(ctx, g.v, viml_inertial_out{}, g.csr, true);
+  rc = enqueue_inertial_at(ctx, g.v, a.poses, a.ex_pose, extra, g.csr);
   if (rc != VIML_OK) return rc;
   g.pf_window_offset = a.pf_window_offset, g.pf_idx = a.pf_idx, g.pf_obs = a.pf_obs, g.pf_pts_i_z = a.pf_pts_i_z;
   rc = viml_launch_marg_select(ctx, g);
@@ -546,11 +554,7 @@ int viml_marginalize_vi(viml_ctx* ctx, const viml_window_batch* in, const viml_i
   a.pf_window_offset = g.sel_offset, a.pf_idx = g.sel_idx, a.pf_obs = g.sel_obs, a.pf_pts_i_z = g.sel_z;
   rc = viml_launch_linearize(ctx, a);
   if (rc != VIML_OK) return rc;
-  DenseArgs dn{};
-  dn.X = X, dn.ND = (int64_t)W + g.v.NI;   // an upper bound: the kernels read ND only as "any dense factors"
-  dn.window_offset = g.csr.window_offset, dn.row_offset = g.csr.row_offset, dn.col_offset = g.csr.col_offset;
-  dn.jac_offset = g.csr.jac_offset, dn.col_index = g.csr.col_index, dn.residual = g.csr.residual, dn.jacobian = g.csr.jacobian;
-  rc = viml_launch_reduced(ctx, W, D, dn, a.out.S, a.out.g, Sx, gx);
+  rc = viml_launch_reduced(ctx, W, D, dense_view(g.v, g.csr), a.out.S, a.out.g, Sx, gx);
   if (rc != VIML_OK) return rc;
   g.Sx = Sx, g.gx = gx;
   rc = viml_launch_marg_gather(ctx, g);
@@ -567,8 +571,7 @@ int viml_slide_vi(viml_ctx* ctx, const viml_window_batch* in, const double* extr
   if (!out) return fail(ctx, VIML_ERR_INVALID, "null output struct");
   const bool dev = (flags & VIML_PTRS_DEVICE) != 0;
   BatchForm form;
-  int rc = check_window_batch(ctx, in, dev, &form);
-  if (rc == VIML_OK && !dev && in->n_windows > 0) rc = check_batch_indices(ctx, in, form, 0, in->n_point_factors, 0, in->n_line_factors);
+  int rc = check_batch(ctx, in, dev, &form);
   if (rc != VIML_OK) return rc;
   const int W = in->n_windows, P = in->poses_per_window, F = in->feats_per_window, X = extra_dim;
   if (P < 2) return fail(ctx, VIML_ERR_INVALID, "viml_slide_vi: needs P >= 2");
@@ -583,12 +586,8 @@ int viml_slide_vi(viml_ctx* ctx, const viml_window_batch* in, const double* extr
   }
   VIML_TRY_CUDA(ctx, cudaSetDevice(ctx->device));
   Stager st{ctx, dev};
-  viml_window_batch pts = *in;   // line factors take no part
-  pts.n_line_factors = 0;
-  BatchForm pform = form;
-  pform.line_table = false;
   StagedBatch b;
-  stage_batch(ctx, st, &pts, pform, 0, &b);
+  stage_point_batch(ctx, st, in, form, 0, &b);
   SlideArgs s{};
   s.W = W, s.P = P, s.F = F, s.X = X, s.init_depth = init_depth;
   st.in(margin, (size_t)W, &s.margin);

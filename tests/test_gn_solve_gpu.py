@@ -23,6 +23,8 @@ import numpy as np
 import pytest
 import scipy.linalg
 
+from vi_helpers import Guarded
+
 U = 2.0 ** -53
 LD = np.longdouble
 U_LD = float(np.finfo(LD).eps) / 2   # unit roundoff of the extended type the reference computes in
@@ -502,30 +504,6 @@ def test_failure_only_affects_its_window(pkg, ctx, Dx):
 
 
 # ---- (f) viml_reduced_from_schur ------------------------------------------------------------------------------------------------
-class _Guarded:
-    """A device copy of a host array between GUARD bytes of a fixed pattern: check() reads the whole allocation back, fails if a byte
-    outside the array changed, and returns the array."""
-    GUARD = 4096
-
-    def __init__(self, ctx, a):
-        self.ctx, self.a = ctx, np.ascontiguousarray(a)
-        self.img = np.concatenate([np.full(self.GUARD, 0xA5, np.uint8), self.a.view(np.uint8).reshape(-1),
-                                   np.full(self.GUARD, 0x5A, np.uint8)])
-        self.base = ctx.to_device(self.img)
-        self.ptr = self.base + self.GUARD
-
-    def check(self):
-        back = np.empty_like(self.img)
-        self.ctx.d2h(back, self.base)
-        self.ctx.sync()
-        n = self.a.nbytes
-        assert np.all(back[:self.GUARD] == 0xA5) and np.all(back[self.GUARD + n:] == 0x5A), "write outside the buffer"
-        return back[self.GUARD:self.GUARD + n].view(self.a.dtype).reshape(self.a.shape)
-
-    def free(self):
-        self.ctx.device_free(self.base)
-
-
 def schur_case(rng, W, D, X):
     """Random (not symmetric: a transposed copy shows) S, g and factors over ~3/4 of the columns, one of them too large for
     reduced_kernel's stage when Dx allows."""
@@ -567,8 +545,8 @@ def test_reduced_from_schur(pkg, ctx, D, X):
         check_reduced(Ref(Dx, per[w], S[w], g[w]), Sx[w], gx[w], ("from_schur", D, X, w))
     # device pointers: the same bits, nothing written outside Sx / gx, the inputs left as they were
     ins = {"S": S, "g": g, **dense.arrays()}
-    gi = {k: _Guarded(ctx, a) for k, a in ins.items()}
-    go = {"Sx": _Guarded(ctx, np.full((W, Dx, Dx), np.nan)), "gx": _Guarded(ctx, np.full((W, Dx), np.nan))}
+    gi = {k: Guarded(ctx, a) for k, a in ins.items()}
+    go = {"Sx": Guarded(ctx, np.full((W, Dx, Dx), np.nan)), "gx": Guarded(ctx, np.full((W, Dx), np.nan))}
     dd = dense.struct({k: gi[k].ptr for k in dense.arrays()})
     rd = abi.ReducedOut()
     rd.Sx, rd.gx = go["Sx"].ptr, go["gx"].ptr

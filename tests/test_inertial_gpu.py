@@ -9,6 +9,7 @@ import pytest
 
 import inertial_oracle as io
 from conftest import rel_err
+from vi_helpers import device_structs, guard_all, inertial_only, rotate
 
 pytestmark = pytest.mark.gpu
 
@@ -29,15 +30,9 @@ def _case(pkg, W=6, seed=31, extra_pad=0, F=40, gaps=True, perturb=0.0):
         batch.poses[..., :3] += perturb * rng.standard_normal(batch.poses[..., :3].shape)
         for w in range(batch.W):
             for p in range(batch.P):
-                batch.poses[w, p] = _rotate(batch.poses[w, p], 0.5 * perturb * rng.standard_normal(3))
+                batch.poses[w, p] = rotate(batch.poses[w, p], 0.5 * perturb * rng.standard_normal(3))
         extra = extra + perturb * rng.standard_normal(extra.shape)
     return batch, vi, extra
-
-
-def _rotate(x, th):
-    q = io.qmul(io.quat(x), (1.0, th[0] / 2, th[1] / 2, th[2] / 2))
-    n = np.sqrt(sum(c * c for c in q))
-    return np.array([x[0], x[1], x[2], q[1] / n, q[2] / n, q[3] / n, q[0] / n])
 
 
 def _check_eval(got, ref, vi):
@@ -59,38 +54,6 @@ def test_evaluate_parity_host(pkg, orc, ctx):
     _check_eval(got, ref, vi)
 
 
-class _Guarded:
-    """A device copy of a host array with GUARD bytes of a fixed pattern on either side: after a call, check() reads the whole
-    allocation back and fails if a byte outside the array changed (a write out of bounds by the kernels of the call)."""
-    GUARD = 4096
-
-    def __init__(self, ctx, a):
-        self.ctx, self.a = ctx, np.ascontiguousarray(a)
-        self.n = self.a.nbytes
-        self.img = np.concatenate([np.full(self.GUARD, 0xA5, np.uint8), self.a.view(np.uint8).reshape(-1),
-                                   np.full(self.GUARD, 0x5A, np.uint8)])
-        self.base = ctx.to_device(self.img)
-        self.ptr = self.base + self.GUARD
-
-    def check(self):
-        back = np.empty_like(self.img)
-        self.ctx.d2h(back, self.base)
-        self.ctx.sync()
-        assert np.all(back[:self.GUARD] == 0xA5) and np.all(back[self.GUARD + self.n:] == 0x5A), "write outside the buffer"
-        return back[self.GUARD:self.GUARD + self.n].view(self.a.dtype).reshape(self.a.shape)
-
-    def free(self):
-        self.ctx.device_free(self.base)
-
-
-def _guard_all(ctx, arrays):
-    return {k: (None if a is None else _Guarded(ctx, a)) for k, a in arrays.items()}
-
-
-def _ptrs(g):
-    return {k: (None if v is None else v.ptr) for k, v in g.items()}
-
-
 def _check_inputs(g, arrays):
     """Inputs come back unchanged and nothing around them was written."""
     for k, v in g.items():
@@ -103,13 +66,13 @@ def test_evaluate_parity_device(pkg, orc, ctx):
     batch, vi, extra = _case(pkg, seed=41, extra_pad=3)
     ref = io.inertial_evaluate(orc, batch.poses, batch.ex_pose, extra, vi)
     ins = {"poses": batch.poses, "ex_pose": batch.ex_pose, "extra": extra, **vi.arrays()}
-    gi = _guard_all(ctx, ins)
+    gi = guard_all(ctx, ins)
     s = batch.struct({**batch.arrays(), "poses": gi["poses"].ptr, "ex_pose": gi["ex_pose"].ptr})
     v = vi.struct({k: gi[k].ptr for k in vi.arrays()})
     got = {"imu_residual": np.full((vi.NI, 15), np.nan), "imu_jac_pose_i": np.full((vi.NI, 15, 7), np.nan),
            "imu_jac_sb_i": np.full((vi.NI, 15, 9), np.nan), "imu_jac_pose_j": np.full((vi.NI, 15, 7), np.nan),
            "imu_jac_sb_j": np.full((vi.NI, 15, 9), np.nan), "prior_residual": np.full((vi.W, vi.n_max), np.nan)}
-    go = _guard_all(ctx, got)
+    go = guard_all(ctx, got)
     o = pkg._abi.InertialOut()
     for k in got:
         setattr(o, k, go[k].ptr)
@@ -130,15 +93,11 @@ def test_evaluate_parity_device(pkg, orc, ctx):
 def _gn_step_vi_device(pkg, ctx, batch, vi, extra, flags, lam):
     """viml_gn_step_vi with VIML_PTRS_DEVICE on guarded device copies of every input and output."""
     X, W, Dx = vi.X, batch.W, batch.D + vi.X
-    b_in = {k: a for k, a in batch.arrays().items() if a is not None}
-    ins = {**{"b_" + k: a for k, a in b_in.items()}, **{"v_" + k: a for k, a in vi.arrays().items()}, "extra": extra}
-    gi = _guard_all(ctx, ins)
-    s = batch.struct({**batch.arrays(), **{k: gi["b_" + k].ptr for k in b_in}})
-    v = vi.struct({k: gi["v_" + k].ptr for k in vi.arrays()})
+    ins, gi, s, v = device_structs(ctx, batch, vi, extra)
     outs = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
             "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, X), np.nan),
             "dx": np.full((W, Dx), np.nan), "cost": np.full((W, 3), np.nan), "solved": np.full(W, -1, dtype=np.int32)}
-    go = _guard_all(ctx, outs)
+    go = guard_all(ctx, outs)
     opt = pkg._abi.GnOptions()
     opt.lambda_ = lam
     o = pkg._abi.GnOut()
@@ -154,19 +113,13 @@ def _gn_step_vi_device(pkg, ctx, batch, vi, extra, flags, lam):
     return res
 
 
-def _inertial_only(pkg, batch):
-    W = batch.W
-    return pkg._abi.Batch(batch.poses, batch.ex_pose, batch.inv_depth, np.zeros(W + 1, dtype=np.int32),
-                          np.zeros(0, dtype=np.uint32), np.zeros((0, 4)))
-
-
 def test_gn_step_vi_device_pointers(pkg, ctx):
     """VIML_PTRS_DEVICE against the host-pointer flavour on the same inputs: bit for bit without point / line factors (every
     kernel on the path is then order-deterministic), to 1e-12 with them (the visual pose blocks are summed through shared-memory
     atomics).  Outputs are written inside their buffers only, inputs are left unchanged."""
     batch, vi, extra = _case(pkg, seed=91, gaps=False, perturb=0.01)
     flags = pkg.LOSS_CAUCHY
-    for b_, exact in ((_inertial_only(pkg, batch), True), (batch, False)):
+    for b_, exact in ((inertial_only(pkg, batch), True), (batch, False)):
         h = ctx.gn_step_vi(b_, vi, extra, flags, lam=1e-3)
         d = _gn_step_vi_device(pkg, ctx, b_, vi, extra, flags, 1e-3)
         assert h["solved"].all() and np.array_equal(h["solved"], d["solved"])
@@ -183,10 +136,9 @@ def test_gn_step_vi_equals_gn_step_on_evaluated_blocks(pkg, ctx):
     summed through shared-memory atomics in whatever order the warps finish (two viml_gn_step calls repeat to rounding only), so
     the full batch is held to 1e-12."""
     batch, vi, extra = _case(pkg, seed=51, gaps=False, perturb=0.01)
-    inertial_only = _inertial_only(pkg, batch)
     flags = pkg.LOSS_CAUCHY
     dense = vi.to_dense(ctx.inertial_evaluate(batch, extra, vi))
-    for b_, exact in ((inertial_only, True), (batch, False)):
+    for b_, exact in ((inertial_only(pkg, batch), True), (batch, False)):
         a = ctx.gn_step_vi(b_, vi, extra, flags, lam=1e-3)
         b = ctx.gn_step(b_, dense, extra, flags, lam=1e-3)
         assert a["solved"].all() and np.array_equal(a["solved"], b["solved"])

@@ -12,7 +12,7 @@ import pytest
 
 import inertial_oracle as io
 import marg_vi_policy as mp
-from test_solve_vi_gpu import _bits, _guard_all, _inertial_only, _slice_vi
+from vi_helpers import bits, guard_all, inertial_only, slice_vi
 
 pytestmark = pytest.mark.gpu
 
@@ -92,7 +92,7 @@ def _check_window(pkg, got, w, r, JtJ, Jtr, batch, extra, tol=1e-8):
     assert got["prior_n"][w] == n and got["prior_n_blocks"][w] == len(r["keep"])
     assert np.array_equal(got["prior_block"][w, :len(r["keep"])], np.array(r["keep"], dtype=np.int32).reshape(-1, 4))
     x0 = mp.x0_rows(batch.P, r["src"], batch.poses[w], batch.ex_pose[w], extra[w])
-    assert np.array_equal(_bits(got["prior_x0"][w, :len(r["keep"])]), _bits(x0))
+    assert np.array_equal(bits(got["prior_x0"][w, :len(r["keep"])]), bits(x0))
     J, res = got["prior_jacobian"][w, :n, :n], got["prior_residual"][w, :n]
     e1 = pkg.parity.unit_err("S", _pad6(J.T @ J)[None], _pad6(JtJ)[None])
     e2 = pkg.parity.unit_err("g", _pad6(J.T @ res)[None], _pad6(Jtr)[None])
@@ -168,13 +168,13 @@ def test_mixed_batch_equals_one_window_calls(pkg, ctx):
     assert np.array_equal(got["prior_block"][7, :nb7], vi.prior_block[7, :nb7]) and np.array_equal(got["prior_x0"][7, :nb7], vi.prior_x0[7, :nb7])
     exact = {1, 4, 7}   # MARGIN_SECOND_NEW: the prior alone
     for w in range(batch.W):
-        one = ctx.marginalize_vi(batch.slice_windows(w, w + 1), _slice_vi(pkg, vi, w), extra[w:w + 1], margin[w:w + 1], FLAGS)
+        one = ctx.marginalize_vi(batch.slice_windows(w, w + 1), slice_vi(pkg, vi, w), extra[w:w + 1], margin[w:w + 1], FLAGS)
         n = int(one["prior_n"][0])
         for k in ("prior_n", "prior_n_blocks", "prior_block", "prior_x0"):
-            assert np.array_equal(_bits(got[k][w]), _bits(one[k][0])), (w, k)
+            assert np.array_equal(bits(got[k][w]), bits(one[k][0])), (w, k)
         J, r, J1, r1 = got["prior_jacobian"][w, :n, :n], got["prior_residual"][w, :n], one["prior_jacobian"][0, :n, :n], one["prior_residual"][0, :n]
         if w in exact:
-            assert np.array_equal(_bits(J), _bits(J1)) and np.array_equal(_bits(r), _bits(r1)), w
+            assert np.array_equal(bits(J), bits(J1)) and np.array_equal(bits(r), bits(r1)), w
         else:
             assert pkg.parity.unit_err("S", _pad6(J.T @ J)[None], _pad6(J1.T @ J1)[None]) < 1e-9, w
             assert pkg.parity.unit_err("g", _pad6(J.T @ r)[None], _pad6(J1.T @ r1)[None]) < 1e-9, w
@@ -207,7 +207,7 @@ def test_two_frame_chain_device_pointers(pkg, ctx):
     """solve, marginalise with device pointers, slide (numpy), solve with the new prior: equal to the host-pointer chain bit for bit
     (no point factors: every kernel is order-deterministic), and no window fails because of the prior."""
     batch, vi, extra = _case(pkg, W=6, seed=23)
-    b = _inertial_only(pkg, batch)
+    b = inertial_only(pkg, batch)
     margin = np.array([0, 0, 1, 0, 1, 0], np.int32)
 
     def chain(device):
@@ -230,9 +230,9 @@ def test_two_frame_chain_device_pointers(pkg, ctx):
     p_host, s_host = chain(False)
     p_dev, s_dev = chain(True)
     for k in PRIOR:
-        assert np.array_equal(_bits(p_dev[k]), _bits(p_host[k])), k
+        assert np.array_equal(bits(p_dev[k]), bits(p_host[k])), k
     for k in s_host:
-        assert np.array_equal(_bits(s_dev[k]), _bits(s_host[k])), k
+        assert np.array_equal(bits(s_dev[k]), bits(s_host[k])), k
     assert (s_host["status"] != pkg._abi.SOLVE_FAILURE).all() and (s_host["accepted"] > 0).all()
 
 
@@ -244,12 +244,12 @@ def _marg_device(pkg, ctx, batch, vi, extra, margin, n_max=None):
     b_in = {k: a for k, a in batch.arrays().items() if a is not None}
     ins = {**{"b_" + k: a for k, a in b_in.items()}, **{"v_" + k: a for k, a in vi.arrays().items()}, "extra": extra,
            "margin": np.ascontiguousarray(margin, np.int32)}
-    gi = _guard_all(ctx, ins)
+    gi = guard_all(ctx, ins)
     s = batch.struct({**batch.arrays(), **{k: gi["b_" + k].ptr for k in b_in}})
     v = vi.struct({k: gi["v_" + k].ptr for k in vi.arrays()})
     outs = {"prior_n": np.full(W, -1, np.int32), "prior_jacobian": np.full((W, n_max, n_max), np.nan), "prior_residual": np.full((W, n_max), np.nan),
             "prior_n_blocks": np.full(W, -1, np.int32), "prior_block": np.full((W, mb, 4), -1, np.int32), "prior_x0": np.full((W, mb, 9), np.nan)}
-    go = _guard_all(ctx, outs)
+    go = guard_all(ctx, outs)
     o = pkg._abi.PriorOut()
     o.prior_n_max, o.prior_max_blocks = n_max, mb
     for k in outs:
@@ -258,7 +258,7 @@ def _marg_device(pkg, ctx, batch, vi, extra, margin, n_max=None):
                                            FLAGS | pkg.PTRS_DEVICE))
     ctx.sync()
     res = {k: g.check() for k, g in go.items()}
-    same = all(np.array_equal(_bits(g.check()), _bits(ins[k])) for k, g in gi.items())
+    same = all(np.array_equal(bits(g.check()), bits(ins[k])) for k, g in gi.items())
     for g in list(gi.values()) + list(go.values()):
         g.free()
     return res, same
@@ -267,12 +267,12 @@ def _marg_device(pkg, ctx, batch, vi, extra, margin, n_max=None):
 def test_device_pointers_guard_bands(pkg, ctx):
     batch, vi, extra = _case(pkg, W=5, seed=29, no_imu=(1,), no_prior=(2,))
     margin = np.array([0, 0, 0, 1, 1], np.int32)
-    b = _inertial_only(pkg, batch)   # deterministic kernels: the flavours agree bit for bit
+    b = inertial_only(pkg, batch)   # deterministic kernels: the flavours agree bit for bit
     host = ctx.marginalize_vi(b, vi, extra, margin, FLAGS)
     dev, same = _marg_device(pkg, ctx, b, vi, extra, margin)
     assert same, "an input changed"
     for k in PRIOR:
-        assert np.array_equal(_bits(dev[k]), _bits(host[k])), k
+        assert np.array_equal(bits(dev[k]), bits(host[k])), k
     # with point factors (the observation table too): inputs untouched, nothing written outside the outputs
     dev, same = _marg_device(pkg, ctx, batch, vi, extra, margin)
     assert same and (dev["prior_n"] >= 0).all()
@@ -302,7 +302,7 @@ def test_validation(pkg, ctx):
     refused(mg=np.array([0, 2], np.int32))
     refused(n_max=60)                       # the kept dimension (75) does not fit
     refused(max_blocks=4)                   # nor the block count (12)
-    v = _slice_vi(pkg, vi, 0)
+    v = slice_vi(pkg, vi, 0)
     v = pkg._abi.Inertial(1, v.P, v.X, v.gravity, v.imu_window_offset, v.imu_pose, v.imu_sb.copy(), v.imu_preint, v.imu_jacobian,
                           v.imu_sqrt_info, v.prior_n, v.prior_jacobian, v.prior_residual, v.prior_n_blocks, v.prior_block.copy(), v.prior_x0)
     b1, e1 = batch.slice_windows(0, 1), extra[:1]

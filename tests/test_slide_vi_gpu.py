@@ -11,7 +11,7 @@ import pytest
 import marg_vi_policy as mp
 import slide_policy as sp
 from conftest import rel_err
-from test_solve_vi_gpu import _bits, _guard_all, _inertial_only
+from vi_helpers import bits, guard_all, inertial_only
 
 pytestmark = pytest.mark.gpu
 
@@ -27,7 +27,7 @@ def _case(pkg, W=4, seed=3, F=40, **kw):
 
 def _check_bits(got, ref):
     for k in STATE:
-        assert got[k].shape == ref[k].shape and np.array_equal(_bits(got[k]), _bits(ref[k])), k
+        assert got[k].shape == ref[k].shape and np.array_equal(bits(got[k]), bits(ref[k])), k
 
 
 def _n_moved(batch, got):
@@ -68,7 +68,7 @@ def test_mixed_batch(pkg, ctx):
     margin = np.array([0, 1, 0, 0, 1, 0], np.int32)
     got = ctx.slide_vi(batch, extra, margin, 0)
     _check_bits(got, sp.slide_batch(batch, extra, margin))
-    assert np.array_equal(_bits(got["inv_depth"][2]), _bits(batch.inv_depth[2]))
+    assert np.array_equal(bits(got["inv_depth"][2]), bits(batch.inv_depth[2]))
     assert got["inv_depth"][3, f] == batch.inv_depth[3, f]
     assert not np.array_equal(got["inv_depth"][0], batch.inv_depth[0])
 
@@ -90,11 +90,11 @@ def _slide_device(pkg, ctx, batch, extra, margin, init_depth=5.0, obs_table=Fals
     arrs = batch.arrays() if arrs is None else arrs
     b_in = {k: a for k, a in arrs.items() if a is not None}
     ins = {**{"b_" + k: a for k, a in b_in.items()}, "extra": extra, "margin": np.ascontiguousarray(margin, np.int32)}
-    gi = _guard_all(ctx, ins)
+    gi = guard_all(ctx, ins)
     s = batch.struct({**{k: None for k in arrs}, **{k: gi["b_" + k].ptr for k in b_in}})
     outs = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
             "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full_like(extra, np.nan)}
-    go = _guard_all(ctx, outs)
+    go = guard_all(ctx, outs)
     o = pkg._abi.SlideOut()
     for k in outs:
         setattr(o, k, go[k].ptr)
@@ -102,7 +102,7 @@ def _slide_device(pkg, ctx, batch, extra, margin, init_depth=5.0, obs_table=Fals
                                      pkg.PTRS_DEVICE))
     ctx.sync()
     res = {k: g.check() for k, g in go.items()}
-    same = all(np.array_equal(_bits(g.check()), _bits(ins[k])) for k, g in gi.items())
+    same = all(np.array_equal(bits(g.check()), bits(ins[k])) for k, g in gi.items())
     for g in list(gi.values()) + list(go.values()):
         g.free()
     return res, same
@@ -241,7 +241,7 @@ def test_two_frame_chain_device_pointers(pkg, ctx, points):
     pose blocks are summed through shared-memory atomics: the 1e-9 per-unit bar."""
     batch = pkg.synth.make_windows(6, seed=23, F=40, lines_per_frame=0)
     vi, extra = pkg.synth.make_inertial_factors(batch, seed=24)
-    b = batch if points else _inertial_only(pkg, batch)
+    b = batch if points else inertial_only(pkg, batch)
     margin = np.array([0, 0, 1, 0, 1, 0], np.int32)
     nxt = sp.next_structure_batch(b, margin)
     h1, h2 = _chain_host(pkg, ctx, b, vi, extra, margin, nxt)
@@ -251,7 +251,7 @@ def test_two_frame_chain_device_pointers(pkg, ctx, points):
     for h, d in ((h1, d1), (h2, d2)):
         for k in SOLVE_OUT:
             if not points:
-                assert np.array_equal(_bits(d[k]), _bits(h[k])), k
+                assert np.array_equal(bits(d[k]), bits(h[k])), k
             elif k in STATE + ("cost",):
                 for w in range(b.W):
                     assert rel_err(d[k][w], h[k][w]) < 1e-9, (k, w)

@@ -6,7 +6,6 @@ prior factors' J^T J, the damped system solved densely, x+ by pose_plus, f(x+) f
 the scalar step and policy of tests/dogleg_policy.py.  The device eliminates the landmarks and solves the reduced system with a
 blocked Cholesky, so values agree to 1e-9 and the decisions exactly; bit-exact checks are only made between device runs."""
 import copy
-import ctypes as C
 import math
 
 import numpy as np
@@ -15,18 +14,13 @@ import pytest
 import dogleg_policy as dp
 import inertial_oracle as io
 from conftest import rel_err
+from vi_helpers import bits, inertial_only, rotate, slice_vi, solve_device
 
 pytestmark = pytest.mark.gpu
 
 CAUCHY, OUT_HB = 0x10, 0x02
 STATE = ("poses", "ex_pose", "inv_depth", "extra")
 EPS = 1e-8
-
-
-def _rotate(x, th):
-    q = io.qmul(io.quat(x), (1.0, th[0] / 2, th[1] / 2, th[2] / 2))
-    n = np.sqrt(sum(c * c for c in q))
-    return np.array([x[0], x[1], x[2], q[1] / n, q[2] / n, q[3] / n, q[0] / n])
 
 
 def _case(pkg, W=6, seed=5, P=11, F=40, no_imu=(), perturb=(0.002, 0.01, 0.05, 0.5, 1.0)):
@@ -38,27 +32,9 @@ def _case(pkg, W=6, seed=5, P=11, F=40, no_imu=(), perturb=(0.002, 0.01, 0.05, 0
         s = perturb[w % len(perturb)]
         batch.poses[w, :, :3] += s * rng.standard_normal((P, 3))
         for p in range(P):
-            batch.poses[w, p] = _rotate(batch.poses[w, p], 0.5 * s * rng.standard_normal(3))
+            batch.poses[w, p] = rotate(batch.poses[w, p], 0.5 * s * rng.standard_normal(3))
         extra[w] += s * rng.standard_normal(extra.shape[1])
     return batch, vi, extra
-
-
-def _inertial_only(pkg, batch):
-    W = batch.W
-    return pkg._abi.Batch(batch.poses, batch.ex_pose, batch.inv_depth, np.zeros(W + 1, dtype=np.int32),
-                          np.zeros(0, dtype=np.uint32), np.zeros((0, 4)))
-
-
-def _slice_vi(pkg, vi, w):
-    k0, k1 = int(vi.imu_window_offset[w]), int(vi.imu_window_offset[w + 1])
-    return pkg._abi.Inertial(1, vi.P, vi.X, vi.gravity, np.array([0, k1 - k0]), vi.imu_pose[k0:k1], vi.imu_sb[k0:k1],
-                             vi.imu_preint[k0:k1], vi.imu_jacobian[k0:k1], vi.imu_sqrt_info[k0:k1], vi.prior_n[w:w + 1],
-                             vi.prior_jacobian[w:w + 1], vi.prior_residual[w:w + 1], vi.prior_n_blocks[w:w + 1],
-                             vi.prior_block[w:w + 1], vi.prior_x0[w:w + 1])
-
-
-def _bits(a):
-    return np.ascontiguousarray(a).view(np.uint8)
 
 
 # ---- the numpy reference ------------------------------------------------------------------------------------------------------
@@ -158,7 +134,7 @@ def _reference(system, cost, batch1, extra1, X, opt):
 def _library_reference(pkg, ctx, batch, vi, extra, opt):
     ref = []
     for w in range(batch.W):
-        vi1 = _slice_vi(pkg, vi, w)
+        vi1 = slice_vi(pkg, vi, w)
 
         def system(b, ex):
             lin = ctx.linearize(b, OUT_HB | CAUCHY)
@@ -211,7 +187,7 @@ def _run_against_reference(pkg, ctx, batch, vi, extra):
 
 def test_against_numpy_inertial_only(pkg, ctx):
     batch, vi, extra = _case(pkg, W=5, seed=5)
-    cases, reused = _run_against_reference(pkg, ctx, _inertial_only(pkg, batch), vi, extra)
+    cases, reused = _run_against_reference(pkg, ctx, inertial_only(pkg, batch), vi, extra)
     assert {1, 2, 3} <= cases and reused > 0
 
 
@@ -227,7 +203,7 @@ def test_against_cpu_oracle(pkg, orc, ctx, cfg):
     opt = dp.Options(max_iterations=5, initial_radius=1e-2)
     got = _solve(pkg, ctx, batch, vi, extra, opt)
     for w in range(2):
-        vi1 = _slice_vi(pkg, vi, w)
+        vi1 = slice_vi(pkg, vi, w)
 
         def system(b, ex):
             lin = orc.linearize_batch(cfg, b, OUT_HB | CAUCHY)
@@ -244,7 +220,7 @@ def test_unfused(pkg, ctx):
     """Dx = 201 (P = 13): the separate reduced-system and solve kernels."""
     batch, vi, extra = _case(pkg, W=3, seed=33, P=13, F=20)
     assert batch.D + vi.X == 201
-    b = _inertial_only(pkg, batch)
+    b = inertial_only(pkg, batch)
     opt = dp.Options(max_iterations=8, initial_radius=1e-2)
     got = _solve(pkg, ctx, b, vi, extra, opt)
     _check_close(got, _library_reference(pkg, ctx, b, vi, extra, opt), opt)
@@ -254,18 +230,18 @@ def test_unfused(pkg, ctx):
 def test_window_independence(pkg, ctx):
     """Without point and line factors a window solved in a batch equals the same window solved alone, bit for bit."""
     batch, vi, extra = _case(pkg, W=5, seed=71)
-    b = _inertial_only(pkg, batch)
+    b = inertial_only(pkg, batch)
     opt = dp.Options(max_iterations=10, initial_radius=1e-2)
     got = _solve(pkg, ctx, b, vi, extra, opt)
     for w in range(b.W):
-        one = _solve(pkg, ctx, b.slice_windows(w, w + 1), _slice_vi(pkg, vi, w), extra[w:w + 1], opt)
+        one = _solve(pkg, ctx, b.slice_windows(w, w + 1), slice_vi(pkg, vi, w), extra[w:w + 1], opt)
         for k in one:
-            assert np.array_equal(_bits(got[k][w]), _bits(one[k][0])), (w, k)
+            assert np.array_equal(bits(got[k][w]), bits(one[k][0])), (w, k)
 
 
 def test_nan_in_one_window(pkg, ctx):
     batch, vi, extra = _case(pkg, W=6, seed=51)
-    b = _inertial_only(pkg, batch)
+    b = inertial_only(pkg, batch)
     opt = dp.Options(max_iterations=6, initial_radius=1e-2)
     clean = _solve(pkg, ctx, b, vi, extra, opt)
     bad = copy.deepcopy(b)
@@ -275,10 +251,10 @@ def test_nan_in_one_window(pkg, ctx):
     assert np.isnan(got["cost"][3]).all() and np.isnan(got["trace"][3]).all() and got["radius"][3] == 1e-2
     start = {"poses": bad.poses, "ex_pose": bad.ex_pose, "inv_depth": bad.inv_depth, "extra": extra}
     for k in STATE:
-        assert np.array_equal(_bits(got[k][3]), _bits(start[k][3])), k
+        assert np.array_equal(bits(got[k][3]), bits(start[k][3])), k
     others = [w for w in range(b.W) if w != 3]
     for k in clean:
-        assert np.array_equal(_bits(got[k][others]), _bits(clean[k][others])), k
+        assert np.array_equal(bits(got[k][others]), bits(clean[k][others])), k
 
 
 def test_prior_only_window(pkg, ctx):
@@ -286,7 +262,7 @@ def test_prior_only_window(pkg, ctx):
     mu 1e-6 / s^2 (Ceres' clamp of the scaled diagonal), so the window still converges: its state stays finite, its cost does not
     rise, and the windows beside it are those of the batch without it."""
     batch, vi, extra = _case(pkg, W=4, seed=5, no_imu=(2,))
-    b = _inertial_only(pkg, batch)
+    b = inertial_only(pkg, batch)
     opt = dp.Options(max_iterations=12)
     got = _solve(pkg, ctx, b, vi, extra, opt)
     assert got["status"][2] != dp.FAILURE and got["accepted"][2] > 0
@@ -294,71 +270,20 @@ def test_prior_only_window(pkg, ctx):
         assert np.isfinite(got[k][2]).all(), k
     assert got["cost"][2, 1] <= got["cost"][2, 0]
     for w in (0, 1, 3):
-        one = _solve(pkg, ctx, b.slice_windows(w, w + 1), _slice_vi(pkg, vi, w), extra[w:w + 1], opt)
+        one = _solve(pkg, ctx, b.slice_windows(w, w + 1), slice_vi(pkg, vi, w), extra[w:w + 1], opt)
         for k in one:
-            assert np.array_equal(_bits(got[k][w]), _bits(one[k][0])), (w, k)
-
-
-class _Guarded:
-    """A device copy of a host array with GUARD bytes of a fixed pattern on either side: check() reads the allocation back and fails
-    if a byte outside the array changed."""
-    GUARD = 4096
-
-    def __init__(self, ctx, a):
-        self.ctx, self.a = ctx, np.ascontiguousarray(a)
-        self.n = self.a.nbytes
-        self.img = np.concatenate([np.full(self.GUARD, 0xA5, np.uint8), self.a.view(np.uint8).reshape(-1),
-                                   np.full(self.GUARD, 0x5A, np.uint8)])
-        self.base = ctx.to_device(self.img)
-        self.ptr = self.base + self.GUARD
-
-    def check(self):
-        back = np.empty_like(self.img)
-        self.ctx.d2h(back, self.base)
-        self.ctx.sync()
-        assert np.all(back[:self.GUARD] == 0xA5) and np.all(back[self.GUARD + self.n:] == 0x5A), "write outside the buffer"
-        return back[self.GUARD:self.GUARD + self.n].view(self.a.dtype).reshape(self.a.shape)
-
-    def free(self):
-        self.ctx.device_free(self.base)
-
-
-def _solve_device(pkg, ctx, batch, vi, extra, opt):
-    b_in = {k: a for k, a in batch.arrays().items() if a is not None}
-    ins = {**{"b_" + k: a for k, a in b_in.items()}, **{"v_" + k: a for k, a in vi.arrays().items()}, "extra": extra}
-    gi = {k: _Guarded(ctx, a) for k, a in ins.items()}
-    s = batch.struct({**batch.arrays(), **{k: gi["b_" + k].ptr for k in b_in}})
-    v = vi.struct({k: gi["v_" + k].ptr for k in vi.arrays()})
-    W, M = batch.W, opt.max_iterations
-    outs = {"poses": np.full_like(batch.poses, np.nan), "ex_pose": np.full_like(batch.ex_pose, np.nan),
-            "inv_depth": np.full_like(batch.inv_depth, np.nan), "extra": np.full((W, vi.X), np.nan),
-            "status": np.full(W, -1, np.int32), "iterations": np.full(W, -1, np.int32), "accepted": np.full(W, -1, np.int32),
-            "cost": np.full((W, 2), np.nan), "radius": np.full(W, np.nan), "trace": np.full((W, M, 4), -1.0)}
-    go = {k: _Guarded(ctx, a) for k, a in outs.items()}
-    o = pkg._abi.SolveOut()
-    for k in outs:
-        setattr(o, k, go[k].ptr)
-    so = ctx.solve_options(**vars(opt))
-    ctx._check(ctx.lib.viml_solve_vi(ctx.h, C.byref(s), C.byref(v), gi["extra"].ptr, C.byref(so), C.byref(o),
-                                     CAUCHY | pkg.SOLVE_DOGLEG | pkg.PTRS_DEVICE))
-    ctx.sync()
-    res = {k: g.check() for k, g in go.items()}
-    for k, g in gi.items():
-        assert np.array_equal(_bits(g.check()), _bits(ins[k])), k
-    for g in list(gi.values()) + list(go.values()):
-        g.free()
-    return res
+            assert np.array_equal(bits(got[k][w]), bits(one[k][0])), (w, k)
 
 
 def test_device_pointers(pkg, ctx):
     """Guarded device buffers: nothing is written outside the outputs, the inputs stay untouched, and two calls agree with each
     other and with the host flavour bit for bit (no point or line factors, whose pose blocks are summed through atomics)."""
     batch, vi, extra = _case(pkg, W=6, seed=41)
-    b = _inertial_only(pkg, batch)
+    b = inertial_only(pkg, batch)
     opt = dp.Options(max_iterations=8, initial_radius=1e-2)
     host = _solve(pkg, ctx, b, vi, extra, opt)
     for _ in range(2):
-        dev = _solve_device(pkg, ctx, b, vi, extra, opt)
+        dev = solve_device(pkg, ctx, b, vi, extra, opt, CAUCHY | pkg.SOLVE_DOGLEG)
         for k in host:
-            assert np.array_equal(_bits(dev[k]), _bits(host[k])), k
+            assert np.array_equal(bits(dev[k]), bits(host[k])), k
     assert (host["accepted"] > 0).all()
